@@ -1,12 +1,15 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: mLSTM chunkwise fwd+bwd (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one forward + one backward of the chunkwise mLSTM over one batch of synthetic
 input: bf16, B=32 NH=4 S=1600 DH=64 chunk=64 per GPU (weak scaling: every rank runs the same
 per-GPU workload on its own data; the op has no cross-sample term, so there is no data-path
 collective -- SURVEY.md §8e).  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy in float32, so that two
+builds can be compared output for output: the inputs are seeded, identical from run to run.
 
 Metric: algorithmic TFLOP/s = 14*L*d*(L+d) FLOP per chunk (SURVEY.md §8d) x chunks / time.
 """
@@ -28,6 +31,7 @@ CFG = dict(B=32, NH=4, S=1600, DK=64, DV=64, L=64)
 WORKLOAD = "mlstm_chunkwise_fwbw bf16 B=32 NH=4 S=1600 DH=64 chunk=64 (BASELINE configs[1])"
 METRIC = "mLSTM chunkwise fwd+bwd TFLOP/s (algorithmic, 14*L*d*(L+d) per chunk)"
 N_SETS = 4  # rotating input sets: ~105 MB of inputs + ~105 MB of outputs per step >> 126 MB L2 over a rotation
+DUMP_BYTES = 60_000_000  # --dump-outputs stays under 64 MB: one step's outputs are ~213 MB in float32
 
 
 def flops_and_bytes(c, itemsize=2):
@@ -42,6 +46,22 @@ def flops_and_bytes(c, itemsize=2):
     fw_bytes = 2 * qk + v + 2 * gate + v + 2 * vec32  # read q,k,v,i,f; write h,n_out,m_out
     bw_bytes = 2 * qk + v + v + 2 * gate + 2 * vec32 + 2 * qk + v + 2 * gate  # read q,k,v,dh,i,f,n,m; write dq,dk,dv,di,df
     return bh * nc * fwd, bh * nc * bwd, fw_bytes, bw_bytes
+
+
+def dump_outputs(out_dir, outs, seed=0):
+    """Write each (B, NH, ...) output as out_dir/<name>.npy in float32, its (batch, head) rows flattened into one
+    leading axis.  Where all rows do not fit DUMP_BYTES, every array keeps the same fixed, seeded subset of rows
+    (ascending (batch, head) order), so that row r of every file belongs to the same (batch, head)."""
+    import numpy as np
+
+    rows = {name: t.detach().flatten(0, 1) for name, t in outs.items()}
+    n_rows = next(iter(rows.values())).shape[0]
+    row_bytes = sum(t[0].numel() * 4 for t in rows.values())
+    keep = min(n_rows, DUMP_BYTES // row_bytes)
+    idx = torch.randperm(n_rows, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in rows.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t[idx.to(t.device)].float().cpu().numpy())
 
 
 def peaks():
@@ -477,7 +497,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-model-calls", action="store_true")
     ap.add_argument("--no-model-train", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (h, n_out, m_out, dq, dk, dv, di, df) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -544,6 +570,7 @@ def main():
     # One CUDA graph per rotating input set: the step is two ~100 us kernels, so eager Python/ctypes
     # launch gaps would dominate.  Outputs live in the graphs' private pools.
     graphs, fw_graphs, bw_graphs, keep = [], [], [], []
+    multi_out, single_out = [], []  # (forward, backward) results of the timed graphs, per input set
     side = torch.cuda.Stream()
     REP = 4  # launches per input set in the per-kernel graphs below
     with torch.cuda.stream(side):
@@ -553,7 +580,7 @@ def main():
         with torch.cuda.graph(g_multi, stream=side):
             for r in range(N_SETS):
                 saved = fw_only(sets[r])
-                keep.append((saved, bw_only(sets[r], saved)))
+                multi_out.append((saved, bw_only(sets[r], saved)))
         # per-kernel graphs: REP * N_SETS back-to-back launches of ONE kernel over the rotating sets, so that the
         # roofline's per-launch duration is the kernel period, not kernel + graph launch + event overhead
         saved_all = [fw_only(sets[r]) for r in range(N_SETS)]
@@ -571,7 +598,7 @@ def main():
                 saved = fw_only(sets[r])
                 out = bw_only(sets[r], saved)
             graphs.append(g)
-            keep.append((saved, out))
+            single_out.append((saved, out))
             gf = torch.cuda.CUDAGraph()
             with torch.cuda.graph(gf, stream=side):
                 saved_f = fw_only(sets[r])
@@ -605,6 +632,10 @@ def main():
 
     ms_step = replicas.max_over_ranks(e0.elapsed_time(e1), dev) / args.steps  # slowest rank
     value = replicas.sum_over_ranks(ff + fb, dev) / (ms_step * 1e-3) / 1e12    # all ranks' work over that time
+    if args.dump_outputs and rank == 0:
+        rem = args.steps % N_SETS  # the last timed step is graphs[rem - 1], or the last set of g_multi
+        (h, n_out, m_out, _, _), (dq, dk, dv, di, df, _) = single_out[rem - 1] if rem else multi_out[-1]
+        dump_outputs(args.dump_outputs, dict(h=h, n_out=n_out, m_out=m_out, dq=dq, dk=dk, dv=dv, di=di, df=df))
 
     # ---- per-kernel timing for the roofline: CUDA events on the launching stream, one kernel per graph
     fw_ms, bw_ms = [], []
@@ -727,7 +758,7 @@ def main():
     sync_all()
     e2e_ms = replicas.max_over_ranks(e0.elapsed_time(e1), dev) / e_steps
     e2e_val = replicas.sum_over_ranks(ff + fb, dev) / (e2e_ms * 1e-3) / 1e12
-    e2e_check = float((host_out["h"].float() - keep[0][0][0].float().cpu()).abs().max())  # same inputs as set 0
+    e2e_check = float((host_out["h"].float() - multi_out[0][0][0].float().cpu()).abs().max())  # same inputs as set 0
 
     del pipe
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)

@@ -1,10 +1,11 @@
-"""Generate golden vectors from the UNMODIFIED reference (run in the build container only).
+"""Generate golden vectors from the UNMODIFIED reference.
 
+    sh tools/stage_reference.sh <checkout of xlstm-yolo-clean>
     PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
 
-Imports ``mlstm_kernels`` from /root/reference (read-only; it does not exist on the
-GPU box, which is why the outputs are committed as ``tests/golden/*.npz``).  Every
-case runs the reference in float64 on seeded inputs:
+Imports ``mlstm_kernels`` from the staged copy under baseline/_ref (read-only; the
+repository does not carry the reference, which is why the outputs are committed as
+``tests/golden/*.npz``).  Every case runs the reference in float64 on seeded inputs:
 
   * ``mlstm_chunkwise__native_custbw`` through autograd (the user-facing API whose
     backward is the spec, native/fwbw.py:228-263) -> h, last states, dq dk dv di df dc0
@@ -22,7 +23,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.path.join(HERE, "..", "..", "baseline", "_ref"))
 sys.dont_write_bytecode = True
 
 from mlstm_kernels.torch import get_mlstm_kernel  # noqa: E402

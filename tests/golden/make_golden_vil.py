@@ -1,4 +1,4 @@
-"""Golden vectors of the UNMODIFIED reference ViLLayer.mlstm_branch (run in the build container only).
+"""Golden vectors of the UNMODIFIED reference ViLLayer.mlstm_branch (staged under baseline/_ref by tools/stage_reference.sh).
 
     PYTHONDONTWRITEBYTECODE=1 YOLO_CONFIG_DIR=/tmp/yolo_cfg python tests/golden/make_golden_vil.py
 
@@ -18,7 +18,7 @@ import types
 import numpy as np
 import torch
 
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", "baseline", "_ref"))
 sys.dont_write_bytecode = True
 os.environ.setdefault("YOLO_CONFIG_DIR", "/tmp/yolo_cfg")
 for name in ("matplotlib", "matplotlib.pyplot"):

@@ -109,12 +109,13 @@ def test_compute_call_without_device_returns_error(lib):
 
 def test_registry_drop_in():
     """register() makes 'chunkwise--b200' resolvable through the reference's get_mlstm_kernel
-    (only where the reference package is importable, i.e. the build container)."""
+    (only where the reference is staged under baseline/_ref, tools/stage_reference.sh)."""
     import sys
 
-    if not os.path.isdir("/root/reference/mlstm_kernels"):
-        pytest.skip("reference package not present on this box")
-    sys.path.insert(0, "/root/reference")
+    ref = os.path.join(ROOT, "baseline", "_ref")
+    if not os.path.isdir(os.path.join(ref, "mlstm_kernels")):
+        pytest.skip("reference not staged under baseline/_ref (tools/stage_reference.sh)")
+    sys.path.insert(0, ref)
     sys.dont_write_bytecode = True
     try:
         import xlstm_yolo_clean_b200 as pkg
@@ -129,7 +130,7 @@ def test_registry_drop_in():
         with pytest.raises(RuntimeError, match="no CPU path"):  # routed to our kernel, which refuses CPU
             be(q=q, k=q, v=q, i=g, f=g)
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(ref)
 
 
 def test_rotated_conv_equals_flip_conv_flip():

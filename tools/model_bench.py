@@ -31,7 +31,7 @@ import torch  # noqa: E402
 
 def _import_reference():
     if not os.path.isdir(os.path.join(REF, "mlstm_kernels")):
-        raise SystemExit("baseline/_ref is missing: run tools/stage_reference.sh in the build container first")
+        raise SystemExit("baseline/_ref is missing: run `sh tools/stage_reference.sh <checkout of xlstm-yolo-clean>` first")
     sys.path.insert(0, REF)
     os.environ.setdefault("YOLO_CONFIG_DIR", "/tmp/yolo_cfg")
     for name in ("matplotlib", "matplotlib.pyplot"):  # hard import at ultralytics/utils/__init__.py:24
