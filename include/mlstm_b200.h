@@ -166,8 +166,9 @@ size_t mlstm_b200_workspace_bytes(const mlstm_b200_shape* shape, int backward);
 size_t mlstm_b200_states_bytes(const mlstm_b200_shape* shape);
 
 /* 1 if the tensor-core (tcgen05) kernels cover this shape/dtype forward AND backward, else 0
- * (16-bit dtypes, DHQK == DHHV in {32, 64, 128}, S % 4 == 0; the head-dim-128 backward runs as four
- * head-dim-64 block problems inside the call). */
+ * (16-bit dtypes, S % 4 == 0, and DHQK == DHHV in {32, 64, 128} or (DHQK, DHHV) in {(32, 64), (64, 128)}; the
+ * head-dim-128 backward runs as four head-dim-64 block problems inside the call, a rectangular (D, 2 D) call as two
+ * square head-dim-D problems on the two column halves of v / h / dh / dv). */
 int mlstm_b200_tensor_path_supported(const mlstm_b200_shape* shape);
 
 /* Forward: h, n_out, m_out and optionally the last (C, n, m) states. */
@@ -196,7 +197,8 @@ void mlstm_b200_debug_set_clock_buffer(void* dev_ptr);
  * which the reference's inference wrapper runs for the tokens that do not fill a chunk
  * (wrap_chunkwise__arbitrary_sequence_length, mlstm_kernels/torch/kernel_wrappers.py:12-201).
  *   q, k (B, NH, S, DHQK), v, h (B, NH, S, DHHV), i, f (B, NH, S): element strides [b, head, s, 1] / [b, head, s];
- *   DHQK == DHHV in {32, 64, 128}; dtype of q / k / v / i / f / h; states contiguous fp32 as in the chunkwise calls
+ *   DHQK == DHHV in {32, 64, 128} or (DHQK, DHHV) in {(32, 64), (64, 128)}; dtype of q / k / v / i / f / h; states
+ *   contiguous fp32 as in the chunkwise calls
  *   (m is (B, NH)).  Initial states: all three or none (none = zeros); last states: all three or none; the last
  *   states may alias the initial ones (in-place update).  siging = 1: sigmoid input gate, m stays 0.
  *   Forward only (the reference's recurrent kernels have no backward).

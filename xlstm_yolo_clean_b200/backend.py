@@ -411,9 +411,10 @@ def _bw_launch(q, k, v, i, f, n_ptr, m_ptr, dh, c0, n0, m0, dcl, qk_scale, chunk
             a.dq.stride[:4] = a.dk.stride[:4] = (NH * S * DK, S * DK, DK, 1)
             a.dv.stride[:4] = (NH * S * DV, S * DV, DV, 1)
             a.di.stride[:3] = a.df.stride[:3] = (NH * S, S, 1)
-        # the tensor-core route only needs scratch to recompute the states (or for the head-dim-128 block problems)
+        # the tensor-core route only needs scratch to recompute the states (or for the block problems of head dim 128
+        # and of rectangular heads)
         plan.ws_bytes = lib.mlstm_b200_workspace_bytes(C.byref(a.shape), 1)
-        if plan.tensor_route and c_states is not None and DK != 128:
+        if plan.tensor_route and c_states is not None and DK != 128 and DK == DV:
             plan.ws_bytes = 0
         plan.gshape_qk, plan.gshape_v, plan.gshape_g = (B, NH, S, DK), (B, NH, S, DV), (B, NH, S)
         for name, t in (("q", q), ("k", k), ("v", v), ("i", i), ("f", f), ("dh", dh)):

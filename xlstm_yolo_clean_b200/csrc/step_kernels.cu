@@ -125,14 +125,24 @@ __global__ void __launch_bounds__(kStepThreads) k_recurrent(StepParams p) {
   }
 }
 
+// (DHQK, DHHV) pairs with a k_recurrent instantiation
+bool recurrent_pair_ok(int DK, int DV) {
+  return (DK == DV && (DK == 32 || DK == 64 || DK == 128)) || (DK == 32 && DV == 64) || (DK == 64 && DV == 128);
+}
+
 template <typename T>
-int launch(const StepParams& p, int D, cudaStream_t st) {
+int launch(const StepParams& p, int DK, int DV, cudaStream_t st) {
   const int grid = p.B * p.NH;
-  switch (D) {
-    case 32: k_recurrent<T, 32, 32><<<grid, kStepThreads, 0, st>>>(p); break;
-    case 64: k_recurrent<T, 64, 64><<<grid, kStepThreads, 0, st>>>(p); break;
-    case 128: k_recurrent<T, 128, 128><<<grid, kStepThreads, 0, st>>>(p); break;
-    default: set_error("recurrent kernels cover head dims 32, 64 and 128 (got %d)", D); return MLSTM_B200_EUNSUPPORTED;
+  if (DK == DV) {
+    switch (DK) {
+      case 32: k_recurrent<T, 32, 32><<<grid, kStepThreads, 0, st>>>(p); break;
+      case 64: k_recurrent<T, 64, 64><<<grid, kStepThreads, 0, st>>>(p); break;
+      case 128: k_recurrent<T, 128, 128><<<grid, kStepThreads, 0, st>>>(p); break;
+    }
+  } else if (DK == 32) {
+    k_recurrent<T, 32, 64><<<grid, kStepThreads, 0, st>>>(p);
+  } else {
+    k_recurrent<T, 64, 128><<<grid, kStepThreads, 0, st>>>(p);
   }
   count_launch();
   MLSTM_CUDA_CHECK(cudaGetLastError());
@@ -142,8 +152,9 @@ int launch(const StepParams& p, int D, cudaStream_t st) {
 }  // namespace
 
 int recurrent_sequence(const mlstm_b200_recurrent_args& a, cudaStream_t st) {
-  if (a.DHQK != a.DHHV) {
-    set_error("recurrent kernels need DHQK == DHHV (got %d, %d)", a.DHQK, a.DHHV);
+  if (!recurrent_pair_ok(a.DHQK, a.DHHV)) {
+    set_error("recurrent kernels cover (DHQK, DHHV) = (32, 32), (64, 64), (128, 128), (32, 64) and (64, 128) (got %d, %d)",
+              a.DHQK, a.DHHV);
     return MLSTM_B200_EUNSUPPORTED;
   }
   if (!a.q.ptr || !a.k.ptr || !a.v.ptr || !a.i.ptr || !a.f.ptr || !a.h.ptr) {
@@ -173,7 +184,7 @@ int recurrent_sequence(const mlstm_b200_recurrent_args& a, cudaStream_t st) {
   p.h = a.h.ptr; p.h_sb = a.h.stride[0]; p.h_sh = a.h.stride[1]; p.h_ss = a.h.stride[2];
   p.c0 = a.c_initial; p.n0 = a.n_initial; p.m0 = a.m_initial;
   p.c1 = a.c_last; p.n1 = a.n_last; p.m1 = a.m_last;
-  MLSTM_DISPATCH_DTYPE(a.dtype, T, return launch<T>(p, a.DHQK, st));
+  MLSTM_DISPATCH_DTYPE(a.dtype, T, return launch<T>(p, a.DHQK, a.DHHV, st));
   return 0;
 }
 

@@ -464,11 +464,13 @@ struct FwSmem {
   static_assert(cDN + 8 <= kTmemCols, "TMEM budget");
 };
 
-template <typename T, int D, bool REV, bool EPI>
-__global__ void __launch_bounds__(kTcThreads, D == 32 ? 2 : 1)
-tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
-          const __grid_constant__ CUtensorMap mapV, const __grid_constant__ CUtensorMap mapH,
-          const __grid_constant__ CUtensorMap mapCs, TcFwParams p) {
+// VB > 1: rectangular heads, DHQK = D and DHHV = VB * D.  CTA x runs the square problem of (batch, head) x / VB on
+// the D-wide column block vb = x % VB of v / h / C (see tc_fw_rect); n and m do not depend on v, so every block
+// computes them and block 0 writes them.
+template <typename T, int D, bool REV, bool EPI, int VB>
+__device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtensorMap& mapK, const CUtensorMap& mapV,
+                                           const CUtensorMap& mapH, const CUtensorMap& mapCs, const TcFwParams& p) {
+  static_assert(VB == 1 || !EPI, "the fused epilogue needs the whole h row");
   constexpr bool kBf16 = std::is_same<T, __nv_bfloat16>::value;
   using SM = FwSmem<D>;
   using L = Lay<D>;
@@ -488,7 +490,7 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
 
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);  // provably warp-uniform: role branches stay uniform
-  const int bh = blockIdx.x, b = bh / p.NH, hh = bh % p.NH;
+  const int bh = blockIdx.x / VB, vb = blockIdx.x % VB, b = bh / p.NH, hh = bh % p.NH;
 
   const T* ip = (const T*)p.ig + b * p.ig_sb + hh * p.ig_sh;
   const T* fp = (const T*)p.fg + b * p.fg_sb + hh * p.fg_sh;
@@ -500,7 +502,7 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
     mbar_expect_tx(&bar_full[s], kStageBytes);
     tma_load_4d(smem + SM::oQ + s * SM::kTile, &mapQ, &bar_full[s], 0, mt(c) * LT, hh, b);
     tma_load_4d(smem + SM::oK + s * SM::kTile, &mapK, &bar_full[s], 0, mt(c) * LT, hh, b);
-    tma_load_4d(smem + SM::oV + s * SM::kTile, &mapV, &bar_full[s], 0, mt(c) * LT, hh, b);
+    tma_load_4d(smem + SM::oV + s * SM::kTile, &mapV, &bar_full[s], vb * D, mt(c) * LT, hh, b);
   };
   // cold start: the first Q / K / V tiles are requested before anything else happens in the CTA.  Under
   // programmatic dependent launch every thread passes griddepcontrol.wait before ITS first global access (a no-op
@@ -542,7 +544,7 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
   for (int j = 0; j < CW; ++j) Creg[j] = 0.f;
   if (warp < kCtlWarp) {
     if (p.c0 && owns_c) {
-      const float* src = p.c0 + ((int64_t)bh * D + drow) * D + ch * CW;
+      const float* src = p.c0 + ((int64_t)bh * D + drow) * (VB * D) + vb * D + ch * CW;
 #pragma unroll
       for (int j = 0; j < CW; ++j) Creg[j] = src[j];
     }
@@ -610,7 +612,7 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
       umma_commit(&bar_s);
     };
     if (lane == 0 && p.store_states) {  // state entering tile 0 (bf16 operand copy) -> c_states[b, h, 0]
-      tma_store_4d(&mapCs, sC, 0, mt(0) * D, hh, b);
+      tma_store_4d(&mapCs, sC, 0, mt(0) * (VB * D) + vb * D, hh, b);
       tma_store_commit();
     }
     __syncwarp();
@@ -668,10 +670,10 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
       if (lane == 0) {
         TC_PROF(c, 14);
         if (p.store_states && c + 1 < p.NT) {  // state entering tile c+1; its own, OLDER group than h(c): see the wait above
-          tma_store_4d(&mapCs, sC, 0, mt(c + 1) * D, hh, b);
+          tma_store_4d(&mapCs, sC, 0, mt(c + 1) * (VB * D) + vb * D, hh, b);
           tma_store_commit();
         }
-        tma_store_4d(&mapH, sH + (SM::kHBuf == 2 ? (c & 1) * SM::kTile : 0), 0, mt(c) * LT, hh, b);
+        tma_store_4d(&mapH, sH + (SM::kHBuf == 2 ? (c & 1) * SM::kTile : 0), vb * D, mt(c) * LT, hh, b);
         tma_store_commit();
         if (c + NSTAGE < p.NT) load_stage(s, c + NSTAGE);
         TC_PROF(c, 15);
@@ -819,7 +821,7 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
         for (int j = 0; j < CW; ++j) o[j] = (__uint_as_float(hi[j]) + bq * __uint_as_float(hx[j])) * inv;  // fw.py:200-212
         uint8_t* sHc = sH + (SM::kHBuf == 2 ? (c & 1) * SM::kTile : 0);
         store_cols<T, D>(sHc, row, ch * CW, o);
-        if (ch == 0 && row < n_valid) {
+        if (ch == 0 && row < n_valid && vb == 0) {
           p.n_out[(int64_t)bh * p.S + t0 + row] = nmax;
           p.m_out[(int64_t)bh * p.S + t0 + row] = m_t;
         }
@@ -864,12 +866,12 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
     // final states (fw.py:302-309)
     if (p.c_last) {
       if (owns_c) {
-        float* dst = p.c_last + ((int64_t)bh * D + drow) * D + ch * CW;
+        float* dst = p.c_last + ((int64_t)bh * D + drow) * (VB * D) + vb * D + ch * CW;
 #pragma unroll
         for (int j = 0; j < CW; ++j) dst[j] = Creg[j];
       }
-      if (owns_c && ch == 0) p.n_last[(int64_t)bh * D + drow] = n_reg;
-      if (tid == 0) p.m_last[bh] = m_run;
+      if (owns_c && ch == 0 && vb == 0) p.n_last[(int64_t)bh * D + drow] = n_reg;
+      if (tid == 0 && vb == 0) p.m_last[bh] = m_run;
     }
   }
   TC_PROF(200, 1);  // this role is done
@@ -878,6 +880,26 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
   TC_PROF(200, 2);
   TC_PROF_CTA(1);
   if (warp == kCtlWarp) tmem_dealloc<SM::kTmemCols>(tmem);
+}
+
+template <typename T, int D, bool REV, bool EPI>
+__global__ void __launch_bounds__(kTcThreads, D == 32 ? 2 : 1)
+tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
+          const __grid_constant__ CUtensorMap mapV, const __grid_constant__ CUtensorMap mapH,
+          const __grid_constant__ CUtensorMap mapCs, TcFwParams p) {
+  tc_fw_body<T, D, REV, EPI, 1>(mapQ, mapK, mapV, mapH, mapCs, p);
+}
+
+// Rectangular heads DHQK = D, DHHV = 2 D: the two square column-block problems of every (batch, head) in one launch
+// (grid 2 B NH, the two blocks of a head on adjacent CTAs so that their Q / K reads meet in L2).  Shared memory, TMEM
+// columns and CTAs per SM are those of tc_fw<T, D>; mapV / mapH are DHHV wide with D-wide boxes, and mapCs is the
+// block layout of make_states_map_blocks (the state entering tile c, column block vb, at rows (2 c + vb) D).
+template <typename T, int D, bool REV>
+__global__ void __launch_bounds__(kTcThreads, D == 32 ? 2 : 1)
+tc_fw_rect(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
+           const __grid_constant__ CUtensorMap mapV, const __grid_constant__ CUtensorMap mapH,
+           const __grid_constant__ CUtensorMap mapCs, TcFwParams p) {
+  tc_fw_body<T, D, REV, false, 2>(mapQ, mapK, mapV, mapH, mapCs, p);
 }
 
 // =============================================================================================
@@ -1022,7 +1044,7 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
     };
     // State entering tile c, for the backward: the 16-bit operand copy of C is stored as its four 64 x 64 blocks
     // (block = 2 * (dqk half) + (dv half)), 256 rows of 64 columns per tile, which is what the four head-dim-64
-    // block problems of the backward load (bw128_by_blocks).  sC holds two [128][64] column halves; a block is
+    // block problems of the backward load (bw_by_blocks).  sC holds two [128][64] column halves; a block is
     // 64 consecutive rows (8 KB) of one half.
     auto store_state = [&](int c) {
 #pragma unroll
@@ -1993,6 +2015,18 @@ int launch_fw(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk,
   return 0;
 }
 
+template <typename T, int D>
+int launch_fw_rect(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
+                   const CUtensorMap& mh, const CUtensorMap& mcs, cudaStream_t st) {
+  using SM = FwSmem<D>;
+  auto kern = p.rev ? tc_fw_rect<T, D, true> : tc_fw_rect<T, D, false>;
+  MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytes));
+  MLSTM_CUDA_CHECK(launch_pdl(pdl_mode() != 0, kern, 2 * p.B * p.NH, kTcThreads, SM::kBytes, st, mq, mk, mv, mh, mcs, p));
+  count_launch();
+  MLSTM_CUDA_CHECK(cudaGetLastError());
+  return 0;
+}
+
 template <typename T>
 int launch_fw_d128(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
                    const CUtensorMap& mh, const CUtensorMap& mcs, cudaStream_t st) {
@@ -2022,10 +2056,11 @@ bool tma_ok(const mlstm_b200_tensor& t) {
          (t.stride[2] % 8) == 0;
 }
 
-// [128 tokens][min(D, 64)] boxes: D = 32 -> 64-byte rows / SWIZZLE_64B, otherwise 128-byte rows / SWIZZLE_128B
-int make_map(CUtensorMap* m, const mlstm_b200_tensor& t, const mlstm_b200_shape& s, int D) {
+// [128 tokens][min(D, 64)] boxes: D = 32 -> 64-byte rows / SWIZZLE_64B, otherwise 128-byte rows / SWIZZLE_128B.
+// `box` < D: D-wide rows read or written in box-wide column blocks (v / h of the rectangular forward).
+int make_map(CUtensorMap* m, const mlstm_b200_tensor& t, const mlstm_b200_shape& s, int D, int box = 0) {
   return sm100_host::make_map_bhsd(m, t.ptr, s.dtype == MLSTM_B200_BF16, s.B, s.NH, s.S, D, t.stride[0], t.stride[1],
-                                   t.stride[2], LT, D == 32 ? 32 : 64);
+                                   t.stride[2], LT, box ? box : D == 32 ? 32 : 64);
 }
 // c_states: (B, NH, NT, D, D) 16-bit, one [D][D] box per tile
 int make_states_map(CUtensorMap* m, const void* ptr, const mlstm_b200_shape& s) {
@@ -2034,12 +2069,15 @@ int make_states_map(CUtensorMap* m, const void* ptr, const mlstm_b200_shape& s) 
                                    (int64_t)NT * D * D, D, D, D);
 }
 
-// head dim 128: (B, NH, NT * 256, 64) -- four 64 x 64 blocks per tile (see tc_fw_d128::store_state)
-int make_states_map_blocks(CUtensorMap* m, const void* ptr, const mlstm_b200_shape& s) {
+// states stored as bd x bd blocks: (B, NH, NT * rows, bd), `rows` = (DHQK / bd) (DHHV / bd) bd rows per tile, block
+// (a, b) of a tile at rows (a DHHV / bd + b) bd.  Head dim 128: bd = 64, four blocks (see tc_fw_d128::store_state);
+// rectangular heads (D, 2 D): bd = D, two blocks (tc_fw_rect).
+int make_states_map_blocks(CUtensorMap* m, const void* ptr, const mlstm_b200_shape& s, int rows, int bd) {
   const int NT = (s.S + LT - 1) / LT;
-  return sm100_host::make_map_bhsd(m, ptr, s.dtype == MLSTM_B200_BF16, s.B, s.NH, NT * 256, 64, (int64_t)s.NH * NT * 256 * 64,
-                                   (int64_t)NT * 256 * 64, 64, 64, 64);
+  return sm100_host::make_map_bhsd(m, ptr, s.dtype == MLSTM_B200_BF16, s.B, s.NH, NT * rows, bd, (int64_t)s.NH * NT * rows * bd,
+                                   (int64_t)NT * rows * bd, bd, bd, bd);
 }
+bool rect_heads(const mlstm_b200_shape& s) { return s.DHQK != s.DHHV; }
 
 int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   const mlstm_b200_shape& s = a.shape;
@@ -2048,6 +2086,10 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   const mlstm_b200_tensor& out = ep ? ep->y : a.h;
   if (!tma_ok(a.q) || !tma_ok(a.k) || !tma_ok(a.v) || !tma_ok(out)) {
     set_error("tensor path needs 16-byte aligned q/k/v/h with strides that are multiples of 8 elements");
+    return MLSTM_B200_EUNSUPPORTED;
+  }
+  if (ep && rect_heads(s)) {
+    set_error("fused epilogue: DHQK == DHHV only");
     return MLSTM_B200_EUNSUPPORTED;
   }
   if (ep) {
@@ -2063,11 +2105,15 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   CUtensorMap mq, mk, mv, mh, mcs;
   mlstm_b200_shape so = s;  // the y map carries y's element type
   if (ep) so.dtype = ep->xy_dtype;
-  int r = make_map(&mq, a.q, s, s.DHQK) | make_map(&mk, a.k, s, s.DHQK) | make_map(&mv, a.v, s, s.DHHV) |
-          make_map(&mh, out, so, s.DHHV);
+  const bool rect = rect_heads(s);
+  const int vbox = rect ? s.DHQK : 0;  // rectangular heads: v / h in DHQK-wide column blocks
+  int r = make_map(&mq, a.q, s, s.DHQK) | make_map(&mk, a.k, s, s.DHQK) | make_map(&mv, a.v, s, s.DHHV, vbox) |
+          make_map(&mh, out, so, s.DHHV, vbox);
   // without a c_states buffer the map is never used by the kernel; point it at the output to keep it valid
-  r |= !c_states ? make_map(&mcs, out, so, s.DHHV)
-                 : s.DHQK == 128 ? make_states_map_blocks(&mcs, c_states, s) : make_states_map(&mcs, c_states, s);
+  r |= !c_states ? make_map(&mcs, out, so, s.DHHV, vbox)
+       : s.DHQK == 128 ? make_states_map_blocks(&mcs, c_states, s, 256, 64)
+       : rect          ? make_states_map_blocks(&mcs, c_states, s, s.DHHV, s.DHQK)
+                       : make_states_map(&mcs, c_states, s);
   if (r) {
     set_error("cuTensorMapEncodeTiled failed (%d)", r);
     return MLSTM_B200_ENODEVICE;
@@ -2094,6 +2140,13 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
     p.h_plain = a.h.ptr; p.h_sb = a.h.stride[0]; p.h_sh = a.h.stride[1]; p.h_ss = a.h.stride[2];
   }
   TC_SET_PROF(p, 0);
+  if (rect) {
+    if (s.DHQK == 32)
+      return s.dtype == MLSTM_B200_BF16 ? launch_fw_rect<__nv_bfloat16, 32>(p, mq, mk, mv, mh, mcs, st)
+                                        : launch_fw_rect<__half, 32>(p, mq, mk, mv, mh, mcs, st);
+    return s.dtype == MLSTM_B200_BF16 ? launch_fw_rect<__nv_bfloat16, 64>(p, mq, mk, mv, mh, mcs, st)
+                                      : launch_fw_rect<__half, 64>(p, mq, mk, mv, mh, mcs, st);
+  }
   if (s.DHQK == 128) {
     if (s.dtype == MLSTM_B200_BF16) return launch_fw_d128<__nv_bfloat16>(p, mq, mk, mv, mh, mcs, st);
     return launch_fw_d128<__half>(p, mq, mk, mv, mh, mcs, st);
@@ -2122,105 +2175,106 @@ BwWs bw_ws(const mlstm_b200_shape& s) {
 
 
 // ---------------------------------------------------------------------------------------------
-// Head dim 128 backward (640-base384) as four d = 64 block problems.
+// Head dim 128 and rectangular-head backward as square block problems.
 //
 // With n_out and every max state held constant (the definition of this backward, native/bw.py:44-47) every term
-// of bw.py:106-203 is bilinear in (a 64-wide block of q / k, a 64-wide block of v / dh): dS = (dH V^T) . D and
-// S = (Q K^T) . D are sums over column blocks, the state gradient dC (dqk x dv) splits into four independent
-// 64 x 64 blocks with the same decay, and the stabilisers depend on the gates only.  A 128-wide tile set does not
-// fit the backward's shared memory with 128-token tiles, so the 128 x 128 problem runs as the sum of four
-// tc_bw<64> problems on strided views of the same tensors (no copies of q/k/v/dh; qk_scale = 128^-1/2; each loads its
-// block of the forward's saved states or recomputes it, bw.py:251-266).  The first partial of every output block is
-// written in place, the second is added by the kernel that produces it (TMA reduce-add stores).
-// 64 x 64 block (a, b) of a (BH, 128, 128) fp32 state <-> contiguous (BH, 64, 64); vec: (BH, 128) <-> (BH, 64)
-__global__ void k_state_block(float* __restrict__ blk, float* __restrict__ full, int a, int b, int64_t n, int scatter) {
+// of bw.py:106-203 is bilinear in (a bd-wide block of q / k, a bd-wide block of v / dh): dS = (dH V^T) . D and
+// S = (Q K^T) . D are sums over column blocks, the state gradient dC (dqk x dv) splits into independent bd x bd
+// blocks with the same decay, and the stabilisers depend on the gates only.  So a (DHQK, DHHV) problem is the sum of
+// (DHQK / bd) x (DHHV / bd) tc_bw<bd> problems on strided views of the same tensors (no copies of q/k/v/dh;
+// qk_scale = DHQK^-1/2 of the whole problem; each loads its block of the forward's saved states or recomputes it,
+// bw.py:251-266).  Head dim 128: bd = 64, a 2 x 2 grid (a 128-wide tile set does not fit the backward's shared memory
+// with 128-token tiles).  Rectangular heads (D, 2 D): bd = D, a 1 x 2 grid.  The first partial of every output block
+// is written in place, the second is added by the kernel that produces it (TMA reduce-add stores).
+// bd x bd block (a, b) of a (BH, DK, DV) fp32 state <-> contiguous (BH, bd, bd); vec: (BH, DK) <-> (BH, bd)
+__global__ void k_state_block(float* __restrict__ blk, float* __restrict__ full, int a, int b, int bd, int DK, int DV,
+                              int64_t n, int scatter) {
   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (idx >= n) return;
-  const int64_t bh = idx >> 12;
-  const int r = (int)((idx >> 6) & 63), c = (int)(idx & 63);
-  float* f = full + (bh * 128 + a * 64 + r) * 128 + b * 64 + c;
+  const int64_t bh = idx / ((int64_t)bd * bd);
+  const int r = (int)(idx / bd % bd), c = (int)(idx % bd);
+  float* f = full + (bh * DK + a * bd + r) * DV + b * bd + c;
   if (scatter) *f = blk[idx]; else blk[idx] = *f;
 }
-__global__ void k_state_vec_block(float* __restrict__ blk, const float* __restrict__ full, int a, int64_t n) {
+__global__ void k_state_vec_block(float* __restrict__ blk, const float* __restrict__ full, int a, int bd, int DK, int64_t n) {
   const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (idx >= n) return;
-  blk[idx] = full[(idx >> 6) * 128 + a * 64 + (idx & 63)];
+  blk[idx] = full[(idx / bd) * DK + a * bd + idx % bd];
 }
 
 }  // namespace
-int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, cudaStream_t st, int acc_qk = 0, int acc_v = 0,
-           int acc_g = 0);
-int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int block, cudaStream_t st, int acc_qk, int acc_v,
-                     int acc_g);
+int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, int nblocks, cudaStream_t st, int acc_qk = 0,
+           int acc_v = 0, int acc_g = 0);
+int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int block, int nblocks, cudaStream_t st, int acc_qk,
+                     int acc_v, int acc_g);
 namespace {
 
+int block_dim(const mlstm_b200_shape& s) { return s.DHQK == 128 ? 64 : s.DHQK; }
 mlstm_b200_shape block_shape(const mlstm_b200_shape& s) {
   mlstm_b200_shape b = s;
-  b.DHQK = b.DHHV = 64;
-  b.qk_scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf(128.f);
+  b.DHQK = b.DHHV = block_dim(s);
+  b.qk_scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf((float)s.DHQK);
   return b;
 }
-struct Bw128Ws {
-  size_t off_sub, sub_bytes, off_tq, off_tk, off_tv, off_ti, off_tf, off_c0, off_n0, off_dcl, off_dc0, total;
+struct BlocksWs {
+  size_t off_sub, sub_bytes, off_c0, off_n0, off_dcl, off_dc0, total;
 };
-Bw128Ws bw128_ws(const mlstm_b200_shape& s) {
-  Bw128Ws w{};
-  const size_t tok = (size_t)s.B * s.NH * s.S, bh = (size_t)s.B * s.NH;
+BlocksWs blocks_ws(const mlstm_b200_shape& s) {
+  BlocksWs w{};
+  const size_t bh = (size_t)s.B * s.NH, bd = block_dim(s);
   size_t o = 0;
   w.sub_bytes = bw_ws(block_shape(s)).total;
   w.off_sub = o; o += align_up(w.sub_bytes, 256);
-  w.off_tq = w.off_tk = w.off_tv = w.off_ti = w.off_tf = o;  // (partial sums are accumulated in-kernel: no scratch)
-  w.off_c0 = o; o += align_up(bh * 64 * 64 * 4, 256);
-  w.off_n0 = o; o += align_up(bh * 64 * 4, 256);
-  w.off_dcl = o; o += align_up(bh * 64 * 64 * 4, 256);
-  w.off_dc0 = o; o += align_up(bh * 64 * 64 * 4, 256);
+  w.off_c0 = o; o += align_up(bh * bd * bd * 4, 256);
+  w.off_n0 = o; o += align_up(bh * bd * 4, 256);
+  w.off_dcl = o; o += align_up(bh * bd * bd * 4, 256);
+  w.off_dc0 = o; o += align_up(bh * bd * bd * 4, 256);
   w.total = o;
   return w;
 }
 
 template <typename T>
-int bw128_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
+int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
   const mlstm_b200_shape& s = a.shape;
-  const Bw128Ws w = bw128_ws(s);
+  const BlocksWs w = blocks_ws(s);
   if (!a.workspace || a.workspace_bytes < w.total) {
     set_error("workspace too small: need %zu bytes, got %zu", w.total, a.workspace_bytes);
     return MLSTM_B200_EWORKSPACE;
   }
   char* ws = (char*)a.workspace;
-  const int64_t tok = (int64_t)s.B * s.NH * s.S, bh = (int64_t)s.B * s.NH;
-  auto dense = [&](size_t off, int width) {  // contiguous (B, NH, S, width) scratch tensor
-    mlstm_b200_tensor t{};
-    t.ptr = ws + off;
-    t.stride[0] = (int64_t)s.NH * s.S * width, t.stride[1] = (int64_t)s.S * width, t.stride[2] = width, t.stride[3] = 1;
-    return t;
-  };
-  auto cols = [&](const mlstm_b200_tensor& t, int j) {  // columns 64 j .. 64 j + 63 of a 128-wide tensor: a view
+  const int bd = block_dim(s), nq = s.DHQK / bd, nv = s.DHHV / bd;
+  const int64_t bh = (int64_t)s.B * s.NH, nst = bh * bd * bd, nvec = bh * bd;
+  auto cols = [&](const mlstm_b200_tensor& t, int j) {  // columns bd j .. bd j + bd - 1 of a wider tensor: a view
     mlstm_b200_tensor v = t;
-    v.ptr = (char*)t.ptr + (size_t)j * 64 * sizeof(T);
+    v.ptr = (char*)t.ptr + (size_t)j * bd * sizeof(T);
     return v;
   };
-  const int thr = 256;
+  auto state_block = [&](size_t off, const float* full, int qa, int vb, int scatter) {
+    k_state_block<<<(unsigned)((nst + 255) / 256), 256, 0, st>>>((float*)(ws + off), (float*)full, qa, vb, bd, s.DHQK, s.DHHV,
+                                                                  nst, scatter);
+  };
   int launches = 0;
   bool first = true;
-  for (int qa = 0; qa < 2; ++qa) {
-    for (int vb = 0; vb < 2; ++vb) {
+  for (int qa = 0; qa < nq; ++qa) {
+    for (int vb = 0; vb < nv; ++vb) {
       mlstm_b200_bw_args sub = a;
       sub.shape = block_shape(s);
       sub.q = cols(a.q, qa); sub.k = cols(a.k, qa); sub.v = cols(a.v, vb); sub.dh = cols(a.dh, vb);
-      // With the forward's saved states (tc_fw_d128 stores them block-wise) every problem loads its block; without
-      // them it recomputes its slice.
+      // With the forward's saved states (tc_fw_d128 / tc_fw_rect store them block-wise) every problem loads its
+      // block; without them it recomputes its slice.
       const bool saved = a.c_states != nullptr;
       sub.c_states = nullptr;
       sub.workspace = ws + w.off_sub; sub.workspace_bytes = w.sub_bytes;
       if (a.c_initial && !saved) {
-        k_state_block<<<(unsigned)((bh * 4096 + thr - 1) / thr), thr, 0, st>>>((float*)(ws + w.off_c0), (float*)a.c_initial, qa, vb, bh * 4096, 0);
-        k_state_vec_block<<<(unsigned)((bh * 64 + thr - 1) / thr), thr, 0, st>>>((float*)(ws + w.off_n0), a.n_initial, qa, bh * 64);
+        state_block(w.off_c0, a.c_initial, qa, vb, 0);
+        k_state_vec_block<<<(unsigned)((nvec + 255) / 256), 256, 0, st>>>((float*)(ws + w.off_n0), a.n_initial, qa, bd, s.DHQK,
+                                                                            nvec);
         sub.c_initial = (const float*)(ws + w.off_c0);
         sub.n_initial = (const float*)(ws + w.off_n0);
         launches += 2;
       }
       if (a.dc_last) {
-        k_state_block<<<(unsigned)((bh * 4096 + thr - 1) / thr), thr, 0, st>>>((float*)(ws + w.off_dcl), (float*)a.dc_last, qa, vb, bh * 4096, 0);
+        state_block(w.off_dcl, a.dc_last, qa, vb, 0);
         sub.dc_last = (const float*)(ws + w.off_dcl);
         ++launches;
       }
@@ -2234,10 +2288,11 @@ int bw128_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
       sub.dv = cols(a.dv, vb);
       sub.di = a.di;
       sub.df = a.df;
-      if (int e = tensor_bw_blocks(sub, saved ? a.c_states : nullptr, saved ? 2 * qa + vb : -1, st, vb == 1, qa == 1, !first))
+      if (int e = tensor_bw_blocks(sub, saved ? a.c_states : nullptr, saved ? qa * nv + vb : -1, nq * nv, st, vb > 0, qa > 0,
+                                   !first))
         return e;
       if (a.dc_initial) {
-        k_state_block<<<(unsigned)((bh * 4096 + thr - 1) / thr), thr, 0, st>>>((float*)(ws + w.off_dc0), a.dc_initial, qa, vb, bh * 4096, 1);
+        state_block(w.off_dc0, a.dc_initial, qa, vb, 1);
         ++launches;
       }
       first = false;
@@ -2267,10 +2322,12 @@ void tensor_set_clock_buffer(void* dev_ptr) {
 }
 bool tensor_context_is_current() { return sm100_host::context_is_current(); }
 
-// forward: d = 32, 64 and 128; backward: d = 32 and 64 natively, d = 128 as four d = 64 block problems (bw128_by_blocks)
+// forward: d = 32, 64 and 128; backward: d = 32 and 64 natively, d = 128 as four d = 64 block problems (bw_by_blocks).
+// Rectangular heads (DHQK, DHHV) = (32, 64) and (64, 128): the forward as two square column-block problems in one launch
+// (tc_fw_rect), the backward as two tc_bw<DHQK> block problems.
 bool tensor_supported(const mlstm_b200_shape& s, int backward) {
   if (s.dtype != MLSTM_B200_BF16 && s.dtype != MLSTM_B200_F16) return false;
-  if (s.DHQK != s.DHHV) return false;
+  if (s.DHQK != s.DHHV && !((s.DHQK == 32 || s.DHQK == 64) && s.DHHV == 2 * s.DHQK)) return false;
   if (s.DHQK != 64 && s.DHQK != 32 && s.DHQK != 128) return false;  // d = 128 backward: four d = 64 block problems
   // Tiles are 128 tokens whatever chunk_size is (h and the states do not depend on it: the stabiliser equals the
   // step-recurrent one), and ragged last tiles are handled in-kernel (TMA zero-fill, gates masked at scan time),
@@ -2283,30 +2340,31 @@ bool tensor_supported(const mlstm_b200_shape& s, int backward) {
 size_t tensor_states_bytes(const mlstm_b200_shape& s) {
   if (!tensor_supported(s, 1)) return 0;
   const size_t NT = (s.S + LT - 1) / LT;
-  return (size_t)s.B * s.NH * NT * s.DHQK * s.DHQK * 2;
+  return (size_t)s.B * s.NH * NT * s.DHQK * s.DHHV * 2;
 }
 
 // forward needs no scratch; backward needs room to recompute the states when c_states is absent
 size_t tensor_workspace_bytes(const mlstm_b200_shape& s, int backward) {
   if (!backward) return 256;
-  return s.DHQK == 128 ? bw128_ws(s).total : bw_ws(s).total;
+  return s.DHQK == 128 || rect_heads(s) ? blocks_ws(s).total : bw_ws(s).total;
 }
 
 int tensor_fw(const mlstm_b200_fw_args& a, cudaStream_t st) { return run_fw(a, a.c_states, st); }
 
-int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st) { return tensor_bw_blocks(a, a.c_states, -1, st, 0, 0, 0); }
+int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st) { return tensor_bw_blocks(a, a.c_states, -1, 1, st, 0, 0, 0); }
 
-// c_states: the forward's saved states (block < 0: this problem's own; block = 0..3: block `block` of a head-dim-128
-// forward's buffer) or NULL = recompute; acc_*: add into dq / dk, dv, di / df instead of overwriting them
-int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int block, cudaStream_t st, int acc_qk, int acc_v,
-                     int acc_g) {
+// c_states: the forward's saved states (block < 0: this problem's own; block = 0 .. nblocks - 1: block `block` of the
+// block-wise buffer of a head-dim-128 or rectangular forward) or NULL = recompute; acc_*: add into dq / dk, dv, di / df
+// instead of overwriting them
+int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int block, int nblocks, cudaStream_t st, int acc_qk,
+                     int acc_v, int acc_g) {
   const mlstm_b200_shape& s = a.shape;
   if (!tma_ok(a.q) || !tma_ok(a.k) || !tma_ok(a.v) || !tma_ok(a.dh) || !tma_ok(a.dq) || !tma_ok(a.dk) || !tma_ok(a.dv)) {
     set_error("tensor path needs 16-byte aligned q/k/v/dh/dq/dk/dv with strides that are multiples of 8 elements");
     return MLSTM_B200_EUNSUPPORTED;
   }
-  if (s.DHQK == 128)
-    return s.dtype == MLSTM_B200_BF16 ? bw128_by_blocks<__nv_bfloat16>(a, st) : bw128_by_blocks<__half>(a, st);
+  if (s.DHQK == 128 || rect_heads(s))
+    return s.dtype == MLSTM_B200_BF16 ? bw_by_blocks<__nv_bfloat16>(a, st) : bw_by_blocks<__half>(a, st);
   const void* c_states = c_states_in;
   if (!c_states) {  // recompute the states with a forward pass into the workspace (bw.py:251-266)
     block = -1;
@@ -2327,12 +2385,14 @@ int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int b
     if (int e = run_fw(f, ws + w.off_states, st)) return e;
     c_states = ws + w.off_states;
   }
-  return run_bw(a, c_states, block, st, acc_qk, acc_v, acc_g);
+  return run_bw(a, c_states, block, nblocks, st, acc_qk, acc_v, acc_g);
 }
 
-// block < 0: c_states holds this problem's own (B, NH, NT, D, D) states.  block = 0..3: c_states is the head-dim-128
-// forward's buffer (four 64 x 64 blocks per tile) and this head-dim-64 problem reads block `block` of every tile.
-int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, cudaStream_t st, int acc_qk, int acc_v, int acc_g) {
+// block < 0: c_states holds this problem's own (B, NH, NT, D, D) states.  block = 0 .. nblocks - 1: c_states is a
+// block-wise buffer (nblocks D x D blocks per tile, make_states_map_blocks) and this problem reads block `block` of
+// every tile.
+int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, int nblocks, cudaStream_t st, int acc_qk, int acc_v,
+           int acc_g) {
   const mlstm_b200_shape& s = a.shape;
   CUtensorMap mq, mk, mv, mdh, mcs, mdq, mdk, mdv;
   const int D = s.DHQK;
@@ -2340,7 +2400,7 @@ int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, cudaStr
   if (s.grad_dtype) sg.dtype = s.grad_dtype;
   const bool mixed = sg.dtype != s.dtype;
   int r = make_map(&mq, a.q, s, D) | make_map(&mk, a.k, s, D) | make_map(&mv, a.v, s, D) | make_map(&mdh, a.dh, s, D) |
-          (block < 0 ? make_states_map(&mcs, c_states, s) : make_states_map_blocks(&mcs, c_states, s)) |
+          (block < 0 ? make_states_map(&mcs, c_states, s) : make_states_map_blocks(&mcs, c_states, s, nblocks * D, D)) |
           make_map(&mdq, a.dq, sg, D) | make_map(&mdk, a.dk, sg, D) | make_map(&mdv, a.dv, sg, D);
   if (r) {
     set_error("cuTensorMapEncodeTiled failed (%d)", r);
@@ -2361,8 +2421,8 @@ int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, cudaStr
   p.sig = s.siging ? 1 : 0;
   p.cap = s.gate_soft_cap;
   p.acc_qk = acc_qk; p.acc_v = acc_v; p.acc_g = acc_g;
-  p.cs_rows = block < 0 ? D : 256;
-  p.cs_off = block < 0 ? 0 : 64 * block;
+  p.cs_rows = block < 0 ? D : nblocks * D;
+  p.cs_off = block < 0 ? 0 : D * block;
   TC_SET_PROF(p, 4096);
   int e;
   if (mixed) {  // kernel operands in one 16-bit dtype, gradients rounded once from fp32 to the other
