@@ -100,7 +100,9 @@ typedef struct mlstm_b200_shape {
  * y and x are (B, NH, S, DHHV) views given by element strides, innermost stride 1, 16-byte aligned with strides that are
  * multiples of 8 elements (y goes out through a TMA tensor map); both are 16-bit, of dtype xy_dtype (BF16 or F16), which
  * may differ from shape.dtype (bf16 kernel under fp16 autocast).  weight / bias / skip: contiguous fp32 (NH*DHHV), each
- * may be NULL (1 / 0 / 0); x.ptr may be NULL.  Tensor-core route only. */
+ * may be NULL (1 / 0 / 0); x.ptr may be NULL.  Tensor-core route only, every head geometry it covers: DHQK == DHHV and
+ * the rectangular (DHQK, DHHV) = (32, 64), (64, 128), whose two DHQK-wide column blocks per head run as one two-CTA
+ * cluster that exchanges the row statistics (mean and rstd are those of the whole DHHV row). */
 typedef struct mlstm_b200_fw_epilogue {
   mlstm_b200_tensor y; /* out */
   mlstm_b200_tensor x; /* optional skip input */
@@ -168,7 +170,8 @@ size_t mlstm_b200_states_bytes(const mlstm_b200_shape* shape);
 /* 1 if the tensor-core (tcgen05) kernels cover this shape/dtype forward AND backward, else 0
  * (16-bit dtypes, S % 4 == 0, and DHQK == DHHV in {32, 64, 128} or (DHQK, DHHV) in {(32, 64), (64, 128)}; the
  * head-dim-128 backward runs as four head-dim-64 block problems inside the call, a rectangular (D, 2 D) call as two
- * square head-dim-D problems on the two column halves of v / h / dh / dv). */
+ * square head-dim-D problems on the two column halves of v / h / dh / dv).  The forward's fused cell-output epilogue
+ * (mlstm_b200_fw_epilogue) is available for every shape this returns 1 for. */
 int mlstm_b200_tensor_path_supported(const mlstm_b200_shape* shape);
 
 /* Forward: h, n_out, m_out and optionally the last (C, n, m) states. */
@@ -187,6 +190,11 @@ int mlstm_b200_last_launch_count(void);
  * boundaries (forward at [tile*16 + slot], backward at [4096 + tile*16 + slot]).  NULL disables it.
  * In the product library this is a no-op: the product build holds no process-global mutable state. */
 void mlstm_b200_debug_set_clock_buffer(void* dev_ptr);
+
+/* How many {2, 1, 1} clusters of the forward with the fused epilogue for rectangular heads (shape.DHQK != DHHV; see
+ * mlstm_b200_fw_epilogue) the current device can hold at once (cudaOccupancyMaxActiveClusters); 0 for a shape that does
+ * not launch as clusters, -1 on error. */
+int mlstm_b200_debug_fw_epilogue_clusters(const mlstm_b200_shape* shape);
 
 /* ---------------------------------------------------------------------------------------------
  * Recurrent form (SURVEY.md section 8(f) #4): S token-by-token steps of the mLSTM with the (C, n, m) state kept on

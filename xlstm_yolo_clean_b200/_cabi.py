@@ -24,6 +24,7 @@ EXPORTS = (
     "mlstm_b200_chunkwise_bw",
     "mlstm_b200_last_launch_count",
     "mlstm_b200_debug_set_clock_buffer",
+    "mlstm_b200_debug_fw_epilogue_clusters",
     "mlstm_b200_recurrent_sequence",
     "mlstm_b200_cellout_workspace_bytes",
     "mlstm_b200_cellout_fw",
@@ -162,6 +163,8 @@ def load_library(path: str | None = None):
     lib.mlstm_b200_last_launch_count.restype = C.c_int
     lib.mlstm_b200_debug_set_clock_buffer.restype = None
     lib.mlstm_b200_debug_set_clock_buffer.argtypes = [C.c_void_p]
+    lib.mlstm_b200_debug_fw_epilogue_clusters.restype = C.c_int
+    lib.mlstm_b200_debug_fw_epilogue_clusters.argtypes = [C.POINTER(Shape)]
     lib.mlstm_b200_recurrent_sequence.restype = C.c_int
     lib.mlstm_b200_recurrent_sequence.argtypes = [C.POINTER(RecurrentArgs), C.c_void_p]
     lib.mlstm_b200_cellout_workspace_bytes.restype = C.c_size_t

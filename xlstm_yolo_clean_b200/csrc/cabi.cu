@@ -98,6 +98,16 @@ int mlstm_b200_last_launch_count(void) { return g_launches; }
 
 void mlstm_b200_debug_set_clock_buffer(void* dev_ptr) { tensor_set_clock_buffer(dev_ptr); }
 
+int mlstm_b200_debug_fw_epilogue_clusters(const mlstm_b200_shape* shape) {
+  g_err[0] = 0;
+  if (!shape) {
+    set_error("shape is NULL");
+    return -1;
+  }
+  if (require_device()) return -1;
+  return tensor_fw_epilogue_clusters(*shape);
+}
+
 int mlstm_b200_tensor_path_supported(const mlstm_b200_shape* shape) {
   if (!shape) return 0;
   return (tensor_supported(*shape, 0) && tensor_supported(*shape, 1)) ? 1 : 0;

@@ -186,6 +186,7 @@ bool tensor_context_is_current();  // a CUDA context is current on the calling t
 bool tensor_fw_views_ok(const mlstm_b200_fw_args& a);
 bool tensor_bw_views_ok(const mlstm_b200_bw_args& a);
 int tensor_fw(const mlstm_b200_fw_args& a, cudaStream_t st);
+int tensor_fw_epilogue_clusters(const mlstm_b200_shape& s);
 int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st);
 
 

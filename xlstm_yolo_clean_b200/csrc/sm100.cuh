@@ -1,5 +1,5 @@
 // Inline-PTX wrappers for the Blackwell (sm_100a) primitives the tensor-core kernels use:
-// mbarrier, TMA (cp.async.bulk.tensor), tcgen05.mma / commit / ld, TMEM alloc, proxy fences.
+// mbarrier, TMA (cp.async.bulk.tensor), tcgen05.mma / commit / ld, TMEM alloc, proxy fences, cluster / DSMEM.
 // Descriptor bit layouts follow the PTX ISA "tcgen05 matrix / instruction descriptor" tables.
 #pragma once
 
@@ -64,6 +64,45 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, int ta
   if (mbar_try_wait(bar, parity)) return;
   if (mbar_try_wait(bar, parity)) return;  // try_wait suspends for a while by itself; retry once inline
   mbar_wait_slow(bar, parity, tag);
+}
+
+// ---------------------------------------------------------------- thread-block clusters / distributed shared memory
+// shared::cluster address of the variable at `p` (own shared memory) in the CTA of cluster rank `rank`
+__device__ __forceinline__ uint32_t cluster_map(const void* p, uint32_t rank) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
+  return r;
+}
+__device__ __forceinline__ void st_cluster_f2(uint32_t caddr, float a, float b) {
+  asm volatile("st.shared::cluster.v2.f32 [%0], {%1, %2};" ::"r"(caddr), "f"(a), "f"(b) : "memory");
+}
+// arrive on an mbarrier of another CTA of the cluster; release: this thread's earlier writes (and those it has observed,
+// e.g. through __syncwarp) are visible to whoever acquires the completed phase
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t caddr) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(caddr) : "memory");
+}
+__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {
+  uint32_t ok;
+  asm volatile(
+      "{\n\t.reg .pred P;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2;\n\tselp.u32 %0, 1, 0, P;\n\t}\n"
+      : "=r"(ok)
+      : "r"(smem_u32(bar)), "r"(parity)
+      : "memory");
+  return ok != 0;
+}
+// bounded like mbar_wait: a lost remote arrival traps instead of hanging the GPU
+__device__ __noinline__ void mbar_wait_cluster_slow(uint64_t* bar, uint32_t parity) {
+  const long long t0 = clock64();
+  while (!mbar_try_wait_cluster(bar, parity))
+    if (clock64() - t0 > SM100_WAIT_CYCLES) __trap();
+}
+__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
+  if (mbar_try_wait_cluster(bar, parity)) return;
+  mbar_wait_cluster_slow(bar, parity);
+}
+// every thread of every CTA of the cluster; release / acquire order the shared-memory accesses around it cluster-wide
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 
 // ---------------------------------------------------------------- programmatic dependent launch

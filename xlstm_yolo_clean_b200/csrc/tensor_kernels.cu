@@ -340,10 +340,16 @@ __device__ __forceinline__ void prefetch_rows_l2(const uint16_t* base, int64_t s
 // tile earlier), so its latency hides under the statistics.  The slice is then overwritten in place with
 // y = (h - mean) rstd w + b + skip x in the y dtype.  (sstat is reused by the next tile only after every worker has
 // passed that tile's control-warp barriers, so one barrier per tile is enough.)
-template <typename T, int D, int NC, typename SwzFn>
+// `row_var` turns the CTA's (mean, M2) over its D columns into the variance of the whole LayerNorm row (and may update
+// mean): the row is these D columns (LnRowLocal), or, for rectangular heads, also the partner CTA's (tc_fw_body).
+template <int D>
+struct LnRowLocal {
+  __device__ __forceinline__ float operator()(float&, float m2) const { return m2 * (1.f / D); }
+};
+template <typename T, int D, int NC, typename SwzFn, typename RowVar = LnRowLocal<D>>
 __device__ __forceinline__ void ln_epilogue_slice(uint8_t* tile_slice_base, SwzFn swz, int row, int col0, int ch, int pair_bar,
                                                   float* sstat, const float* spar, const void* xrow, bool xy_f16, float ln_eps,
-                                                  bool row_valid) {
+                                                  bool row_valid, RowVar row_var = RowVar{}) {
   // spar: [3][D] = weight, bias, skip of this head; sstat: [2][LT] means, [2][LT] centred sums of squares, by column half
   constexpr int NV = NC / 8;        // 16-byte vectors in the slice
   constexpr int XE = NV < 4 ? NV : 4;  // skip-input vectors requested up front (the rest while the first are consumed)
@@ -372,9 +378,10 @@ __device__ __forceinline__ void ln_epilogue_slice(uint8_t* tile_slice_base, SwzF
   sstat[2 * LT + ch * LT + row] = s2;
   named_sync(pair_bar, 64);
   const float mean_b = sstat[(ch ^ 1) * LT + row], s2_b = sstat[2 * LT + (ch ^ 1) * LT + row];
-  const float mean = 0.5f * (mean_a + mean_b), dm = mean_a - mean_b;
+  float mean = 0.5f * (mean_a + mean_b);
+  const float dm = mean_a - mean_b;
   // (symmetric in a / b: both threads of the row get bit-identical statistics)
-  const float rstd = rsqrtf(((s2 + s2_b) + dm * dm * (0.5f * NC)) * (1.f / D) + ln_eps);
+  const float rstd = rsqrtf(row_var(mean, (s2 + s2_b) + dm * dm * (0.5f * NC)) + ln_eps);
 #pragma unroll
   for (int j = 0; j < NV; ++j) {
     uint4* slot = reinterpret_cast<uint4*>(tile_slice_base + swz(row, col0 + 8 * j));
@@ -452,6 +459,12 @@ struct FwSmem {
   static constexpr int fGates = 0, fRs = 2 * GateBuf::kFloats, fStat = fRs + 4 * LT, fPar = fStat + 4 * LT,
                        kSmallFloats = fPar + 3 * D;
   static constexpr int kBytes = oSmall + kSmallFloats * 4 + 1024 /*alignment slack*/;
+  // rectangular heads with the fused epilogue only (tc_fw_rect<..., EPI = true>, launched with kBytesPair): the partner
+  // CTA's (mean, M2) of every row, [2 slots by tile parity][LT] float2, and one mbarrier per slot, behind everything else.
+  // 2 KB more: by shared memory D = 32 still fits two CTAs per SM (2 x 112 KB), D = 64 one (212 KB).
+  static constexpr int oXst = oSmall + kSmallFloats * 4, oXbar = oXst + 2 * LT * 8, kBytesPair = kBytes + 2 * LT * 8 + 16;
+  static_assert(oXst % 16 == 0, "float2 slots");
+  static_assert((D == 32 ? 2 : 1) * (kBytesPair + 1024 /*per-CTA reserve*/ + 256 /*static*/) <= 228 * 1024, "CTAs per SM");
   // TMEM columns.  D = 64: S double-buffered by tile parity (512 columns, one CTA per SM).  D = 32: one S
   // buffer, 256 columns, so that two CTAs share an SM (S(k+1) is issued behind the MMAs that read P(k)).
   // P (16-bit, the A operand of P V) never goes through shared memory: each thread packs its S row in
@@ -466,11 +479,13 @@ struct FwSmem {
 
 // VB > 1: rectangular heads, DHQK = D and DHHV = VB * D.  CTA x runs the square problem of (batch, head) x / VB on
 // the D-wide column block vb = x % VB of v / h / C (see tc_fw_rect); n and m do not depend on v, so every block
-// computes them and block 0 writes them.
+// computes them and block 0 writes them.  With the fused epilogue the two blocks of a head are one {2, 1, 1} cluster
+// (cluster rank = vb) and exchange the LayerNorm row statistics through distributed shared memory.
 template <typename T, int D, bool REV, bool EPI, int VB>
 __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtensorMap& mapK, const CUtensorMap& mapV,
                                            const CUtensorMap& mapH, const CUtensorMap& mapCs, const TcFwParams& p) {
-  static_assert(VB == 1 || !EPI, "the fused epilogue needs the whole h row");
+  static_assert(VB == 1 || VB == 2, "one or two column blocks");
+  constexpr bool kPair = EPI && VB == 2;  // cluster launch, partner statistics
   constexpr bool kBf16 = std::is_same<T, __nv_bfloat16>::value;
   using SM = FwSmem<D>;
   using L = Lay<D>;
@@ -520,6 +535,10 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
     mbar_init(&bar_hx, 1);
     mbar_init(&bar_g[0], 1);
     mbar_init(&bar_g[1], 1);
+    if constexpr (kPair) {  // partner statistics of tiles of parity 0 / 1: one remote arrive per ch == 0 worker warp
+      mbar_init(reinterpret_cast<uint64_t*>(smem + SM::oXbar), 4);
+      mbar_init(reinterpret_cast<uint64_t*>(smem + SM::oXbar) + 1, 4);
+    }
     fence_mbar_init();
   }
   if (warp == kCtlWarp) {
@@ -554,12 +573,12 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
       const uint32_t one2 = pack2<T>(1.f, 1.f);
       for (int e = tid; e < 2048 / 16; e += kWorkers) reinterpret_cast<uint4*>(sOnes)[e] = make_uint4(one2, one2, one2, one2);
     }
-    if (EPI) {  // per-channel parameters of the fused cell-output epilogue for this head
+    if (EPI) {  // per-channel parameters of the fused cell-output epilogue for this head's column block
       float* spar = fsm + SM::fPar;
       for (int e = tid; e < D; e += kWorkers) {
-        spar[e] = p.ln_w ? p.ln_w[hh * D + e] : 1.f;
-        spar[D + e] = p.ln_b ? p.ln_b[hh * D + e] : 0.f;
-        spar[2 * D + e] = p.ln_skip ? p.ln_skip[hh * D + e] : 0.f;
+        spar[e] = p.ln_w ? p.ln_w[hh * (VB * D) + vb * D + e] : 1.f;
+        spar[D + e] = p.ln_b ? p.ln_b[hh * (VB * D) + vb * D + e] : 0.f;
+        spar[2 * D + e] = p.ln_skip ? p.ln_skip[hh * (VB * D) + vb * D + e] : 0.f;
       }
     }
     named_sync(NB_PAIR0, kWorkers);  // sNt zeroed before the owners write column 0
@@ -579,6 +598,7 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
+  if constexpr (kPair) cluster_sync();  // the partner's mbarriers are initialised before the first remote arrive
   const uint32_t tmem = tmem_base_s;
   const uint32_t tS0 = tmem + SM::cS0, tS1 = tmem + SM::cS1, tHi = tmem + SM::cHi, tHx = tmem + SM::cHx, tDC = tmem + SM::cDC,
                  tDN = tmem + SM::cDN;
@@ -692,7 +712,7 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
       return load_gate_raw<T>(ip + (int64_t)t1 * p.ig_ss, p.ig_ss, fp + (int64_t)t1 * p.fg_ss, p.fg_ss, min(LT, p.S - t1));
     };
     // skip-input rows of this head (fused epilogue): pulled into L2 two tiles before the workers read them
-    const uint16_t* xbase = p.x ? (const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh : nullptr;
+    const uint16_t* xbase = p.x ? (const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh + vb * D : nullptr;
     GateRaw<T> raw = raw_of(0);
     for (int n = 0; n < p.NT; ++n) {  // vectors of tile n; tiles 0 and 1 need no buffer hand-back
       if (EPI && p.x) prefetch_rows_l2<D * 2>(xbase, p.x_ss, mt(n) * LT, min(LT, p.S - mt(n) * LT), lane);
@@ -829,14 +849,44 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
           // fused cell output (mlstm_b200_fw_epilogue): the un-normalised row goes out from the staged copy (training:
           // the LayerNorm backward needs it), then the staged slice becomes y = LN(h) w + b + skip x
           const int64_t tok = (int64_t)(t0 + row);
+          const int col = vb * D + ch * CW;  // first column of this thread's slice in the DHHV-wide row
           if (p.h_plain && row < n_valid) {
-            uint4* dst = reinterpret_cast<uint4*>((T*)p.h_plain + b * p.h_sb + hh * p.h_sh + tok * p.h_ss + ch * CW);
+            uint4* dst = reinterpret_cast<uint4*>((T*)p.h_plain + b * p.h_sb + hh * p.h_sh + tok * p.h_ss + col);
 #pragma unroll
             for (int j = 0; j < CW / 8; ++j) dst[j] = *reinterpret_cast<const uint4*>(sHc + L::swz(row, ch * CW + 8 * j));
           }
-          const void* xrow = p.x ? (const void*)((const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh + tok * p.x_ss + ch * CW) : nullptr;
-          ln_epilogue_slice<T, D, CW>(sHc, [](int r, int cc) { return L::swz(r, cc); }, row, ch * CW, ch, NB_PAIR0 + rb,
-                                      fsm + SM::fStat, fsm + SM::fPar, xrow, p.xy_f16 != 0, p.ln_eps, row < n_valid);
+          const void* xrow = p.x ? (const void*)((const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh + tok * p.x_ss + col) : nullptr;
+          if constexpr (!kPair) {
+            ln_epilogue_slice<T, D, CW>(sHc, [](int r, int cc) { return L::swz(r, cc); }, row, ch * CW, ch, NB_PAIR0 + rb,
+                                        fsm + SM::fStat, fsm + SM::fPar, xrow, p.xy_f16 != 0, p.ln_eps, row < n_valid);
+          } else {
+            // The row's other D columns are in the partner CTA (cluster rank vb ^ 1).  The ch == 0 thread of every row
+            // -- every row, valid or not, so that each tile sees its 4 arrivals -- writes this block's (mean, M2) into
+            // the partner's slot of the tile's parity, and each of the 4 ch == 0 warps then arrives once on the partner's
+            // mbarrier of that slot; both threads of the row wait for the partner's arrivals on the local one and combine
+            // the two blocks in block order (bit-identical mean and rstd in both CTAs), exactly as the in-CTA halves.
+            // Two slots are enough: the partner writes tile c + 2 into this slot only after it has received our tile
+            // c + 1 statistics, which the ch == 0 thread sends after this tile's pair barrier of tile c + 1 -- that is,
+            // after both threads of the row have read the slot for tile c.  The same ordering keeps each mbarrier at
+            // most one phase ahead of its waiters, so the parity wait cannot skip a phase.
+            auto pair_var = [&](float& mean, float m2) {
+              float2* xst = reinterpret_cast<float2*>(smem + SM::oXst) + (c & 1) * LT;
+              uint64_t* xbar = reinterpret_cast<uint64_t*>(smem + SM::oXbar) + (c & 1);
+              if (ch == 0) {  // warp-uniform
+                st_cluster_f2(cluster_map(xst + row, vb ^ 1), mean, m2);
+                __syncwarp();
+                if (lane == 0) mbar_arrive_cluster(cluster_map(xbar, vb ^ 1));
+              }
+              mbar_wait_cluster(xbar, (c >> 1) & 1);
+              const float2 o = xst[row];
+              const float mean0 = vb ? o.x : mean, mean1 = vb ? mean : o.x, m2_0 = vb ? o.y : m2, m2_1 = vb ? m2 : o.y;
+              const float dmb = mean0 - mean1;
+              mean = 0.5f * (mean0 + mean1);
+              return ((m2_0 + m2_1) + dmb * dmb * (0.5f * D)) * (1.f / (2 * D));
+            };
+            ln_epilogue_slice<T, D, CW>(sHc, [](int r, int cc) { return L::swz(r, cc); }, row, ch * CW, ch, NB_PAIR0 + rb,
+                                        fsm + SM::fStat, fsm + SM::fPar, xrow, p.xy_f16 != 0, p.ln_eps, row < n_valid, pair_var);
+          }
         }
       }
       // ---- state update C_k = gbar C_{k-1} + dC; n_k ---------------------------------------------------
@@ -880,6 +930,7 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
   TC_PROF(200, 2);
   TC_PROF_CTA(1);
   if (warp == kCtlWarp) tmem_dealloc<SM::kTmemCols>(tmem);
+  if constexpr (kPair) cluster_sync();  // neither CTA exits while its partner may still write into its shared memory
 }
 
 template <typename T, int D, bool REV, bool EPI>
@@ -894,12 +945,13 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
 // (grid 2 B NH, the two blocks of a head on adjacent CTAs so that their Q / K reads meet in L2).  Shared memory, TMEM
 // columns and CTAs per SM are those of tc_fw<T, D>; mapV / mapH are DHHV wide with D-wide boxes, and mapCs is the
 // block layout of make_states_map_blocks (the state entering tile c, column block vb, at rows (2 c + vb) D).
-template <typename T, int D, bool REV>
+// EPI: fused cell-output epilogue, launched as {2, 1, 1} clusters (launch_fw_rect) with FwSmem<D>::kBytesPair.
+template <typename T, int D, bool REV, bool EPI>
 __global__ void __launch_bounds__(kTcThreads, D == 32 ? 2 : 1)
 tc_fw_rect(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
            const __grid_constant__ CUtensorMap mapV, const __grid_constant__ CUtensorMap mapH,
            const __grid_constant__ CUtensorMap mapCs, TcFwParams p) {
-  tc_fw_body<T, D, REV, false, 2>(mapQ, mapK, mapV, mapH, mapCs, p);
+  tc_fw_body<T, D, REV, EPI, 2>(mapQ, mapK, mapV, mapH, mapCs, p);
 }
 
 // =============================================================================================
@@ -2015,13 +2067,40 @@ int launch_fw(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk,
   return 0;
 }
 
+// The two column blocks of a head (adjacent CTAs) as one {2, 1, 1} cluster: co-scheduled, and each can reach the other's
+// shared memory.  Programmatic stream serialisation as launch_pdl.
+template <typename... KArgs, typename... Args>
+cudaError_t launch_pair_pdl(bool use_pdl, void (*kern)(KArgs...), int grid, int block, size_t smem, cudaStream_t st,
+                            Args&&... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid), cfg.blockDim = dim3(block), cfg.dynamicSmemBytes = smem, cfg.stream = st;
+  cudaLaunchAttribute attr[2];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr, cfg.numAttrs = use_pdl ? 2 : 1;
+  return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
+}
+
+template <typename T, int D>
+auto fw_rect_kernel(bool epi, bool rev) {
+  return epi ? (rev ? tc_fw_rect<T, D, true, true> : tc_fw_rect<T, D, false, true>)
+             : (rev ? tc_fw_rect<T, D, true, false> : tc_fw_rect<T, D, false, false>);
+}
+
 template <typename T, int D>
 int launch_fw_rect(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
                    const CUtensorMap& mh, const CUtensorMap& mcs, cudaStream_t st) {
   using SM = FwSmem<D>;
-  auto kern = p.rev ? tc_fw_rect<T, D, true> : tc_fw_rect<T, D, false>;
-  MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytes));
-  MLSTM_CUDA_CHECK(launch_pdl(pdl_mode() != 0, kern, 2 * p.B * p.NH, kTcThreads, SM::kBytes, st, mq, mk, mv, mh, mcs, p));
+  auto kern = fw_rect_kernel<T, D>(p.epi != 0, p.rev != 0);
+  if (p.epi) {  // fused epilogue: LayerNorm statistics exchanged between the two blocks of a head
+    MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytesPair));
+    MLSTM_CUDA_CHECK(launch_pair_pdl(pdl_mode() != 0, kern, 2 * p.B * p.NH, kTcThreads, SM::kBytesPair, st, mq, mk, mv, mh, mcs, p));
+  } else {
+    MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytes));
+    MLSTM_CUDA_CHECK(launch_pdl(pdl_mode() != 0, kern, 2 * p.B * p.NH, kTcThreads, SM::kBytes, st, mq, mk, mv, mh, mcs, p));
+  }
   count_launch();
   MLSTM_CUDA_CHECK(cudaGetLastError());
   return 0;
@@ -2086,10 +2165,6 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   const mlstm_b200_tensor& out = ep ? ep->y : a.h;
   if (!tma_ok(a.q) || !tma_ok(a.k) || !tma_ok(a.v) || !tma_ok(out)) {
     set_error("tensor path needs 16-byte aligned q/k/v/h with strides that are multiples of 8 elements");
-    return MLSTM_B200_EUNSUPPORTED;
-  }
-  if (ep && rect_heads(s)) {
-    set_error("fused epilogue: DHQK == DHHV only");
     return MLSTM_B200_EUNSUPPORTED;
   }
   if (ep) {
@@ -2350,6 +2425,29 @@ size_t tensor_workspace_bytes(const mlstm_b200_shape& s, int backward) {
 }
 
 int tensor_fw(const mlstm_b200_fw_args& a, cudaStream_t st) { return run_fw(a, a.c_states, st); }
+
+// cudaOccupancyMaxActiveClusters of the rectangular forward with the fused epilogue ({2, 1, 1} clusters) on the current
+// device; 0 for a shape that does not launch it, -1 on a CUDA error
+int tensor_fw_epilogue_clusters(const mlstm_b200_shape& s) {
+  if (!tensor_supported(s, 0) || !rect_heads(s)) return 0;
+  auto query = [&](auto kern, int smem) {
+    if (ensure_smem(kern, smem) != cudaSuccess) return -1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(2 * s.B * s.NH), cfg.blockDim = dim3(kTcThreads), cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr, cfg.numAttrs = 1;
+    int n = 0;
+    return cudaOccupancyMaxActiveClusters(&n, kern, &cfg) == cudaSuccess ? n : -1;
+  };
+  const bool bf = s.dtype == MLSTM_B200_BF16, rev = s.reverse != 0;
+  if (s.DHQK == 32)
+    return bf ? query(fw_rect_kernel<__nv_bfloat16, 32>(true, rev), FwSmem<32>::kBytesPair)
+              : query(fw_rect_kernel<__half, 32>(true, rev), FwSmem<32>::kBytesPair);
+  return bf ? query(fw_rect_kernel<__nv_bfloat16, 64>(true, rev), FwSmem<64>::kBytesPair)
+            : query(fw_rect_kernel<__half, 64>(true, rev), FwSmem<64>::kBytesPair);
+}
 
 int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st) { return tensor_bw_blocks(a, a.c_states, -1, 1, st, 0, 0, 0); }
 

@@ -39,6 +39,17 @@ def cellout_supported(NH: int, D: int) -> bool:
     return D in (32, 64, 128) and (NH * D) % 128 == 0 and NH * D <= 2048
 
 
+# one_launch="auto" for rectangular heads, by (DHQK, DHHV, gradients wanted): True = the cell as one forward launch (the
+# rectangular forward with the fused epilogue, two-CTA clusters), False = the rectangular forward + cell-output pass.
+# Measured on an NVIDIA B200 at 1000 W (profiles/r04_rect_epilogue_bench.jsonl, tools/rect_cell_bench.py; DESIGN.md
+# section 4.3): the one-launch cell is 0-14 % slower without gradients and 17-38 % slower in training at both pairs and
+# both BASELINE call sizes, so "auto" keeps two launches; one_launch="always" still fuses.
+RECT_ONE_LAUNCH = {
+    (32, 64, False): False, (32, 64, True): False,
+    (64, 128, False): False, (64, 128, True): False,
+}
+
+
 def _f32c(t):
     return None if t is None else t.detach().to(torch.float32).contiguous()
 
@@ -184,26 +195,36 @@ def rms_norm_b200(x, weight=None, eps=1e-6, out_dtype=None):
     return _RmsNorm.apply(x, weight, eps, out_dtype)
 
 
-def _grad_dtype(in_dtypes, v_k, NH):
+TENSOR_HEAD_DIMS = ((32, 32), (64, 64), (128, 128), (32, 64), (64, 128))  # (DHQK, DHHV) of the tensor-core kernels
+
+
+def _head_dims(qk, v, NH):
+    """(DHQK, DHHV) of layer-layout tensors: qk (B, S, 2 NH DHQK) = [q | k], v (B, S, NH DHHV)."""
+    return qk.shape[-1] // (2 * NH), v.shape[-1] // NH
+
+
+def _grad_dtype(in_dtypes, qk_k, v_k, NH):
     """dtype the backward kernel writes d_qk / d_v / d_gates in: the dtype the layer's tensors had before they were
     re-rounded to the kernel dtype (fp16 under ultralytics' AMP with the bf16 kernels) when the tensor-core route runs
     and the three agree -- ``shape.grad_dtype`` of the C-ABI -- else the kernel dtype (and a cast afterwards)."""
     kdt, dt = v_k.dtype, in_dtypes[0]
-    S, D = v_k.shape[1], v_k.shape[2] // NH
+    S = v_k.shape[1]
     if (dt is not kdt and dt in (torch.float16, torch.bfloat16) and kdt in (torch.float16, torch.bfloat16)
-            and all(t is dt for t in in_dtypes) and D in (32, 64, 128) and S % 4 == 0
+            and all(t is dt for t in in_dtypes) and _head_dims(qk_k, v_k, NH) in TENSOR_HEAD_DIMS and S % 4 == 0
             and _backend._default_impl != _cabi.IMPL_EXACT):
         return dt
     return kdt
 
 
 def _heads(qk, v, gates, NH):
-    """(B, NH, S, D) / (B, NH, S) views of the layer-layout tensors: no data movement."""
+    """(B, NH, S, DHQK) q / k, (B, NH, S, DHHV) v and (B, NH, S) i / f views of the layer-layout tensors: no data
+    movement.  q / k may be narrower than v (rectangular heads)."""
     B, S, H = v.shape
-    D = H // NH
-    q = qk[..., :H].view(B, S, NH, D).transpose(1, 2)
-    k = qk[..., H:].view(B, S, NH, D).transpose(1, 2)
-    vv = v.view(B, S, NH, D).transpose(1, 2)
+    DK, DV = _head_dims(qk, v, NH)
+    Hqk = NH * DK
+    q = qk[..., :Hqk].view(B, S, NH, DK).transpose(1, 2)
+    k = qk[..., Hqk:].view(B, S, NH, DK).transpose(1, 2)
+    vv = v.view(B, S, NH, DV).transpose(1, 2)
     return q, k, vv, gates[..., :NH].transpose(1, 2), gates[..., NH:].transpose(1, 2)
 
 
@@ -224,7 +245,7 @@ class _MlstmLayerLayout(torch.autograd.Function):
             # themselves (the result does not depend on chunk_size: the stabiliser equals the step-recurrent one),
             # so S = 400 / 100 run as they are with a chunk size that divides them -- no zero-padding copies.
             g = math.gcd(S, chunk_size)
-            if tensor_path_supported(B, NH, S, H // NH, H // NH, kernel_dtype, chunk_size=g):
+            if tensor_path_supported(B, NH, S, *_head_dims(qk, v, NH), kernel_dtype, chunk_size=g):
                 chunk_size = g
         pad = (-S) % chunk_size
         if pad:  # zero padding as wrap_chunkwise__pad_zeros (kernel_wrappers.py:227-247); padded tokens come last
@@ -248,7 +269,7 @@ class _MlstmLayerLayout(torch.autograd.Function):
         NH, reverse, siging, chunk_size, eps, pad, S, soft_cap = ctx.cfg
         if pad:
             dh = F.pad(dh, (0, 0, pad, 0) if reverse else (0, 0, 0, pad))
-        gdt = _grad_dtype(ctx.in_dtypes, v_k, NH)  # the caller's 16-bit dtype: no cast pass over the gradients
+        gdt = _grad_dtype(ctx.in_dtypes, qk_k, v_k, NH)  # the caller's 16-bit dtype: no cast pass over the gradients
         d_qk, d_v, d_g = (torch.empty_like(t, dtype=gdt) for t in (qk_k, v_k, g_k))
         q, k, vv, i, f = _heads(qk_k, v_k, g_k, NH)
         mlstm_chunkwise_bw(q, k, vv, i, f, n_out, m_out, dh, chunk_size=chunk_size, eps=eps, c_states=c_states,
@@ -293,7 +314,7 @@ class _MlstmCellFused(torch.autograd.Function):
     ``_MlstmLayerLayout``) with MultiHeadLayerNorm, the (B, NH, S, D) -> (B, S, H) relayout and the learnable skip done in
     the kernel's epilogue (C-ABI ``mlstm_b200_fw_epilogue``): no separate cell-output pass, and under no_grad h never
     reaches HBM un-normalised.  In training h is also written (the LayerNorm backward needs it); the backward is the
-    stand-alone cell-output backward followed by the mLSTM backward."""
+    stand-alone cell-output backward (over DHHV) followed by the mLSTM backward.  q / k may be narrower than v."""
 
     @staticmethod
     @custom_fwd(device_type="cuda")
@@ -327,7 +348,7 @@ class _MlstmCellFused(torch.autograd.Function):
         NH, reverse, siging, chunk_size, eps, soft_cap, ln_eps, out_dtype = ctx.cfg
         dh, dpar, dx = _cellout_bw_call(h, xs, weight, skip if xs is not None else None, dy, ln_eps, out_dtype,
                                         ctx.needs_input_grad[3])
-        gdt = _grad_dtype(ctx.in_dtypes, v_k, NH)  # the caller's 16-bit dtype: no cast pass over the gradients
+        gdt = _grad_dtype(ctx.in_dtypes, qk_k, v_k, NH)  # the caller's 16-bit dtype: no cast pass over the gradients
         d_qk, d_v, d_g = (torch.empty_like(t, dtype=gdt) for t in (qk_k, v_k, g_k))
         q, k, vv, i, f = _heads(qk_k, v_k, g_k, NH)
         nmp = nm.data_ptr()
@@ -385,11 +406,11 @@ def mlstm_cell_b200(cell, q, k, v, reverse=False, skip=None, x_skip=None, siging
     (fused LayerNorm / skip epilogue); see below."""
     if one_launch not in ("auto", "always", "never"):
         raise ValueError(f"one_launch must be 'auto', 'always' or 'never' (got {one_launch!r})")
-    B, S, H = q.shape
+    B, S, H = v.shape  # q / k (B, S, NH DHQK) may be narrower than v (B, S, NH DHHV); the output is v's width
     if not q.is_cuda:
         raise RuntimeError("mlstm_cell_b200: tensors are on the CPU; this backend has no CPU path")
     NH = cell.num_heads
-    D = H // NH
+    DK, D = q.shape[-1] // NH, H // NH
     if_preact = _gate_preact(cell, q, k, v, qk)
     model_dtype = q.dtype
     if qk is not None:  # layer-layout path: the kernel reads / writes the layer's own tensors
@@ -400,7 +421,8 @@ def mlstm_cell_b200(cell, q, k, v, reverse=False, skip=None, x_skip=None, siging
         # soft_cap (vision_lstm2.py:714-715, 755-756): on the tensor-core route the scan warp of the kernels applies
         # cap * tanh(x / cap) to the pre-activations it reads anyway, and the backward applies its derivative where it
         # stores dI / dF -- no elementwise passes over the gates in either direction (zero padding stays zero: tanh 0 = 0)
-        in_kernel_cap = (kdt in (torch.float16, torch.bfloat16) and D in (32, 64, 128) and _backend._default_impl != _cabi.IMPL_EXACT)
+        in_kernel_cap = (kdt in (torch.float16, torch.bfloat16) and (DK, D) in TENSOR_HEAD_DIMS
+                         and _backend._default_impl != _cabi.IMPL_EXACT)
         gates = if_preact if in_kernel_cap else cell.gate_soft_cap * torch.tanh(if_preact / cell.gate_soft_cap)
         qk_c, v_c, g_c = qk, v, gates
         if cell.use_autocast:
@@ -414,7 +436,11 @@ def mlstm_cell_b200(cell, q, k, v, reverse=False, skip=None, x_skip=None, siging
         # the mLSTM kernel followed by the stand-alone cell-output pass is faster (408 vs 428 us; 327 vs 352 us).
         needs_grad = torch.is_grad_enabled() and any(
             t is not None and t.requires_grad for t in (qk_c, v_c, g_c, x_skip, norm.weight_proxy, norm.bias, skip))
-        fuse = one_launch == "always" or (one_launch == "auto" and not needs_grad and D in (32, 64))
+        if DK == D:
+            auto_fuse = not needs_grad and D in (32, 64)
+        else:  # rectangular heads: RECT_ONE_LAUNCH, measured separately (the epilogue runs as two-CTA clusters)
+            auto_fuse = RECT_ONE_LAUNCH.get((DK, D, needs_grad), False)
+        fuse = one_launch == "always" or (one_launch == "auto" and auto_fuse)
         if (fuse and in_kernel_cap and S % 4 == 0 and out_dtype in (torch.float16, torch.bfloat16)
                 and cellout_supported(NH, D) and (x_skip is None or x_skip.shape == (B, S, H))):
             return _MlstmCellFused.apply(qk_c, v_c, g_c, x_skip if skip is not None else None, norm.weight_proxy, norm.bias,
@@ -426,7 +452,7 @@ def mlstm_cell_b200(cell, q, k, v, reverse=False, skip=None, x_skip=None, siging
         capped = cell.gate_soft_cap * torch.tanh(if_preact / cell.gate_soft_cap)  # soft_cap, vision_lstm2.py:755-756
         i_pre, f_pre = torch.chunk(capped, 2, dim=-1)
         i, f = i_pre.transpose(-1, -2), f_pre.transpose(-1, -2)  # (B, NH, S) views
-        qh, kh, vh = (t.view(B, S, NH, D).transpose(1, 2) for t in (q, k, v))  # (B, NH, S, D) views, no copy
+        qh, kh, vh = (t.view(B, S, NH, t.shape[-1] // NH).transpose(1, 2) for t in (q, k, v))  # (B, NH, S, D) views, no copy
         if cell.use_autocast:
             qh, kh, vh, i, f = (t.to(cell.autocast_dtype) for t in (qh, kh, vh, i, f))
         pad = (-S) % chunk_size
