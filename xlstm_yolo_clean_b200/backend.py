@@ -322,6 +322,8 @@ def convert16(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     goes through torch."""
     if x.dtype is dtype:
         return x
+    if torch.compiler.is_compiling():
+        return _ops.convert16(x, dtype)
     if (not x.is_cuda or {x.dtype, dtype} != {torch.float16, torch.bfloat16} or x.numel() == 0
             or not _is_dense(x)):
         return x.to(dtype)
@@ -352,9 +354,10 @@ def mlstm_chunkwise_fw(q, k, v, i, f, c_initial=None, n_initial=None, m_initial=
     if c_initial is None and (n_initial is not None or m_initial is not None):
         B, NH, S, DK = q.shape
         c_initial = torch.zeros(B, NH, DK, v.shape[-1], device=q.device)
-    h, nm, last, c_states = _fw_launch(q, k, v, i, f, c_initial, n_initial, m_initial, qk_scale, bool(return_last_states),
-                                       int(chunk_size), float(eps), impl, bool(save_states), bool(reverse), bool(siging),
-                                       float(gate_soft_cap or 0.0))
+    launch = _ops.fw_launch if torch.compiler.is_compiling() else _fw_launch
+    h, nm, last, c_states = launch(q, k, v, i, f, c_initial, n_initial, m_initial, qk_scale, bool(return_last_states),
+                                   int(chunk_size), float(eps), impl, bool(save_states), bool(reverse), bool(siging),
+                                   float(gate_soft_cap or 0.0))
     return h, nm[0], nm[1], last, c_states
 
 
@@ -480,6 +483,10 @@ def mlstm_chunkwise_bw(q, k, v, i, f, n_out, m_out, dh, c_initial=None, n_initia
     if c_initial is None and (n_initial is not None or m_initial is not None):
         B, NH, S, DK = q.shape
         c_initial = torch.zeros(B, NH, DK, v.shape[-1], device=q.device)
+    if torch.compiler.is_compiling():
+        return _ops.bw_launch(q, k, v, i, f, n_out, m_out, dh, c_initial, n_initial, m_initial, dc_last, qk_scale,
+                              int(chunk_size), float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), bool(siging),
+                              out, float(gate_soft_cap or 0.0), grad_dtype)
     n_out = n_out if n_out.is_contiguous() else n_out.contiguous()
     m_out = m_out if m_out.is_contiguous() else m_out.contiguous()
     return _bw_launch(q, k, v, i, f, n_out.data_ptr(), m_out.data_ptr(), dh, c_initial, n_initial, m_initial, dc_last, qk_scale,
@@ -568,6 +575,8 @@ def mlstm_chunkwise__b200(
     if autocast_kernel_dtype not in _FUNCTIONS:
         raise ValueError(f"Unsupported kernel dtype {autocast_kernel_dtype}.")
     fn = _FUNCTIONS[autocast_kernel_dtype]
+    if torch.compiler.is_compiling():
+        fn = _ops.chunkwise_function(autocast_kernel_dtype)
     h, c_last, n_last, m_last = fn.apply(q, k, v, i, f, c_initial, n_initial, m_initial, bool(return_last_states),
                                          int(chunk_size), float(eps), bool(reverse), False,
                                          _caller_grad_dtype(autocast_kernel_dtype, q, k, v, i, f))
@@ -602,6 +611,8 @@ def mlstm_siging_chunkwise__b200(
     if autocast_kernel_dtype not in _FUNCTIONS:
         raise ValueError(f"Unsupported kernel dtype {autocast_kernel_dtype}.")
     fn = _FUNCTIONS[autocast_kernel_dtype]
+    if torch.compiler.is_compiling():
+        fn = _ops.chunkwise_function(autocast_kernel_dtype)
     need_states = c_initial is not None or n_initial is not None
     m_initial = None
     if need_states:
@@ -626,6 +637,9 @@ def mlstm_recurrent_sequence__b200(q, k, v, i, f, c_initial=None, n_initial=None
     ``mlstm_recurrent_sequence__native_fw`` (mlstm_kernels/torch/recurrent/native_sequence.py:133-175; registry name
     ``native_sequence__native``).  q, k (B, NH, S, DHQK), v (B, NH, S, DHHV), i, f (B, NH, S).
     Returns h, or (h, (C, n, m)) with ``return_last_states`` -- the reference's convention; forward only."""
+    if torch.compiler.is_compiling():
+        return _ops.recurrent_sequence(q, k, v, i, f, c_initial, n_initial, m_initial, bool(return_last_states), float(eps),
+                                       dtype_state, bool(siging))
     lib = _cabi.load_library()
     for name, t in (("q", q), ("k", k), ("v", v), ("i", i), ("f", f)):
         if not t.is_cuda:
@@ -749,3 +763,6 @@ def patch_model(model: torch.nn.Module, name: str = KERNEL_NAME, mode: str = "tr
 
         vil.patch_layers(model, siging=siging, kernel_dtype=kernel_dtype, graphs=graphs)
     return n
+
+
+from . import ops as _ops  # noqa: E402  (the torch.library ops are built on this module's launchers)

@@ -29,6 +29,7 @@ import torch.nn.functional as F
 
 from . import _cabi
 from . import backend as _backend
+from . import ops as _ops
 from torch.amp import custom_bwd, custom_fwd
 
 from .backend import (_DTYPES, _cell_uses_siging, _on_device, _tensor, mlstm_chunkwise__b200, mlstm_chunkwise_bw, mlstm_chunkwise_fw,
@@ -58,62 +59,46 @@ def _vec_ok(t: torch.Tensor) -> bool:
     return t.stride(-1) == 1 and all(s % 4 == 0 for s in t.stride()[:-1]) and t.data_ptr() % 16 == 0
 
 
+def _cellout_fw_call(h, x, weight, bias, skip, eps, out_dtype):
+    """mlstm_b200_cellout_fw: y (B, S, NH*D) in ``out_dtype``.  ``h`` passes ``_vec_ok``; ``x`` is None or contiguous in
+    ``out_dtype``."""
+    lib = _cabi.load_library()
+    B, NH, S, D = h.shape
+    w32, b32, s32 = _f32c(weight), _f32c(bias), _f32c(skip)
+    with _on_device(h.device):
+        y = torch.empty(B, S, NH * D, dtype=out_dtype, device=h.device)
+        a = _cabi.CellOutArgs()
+        a.B, a.NH, a.S, a.D = B, NH, S, D
+        a.h_dtype, a.x_dtype, a.y_dtype = _DTYPES[h.dtype], _DTYPES[out_dtype], _DTYPES[out_dtype]
+        a.eps = float(eps)
+        a.h, a.x, a.y = _tensor(h), _tensor(x), _tensor(y)
+        a.weight = None if w32 is None else w32.data_ptr()
+        a.bias = None if b32 is None else b32.data_ptr()
+        a.skip = None if s32 is None else s32.data_ptr()
+        st = lib.mlstm_b200_cellout_fw(C.byref(a), C.c_void_p(torch.cuda.current_stream(h.device).cuda_stream))
+        _cabi.check(st, "mlstm_b200_cellout_fw")
+    return y
+
+
 class _CellOut(torch.autograd.Function):
     """y = MultiHeadLayerNorm(h) [+ skip * x], h (B,NH,S,D) -> y (B,S,NH*D)."""
 
     @staticmethod
     def forward(ctx, h, weight, bias, skip, x, eps, out_dtype):
-        lib = _cabi.load_library()
         if not h.is_cuda:
             raise RuntimeError("cell_out: h is on the CPU; this backend has no CPU path")
-        B, NH, S, D = h.shape
         h = h if _vec_ok(h) else h.contiguous()
         if x is not None:  # x, y, dy, dx all move as dense (B, S, H) rows
             x = x if (x.dtype == out_dtype and x.is_contiguous() and x.data_ptr() % 16 == 0) else x.to(out_dtype).contiguous()
-        w32, b32, s32 = _f32c(weight), _f32c(bias), _f32c(skip)
-        with _on_device(h.device):
-            y = torch.empty(B, S, NH * D, dtype=out_dtype, device=h.device)
-            a = _cabi.CellOutArgs()
-            a.B, a.NH, a.S, a.D = B, NH, S, D
-            a.h_dtype, a.x_dtype, a.y_dtype = _DTYPES[h.dtype], _DTYPES[out_dtype], _DTYPES[out_dtype]
-            a.eps = float(eps)
-            a.h, a.x, a.y = _tensor(h), _tensor(x), _tensor(y)
-            a.weight = None if w32 is None else w32.data_ptr()
-            a.bias = None if b32 is None else b32.data_ptr()
-            a.skip = None if s32 is None else s32.data_ptr()
-            st = lib.mlstm_b200_cellout_fw(C.byref(a), C.c_void_p(torch.cuda.current_stream(h.device).cuda_stream))
-            _cabi.check(st, "mlstm_b200_cellout_fw")
+        y = _cellout_fw_call(h, x, weight, bias, skip, eps, out_dtype)
         ctx.save_for_backward(h, x, weight, bias, skip)
         ctx.eps, ctx.out_dtype = float(eps), out_dtype
         return y
 
     @staticmethod
     def backward(ctx, dy):
-        lib = _cabi.load_library()
         h, x, weight, bias, skip = ctx.saved_tensors
-        B, NH, S, D = h.shape
-        dy = dy if (dy.dtype == ctx.out_dtype and dy.is_contiguous() and dy.data_ptr() % 16 == 0) else dy.to(ctx.out_dtype).contiguous()
-        w32, s32 = _f32c(weight), _f32c(skip)
-        dev = h.device
-        with _on_device(dev):
-            dh = torch.empty_strided(h.shape, h.stride(), dtype=h.dtype, device=dev)  # the kernel walks h and dh together
-            dx = torch.empty_like(dy) if (x is not None and ctx.needs_input_grad[4]) else None
-            dpar = torch.empty(3, NH * D, dtype=torch.float32, device=dev)
-            b = _cabi.CellOutBwArgs()
-            a = b.fw
-            a.B, a.NH, a.S, a.D = B, NH, S, D
-            a.h_dtype, a.x_dtype, a.y_dtype = _DTYPES[h.dtype], _DTYPES[ctx.out_dtype], _DTYPES[ctx.out_dtype]
-            a.eps = ctx.eps
-            a.h, a.x = _tensor(h), _tensor(x)
-            a.weight = None if w32 is None else w32.data_ptr()
-            a.skip = None if s32 is None else s32.data_ptr()
-            b.dy, b.dh, b.dx = _tensor(dy), _tensor(dh), _tensor(dx)
-            b.dweight, b.dbias, b.dskip = dpar[0].data_ptr(), dpar[1].data_ptr(), dpar[2].data_ptr()
-            ws_bytes = lib.mlstm_b200_cellout_workspace_bytes(C.byref(a))
-            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            b.workspace, b.workspace_bytes = ws.data_ptr(), ws_bytes
-            st = lib.mlstm_b200_cellout_bw(C.byref(b), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
-            _cabi.check(st, "mlstm_b200_cellout_bw")
+        dh, dpar, dx = _cellout_bw_call(h, x, weight, skip, dy, ctx.eps, ctx.out_dtype, ctx.needs_input_grad[4])
         return (dh,
                 None if weight is None else dpar[0].to(weight.dtype),
                 None if bias is None else dpar[1].to(bias.dtype),
@@ -125,10 +110,52 @@ def cell_out(h, weight=None, bias=None, skip=None, x=None, eps=1e-6, out_dtype=N
     """Fused MultiHeadLayerNorm (+ skip): see the module docstring.  ``weight`` is the effective scale
     (the reference's ``weight_proxy`` = 1 + weight, vision_lstm2.py:900-907)."""
     out_dtype = out_dtype or (x.dtype if x is not None else h.dtype)
+    if torch.compiler.is_compiling():
+        return _ops.cell_out(h, weight, bias, skip, x, eps, out_dtype)
     return _CellOut.apply(h, weight, bias, skip, x, eps, out_dtype)
 
 
 RMSNORM_DIMS = (192, 256, 384, 512)
+
+
+def _rmsnorm_fw_call(x2, weight, eps, out_dtype):
+    """mlstm_b200_rmsnorm_fw on contiguous (rows, C) ``x2``: returns y (rows, C) in ``out_dtype`` and rstd (rows,) fp32."""
+    lib = _cabi.load_library()
+    rows, Cdim = x2.shape
+    w32 = _f32c(weight)
+    with _on_device(x2.device):
+        y = torch.empty(rows, Cdim, dtype=out_dtype, device=x2.device)
+        rstd = torch.empty(rows, dtype=torch.float32, device=x2.device)
+        a = _cabi.RmsNormArgs()
+        a.rows, a.C, a.x_dtype, a.y_dtype, a.eps = rows, Cdim, _DTYPES[x2.dtype], _DTYPES[out_dtype], float(eps)
+        a.x, a.y, a.rstd = x2.data_ptr(), y.data_ptr(), rstd.data_ptr()
+        a.weight = None if w32 is None else w32.data_ptr()
+        st = lib.mlstm_b200_rmsnorm_fw(C.byref(a), C.c_void_p(torch.cuda.current_stream(x2.device).cuda_stream))
+        _cabi.check(st, "mlstm_b200_rmsnorm_fw")
+    return y, rstd
+
+
+def _rmsnorm_bw_call(x2, weight, rstd, dy2, eps, out_dtype):
+    """mlstm_b200_rmsnorm_bw: dx (rows, C) in x2's dtype and dweight (C,) fp32; ``dy2`` contiguous in ``out_dtype``."""
+    lib = _cabi.load_library()
+    rows, Cdim = x2.shape
+    w32 = _f32c(weight)
+    dev = x2.device
+    with _on_device(dev):
+        dx = torch.empty_like(x2)
+        dw = torch.empty(Cdim, dtype=torch.float32, device=dev)
+        b = _cabi.RmsNormBwArgs()
+        a = b.fw
+        a.rows, a.C, a.x_dtype, a.y_dtype, a.eps = rows, Cdim, _DTYPES[x2.dtype], _DTYPES[out_dtype], eps
+        a.x, a.rstd = x2.data_ptr(), rstd.data_ptr()
+        a.weight = None if w32 is None else w32.data_ptr()
+        b.dy, b.dx, b.dweight = dy2.data_ptr(), dx.data_ptr(), dw.data_ptr()
+        nws = lib.mlstm_b200_rmsnorm_workspace_bytes(C.byref(a))
+        ws = torch.empty(nws, dtype=torch.uint8, device=dev)
+        b.workspace, b.workspace_bytes = ws.data_ptr(), nws
+        st = lib.mlstm_b200_rmsnorm_bw(C.byref(b), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+        _cabi.check(st, "mlstm_b200_rmsnorm_bw")
+    return dx, dw
 
 
 class _RmsNorm(torch.autograd.Function):
@@ -137,50 +164,23 @@ class _RmsNorm(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, eps, out_dtype):
-        lib = _cabi.load_library()
         if not x.is_cuda:
             raise RuntimeError("rms_norm_b200: x is on the CPU; this backend has no CPU path")
         shp = x.shape
         x2 = x.reshape(-1, shp[-1])
         x2 = x2 if x2.is_contiguous() else x2.contiguous()
-        rows, Cdim = x2.shape
-        w32 = _f32c(weight)
-        with _on_device(x.device):
-            y = torch.empty(rows, Cdim, dtype=out_dtype, device=x.device)
-            rstd = torch.empty(rows, dtype=torch.float32, device=x.device)
-            a = _cabi.RmsNormArgs()
-            a.rows, a.C, a.x_dtype, a.y_dtype, a.eps = rows, Cdim, _DTYPES[x2.dtype], _DTYPES[out_dtype], float(eps)
-            a.x, a.y, a.rstd = x2.data_ptr(), y.data_ptr(), rstd.data_ptr()
-            a.weight = None if w32 is None else w32.data_ptr()
-            st = lib.mlstm_b200_rmsnorm_fw(C.byref(a), C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream))
-            _cabi.check(st, "mlstm_b200_rmsnorm_fw")
+        y, rstd = _rmsnorm_fw_call(x2, weight, eps, out_dtype)
         ctx.save_for_backward(x2, weight, rstd)
         ctx.eps, ctx.out_dtype, ctx.shp = float(eps), out_dtype, shp
         return y.view(shp)
 
     @staticmethod
     def backward(ctx, dy):
-        lib = _cabi.load_library()
         x2, weight, rstd = ctx.saved_tensors
         rows, Cdim = x2.shape
         dy2 = dy.reshape(rows, Cdim)
         dy2 = dy2 if (dy2.dtype == ctx.out_dtype and dy2.is_contiguous()) else dy2.to(ctx.out_dtype).contiguous()
-        w32 = _f32c(weight)
-        dev = x2.device
-        with _on_device(dev):
-            dx = torch.empty_like(x2)
-            dw = torch.empty(Cdim, dtype=torch.float32, device=dev)
-            b = _cabi.RmsNormBwArgs()
-            a = b.fw
-            a.rows, a.C, a.x_dtype, a.y_dtype, a.eps = rows, Cdim, _DTYPES[x2.dtype], _DTYPES[ctx.out_dtype], ctx.eps
-            a.x, a.rstd = x2.data_ptr(), rstd.data_ptr()
-            a.weight = None if w32 is None else w32.data_ptr()
-            b.dy, b.dx, b.dweight = dy2.data_ptr(), dx.data_ptr(), dw.data_ptr()
-            nws = lib.mlstm_b200_rmsnorm_workspace_bytes(C.byref(a))
-            ws = torch.empty(nws, dtype=torch.uint8, device=dev)
-            b.workspace, b.workspace_bytes = ws.data_ptr(), nws
-            st = lib.mlstm_b200_rmsnorm_bw(C.byref(b), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
-            _cabi.check(st, "mlstm_b200_rmsnorm_bw")
+        dx, dw = _rmsnorm_bw_call(x2, weight, rstd, dy2, ctx.eps, ctx.out_dtype)
         return dx.view(ctx.shp), (None if weight is None else dw.to(weight.dtype)), None, None
 
 
@@ -192,6 +192,8 @@ def rms_norm_b200(x, weight=None, eps=1e-6, out_dtype=None):
             out_dtype = torch.get_autocast_dtype("cuda")
         else:
             out_dtype = x.dtype  # torch.rms_norm returns the input dtype
+    if torch.compiler.is_compiling():
+        return _ops.rms_norm(x, weight, eps, out_dtype)
     return _RmsNorm.apply(x, weight, eps, out_dtype)
 
 
@@ -207,10 +209,14 @@ def _grad_dtype(in_dtypes, qk_k, v_k, NH):
     """dtype the backward kernel writes d_qk / d_v / d_gates in: the dtype the layer's tensors had before they were
     re-rounded to the kernel dtype (fp16 under ultralytics' AMP with the bf16 kernels) when the tensor-core route runs
     and the three agree -- ``shape.grad_dtype`` of the C-ABI -- else the kernel dtype (and a cast afterwards)."""
-    kdt, dt = v_k.dtype, in_dtypes[0]
-    S = v_k.shape[1]
+    return _grad_dtype_of(in_dtypes, v_k.dtype, _head_dims(qk_k, v_k, NH), v_k.shape[1])
+
+
+def _grad_dtype_of(in_dtypes, kdt, head_dims, S):
+    """``_grad_dtype`` from the kernel dtype, (DHQK, DHHV) and S alone."""
+    dt = in_dtypes[0]
     if (dt is not kdt and dt in (torch.float16, torch.bfloat16) and kdt in (torch.float16, torch.bfloat16)
-            and all(t is dt for t in in_dtypes) and _head_dims(qk_k, v_k, NH) in TENSOR_HEAD_DIMS and S % 4 == 0
+            and all(t is dt for t in in_dtypes) and head_dims in TENSOR_HEAD_DIMS and S % 4 == 0
             and _backend._default_impl != _cabi.IMPL_EXACT):
         return dt
     return kdt
@@ -443,10 +449,12 @@ def mlstm_cell_b200(cell, q, k, v, reverse=False, skip=None, x_skip=None, siging
         fuse = one_launch == "always" or (one_launch == "auto" and auto_fuse)
         if (fuse and in_kernel_cap and S % 4 == 0 and out_dtype in (torch.float16, torch.bfloat16)
                 and cellout_supported(NH, D) and (x_skip is None or x_skip.shape == (B, S, H))):
-            return _MlstmCellFused.apply(qk_c, v_c, g_c, x_skip if skip is not None else None, norm.weight_proxy, norm.bias,
+            fused = _ops.cell_fused if torch.compiler.is_compiling() else _MlstmCellFused.apply
+            return fused(qk_c, v_c, g_c, x_skip if skip is not None else None, norm.weight_proxy, norm.bias,
                                          skip, NH, bool(reverse), bool(siging), int(chunk_size), float(eps), kdt,
                                          float(cell.gate_soft_cap), float(norm.eps), out_dtype)
-        h = _MlstmLayerLayout.apply(qk_c, v_c, g_c, NH, bool(reverse), bool(siging), int(chunk_size), float(eps), kdt,
+        layer = _ops.layer_layout if torch.compiler.is_compiling() else _MlstmLayerLayout.apply
+        h = layer(qk_c, v_c, g_c, NH, bool(reverse), bool(siging), int(chunk_size), float(eps), kdt,
                                     float(cell.gate_soft_cap) if in_kernel_cap else 0.0)
     else:
         capped = cell.gate_soft_cap * torch.tanh(if_preact / cell.gate_soft_cap)  # soft_cap, vision_lstm2.py:755-756
@@ -577,6 +585,8 @@ class _Graphed:
         raise NotImplementedError
 
     def _graphable(self, x) -> bool:
+        if torch.compiler.is_compiling():  # torch.compile traces the eager layer (its ops are graph nodes)
+            return False
         if (torch.distributed.is_available() and torch.distributed.is_initialized()
                 and torch.distributed.get_world_size() > 1):
             # single-process training only: a capture started lazily inside DDP's forward is invalidated by the
