@@ -75,7 +75,12 @@ typedef struct mlstm_b200_shape {
                          initial / last states then refer to the END / START of the sequence in memory */
   int32_t siging;     /* 1: sigmoid input gate, no max state, denominator max(|n|, 1) -- the variant the
                          reference's CUDA model path uses (triton_xl_chunk_siging/fwbw.py:211-268,
-                         parallel/native_siging/fw.py:15-74); m_initial / m_last are then ignored / zero */
+                         parallel/native_siging/fw.py:15-74); m_initial / m_last are then ignored / zero.
+                         2: the same sigmoid input gate WITHOUT the normaliser (the reference's normalize=False,
+                         triton_xl_chunk_siging/fwbw.py:211-268): h = q C + sum_s P_ts v_s is the numerator, eps does not
+                         enter it, and the backward uses dh as it is and never reads n_out (the forward still writes
+                         n_out / m_out and carries n, so the last states are those of siging = 1).  Not with the fused
+                         cell-output epilogue (MLSTM_B200_EUNSUPPORTED).  Any other value: MLSTM_B200_EINVAL. */
   float eps;
   float qk_scale;     /* <= 0 selects DHQK^-0.5 (native/fw.py:263-264) */
   float gate_soft_cap;/* > 0: i and f are gate PRE-activations and the kernels apply the cell's soft cap
@@ -208,7 +213,8 @@ int mlstm_b200_debug_fw_epilogue_clusters(const mlstm_b200_shape* shape);
  *   DHQK == DHHV in {32, 64, 128} or (DHQK, DHHV) in {(32, 64), (64, 128)}; dtype of q / k / v / i / f / h; states
  *   contiguous fp32 as in the chunkwise calls
  *   (m is (B, NH)).  Initial states: all three or none (none = zeros); last states: all three or none; the last
- *   states may alias the initial ones (in-place update).  siging = 1: sigmoid input gate, m stays 0.
+ *   states may alias the initial ones (in-place update).  siging = 1: sigmoid input gate, m stays 0; siging = 2: the
+ *   same without the normaliser (h = q . C_t, as mlstm_b200_shape::siging = 2).
  *   Forward only (the reference's recurrent kernels have no backward).
  */
 typedef struct mlstm_b200_recurrent_args {

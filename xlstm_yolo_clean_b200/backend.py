@@ -70,7 +70,17 @@ class _on_device:
             self.ctx.__exit__(*a)
 
 
-def _shape(q, v, chunk_size, eps, impl, qk_scale=None, reverse=False, siging=False, gate_soft_cap=0.0) -> _cabi.Shape:
+def _siging_mode(siging, normalize=True) -> int:
+    """``mlstm_b200_shape::siging``: 0 exp input gate, 1 sigmoid input gate, 2 sigmoid input gate without the
+    normaliser (``normalize=False``, h = q C + sum_s P_ts v_s).  The exp-gate variant always normalises."""
+    if not normalize:
+        if not siging:
+            raise ValueError("normalize=False exists for the sigmoid input gate only (pass siging=True)")
+        return 2
+    return 1 if siging else 0
+
+
+def _shape(q, v, chunk_size, eps, impl, qk_scale=None, reverse=False, siging=0, gate_soft_cap=0.0) -> _cabi.Shape:
     B, NH, S, DK = q.shape
     s = _cabi.Shape()
     s.B, s.NH, s.S, s.DHQK, s.DHHV = B, NH, S, DK, v.shape[-1]
@@ -78,7 +88,7 @@ def _shape(q, v, chunk_size, eps, impl, qk_scale=None, reverse=False, siging=Fal
     s.dtype = _DTYPES[q.dtype]
     s.impl = _default_impl if impl is None else impl
     s.reverse = 1 if reverse else 0
-    s.siging = 1 if siging else 0
+    s.siging = int(siging)  # _siging_mode
     s.eps = float(eps)
     s.qk_scale = -1.0 if qk_scale is None else float(qk_scale)
     s.gate_soft_cap = float(gate_soft_cap or 0.0)
@@ -199,7 +209,8 @@ def _ws_tensor(nbytes: int, dev):
 def _fw_launch(q, k, v, i, f, c0, n0, m0, qk_scale, return_last_states, chunk_size, eps, impl, save_states, reverse, siging,
                soft_cap=0.0, epi: Optional[FwEpilogue] = None):
     """Returns h, nm (2, B, NH, S) fp32 = [n_out, m_out], last-or-None, c_states-or-None.  With ``epi`` the kernel writes
-    epi.y (fused LayerNorm + skip epilogue) and h is None unless epi.want_h."""
+    epi.y (fused LayerNorm + skip epilogue) and h is None unless epi.want_h.  ``siging``: the C-ABI mode, see
+    ``_siging_mode`` (a bool is mode 0 / 1)."""
     impl = _default_impl if impl is None else impl
     dt = q.dtype
     if i.dtype is not dt:
@@ -343,20 +354,25 @@ def convert16(x: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
 
 def mlstm_chunkwise_fw(q, k, v, i, f, c_initial=None, n_initial=None, m_initial=None, qk_scale=None,
                        return_last_states=False, chunk_size=64, eps=1e-6, impl=None, save_states=True, reverse=False, siging=False,
-                       gate_soft_cap=0.0):
+                       gate_soft_cap=0.0, normalize=True):
     """C-ABI forward.  Returns h, n_out, m_out, last_states-or-None (fp32), c_states-or-None.
+
+    ``normalize=False`` (sigmoid input gate only, ``ValueError`` otherwise): h is the numerator q C + sum_s P_ts v_s,
+    without the division by max(|n|, 1) + eps; n_out / m_out are written as with the normaliser, and the last states
+    are the same.
 
     ``gate_soft_cap`` > 0: ``i`` / ``f`` are gate pre-activations and the kernel applies ``cap * tanh(x / cap)``
     (MatrixLSTMCell.soft_cap, vision_lstm2.py:714-715) while it scans them (tensor-core route only).
 
     ``c_states`` is the opaque per-tile state buffer the tensor-core backward consumes (the
     reference's return_all_states mode, native/fwbw.py:73-101); None when the kernels recompute."""
+    mode = _siging_mode(siging, normalize)
     if c_initial is None and (n_initial is not None or m_initial is not None):
         B, NH, S, DK = q.shape
         c_initial = torch.zeros(B, NH, DK, v.shape[-1], device=q.device)
     launch = _ops.fw_launch if torch.compiler.is_compiling() else _fw_launch
     h, nm, last, c_states = launch(q, k, v, i, f, c_initial, n_initial, m_initial, qk_scale, bool(return_last_states),
-                                   int(chunk_size), float(eps), impl, bool(save_states), bool(reverse), bool(siging),
+                                   int(chunk_size), float(eps), impl, bool(save_states), bool(reverse), mode,
                                    float(gate_soft_cap or 0.0))
     return h, nm[0], nm[1], last, c_states
 
@@ -472,31 +488,37 @@ def _bw_launch(q, k, v, i, f, n_ptr, m_ptr, dh, c0, n0, m0, dcl, qk_scale, chunk
 
 def mlstm_chunkwise_bw(q, k, v, i, f, n_out, m_out, dh, c_initial=None, n_initial=None, m_initial=None,
                        dc_last=None, qk_scale=None, chunk_size=64, eps=1e-6, impl=None, want_dc_initial=False,
-                       c_states=None, reverse=False, siging=False, out=None, gate_soft_cap=0.0, grad_dtype=None):
+                       c_states=None, reverse=False, siging=False, out=None, gate_soft_cap=0.0, grad_dtype=None,
+                       normalize=True):
     """C-ABI backward.  Returns dq, dk, dv, di, df, dc_initial-or-None (fp32).
+
+    ``normalize=False`` (sigmoid input gate only, ``ValueError`` otherwise): the backward of the forward's
+    ``normalize=False``; dh is not scaled by 1 / (n_out + eps) and ``n_out`` is not read.
 
     With ``gate_soft_cap`` > 0 (see the forward) di / df are gradients w.r.t. the gate pre-activations.
 
     ``out`` = (dq, dk, dv, di, df) lets the caller provide the gradient tensors (any batch/head/token strides,
     unit innermost stride for dq/dk/dv), e.g. views into a fused (B, S, 2H) qk gradient.  Their dtype -- or
     ``grad_dtype`` when the gradients are allocated here -- may be the other 16-bit dtype than the kernel's."""
+    mode = _siging_mode(siging, normalize)
     if c_initial is None and (n_initial is not None or m_initial is not None):
         B, NH, S, DK = q.shape
         c_initial = torch.zeros(B, NH, DK, v.shape[-1], device=q.device)
     if torch.compiler.is_compiling():
         return _ops.bw_launch(q, k, v, i, f, n_out, m_out, dh, c_initial, n_initial, m_initial, dc_last, qk_scale,
-                              int(chunk_size), float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), bool(siging),
+                              int(chunk_size), float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), mode,
                               out, float(gate_soft_cap or 0.0), grad_dtype)
     n_out = n_out if n_out.is_contiguous() else n_out.contiguous()
     m_out = m_out if m_out.is_contiguous() else m_out.contiguous()
     return _bw_launch(q, k, v, i, f, n_out.data_ptr(), m_out.data_ptr(), dh, c_initial, n_initial, m_initial, dc_last, qk_scale,
-                      int(chunk_size), float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), bool(siging), out,
+                      int(chunk_size), float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), mode, out,
                       float(gate_soft_cap or 0.0), grad_dtype)
 
 
 def _make_function(autocast_kernel_dtype: torch.dtype):
     class _MlstmChunkwiseB200(torch.autograd.Function):
-        """autograd.Function with the contract of _mlstm_chunkwise_fwbw (native/fwbw.py:35-171)."""
+        """autograd.Function with the contract of _mlstm_chunkwise_fwbw (native/fwbw.py:35-171).  ``siging`` is the
+        C-ABI mode of ``_siging_mode`` (0 / 1 / 2)."""
 
         @staticmethod
         @custom_fwd(device_type="cuda", cast_inputs=autocast_kernel_dtype)
@@ -604,10 +626,9 @@ def mlstm_siging_chunkwise__b200(
     """Sigmoid-input-gate variant: drop-in for ``mlstm_siging_chunkwise__xl_chunk``
     (mlstm_kernels/torch/chunkwise/triton_xl_chunk_siging/fwbw.py:211-268), the kernel the reference's
     CUDA model path selects (vision_lstm2.py:685-697).  No max state: last states are (C, n).
-    The Triton tile-size kwargs are accepted and ignored.
+    ``normalize=False`` drops the normaliser: h = q C + sum_s P_ts v_s, with no division by max(|n|, 1) + eps (n is
+    still carried and returned).  The Triton tile-size kwargs are accepted and ignored.
     """
-    if not normalize:
-        raise NotImplementedError("normalize=False is not supported by the B200 siging kernel")
     if autocast_kernel_dtype not in _FUNCTIONS:
         raise ValueError(f"Unsupported kernel dtype {autocast_kernel_dtype}.")
     fn = _FUNCTIONS[autocast_kernel_dtype]
@@ -623,7 +644,7 @@ def mlstm_siging_chunkwise__b200(
         if n_initial is None:
             n_initial = torch.zeros(B, NH, q.shape[-1], dtype=q.dtype, device=q.device)
     h, c_last, n_last, _ = fn.apply(q, k, v, i, f, c_initial, n_initial, m_initial, bool(return_last_states),
-                                    int(chunk_size), float(eps), bool(reverse), True,
+                                    int(chunk_size), float(eps), bool(reverse), _siging_mode(True, normalize),
                                     _caller_grad_dtype(autocast_kernel_dtype, q, k, v, i, f))
     if return_last_states:
         return h, (c_last, n_last)
@@ -632,14 +653,18 @@ def mlstm_siging_chunkwise__b200(
 
 def mlstm_recurrent_sequence__b200(q, k, v, i, f, c_initial=None, n_initial=None, m_initial=None,
                                    return_last_states: bool = False, eps: float = 1e-6,
-                                   dtype_state: torch.dtype = torch.float32, siging: bool = False, **kwargs):
+                                   dtype_state: torch.dtype = torch.float32, siging: bool = False, normalize: bool = True,
+                                   **kwargs):
     """Token-by-token mLSTM over a whole sequence in ONE launch, state on chip: drop-in for
     ``mlstm_recurrent_sequence__native_fw`` (mlstm_kernels/torch/recurrent/native_sequence.py:133-175; registry name
     ``native_sequence__native``).  q, k (B, NH, S, DHQK), v (B, NH, S, DHHV), i, f (B, NH, S).
+    ``siging=True, normalize=False``: the sigmoid-input-gate cell without the normaliser (h = q . C_t), so that a
+    ``return_last_states`` prefix of ``mlstm_siging_chunkwise__b200(normalize=False)`` continues here.
     Returns h, or (h, (C, n, m)) with ``return_last_states`` -- the reference's convention; forward only."""
+    mode = _siging_mode(siging, normalize)
     if torch.compiler.is_compiling():
         return _ops.recurrent_sequence(q, k, v, i, f, c_initial, n_initial, m_initial, bool(return_last_states), float(eps),
-                                       dtype_state, bool(siging))
+                                       dtype_state, bool(siging), normalize=bool(normalize))
     lib = _cabi.load_library()
     for name, t in (("q", q), ("k", k), ("v", v), ("i", i), ("f", f)):
         if not t.is_cuda:
@@ -654,7 +679,7 @@ def mlstm_recurrent_sequence__b200(q, k, v, i, f, c_initial=None, n_initial=None
     dev = q.device
     with _on_device(dev):
         a = _cabi.RecurrentArgs()
-        a.B, a.NH, a.S, a.DHQK, a.DHHV, a.dtype, a.siging, a.eps = B, NH, S, DK, DV, _DTYPES[dt], int(bool(siging)), float(eps)
+        a.B, a.NH, a.S, a.DHQK, a.DHHV, a.dtype, a.siging, a.eps = B, NH, S, DK, DV, _DTYPES[dt], mode, float(eps)
         h = torch.empty(B, NH, S, DV, dtype=dt, device=dev)
         a.q, a.k, a.v, a.i, a.f, a.h = (_tensor(t) for t in (q, k, v, i, f, h))
         keep = []
@@ -678,13 +703,13 @@ def mlstm_recurrent_sequence__b200(q, k, v, i, f, c_initial=None, n_initial=None
 
 
 def mlstm_recurrent_step__b200(q, k, v, i, f, c, n, m, eps: float = 1e-6, dtype_state: torch.dtype = torch.float32,
-                               siging: bool = False, **kwargs):
+                               siging: bool = False, normalize: bool = True, **kwargs):
     """One recurrent step: drop-in for ``mlstm_recurrent_step__native`` (recurrent/native_step.py:104-132; registry name
     ``native``).  q, k (B, NH, DHQK), v (B, NH, DHHV), i, f (B, NH, 1); states c (B, NH, DHQK, DHHV), n (B, NH, DHQK),
     m (B, NH, 1).  Returns h (B, NH, DHHV), (c_new, n_new, m_new)."""
     h, last = mlstm_recurrent_sequence__b200(q.unsqueeze(2), k.unsqueeze(2), v.unsqueeze(2), i.reshape(*i.shape[:2], 1),
                                              f.reshape(*f.shape[:2], 1), c, n, m, return_last_states=True, eps=eps,
-                                             dtype_state=dtype_state, siging=siging)
+                                             dtype_state=dtype_state, siging=siging, normalize=normalize)
     return h.squeeze(2), last
 
 

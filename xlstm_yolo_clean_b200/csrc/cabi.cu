@@ -40,6 +40,14 @@ int check_vec(const mlstm_b200_tensor& t, const char* name) {
   return 0;
 }
 
+int check_siging(int32_t siging) {
+  if (siging < 0 || siging > 2) {
+    set_error("siging must be 0, 1 or 2 (got %d)", siging);
+    return MLSTM_B200_EINVAL;
+  }
+  return 0;
+}
+
 int require_device() {
   int dev = -1;
   cudaError_t e = cudaGetDevice(&dev);
@@ -160,6 +168,11 @@ int mlstm_b200_chunkwise_fw(const mlstm_b200_fw_args* a, void* stream) {
     set_error("Sequence length %d is not divisible by chunk size %d.", a->shape.S, a->shape.chunk_size);
     return MLSTM_B200_EINVAL;
   }
+  if (int e = check_siging(a->shape.siging)) return e;
+  if (a->epilogue && a->shape.siging == 2) {  // the cell it fuses (MatrixLSTMCell) always normalises
+    set_error("the fused cell-output epilogue does not cover siging = 2 (no normaliser)");
+    return MLSTM_B200_EUNSUPPORTED;
+  }
   if (int e = require_device()) return e;
   int err = 0;
   bool tc = use_tensor(a->shape, 0, &err);
@@ -210,6 +223,7 @@ int mlstm_b200_chunkwise_bw(const mlstm_b200_bw_args* a, void* stream) {
     set_error("Sequence length %d is not divisible by chunk size %d.", a->shape.S, a->shape.chunk_size);
     return MLSTM_B200_EINVAL;
   }
+  if (int e = check_siging(a->shape.siging)) return e;
   if (int e = require_device()) return e;
   int err = 0;
   bool tc = use_tensor(a->shape, 1, &err);
@@ -240,6 +254,7 @@ int mlstm_b200_recurrent_sequence(const mlstm_b200_recurrent_args* a, void* stre
     set_error("args is NULL");
     return MLSTM_B200_EINVAL;
   }
+  if (int e = check_siging(a->siging)) return e;
   if (int e = require_device()) return e;
   return recurrent_sequence(*a, (cudaStream_t)stream);
 }

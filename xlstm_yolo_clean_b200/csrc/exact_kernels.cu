@@ -49,7 +49,7 @@ struct ExactParams {
   float* dc0;
   int DVT;  // dv slice width of the recurrent kernels
   int rev;  // 1: anti-causal scan -- processing index t lives at memory token S-1-t (no data is moved)
-  int sig;  // 1: sigmoid input gate, every max state is 0 (siging variant)
+  int sig;  // mlstm_b200_shape::siging: 1 sigmoid input gate, every max state 0; 2 the same without the normaliser
 };
 // memory token of processing index t, and the signed token step
 __device__ __forceinline__ int64_t tok(const ExactParams& p, int64_t t) { return p.rev ? (int64_t)p.S - 1 - t : t; }
@@ -259,7 +259,7 @@ __global__ void __launch_bounds__(kThreads) k_fw_h(ExactParams p) {
     float den = bq * qn + rs;                             // fw.py:204-206
     float nmax = fmaxf(fabsf(den), expf(-smt[t]));        // fw.py:208-210
     sbq[t] = bq;
-    sden[t] = nmax + p.eps;
+    sden[t] = p.sig == 2 ? 1.f : nmax + p.eps;  // siging = 2: h is the numerator
     p.n_out[(int64_t)bh * p.S + t0 + sg * t] = nmax;  // saved vectors are indexed by memory token
     p.m_out[(int64_t)bh * p.S + t0 + sg * t] = smt[t];
   }
@@ -339,9 +339,11 @@ __global__ void __launch_bounds__(kThreads) k_bw_dc(ExactParams p) {
       float bq = expf(sb[t] + m_prev - p.m_out_in[(int64_t)bh * p.S + t0 + sg * t]) * p.scale;  // bw.py:79-86
       sQ[t * ldk + d] *= bq;
     }
-    for (int e = threadIdx.x; e < L * DVT; e += blockDim.x) {
-      int t = e / DVT, x = e - t * DVT;
-      sH[t * ldv + x] /= (p.n_out_in[(int64_t)bh * p.S + t0 + sg * t] + p.eps);  // bw.py:88-90
+    if (p.sig != 2) {  // siging = 2: no normaliser, dh is used as it is
+      for (int e = threadIdx.x; e < L * DVT; e += blockDim.x) {
+        int t = e / DVT, x = e - t * DVT;
+        sH[t * ldv + x] /= (p.n_out_in[(int64_t)bh * p.S + t0 + sg * t] + p.eps);  // bw.py:88-90
+      }
     }
     __syncthreads();
     for (int idx = threadIdx.x; idx < MS * NS; idx += blockDim.x) {
@@ -421,9 +423,11 @@ __global__ void __launch_bounds__(kThreads) k_bw_dqkv(ExactParams p) {
     sab[t] = expf(s_g - sb[t] + si[t] - m_next);  // bw.py:181,187
     sbb[t] = expf(sb[t] + m_prev - mt);           // bw.py:186
   }
-  for (int e = threadIdx.x; e < L * DV; e += blockDim.x) {
-    int t = e / DV, x = e - t * DV;
-    sH[t * ldv + x] /= (p.n_out_in[(int64_t)bh * p.S + t0 + sg * t] + p.eps);  // bw.py:135
+  if (p.sig != 2) {  // siging = 2: no normaliser, dh is used as it is
+    for (int e = threadIdx.x; e < L * DV; e += blockDim.x) {
+      int t = e / DV, x = e - t * DV;
+      sH[t * ldv + x] /= (p.n_out_in[(int64_t)bh * p.S + t0 + sg * t] + p.eps);  // bw.py:135
+    }
   }
   __syncthreads();
 
@@ -717,7 +721,7 @@ int exact_fw(const mlstm_b200_fw_args& a, cudaStream_t st) {
   p.c_last = a.c_last; p.n_last = a.n_last; p.m_last = a.m_last;
   p.DVT = pick_dvt(s);
   p.rev = s.reverse ? 1 : 0;
-  p.sig = s.siging ? 1 : 0;
+  p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
   MLSTM_DISPATCH_DTYPE(s.dtype, T, {
     if (int e = launch_states<T>(p, st)) return e;
     size_t sm = smem_fw_h(L, p.DK, p.DV);
@@ -757,7 +761,7 @@ int exact_bw(const mlstm_b200_bw_args& a, cudaStream_t st) {
   p.dc0 = a.dc_initial;
   p.DVT = pick_dvt(s);
   p.rev = s.reverse ? 1 : 0;
-  p.sig = s.siging ? 1 : 0;
+  p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
   MLSTM_DISPATCH_DTYPE(s.dtype, T, {
     if (int e = launch_states<T>(p, st)) return e;  // recompute C/n/m states (bw.py:251-266)
     size_t sm = smem_bw_dc(L, p.DK, p.DVT);

@@ -21,7 +21,7 @@ template <typename T>
 __device__ __forceinline__ float round_to(float x) { return to_f32<T>(from_f32<T>(x)); }
 
 struct StepParams {
-  int B, NH, S, siging;
+  int B, NH, S, siging;  // mlstm_b200_recurrent_args::siging: 0, 1 or 2 (no normaliser)
   float eps, scale;
   const void *q, *k, *v, *ig, *fg;
   int64_t q_sb, q_sh, q_ss, k_sb, k_sh, k_ss, v_sb, v_sh, v_ss, i_sb, i_sh, i_ss, f_sb, f_sh, f_ss;
@@ -111,7 +111,7 @@ __global__ void __launch_bounds__(kStepThreads) k_recurrent(StepParams p) {
 #pragma unroll
     for (int w = 0; w < (DK + 31) / 32; ++w) qn += s_red[w];
     qn = round_to<T>(qn);
-    const float denom = fmaxf(fabsf(qn), expf(-m_new)) + p.eps;  // native_step.py:88-91
+    const float denom = p.siging == 2 ? 1.f : fmaxf(fabsf(qn), expf(-m_new)) + p.eps;  // native_step.py:88-91
     if (rg == 0) hp[(int64_t)t * p.h_ss + j] = from_f32<T>(round_to<T>(acc) / denom);
     m = m_new;
   }
@@ -173,7 +173,7 @@ int recurrent_sequence(const mlstm_b200_recurrent_args& a, cudaStream_t st) {
   }
   if (a.B <= 0 || a.NH <= 0 || a.S <= 0) return 0;
   StepParams p{};
-  p.B = a.B; p.NH = a.NH; p.S = a.S; p.siging = a.siging ? 1 : 0;
+  p.B = a.B; p.NH = a.NH; p.S = a.S; p.siging = a.siging;
   p.eps = a.eps;
   p.scale = 1.f / sqrtf((float)a.DHQK);
   p.q = a.q.ptr; p.q_sb = a.q.stride[0]; p.q_sh = a.q.stride[1]; p.q_ss = a.q.stride[2];

@@ -420,7 +420,8 @@ struct TcFwParams {
   float *n_out, *m_out;
   float *c_last, *n_last, *m_last;
   int rev;           // 1: anti-causal direction (tiles walked from the end, mirrored in-tile mask)
-  int sig;           // 1: sigmoid input gate, all max states are 0 (siging variant)
+  int sig;           // mlstm_b200_shape::siging: 1 sigmoid input gate, all max states 0; 2 the same without the
+                     // normaliser (h = numerator)
   int store_states;  // 1: TMA-store the bf16 copy of C entering every tile (consumed by the backward)
   float cap;         // > 0: gate soft cap applied in the scan warp (mlstm_b200_shape::gate_soft_cap)
   // fused cell-output epilogue (mlstm_b200_fw_epilogue): the tensor map "mapH" then describes y; the plain h (if wanted)
@@ -835,7 +836,7 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
         tmem_ld_wait();
         const float den = bq * __uint_as_float(qn_u) + rs;       // fw.py:204-206
         const float nmax = fmaxf(fabsf(den), __expf(-m_t));    // fw.py:208-210
-        const float inv = 1.f / (nmax + p.eps);
+        const float inv = p.sig == 2 ? 1.f : 1.f / (nmax + p.eps);  // siging = 2: no normaliser
         float o[CW];
 #pragma unroll
         for (int j = 0; j < CW; ++j) o[j] = (__uint_as_float(hi[j]) + bq * __uint_as_float(hx[j])) * inv;  // fw.py:200-212
@@ -1287,7 +1288,7 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
         const float bq = __expf(b_t + m_run - m_t) * p.scale;                          // fw.py:197-198
         const float den = bq * (sqn[row] + sqn[LT + row]) + srs[row] + srs[LT + row];  // fw.py:204-206
         const float nmax = fmaxf(fabsf(den), __expf(-m_t));                            // fw.py:208-210
-        const float inv = 1.f / (nmax + p.eps);
+        const float inv = p.sig == 2 ? 1.f : 1.f / (nmax + p.eps);  // siging = 2: no normaliser
 #pragma unroll 1
         for (int hf = 0; hf < 2; ++hf) {
           uint32_t hi[32], hx[32];
@@ -1380,7 +1381,8 @@ struct TcBwParams {
   int64_t di_sb, di_sh, di_ss, df_sb, df_sh, df_ss;
   float* dc0;
   int rev;  // 1: the forward ran anti-causally; this sweep then walks the memory tiles in ascending order
-  int sig;  // 1: sigmoid input gate (m_out is all zeros, dI picks up sigmoid(-i))
+  int sig;  // 1: sigmoid input gate (m_out is all zeros, dI picks up sigmoid(-i)); 2: the same without the normaliser
+            // (dh is not scaled by 1 / (n + eps), n_out is not read)
   float cap;  // > 0: gate soft cap (see TcFwParams); dI / dF are written w.r.t. the pre-activations
   // head-dim-128 block problems: add into outputs another block problem of the same call has already written
   // (dq / dk / dv through TMA reduce-add, di / df read-modify-write by their one owner thread)
@@ -1681,7 +1683,7 @@ tc_bw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
       r.g = load_gate_raw<T>(ip + (int64_t)t0 * p.ig_ss, p.ig_ss, fp + (int64_t)t0 * p.fg_ss, p.fg_ss, n_valid);
       if (lane * 4 < n_valid) {  // n_valid is a multiple of 4 (tensor_supported)
         r.mt = *reinterpret_cast<const float4*>(mo + t0 + lane * 4);
-        r.nt = *reinterpret_cast<const float4*>(no + t0 + lane * 4);
+        r.nt = p.sig == 2 ? make_float4(1.f, 1.f, 1.f, 1.f) : *reinterpret_cast<const float4*>(no + t0 + lane * 4);
       } else {
         r.mt = make_float4(0.f, 0.f, 0.f, 0.f);
         r.nt = make_float4(1.f, 1.f, 1.f, 1.f);
@@ -1798,7 +1800,7 @@ tc_bw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
       const float g = gb[GateBuf::oScal], m_prev = gb[GateBuf::oScal + 2], m_next = gb[GateBuf::oScal + 3];
       const float b_t = gb[GateBuf::oB + row], i_t = gb[GateBuf::oI + row];
       const float m_t = gb[GateBuf::oMt + row], n_t = gb[GateBuf::oNt + row];
-      const float rinv = valid ? 1.f / (n_t + p.eps) : 0.f;         // bw.py:135
+      const float rinv = !valid ? 0.f : p.sig == 2 ? 1.f : 1.f / (n_t + p.eps);  // bw.py:135 (siging = 2: no normaliser)
       const float bbar = valid ? __expf(b_t + m_prev - m_t) : 0.f;  // bw.py:186
       const float abar = __expf(g - b_t + i_t - m_next);            // bw.py:187 (0 for tail tokens)
       const float gbar = __expf(g + m_prev - m_next);               // bw.py:76
@@ -2203,7 +2205,7 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   p.n_out = a.n_out; p.m_out = a.m_out;
   p.c_last = a.c_last; p.n_last = a.n_last; p.m_last = a.m_last;
   p.rev = s.reverse ? 1 : 0;
-  p.sig = s.siging ? 1 : 0;
+  p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
   p.store_states = c_states != nullptr;
   p.cap = s.gate_soft_cap;
   if (ep) {
@@ -2516,7 +2518,7 @@ int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, int nbl
   p.df = a.df.ptr; p.df_sb = a.df.stride[0]; p.df_sh = a.df.stride[1]; p.df_ss = a.df.stride[2];
   p.dc0 = a.dc_initial;
   p.rev = s.reverse ? 1 : 0;
-  p.sig = s.siging ? 1 : 0;
+  p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
   p.cap = s.gate_soft_cap;
   p.acc_qk = acc_qk; p.acc_v = acc_v; p.acc_g = acc_g;
   p.cs_rows = block < 0 ? D : nblocks * D;

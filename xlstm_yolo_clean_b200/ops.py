@@ -100,21 +100,24 @@ def _bw_grad_dtype(q, v, dt, chunk_size, impl, grad_dtype):
 def chunkwise_fw(q: Tensor, k: Tensor, v: Tensor, i: Tensor, f: Tensor, c_initial: Optional[Tensor],
                  n_initial: Optional[Tensor], m_initial: Optional[Tensor], cast_to: Optional[torch.dtype],
                  qk_scale: Optional[float], return_last_states: bool, chunk_size: int, eps: float, impl: int,
-                 save_states: bool, reverse: bool, siging: bool, soft_cap: float, grad_dtype: Optional[torch.dtype]
-                 ) -> tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+                 save_states: bool, reverse: bool, siging: bool, soft_cap: float, grad_dtype: Optional[torch.dtype],
+                 normalize: bool = True) -> tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     """Returns h, nm = [n_out, m_out] (2, B, NH, S) fp32, C / n / m_last fp32 (0-element unless
     ``return_last_states``), c_states uint8 (0-element unless saved).  ``cast_to``: the custom_fwd rule, every floating
-    input rounded to that dtype first.  ``grad_dtype`` is read by the backward only."""
+    input rounded to that dtype first.  ``grad_dtype`` is read by the backward only.  ``normalize=False``: the
+    sigmoid-input-gate variant without the normaliser (``siging`` must be set)."""
+    mode = _backend._siging_mode(siging, normalize)
     q, k, v, i, f, c0, n0, m0 = _cast(cast_to, q, k, v, i, f, c_initial, n_initial, m_initial)
     h, nm, last, c_states = _backend._fw_launch(q, k, v, i, f, c0, n0, m0, qk_scale, return_last_states, chunk_size, eps,
-                                                impl, save_states, reverse, siging, soft_cap)
+                                                impl, save_states, reverse, mode, soft_cap)
     last = last if last is not None else tuple(_empty(q) for _ in range(3))
     return h, nm, *last, (c_states if c_states is not None else _empty(q, _U8))
 
 
 @chunkwise_fw.register_fake
 def _(q, k, v, i, f, c_initial, n_initial, m_initial, cast_to, qk_scale, return_last_states, chunk_size, eps, impl,
-      save_states, reverse, siging, soft_cap, grad_dtype):
+      save_states, reverse, siging, soft_cap, grad_dtype, normalize=True):
+    _backend._siging_mode(siging, normalize)
     dt = cast_to or q.dtype
     B, NH, S, DK = q.shape
     DV = v.shape[3]
@@ -134,22 +137,24 @@ def chunkwise_bw(q: Tensor, k: Tensor, v: Tensor, i: Tensor, f: Tensor, n_out: T
                  c_initial: Optional[Tensor], n_initial: Optional[Tensor], m_initial: Optional[Tensor],
                  dc_last: Optional[Tensor], c_states: Optional[Tensor], cast_to: Optional[torch.dtype],
                  qk_scale: Optional[float], chunk_size: int, eps: float, impl: int, want_dc_initial: bool, reverse: bool,
-                 siging: bool, soft_cap: float, grad_dtype: Optional[torch.dtype]
+                 siging: bool, soft_cap: float, grad_dtype: Optional[torch.dtype], normalize: bool = True
                  ) -> tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
     """Returns dq, dk, dv, di, df (in ``grad_dtype`` where the kernels write it, else the kernel dtype) and dC_initial
     fp32 (0-element unless ``want_dc_initial``).  A 0-element ``c_states``: the kernels recompute the states."""
+    mode = _backend._siging_mode(siging, normalize)
     q, k, v, i, f, c0, n0, m0 = _cast(cast_to, q, k, v, i, f, c_initial, n_initial, m_initial)
     n_out = n_out if n_out.is_contiguous() else n_out.contiguous()
     m_out = m_out if m_out.is_contiguous() else m_out.contiguous()
     dq, dk, dv, di, df, dc0 = _backend._bw_launch(q, k, v, i, f, n_out.data_ptr(), m_out.data_ptr(), dh, c0, n0, m0, dc_last,
                                                   qk_scale, chunk_size, eps, impl, want_dc_initial, _none(c_states), reverse,
-                                                  siging, None, soft_cap, grad_dtype)
+                                                  mode, None, soft_cap, grad_dtype)
     return dq, dk, dv, di, df, (dc0 if dc0 is not None else _empty(q))
 
 
 @chunkwise_bw.register_fake
 def _(q, k, v, i, f, n_out, m_out, dh, c_initial, n_initial, m_initial, dc_last, c_states, cast_to, qk_scale, chunk_size,
-      eps, impl, want_dc_initial, reverse, siging, soft_cap, grad_dtype):
+      eps, impl, want_dc_initial, reverse, siging, soft_cap, grad_dtype, normalize=True):
+    _backend._siging_mode(siging, normalize)
     gdt = _bw_grad_dtype(q, v, cast_to or q.dtype, chunk_size, impl, grad_dtype)
     B, NH, S, DK = q.shape
     DV = v.shape[3]
@@ -161,15 +166,15 @@ def _(q, k, v, i, f, n_out, m_out, dh, c_initial, n_initial, m_initial, dc_last,
 
 def _chunkwise_setup(ctx, inputs, output):
     (q, k, v, i, f, c0, n0, m0, cast_to, qk_scale, rls, chunk_size, eps, impl, save_states, reverse, siging, soft_cap,
-     grad_dtype) = inputs
+     grad_dtype, normalize) = inputs
     ctx.save_for_backward(q, k, v, i, f, c0, n0, m0, output[1], output[5])
-    ctx.cfg = (cast_to, qk_scale, rls, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype)
+    ctx.cfg = (cast_to, qk_scale, rls, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype, normalize)
     ctx.set_materialize_grads(False)  # nm and c_states carry no gradient: no zero tensors for them
 
 
 def _chunkwise_backward(ctx, dh, dnm, dc_last, dn_last, dm_last, dc_states):
     q, k, v, i, f, c0, n0, m0, nm, c_states = ctx.saved_tensors
-    cast_to, qk_scale, rls, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype = ctx.cfg
+    cast_to, qk_scale, rls, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype, normalize = ctx.cfg
     B, NH, S, DK = q.shape
     DV = v.shape[3]
     if dh is None:
@@ -180,13 +185,13 @@ def _chunkwise_backward(ctx, dh, dnm, dc_last, dn_last, dm_last, dc_states):
         dc_last = q.new_zeros((B, NH, DK, DV), dtype=_F32)
     dq, dk, dv, di, df, dc0 = chunkwise_bw(q, k, v, i, f, nm[0], nm[1], dh, c0, n0, m0, dc_last, c_states, cast_to,
                                            qk_scale, chunk_size, eps, impl, c0 is not None, reverse, siging, soft_cap,
-                                           grad_dtype)
+                                           grad_dtype, normalize)
     # dN / dM_initial are zeros, as in native/bw.py:329-337 (and _MlstmChunkwiseB200)
     return (dq, dk, dv, di, df,
             None if c0 is None else dc0.to(cast_to if _autocast_eligible(c0) and cast_to else c0.dtype),
             None if n0 is None else torch.zeros_like(n0),
             None if m0 is None else torch.zeros_like(m0),
-            None, None, None, None, None, None, None, None, None, None, None)
+            None, None, None, None, None, None, None, None, None, None, None, None)
 
 
 torch.library.register_autograd(chunkwise_fw, _chunkwise_backward, setup_context=_chunkwise_setup)
@@ -194,7 +199,7 @@ torch.library.register_autograd(chunkwise_fw, _chunkwise_backward, setup_context
 
 class _ChunkwiseFunction:
     """What ``backend._FUNCTIONS[kernel_dtype]`` is to eager calls: ``apply`` with ``_MlstmChunkwiseB200.forward``'s
-    arguments, here over ``chunkwise_fw``."""
+    arguments (``siging`` the C-ABI mode 0 / 1 / 2), here over ``chunkwise_fw``."""
 
     def __init__(self, kernel_dtype):
         self.kernel_dtype = kernel_dtype
@@ -208,7 +213,7 @@ class _ChunkwiseFunction:
             c_initial = q.new_zeros((q.shape[0], q.shape[1], q.shape[3], v.shape[3]), dtype=dt)
         h, _, c_last, n_last, m_last, _ = chunkwise_fw(q, k, v, i, f, c_initial, n_initial, m_initial, cast_to, None,
                                                        return_last_states, chunk_size, eps, _backend._default_impl, need_bw,
-                                                       reverse, siging, 0.0, grad_dtype)
+                                                       reverse, siging != 0, 0.0, grad_dtype, siging != 2)
         if not return_last_states:
             return h, None, None, None
         return h, c_last.to(dt), n_last.to(dt), m_last.to(dt)  # native kernels hand states back in the input dtype
@@ -223,24 +228,27 @@ def chunkwise_function(kernel_dtype) -> _ChunkwiseFunction:
 
 def fw_launch(q, k, v, i, f, c0, n0, m0, qk_scale, return_last_states, chunk_size, eps, impl, save_states, reverse, siging,
               soft_cap=0.0):
-    """``backend._fw_launch`` (without the fused epilogue) over ``chunkwise_fw``: what ``mlstm_chunkwise_fw`` calls."""
+    """``backend._fw_launch`` (without the fused epilogue) over ``chunkwise_fw``: what ``mlstm_chunkwise_fw`` calls
+    (``siging`` the C-ABI mode 0 / 1 / 2)."""
     impl = _backend._default_impl if impl is None else impl
     q, k, v, i, f, c0, n0, m0 = (None if t is None else t.detach() for t in (q, k, v, i, f, c0, n0, m0))
     h, nm, c_last, n_last, m_last, c_states = chunkwise_fw(q, k, v, i, f, c0, n0, m0, None, qk_scale, return_last_states,
-                                                           chunk_size, eps, impl, save_states, reverse, siging, soft_cap, None)
+                                                           chunk_size, eps, impl, save_states, reverse, siging != 0, soft_cap,
+                                                           None, siging != 2)
     return h, nm, ((c_last, n_last, m_last) if return_last_states else None), (c_states if save_states else None)
 
 
 def bw_launch(q, k, v, i, f, n_out, m_out, dh, c0, n0, m0, dc_last, qk_scale, chunk_size, eps, impl, want_dc_initial,
               c_states, reverse, siging, out, soft_cap, grad_dtype):
-    """``mlstm_chunkwise_bw`` over ``chunkwise_bw``.  Caller-provided ``out`` tensors receive a copy of the gradients."""
+    """``mlstm_chunkwise_bw`` over ``chunkwise_bw`` (``siging`` the C-ABI mode 0 / 1 / 2).  Caller-provided ``out``
+    tensors receive a copy of the gradients."""
     impl = _backend._default_impl if impl is None else impl
     if out is not None:
         grad_dtype = out[0].dtype
     args = (q, k, v, i, f, n_out, m_out, dh, c0, n0, m0, dc_last, c_states)
     args = tuple(None if t is None else t.detach() for t in args)
-    dq, dk, dv, di, df, dc0 = chunkwise_bw(*args, None, qk_scale, chunk_size, eps, impl, want_dc_initial, reverse, siging,
-                                           soft_cap, grad_dtype)
+    dq, dk, dv, di, df, dc0 = chunkwise_bw(*args, None, qk_scale, chunk_size, eps, impl, want_dc_initial, reverse, siging != 0,
+                                           soft_cap, grad_dtype, siging != 2)
     if out is not None:
         for o, g in zip(out, (dq, dk, dv, di, df)):
             o.copy_(g)
@@ -561,10 +569,10 @@ def convert16(x, dtype):
 @_op("recurrent_sequence")
 def _recurrent_sequence(q: Tensor, k: Tensor, v: Tensor, i: Tensor, f: Tensor, c_initial: Optional[Tensor],
                         n_initial: Optional[Tensor], m_initial: Optional[Tensor], return_last_states: bool, eps: float,
-                        siging: bool) -> tuple[Tensor, Tensor, Tensor, Tensor]:
+                        siging: bool, normalize: bool = True) -> tuple[Tensor, Tensor, Tensor, Tensor]:
     """``mlstm_recurrent_sequence__b200``: h and the last states fp32 (0-element unless ``return_last_states``)."""
     out = _backend.mlstm_recurrent_sequence__b200(q, k, v, i, f, c_initial, n_initial, m_initial, return_last_states, eps,
-                                                  _F32, siging)
+                                                  _F32, siging, normalize)
     if not return_last_states:
         return out, _empty(q), _empty(q), _empty(q)
     h, (c, n, m) = out
@@ -572,7 +580,8 @@ def _recurrent_sequence(q: Tensor, k: Tensor, v: Tensor, i: Tensor, f: Tensor, c
 
 
 @_recurrent_sequence.register_fake
-def _(q, k, v, i, f, c_initial, n_initial, m_initial, return_last_states, eps, siging):
+def _(q, k, v, i, f, c_initial, n_initial, m_initial, return_last_states, eps, siging, normalize=True):
+    _backend._siging_mode(siging, normalize)
     B, NH, S, DK = q.shape
     DV = v.shape[-1]
     h = q.new_empty((B, NH, S, DV))
@@ -582,10 +591,11 @@ def _(q, k, v, i, f, c_initial, n_initial, m_initial, return_last_states, eps, s
             q.new_empty((B, NH, 1), dtype=_F32))
 
 
-def recurrent_sequence(q, k, v, i, f, c_initial, n_initial, m_initial, return_last_states, eps, dtype_state, siging):
+def recurrent_sequence(q, k, v, i, f, c_initial, n_initial, m_initial, return_last_states, eps, dtype_state, siging,
+                       normalize=True):
     """``mlstm_recurrent_sequence__b200`` over the ``recurrent_sequence`` op (forward only, like the eager call)."""
     args = tuple(None if t is None else t.detach() for t in (q, k, v, i, f, c_initial, n_initial, m_initial))
-    h, c, n, m = _recurrent_sequence(*args, return_last_states, eps, siging)
+    h, c, n, m = _recurrent_sequence(*args, return_last_states, eps, siging, normalize)
     if not return_last_states:
         return h
     return h, (c.to(dtype_state), n.to(dtype_state), m.to(dtype_state))
