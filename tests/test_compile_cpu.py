@@ -185,7 +185,7 @@ def test_eager_calls_never_enter_the_ops(pkg, monkeypatch):
 
     for name in ("chunkwise_fw", "chunkwise_bw", "layer_fw", "layer_bw", "chunkwise_fw_epilogue", "cellout_fw", "cellout_bw",
                  "rmsnorm_fw", "rmsnorm_bw", "_convert16", "_recurrent_sequence", "chunkwise_function", "fw_launch",
-                 "bw_launch", "layer_layout", "cell_fused", "cell_out", "rms_norm", "convert16", "recurrent_sequence"):
+                 "bw_launch", "rms_norm", "convert16", "recurrent_sequence"):
         monkeypatch.setattr(O, name, boom)
     q, k, v = (torch.randn(1, 2, 64, 32) for _ in range(3))
     i, f = torch.randn(1, 2, 64), torch.randn(1, 2, 64)
@@ -197,8 +197,10 @@ def test_eager_calls_never_enter_the_ops(pkg, monkeypatch):
         lambda: pkg.mlstm_recurrent_sequence__b200(q, k, v, i, f),
         lambda: pkg.cell_out(torch.randn(1, 2, 8, 64)),
         lambda: pkg.rms_norm_b200(torch.randn(2, 256), torch.ones(256)),
-        lambda: pkg.vil._MlstmLayerLayout.apply(torch.randn(1, 64, 128), torch.randn(1, 64, 64), torch.randn(1, 64, 4), 2,
-                                                False, False, 64, 1e-6, torch.bfloat16),
+        lambda: pkg.vil._layer_layout(torch.randn(1, 64, 128), torch.randn(1, 64, 64), torch.randn(1, 64, 4), 2, False, False,
+                                      64, 1e-6, torch.bfloat16, 0.0),
+        lambda: pkg.vil._cell_fused(torch.randn(1, 64, 128), torch.randn(1, 64, 64), torch.randn(1, 64, 4), None, None, None,
+                                    None, 2, False, False, 64, 1e-6, torch.bfloat16, 0.0, 1e-6, torch.float16),
     ]
     for call in calls:
         with pytest.raises((RuntimeError, AssertionError)) as e:

@@ -364,3 +364,25 @@ def test_rmsnorm_and_cell_out_fullgraph(pkg, C):
     o_c, g_c = _run(torch.compile(f, fullgraph=True), ts, douts)
     _assert_same(o_e, o_c)
     _assert_same(g_e, g_c)
+
+
+@pytest.mark.parametrize("backend", ["inductor", "aot_eager"])
+def test_cell_out_misaligned_skip_input(pkg, backend):
+    """A contiguous skip input 2 bytes past an aligned address (the cell-output kernels need 8): eager and compiled calls
+    both read an aligned copy and agree bit for bit."""
+    n = 3 * 77 * 256
+    xs = torch.randn(n + 1, device=DEV, dtype=torch.float16)[1:].view(3, 77, 256).requires_grad_(True)
+    assert xs.is_leaf and xs.data_ptr() % 8
+    h = torch.randn(3, 4, 77, 64, device=DEV, dtype=torch.bfloat16, requires_grad=True)
+    hw, hb, hs = (torch.randn(256, device=DEV, requires_grad=True) for _ in range(3))
+
+    def f(h, hw, hb, hs, xs):
+        with torch.autocast("cuda", dtype=torch.float16):
+            return pkg.cell_out(h, hw, hb, hs, xs, eps=1e-6)
+
+    ts = [h, hw, hb, hs, xs]
+    douts = [torch.randn(3, 77, 256, device=DEV, dtype=torch.float16)]
+    o_e, g_e = _run(f, ts, douts)
+    o_c, g_c = _run(torch.compile(f, backend=backend, fullgraph=True), ts, douts)
+    _assert_same(o_e, o_c)
+    _assert_same(g_e, g_c)

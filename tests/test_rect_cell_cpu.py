@@ -37,7 +37,8 @@ def test_grad_dtype_takes_head_dims_from_qk_and_v():
     for DK, DV, ok in ((32, 64, True), (64, 128, True), (64, 64, True), (32, 128, False), (48, 96, False)):
         qk = torch.empty(1, S, 2 * NH * DK, dtype=torch.bfloat16)
         v = torch.empty(1, S, NH * DV, dtype=torch.bfloat16)
-        assert vil._grad_dtype(ins, qk, v, NH) == (torch.float16 if ok else torch.bfloat16), (DK, DV)
+        assert vil._layer_grad_dtype(ins, torch.bfloat16, vil._head_dims(qk, v, NH), S) == (
+            torch.float16 if ok else torch.bfloat16), (DK, DV)
 
 
 def test_rect_one_launch_policy_covers_both_pairs_and_grad_modes():

@@ -80,6 +80,39 @@ def _siging_mode(siging, normalize=True) -> int:
     return 1 if siging else 0
 
 
+def _siging_flags(mode: int) -> tuple[bool, bool]:
+    """(siging, normalize) of a C-ABI mode: the inverse of ``_siging_mode``."""
+    return mode != 0, mode != 2
+
+
+_16BIT = (torch.float16, torch.bfloat16)
+
+
+def _grad_dtype(kernel_dtype, caller_dtype, tensor_route: bool):
+    """The dtype the backward writes freshly allocated gradients in: the caller's dtype (``caller_dtype``, None when
+    the caller has no single one) where the tensor-core route rounds its fp32 accumulators straight to it
+    (``shape.grad_dtype``: the two 16-bit dtypes), else the kernel dtype (autograd casts the gradients afterwards)."""
+    if (caller_dtype is None or caller_dtype is kernel_dtype or not tensor_route or caller_dtype not in _16BIT
+            or kernel_dtype not in _16BIT):
+        return kernel_dtype
+    return caller_dtype
+
+
+def _zero_c_initial(q, v, c_initial, n_initial, m_initial):
+    """``c_initial``, or a zero C when only n / m_initial are given: the kernels read initial states only with a C."""
+    if c_initial is None and (n_initial is not None or m_initial is not None):
+        B, NH, S, DK = q.shape
+        return torch.zeros(B, NH, DK, v.shape[-1], device=q.device)
+    return c_initial
+
+
+def _nm_ptrs(nm):
+    """n_out / m_out pointers for the backward from the forward's nm = [n_out, m_out] (2, B, NH, S) fp32, which must be
+    contiguous (as the forward allocates it)."""
+    nmp = nm.data_ptr()
+    return nmp, nmp + nm.stride(0) * 4
+
+
 def _shape(q, v, chunk_size, eps, impl, qk_scale=None, reverse=False, siging=0, gate_soft_cap=0.0) -> _cabi.Shape:
     B, NH, S, DK = q.shape
     s = _cabi.Shape()
@@ -367,9 +400,7 @@ def mlstm_chunkwise_fw(q, k, v, i, f, c_initial=None, n_initial=None, m_initial=
     ``c_states`` is the opaque per-tile state buffer the tensor-core backward consumes (the
     reference's return_all_states mode, native/fwbw.py:73-101); None when the kernels recompute."""
     mode = _siging_mode(siging, normalize)
-    if c_initial is None and (n_initial is not None or m_initial is not None):
-        B, NH, S, DK = q.shape
-        c_initial = torch.zeros(B, NH, DK, v.shape[-1], device=q.device)
+    c_initial = _zero_c_initial(q, v, c_initial, n_initial, m_initial)
     launch = _ops.fw_launch if torch.compiler.is_compiling() else _fw_launch
     h, nm, last, c_states = launch(q, k, v, i, f, c_initial, n_initial, m_initial, qk_scale, bool(return_last_states),
                                    int(chunk_size), float(eps), impl, bool(save_states), bool(reverse), mode,
@@ -407,8 +438,7 @@ def _bw_launch(q, k, v, i, f, n_ptr, m_ptr, dh, c0, n0, m0, dcl, qk_scale, chunk
         plan = _BwPlan()
         plan.tensor_route = _tensor_route(lib, a.shape)
         if gdt is not dt:
-            if out is None and (not plan.tensor_route or gdt not in (torch.float16, torch.bfloat16)):
-                # gradients allocated here: the kernel dtype it is (autograd casts them where it has to)
+            if out is None and _grad_dtype(dt, gdt, plan.tensor_route) is dt:
                 return _bw_launch(q, k, v, i, f, n_ptr, m_ptr, dh, c0, n0, m0, dcl, qk_scale, chunk_size, eps, impl,
                                   want_dc_initial, c_states, reverse, siging, None, soft_cap, None)
             if not plan.tensor_route or gdt not in (torch.float16, torch.bfloat16):
@@ -501,18 +531,19 @@ def mlstm_chunkwise_bw(q, k, v, i, f, n_out, m_out, dh, c_initial=None, n_initia
     unit innermost stride for dq/dk/dv), e.g. views into a fused (B, S, 2H) qk gradient.  Their dtype -- or
     ``grad_dtype`` when the gradients are allocated here -- may be the other 16-bit dtype than the kernel's."""
     mode = _siging_mode(siging, normalize)
-    if c_initial is None and (n_initial is not None or m_initial is not None):
-        B, NH, S, DK = q.shape
-        c_initial = torch.zeros(B, NH, DK, v.shape[-1], device=q.device)
-    if torch.compiler.is_compiling():
-        return _ops.bw_launch(q, k, v, i, f, n_out, m_out, dh, c_initial, n_initial, m_initial, dc_last, qk_scale,
-                              int(chunk_size), float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), mode,
-                              out, float(gate_soft_cap or 0.0), grad_dtype)
-    n_out = n_out if n_out.is_contiguous() else n_out.contiguous()
-    m_out = m_out if m_out.is_contiguous() else m_out.contiguous()
-    return _bw_launch(q, k, v, i, f, n_out.data_ptr(), m_out.data_ptr(), dh, c_initial, n_initial, m_initial, dc_last, qk_scale,
-                      int(chunk_size), float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), mode, out,
-                      float(gate_soft_cap or 0.0), grad_dtype)
+    c_initial = _zero_c_initial(q, v, c_initial, n_initial, m_initial)
+    launch = _ops.bw_launch if torch.compiler.is_compiling() else _chunkwise_bw
+    return launch(q, k, v, i, f, n_out, m_out, dh, c_initial, n_initial, m_initial, dc_last, qk_scale, int(chunk_size),
+                  float(eps), impl, bool(want_dc_initial), c_states, bool(reverse), mode, out, float(gate_soft_cap or 0.0),
+                  grad_dtype)
+
+
+def _chunkwise_bw(q, k, v, i, f, n_out, m_out, dh, c0, n0, m0, dc_last, qk_scale, chunk_size, eps, impl, want_dc_initial,
+                  c_states, reverse, siging, out, soft_cap, grad_dtype):
+    """``_bw_launch`` with n_out / m_out as (B, NH, S) fp32 tensors (copied where they are not contiguous)."""
+    n_out, m_out = n_out.contiguous(), m_out.contiguous()
+    return _bw_launch(q, k, v, i, f, n_out.data_ptr(), m_out.data_ptr(), dh, c0, n0, m0, dc_last, qk_scale, chunk_size, eps,
+                      impl, want_dc_initial, c_states, reverse, siging, out, soft_cap, grad_dtype)
 
 
 def _make_function(autocast_kernel_dtype: torch.dtype):
@@ -526,8 +557,6 @@ def _make_function(autocast_kernel_dtype: torch.dtype):
                     siging, grad_dtype=None):
             need_bw = any(ctx.needs_input_grad[:6])
             ctx.grad_dtype = grad_dtype
-            if c_initial is None and (n_initial is not None or m_initial is not None):
-                c_initial = torch.zeros(q.shape[0], q.shape[1], q.shape[3], v.shape[3], dtype=q.dtype, device=q.device)
             h, nm, last, c_states = _fw_launch(q, k, v, i, f, c_initial, n_initial, m_initial, None, return_last_states,
                                                chunk_size, eps, None, need_bw, reverse, siging)
             ctx.save_for_backward(q, k, v, i, f, c_initial, n_initial, m_initial, nm, c_states)
@@ -541,8 +570,8 @@ def _make_function(autocast_kernel_dtype: torch.dtype):
         @custom_bwd(device_type="cuda")
         def backward(ctx, dh, dc_last, dn_last, dm_last):
             q, k, v, i, f, c0, n0, m0, nm, c_states = ctx.saved_tensors
-            nmp = nm.data_ptr()
-            dq, dk, dv, di, df, dc0 = _bw_launch(q, k, v, i, f, nmp, nmp + nm.stride(0) * 4, dh, c0, n0, m0, dc_last, None,
+            n_ptr, m_ptr = _nm_ptrs(nm)
+            dq, dk, dv, di, df, dc0 = _bw_launch(q, k, v, i, f, n_ptr, m_ptr, dh, c0, n0, m0, dc_last, None,
                                                  ctx.chunk_size, ctx.eps, None, c0 is not None, c_states, ctx.reverse,
                                                  ctx.siging, None, 0.0, ctx.grad_dtype)
             # dn_last / dm_last are ignored and dN/dM_initial are zeros, as in native/bw.py:329-337
@@ -599,6 +628,7 @@ def mlstm_chunkwise__b200(
     fn = _FUNCTIONS[autocast_kernel_dtype]
     if torch.compiler.is_compiling():
         fn = _ops.chunkwise_function(autocast_kernel_dtype)
+    c_initial = _zero_c_initial(q, v, c_initial, n_initial, m_initial)
     h, c_last, n_last, m_last = fn.apply(q, k, v, i, f, c_initial, n_initial, m_initial, bool(return_last_states),
                                          int(chunk_size), float(eps), bool(reverse), False,
                                          _caller_grad_dtype(autocast_kernel_dtype, q, k, v, i, f))
@@ -634,16 +664,8 @@ def mlstm_siging_chunkwise__b200(
     fn = _FUNCTIONS[autocast_kernel_dtype]
     if torch.compiler.is_compiling():
         fn = _ops.chunkwise_function(autocast_kernel_dtype)
-    need_states = c_initial is not None or n_initial is not None
-    m_initial = None
-    if need_states:
-        B, NH = q.shape[:2]
-        m_initial = torch.zeros(B, NH, 1, dtype=q.dtype, device=q.device)
-        if c_initial is None:
-            c_initial = torch.zeros(B, NH, q.shape[-1], v.shape[-1], dtype=q.dtype, device=q.device)
-        if n_initial is None:
-            n_initial = torch.zeros(B, NH, q.shape[-1], dtype=q.dtype, device=q.device)
-    h, c_last, n_last, _ = fn.apply(q, k, v, i, f, c_initial, n_initial, m_initial, bool(return_last_states),
+    c_initial = _zero_c_initial(q, v, c_initial, n_initial, None)  # no max state: the kernels start m at 0
+    h, c_last, n_last, _ = fn.apply(q, k, v, i, f, c_initial, n_initial, None, bool(return_last_states),
                                     int(chunk_size), float(eps), bool(reverse), _siging_mode(True, normalize),
                                     _caller_grad_dtype(autocast_kernel_dtype, q, k, v, i, f))
     if return_last_states:

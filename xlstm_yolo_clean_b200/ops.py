@@ -2,16 +2,17 @@
 ``torch.export`` trace the B200 kernels as opaque graph nodes instead of breaking the graph at every ctypes call.
 
 Dynamo cannot trace what the eager entry points do around a launch (ctypes, ``data_ptr()`` arithmetic, the per-thread
-call plans), so while it traces (``torch.compiler.is_compiling()``) those entry points call the functions at the end of
-this module instead.  They keep every host decision -- tensor route, chunk size, padding, one launch or two, gradient
-dtype -- in Python, where Dynamo guards on it; the decisions depend on sizes, strides and dtypes only.  Eager calls never
-come here.
+call plans), so while it traces (``torch.compiler.is_compiling()``) those entry points call these ops instead of their
+``autograd.Function``s, after the same host decisions -- chunk size, padding, one launch or two, gradient dtype -- made by
+the same functions, in Python, where Dynamo guards on them; the decisions depend on sizes, strides and dtypes only.
+Eager calls never come here.
 
-Each op's real implementation calls the launcher the eager path calls (``backend._fw_launch`` / ``_bw_launch``,
-``vil._cellout_fw_call`` / ``_cellout_bw_call``, ...), with the same plans and view fix-ups, so it runs exactly the
-kernels an eager call runs.  Each fake implementation allocates exactly what the real one does, shapes, dtypes and
-strides, and takes a symbolic batch size.  An op cannot return None: absent outputs are 0-element tensors, mapped back
-to None here.  No output aliases an input.
+Each op's real implementation is the body the eager ``autograd.Function`` calls (``backend._fw_launch`` /
+``_chunkwise_bw``, ``vil._layer_fw`` / ``_layer_bw`` / ``_cell_fused_fw``, ``vil._cellout_fw_call`` / ``_cellout_bw_call``,
+``vil._rmsnorm_fw_call`` / ``_rmsnorm_bw_call``), so it runs exactly the kernels an eager call runs.  Each fake
+implementation allocates exactly what the real one does, shapes, dtypes and strides, and takes a symbolic batch size.
+An op cannot return None: absent outputs are 0-element tensors, mapped back to None by the few wrappers here.  No output
+aliases an input.
 
 Inputs the eager ``autograd.Function``s round to the kernel dtype inside their forward (``custom_fwd(cast_inputs=...)``,
 ``convert16`` of the layer tensors) are rounded inside the ops too, so the gradients reach the caller's tensors through
@@ -21,11 +22,9 @@ copies alive (under autocast: one conversion pass per input and backward).
 from __future__ import annotations
 
 import ctypes as C
-import math
 from typing import Optional
 
 import torch
-import torch.nn.functional as F
 from torch import Tensor
 
 from . import _cabi
@@ -33,7 +32,6 @@ from . import backend as _backend
 from . import vil as _vil
 
 _F32, _U8 = torch.float32, torch.uint8
-_16BIT = (torch.float16, torch.bfloat16)
 # Inductor hands each op exactly the strides its fake saw: dh of the cell-output backward takes h's strides
 _TAGS = (torch._C.Tag.needs_exact_strides,)
 
@@ -73,24 +71,9 @@ def _tensor_route(NH, S, DK, DV, dtype, chunk_size, impl) -> bool:
     return _backend._tensor_route(_cabi.load_library(), _shape_struct(NH, S, DK, DV, dtype, chunk_size, impl))
 
 
-@torch.compiler.assume_constant_result
-def _tensor_path_supported(NH: int, S: int, DK: int, DV: int, dtype: torch.dtype, chunk_size: int) -> bool:
-    """``backend.tensor_path_supported`` as a trace-time constant (a host-only query of the support matrix)."""
-    return _backend.tensor_path_supported(1, NH, S, DK, DV, dtype, chunk_size)
-
-
 def _states_bytes(B, NH, S, DK, DV, dtype, chunk_size, impl):
     """Size of c_states (``mlstm_b200_states_bytes``, a host-only query): linear in B, which may be symbolic."""
     return B * _cabi.load_library().mlstm_b200_states_bytes(C.byref(_shape_struct(NH, S, DK, DV, dtype, chunk_size, impl)))
-
-
-def _bw_grad_dtype(q, v, dt, chunk_size, impl, grad_dtype):
-    """The dtype ``backend._bw_launch`` writes freshly allocated gradients in."""
-    gdt = grad_dtype or dt
-    if gdt is dt:
-        return dt
-    ok = gdt in _16BIT and _tensor_route(q.shape[1], q.shape[2], q.shape[3], v.shape[3], dt, chunk_size, impl)
-    return gdt if ok else dt
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -143,11 +126,9 @@ def chunkwise_bw(q: Tensor, k: Tensor, v: Tensor, i: Tensor, f: Tensor, n_out: T
     fp32 (0-element unless ``want_dc_initial``).  A 0-element ``c_states``: the kernels recompute the states."""
     mode = _backend._siging_mode(siging, normalize)
     q, k, v, i, f, c0, n0, m0 = _cast(cast_to, q, k, v, i, f, c_initial, n_initial, m_initial)
-    n_out = n_out if n_out.is_contiguous() else n_out.contiguous()
-    m_out = m_out if m_out.is_contiguous() else m_out.contiguous()
-    dq, dk, dv, di, df, dc0 = _backend._bw_launch(q, k, v, i, f, n_out.data_ptr(), m_out.data_ptr(), dh, c0, n0, m0, dc_last,
-                                                  qk_scale, chunk_size, eps, impl, want_dc_initial, _none(c_states), reverse,
-                                                  mode, None, soft_cap, grad_dtype)
+    dq, dk, dv, di, df, dc0 = _backend._chunkwise_bw(q, k, v, i, f, n_out, m_out, dh, c0, n0, m0, dc_last, qk_scale,
+                                                     chunk_size, eps, impl, want_dc_initial, _none(c_states), reverse, mode,
+                                                     None, soft_cap, grad_dtype)
     return dq, dk, dv, di, df, (dc0 if dc0 is not None else _empty(q))
 
 
@@ -155,9 +136,11 @@ def chunkwise_bw(q: Tensor, k: Tensor, v: Tensor, i: Tensor, f: Tensor, n_out: T
 def _(q, k, v, i, f, n_out, m_out, dh, c_initial, n_initial, m_initial, dc_last, c_states, cast_to, qk_scale, chunk_size,
       eps, impl, want_dc_initial, reverse, siging, soft_cap, grad_dtype, normalize=True):
     _backend._siging_mode(siging, normalize)
-    gdt = _bw_grad_dtype(q, v, cast_to or q.dtype, chunk_size, impl, grad_dtype)
     B, NH, S, DK = q.shape
     DV = v.shape[3]
+    dt = cast_to or q.dtype
+    route = grad_dtype not in (None, dt) and _tensor_route(NH, S, DK, DV, dt, chunk_size, impl)  # asked only when it matters
+    gdt = _backend._grad_dtype(dt, grad_dtype, route)
     dc0 = q.new_empty((B, NH, DK, DV), dtype=_F32) if want_dc_initial else _empty(q)
     return (q.new_empty((B, NH, S, DK), dtype=gdt), q.new_empty((B, NH, S, DK), dtype=gdt),
             q.new_empty((B, NH, S, DV), dtype=gdt), q.new_empty((B, NH, S), dtype=gdt), q.new_empty((B, NH, S), dtype=gdt),
@@ -209,11 +192,10 @@ class _ChunkwiseFunction:
         cast_to = self.kernel_dtype if torch.is_autocast_enabled("cuda") else None
         dt = cast_to if (cast_to is not None and _autocast_eligible(q)) else q.dtype
         need_bw = torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (q, k, v, i, f, c_initial))
-        if c_initial is None and (n_initial is not None or m_initial is not None):
-            c_initial = q.new_zeros((q.shape[0], q.shape[1], q.shape[3], v.shape[3]), dtype=dt)
+        siging, normalize = _backend._siging_flags(siging)
         h, _, c_last, n_last, m_last, _ = chunkwise_fw(q, k, v, i, f, c_initial, n_initial, m_initial, cast_to, None,
                                                        return_last_states, chunk_size, eps, _backend._default_impl, need_bw,
-                                                       reverse, siging != 0, 0.0, grad_dtype, siging != 2)
+                                                       reverse, siging, 0.0, grad_dtype, normalize)
         if not return_last_states:
             return h, None, None, None
         return h, c_last.to(dt), n_last.to(dt), m_last.to(dt)  # native kernels hand states back in the input dtype
@@ -232,9 +214,10 @@ def fw_launch(q, k, v, i, f, c0, n0, m0, qk_scale, return_last_states, chunk_siz
     (``siging`` the C-ABI mode 0 / 1 / 2)."""
     impl = _backend._default_impl if impl is None else impl
     q, k, v, i, f, c0, n0, m0 = (None if t is None else t.detach() for t in (q, k, v, i, f, c0, n0, m0))
+    siging, normalize = _backend._siging_flags(siging)
     h, nm, c_last, n_last, m_last, c_states = chunkwise_fw(q, k, v, i, f, c0, n0, m0, None, qk_scale, return_last_states,
-                                                           chunk_size, eps, impl, save_states, reverse, siging != 0, soft_cap,
-                                                           None, siging != 2)
+                                                           chunk_size, eps, impl, save_states, reverse, siging, soft_cap,
+                                                           None, normalize)
     return h, nm, ((c_last, n_last, m_last) if return_last_states else None), (c_states if save_states else None)
 
 
@@ -247,8 +230,9 @@ def bw_launch(q, k, v, i, f, n_out, m_out, dh, c0, n0, m0, dc_last, qk_scale, ch
         grad_dtype = out[0].dtype
     args = (q, k, v, i, f, n_out, m_out, dh, c0, n0, m0, dc_last, c_states)
     args = tuple(None if t is None else t.detach() for t in args)
-    dq, dk, dv, di, df, dc0 = chunkwise_bw(*args, None, qk_scale, chunk_size, eps, impl, want_dc_initial, reverse, siging != 0,
-                                           soft_cap, grad_dtype, siging != 2)
+    siging, normalize = _backend._siging_flags(siging)
+    dq, dk, dv, di, df, dc0 = chunkwise_bw(*args, None, qk_scale, chunk_size, eps, impl, want_dc_initial, reverse, siging,
+                                           soft_cap, grad_dtype, normalize)
     if out is not None:
         for o, g in zip(out, (dq, dk, dv, di, df)):
             o.copy_(g)
@@ -259,11 +243,6 @@ def bw_launch(q, k, v, i, f, n_out, m_out, dh, c0, n0, m0, dc_last, qk_scale, ch
 # ------------------------------------------------------------------------------------------------------------------
 # chunkwise mLSTM on the layer's own tensors: vil._MlstmLayerLayout and vil._MlstmCellFused
 # ------------------------------------------------------------------------------------------------------------------
-def _layer_heads(qk, v, gates, NH, kernel_dtype):
-    qk_k, v_k, g_k = (_backend.convert16(t, kernel_dtype) for t in (qk, v, gates))
-    return (qk_k, v_k, g_k), _vil._heads(qk_k, v_k, g_k, NH)
-
-
 @_op("layer_fw")
 def layer_fw(qk: Tensor, v: Tensor, gates: Tensor, NH: int, kernel_dtype: torch.dtype, chunk_size: int, eps: float,
              impl: int, save_states: bool, reverse: bool, siging: bool, soft_cap: float, grad_dtype: torch.dtype
@@ -271,9 +250,8 @@ def layer_fw(qk: Tensor, v: Tensor, gates: Tensor, NH: int, kernel_dtype: torch.
     """The forward of ``vil._MlstmLayerLayout`` on qk (B, S, 2 NH DHQK) = [q | k], v (B, S, NH DHHV) and gates
     (B, S, 2 NH) = [i | f] (S a multiple of ``chunk_size``), rounded to ``kernel_dtype`` here.  Returns h
     (B, NH, S, DHHV), nm, c_states.  ``grad_dtype`` is read by the backward only."""
-    _, (q, k, vv, i, f) = _layer_heads(qk, v, gates, NH, kernel_dtype)
-    h, nm, _, c_states = _backend._fw_launch(q, k, vv, i, f, None, None, None, None, False, chunk_size, eps, impl,
-                                             save_states, reverse, siging, soft_cap)
+    _, h, nm, c_states = _vil._layer_fw(qk, v, gates, NH, kernel_dtype, chunk_size, eps, impl, save_states, reverse, siging,
+                                        soft_cap)
     return h, nm, (c_states if c_states is not None else _empty(v, _U8))
 
 
@@ -291,22 +269,13 @@ def layer_bw(qk: Tensor, v: Tensor, gates: Tensor, nm: Tensor, dh: Tensor, c_sta
              kernel_dtype: torch.dtype, chunk_size: int, eps: float, impl: int, reverse: bool, siging: bool, soft_cap: float,
              grad_dtype: torch.dtype) -> tuple[Tensor, Tensor, Tensor]:
     """Gradients of ``layer_fw`` in the layer's layouts, written by the kernel in ``grad_dtype``: d_qk, d_v, d_gates."""
-    (qk_k, v_k, g_k), (q, k, vv, i, f) = _layer_heads(qk, v, gates, NH, kernel_dtype)
-    d_qk, d_v, d_g = (torch.empty_like(t, dtype=grad_dtype) for t in (qk_k, v_k, g_k))
-    nm = nm if nm.is_contiguous() else nm.contiguous()
-    nmp = nm.data_ptr()
-    _backend._bw_launch(q, k, vv, i, f, nmp, nmp + nm.stride(0) * 4, dh, None, None, None, None, None, chunk_size, eps, impl,
-                        False, _none(c_states), reverse, siging, _vil._heads(d_qk, d_v, d_g, NH), soft_cap)
-    return d_qk, d_v, d_g
+    return _vil._layer_bw(*_vil._kernel_tensors(qk, v, gates, kernel_dtype), nm.contiguous(), dh, _none(c_states), NH,
+                          chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype)
 
 
 @layer_bw.register_fake
 def _(qk, v, gates, nm, dh, c_states, NH, kernel_dtype, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype):
     return tuple(torch.empty_like(t, dtype=grad_dtype) for t in (qk, v, gates))
-
-
-def _to_inputs(grads, inputs):
-    return tuple(g if g.dtype == t.dtype else g.to(t.dtype) for g, t in zip(grads, inputs))
 
 
 def _layer_setup(ctx, inputs, output):
@@ -319,7 +288,8 @@ def _layer_setup(ctx, inputs, output):
 def _layer_backward(ctx, dh, dnm, dc_states):
     qk, v, gates, nm, c_states = ctx.saved_tensors
     grads = layer_bw(qk, v, gates, nm, dh, c_states, *ctx.cfg)
-    return (*_to_inputs(grads, (qk, v, gates)), None, None, None, None, None, None, None, None, None, None)
+    return (*_vil._to_dtypes(grads, (qk.dtype, v.dtype, gates.dtype)), None, None, None, None, None, None, None, None, None,
+            None)
 
 
 torch.library.register_autograd(layer_fw, _layer_backward, setup_context=_layer_setup)
@@ -332,17 +302,10 @@ def chunkwise_fw_epilogue(qk: Tensor, v: Tensor, gates: Tensor, x_skip: Optional
                           soft_cap: float, ln_eps: float, out_dtype: torch.dtype, grad_dtype: torch.dtype
                           ) -> tuple[Tensor, Tensor, Tensor, Tensor]:
     """The forward of ``vil._MlstmCellFused``: ``layer_fw`` with MultiHeadLayerNorm, the relayout and the skip
-    (``x_skip`` (B, S, H) contiguous in ``out_dtype``, or None) in the kernel's epilogue.  Returns y (B, S, NH DHHV),
-    h (0-element unless ``save_states``: the LayerNorm backward reads it), nm, c_states."""
-    B, S, H = v.shape
-    D = H // NH
-    _, (q, k, vv, i, f) = _layer_heads(qk, v, gates, NH, kernel_dtype)
-    y = torch.empty(B, S, H, dtype=out_dtype, device=v.device)
-    as_heads = lambda t: t.view(B, S, NH, D).transpose(1, 2)  # noqa: E731  (B, NH, S, D) view of a (B, S, H) tensor
-    epi = _backend.FwEpilogue(as_heads(y), None if x_skip is None else as_heads(x_skip), _vil._f32c(weight),
-                              _vil._f32c(bias), None if x_skip is None else _vil._f32c(skip), ln_eps, save_states)
-    h, nm, _, c_states = _backend._fw_launch(q, k, vv, i, f, None, None, None, None, False, chunk_size, eps, impl, save_states,
-                                             reverse, siging, soft_cap, epi)
+    (``x_skip`` (B, S, H), or None) in the kernel's epilogue.  Returns y (B, S, NH DHHV), h (0-element unless
+    ``save_states``: the LayerNorm backward reads it), nm, c_states."""
+    _, _, y, h, nm, c_states = _vil._cell_fused_fw(qk, v, gates, x_skip, weight, bias, skip, NH, kernel_dtype, chunk_size,
+                                                   eps, impl, save_states, reverse, siging, soft_cap, ln_eps, out_dtype)
     return (y, (h if h is not None else _empty(v, kernel_dtype)), nm,
             (c_states if c_states is not None else _empty(v, _U8)))
 
@@ -368,63 +331,14 @@ def _epilogue_setup(ctx, inputs, output):
 
 def _epilogue_backward(ctx, dy, dh_unused, dnm, dc_states):
     qk, v, gates, xs, weight, bias, skip, h, nm, c_states = ctx.saved_tensors
-    ln_eps, out_dtype = ctx.ln
-    dh, dpar, dx = cellout_bw(h, xs, weight, skip, dy, ln_eps, out_dtype, ctx.needs_input_grad[3])
+    dh, dpar, dx = cellout_bw(h, xs, weight, skip, dy, *ctx.ln, ctx.needs_input_grad[3])
     grads = layer_bw(qk, v, gates, nm, dh, c_states, *ctx.cfg)
-    return (*_to_inputs(grads, (qk, v, gates)), _none(dx),
-            None if weight is None else dpar[0].to(weight.dtype),
-            None if bias is None else dpar[1].to(bias.dtype),
-            None if skip is None else dpar[2].to(skip.dtype),
-            None, None, None, None, None, None, None, None, None, None, None, None)
+    return (*_vil._to_dtypes(grads, (qk.dtype, v.dtype, gates.dtype)), _none(dx),
+            *_vil._param_grads(dpar, weight, bias, skip), None, None, None, None, None, None, None, None, None, None, None,
+            None)
 
 
 torch.library.register_autograd(chunkwise_fw_epilogue, _epilogue_backward, setup_context=_epilogue_setup)
-
-
-def _layer_chunking(S, NH, head_dims, chunk_size, kernel_dtype):
-    """``_MlstmLayerLayout``'s choice: on the tensor-core route any S % 4 == 0 runs unpadded with a chunk size that
-    divides it; elsewhere the tensors are zero-padded to a multiple of ``chunk_size``.  Returns (chunk_size, pad)."""
-    if S % chunk_size and kernel_dtype in _16BIT:
-        g = math.gcd(S, chunk_size)
-        if _tensor_path_supported(NH, S, *head_dims, kernel_dtype, g):
-            chunk_size = g
-    return chunk_size, (-S) % chunk_size
-
-
-def layer_layout(qk, v, gates, NH, reverse, siging, chunk_size, eps, kernel_dtype, soft_cap=0.0):
-    """``vil._MlstmLayerLayout.apply`` over ``layer_fw`` / ``layer_bw``."""
-    B, S, H = v.shape
-    head_dims = _vil._head_dims(qk, v, NH)
-    in_dtypes = (qk.dtype, v.dtype, gates.dtype)
-    chunk_size, pad = _layer_chunking(S, NH, head_dims, chunk_size, kernel_dtype)
-    if pad:  # zero padding as wrap_chunkwise__pad_zeros (kernel_wrappers.py:227-247); padded tokens come last in scan order
-        pp = (0, 0, pad, 0) if reverse else (0, 0, 0, pad)
-        qk, v, gates = (F.pad(t, pp) for t in (qk, v, gates))
-    need_bw = torch.is_grad_enabled() and any(t.requires_grad for t in (qk, v, gates))
-    gdt = _vil._grad_dtype_of(in_dtypes, kernel_dtype, head_dims, S + pad)
-    h, _, _ = layer_fw(qk, v, gates, NH, kernel_dtype, chunk_size, eps, _backend._default_impl, need_bw, reverse, siging,
-                       soft_cap, gdt)
-    if pad:
-        h = h[:, :, pad:] if reverse else h[:, :, :S]
-    return h
-
-
-def cell_fused(qk, v, gates, x_skip, weight, bias, skip, NH, reverse, siging, chunk_size, eps, kernel_dtype, soft_cap, ln_eps,
-               out_dtype):
-    """``vil._MlstmCellFused.apply`` over ``chunkwise_fw_epilogue``."""
-    B, S, H = v.shape
-    if S % chunk_size:
-        chunk_size = math.gcd(S, chunk_size)  # any S % 4 == 0 runs unpadded (see _MlstmLayerLayout)
-    need_bw = torch.is_grad_enabled() and any(
-        t is not None and t.requires_grad for t in (qk, v, gates, x_skip, weight, bias, skip))
-    xs = None
-    if x_skip is not None and skip is not None:
-        xs = x_skip if (x_skip.dtype == out_dtype and x_skip.is_contiguous()) else x_skip.to(out_dtype).contiguous()
-    gdt = _vil._grad_dtype_of((qk.dtype, v.dtype, gates.dtype), kernel_dtype, _vil._head_dims(qk, v, NH), S)
-    y, _, _, _ = chunkwise_fw_epilogue(qk, v, gates, xs, weight, bias, None if xs is None else skip, NH, kernel_dtype,
-                                       chunk_size, eps, _backend._default_impl, need_bw, reverse, siging, soft_cap, ln_eps,
-                                       out_dtype, gdt)
-    return y
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -433,8 +347,8 @@ def cell_fused(qk, v, gates, x_skip, weight, bias, skip, NH, reverse, siging, ch
 @_op("cellout_fw")
 def cellout_fw(h: Tensor, weight: Optional[Tensor], bias: Optional[Tensor], skip: Optional[Tensor], x: Optional[Tensor],
                eps: float, out_dtype: torch.dtype) -> Tensor:
-    """``vil._CellOut``'s forward: y (B, S, NH D) in ``out_dtype``; ``x`` is None or contiguous in ``out_dtype``."""
-    return _vil._cellout_fw_call(h if _vil._vec_ok(h) else h.contiguous(), x, weight, bias, skip, eps, out_dtype)
+    """``vil._CellOut``'s forward: y (B, S, NH D) in ``out_dtype``."""
+    return _vil._cellout_fw_call(h, x, weight, bias, skip, eps, out_dtype)[0]
 
 
 @cellout_fw.register_fake
@@ -448,10 +362,7 @@ def cellout_bw(h: Tensor, x: Optional[Tensor], weight: Optional[Tensor], skip: O
                out_dtype: torch.dtype, want_dx: bool) -> tuple[Tensor, Tensor, Tensor]:
     """Returns dh (h's strides), dpar (3, H) fp32 = [dweight, dbias, dskip] and dx (0-element unless x and
     ``want_dx``)."""
-    hk = h if _vil._vec_ok(h) else h.contiguous()
-    dh, dpar, dx = _vil._cellout_bw_call(hk, x, weight, skip, dy, eps, out_dtype, want_dx)
-    if hk is not h:
-        dh = torch.empty_strided(h.shape, h.stride(), dtype=h.dtype, device=h.device).copy_(dh)
+    dh, dpar, dx = _vil._cellout_bw_call(h, x, weight, skip, dy, eps, out_dtype, want_dx)
     return dh, dpar, (dx if dx is not None else _empty(dy, out_dtype))
 
 
@@ -471,25 +382,11 @@ def _cellout_setup(ctx, inputs, output):
 
 def _cellout_backward(ctx, dy):
     h, x, weight, bias, skip = ctx.saved_tensors
-    eps, out_dtype = ctx.cfg
-    dh, dpar, dx = cellout_bw(h, x, weight, skip, dy, eps, out_dtype, ctx.needs_input_grad[4])
-    return (dh,
-            None if weight is None else dpar[0].to(weight.dtype),
-            None if bias is None else dpar[1].to(bias.dtype),
-            None if skip is None else dpar[2].to(skip.dtype),
-            _none(dx), None, None)
+    dh, dpar, dx = cellout_bw(h, x, weight, skip, dy, *ctx.cfg, ctx.needs_input_grad[4])
+    return (dh, *_vil._param_grads(dpar, weight, bias, skip), _none(dx), None, None)
 
 
 torch.library.register_autograd(cellout_fw, _cellout_backward, setup_context=_cellout_setup)
-
-
-def cell_out(h, weight, bias, skip, x, eps, out_dtype):
-    """``vil._CellOut.apply`` over ``cellout_fw`` / ``cellout_bw``."""
-    if not h.is_cuda:
-        raise RuntimeError("cell_out: h is on the CPU; this backend has no CPU path")
-    if x is not None and not (x.dtype == out_dtype and x.is_contiguous()):
-        x = x.to(out_dtype).contiguous()  # x, y, dy, dx all move as dense (B, S, H) rows
-    return cellout_fw(h, weight, bias, skip, x, float(eps), out_dtype)
 
 
 @_op("rmsnorm_fw")
@@ -506,7 +403,7 @@ def _(x2, weight, eps, out_dtype):
 @_op("rmsnorm_bw")
 def rmsnorm_bw(x2: Tensor, weight: Optional[Tensor], rstd: Tensor, dy2: Tensor, eps: float, out_dtype: torch.dtype
                ) -> tuple[Tensor, Tensor]:
-    """dx (rows, C) in x2's dtype and dweight (C,) fp32; ``dy2`` contiguous in ``out_dtype``."""
+    """dx (rows, C) in x2's dtype and dweight (C,) fp32."""
     return _vil._rmsnorm_bw_call(x2, weight, rstd, dy2, eps, out_dtype)
 
 
@@ -524,9 +421,7 @@ def _rmsnorm_setup(ctx, inputs, output):
 
 def _rmsnorm_backward(ctx, dy, drstd):
     x2, weight, rstd = ctx.saved_tensors
-    eps, out_dtype = ctx.cfg
-    dy = dy if (dy.dtype == out_dtype and dy.is_contiguous()) else dy.to(out_dtype).contiguous()
-    dx, dw = rmsnorm_bw(x2, weight, rstd, dy, eps, out_dtype)
+    dx, dw = rmsnorm_bw(x2, weight, rstd, dy, *ctx.cfg)
     return dx, (None if weight is None else dw.to(weight.dtype)), None, None
 
 
@@ -534,7 +429,7 @@ torch.library.register_autograd(rmsnorm_fw, _rmsnorm_backward, setup_context=_rm
 
 
 def rms_norm(x, weight, eps, out_dtype):
-    """``vil._RmsNorm.apply`` over ``rmsnorm_fw`` / ``rmsnorm_bw``."""
+    """``vil._RmsNorm.apply`` over ``rmsnorm_fw`` / ``rmsnorm_bw``: the op takes (rows, C) and returns rstd too."""
     if not x.is_cuda:
         raise RuntimeError("rms_norm_b200: x is on the CPU; this backend has no CPU path")
     shp = x.shape

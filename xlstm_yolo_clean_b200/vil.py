@@ -32,8 +32,8 @@ from . import backend as _backend
 from . import ops as _ops
 from torch.amp import custom_bwd, custom_fwd
 
-from .backend import (_DTYPES, _cell_uses_siging, _on_device, _tensor, mlstm_chunkwise__b200, mlstm_chunkwise_bw, mlstm_chunkwise_fw,
-                      mlstm_siging_chunkwise__b200, tensor_path_supported)
+from .backend import (_DTYPES, _cell_uses_siging, _on_device, _tensor, mlstm_chunkwise__b200, mlstm_siging_chunkwise__b200,
+                      tensor_path_supported)
 
 
 def cellout_supported(NH: int, D: int) -> bool:
@@ -59,10 +59,30 @@ def _vec_ok(t: torch.Tensor) -> bool:
     return t.stride(-1) == 1 and all(s % 4 == 0 for s in t.stride()[:-1]) and t.data_ptr() % 16 == 0
 
 
+def _rows(t, dtype):
+    """x, y, dy and dx of the cell-output kernels and of the fused epilogue move as dense (B, S, H) rows in the output
+    dtype at a 16-byte-aligned address: ``t`` as such rows, copied where it is not (None stays None)."""
+    if t is None or (t.dtype == dtype and t.is_contiguous() and t.data_ptr() % 16 == 0):
+        return t
+    t = t.to(dtype).contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()  # a contiguous view at an odd offset of its storage
+
+
+def _param_grads(dpar, weight, bias, skip):
+    """Gradients of weight / bias / skip from dpar (3, H) fp32 = [dweight, dbias, dskip], in the parameters' dtypes."""
+    return tuple(None if p is None else g.to(p.dtype) for g, p in zip(dpar, (weight, bias, skip)))
+
+
+def _to_dtypes(grads, dtypes):
+    return tuple(g if g.dtype == dt else g.to(dt) for g, dt in zip(grads, dtypes))
+
+
 def _cellout_fw_call(h, x, weight, bias, skip, eps, out_dtype):
-    """mlstm_b200_cellout_fw: y (B, S, NH*D) in ``out_dtype``.  ``h`` passes ``_vec_ok``; ``x`` is None or contiguous in
-    ``out_dtype``."""
+    """mlstm_b200_cellout_fw: y (B, S, NH*D) in ``out_dtype``, and the h and x the kernel read (h copied where it fails
+    ``_vec_ok``, x as ``_rows``)."""
     lib = _cabi.load_library()
+    h = h if _vec_ok(h) else h.contiguous()
+    x = _rows(x, out_dtype)
     B, NH, S, D = h.shape
     w32, b32, s32 = _f32c(weight), _f32c(bias), _f32c(skip)
     with _on_device(h.device):
@@ -77,7 +97,40 @@ def _cellout_fw_call(h, x, weight, bias, skip, eps, out_dtype):
         a.skip = None if s32 is None else s32.data_ptr()
         st = lib.mlstm_b200_cellout_fw(C.byref(a), C.c_void_p(torch.cuda.current_stream(h.device).cuda_stream))
         _cabi.check(st, "mlstm_b200_cellout_fw")
-    return y
+    return y, h, x
+
+
+def _cellout_bw_call(h, x, weight, skip, dy, eps, out_dtype, want_dx):
+    """mlstm_b200_cellout_bw: returns dh (h's strides), dpar (3, H) fp32 = [dweight, dbias, dskip] and dx (None unless x
+    and ``want_dx``).  h and x are prepared as in the forward, so the saved inputs of either one can be passed."""
+    lib = _cabi.load_library()
+    hk = h if _vec_ok(h) else h.contiguous()
+    x, dy = _rows(x, out_dtype), _rows(dy, out_dtype)
+    B, NH, S, D = h.shape
+    w32, s32 = _f32c(weight), _f32c(skip)
+    dev = h.device
+    with _on_device(dev):
+        dh = torch.empty_strided(hk.shape, hk.stride(), dtype=h.dtype, device=dev)  # the kernel walks h and dh together
+        dx = torch.empty_like(dy) if (x is not None and want_dx) else None
+        dpar = torch.empty(3, NH * D, dtype=torch.float32, device=dev)
+        b = _cabi.CellOutBwArgs()
+        a = b.fw
+        a.B, a.NH, a.S, a.D = B, NH, S, D
+        a.h_dtype, a.x_dtype, a.y_dtype = _DTYPES[h.dtype], _DTYPES[out_dtype], _DTYPES[out_dtype]
+        a.eps = eps
+        a.h, a.x = _tensor(hk), _tensor(x)
+        a.weight = None if w32 is None else w32.data_ptr()
+        a.skip = None if s32 is None else s32.data_ptr()
+        b.dy, b.dh, b.dx = _tensor(dy), _tensor(dh), _tensor(dx)
+        b.dweight, b.dbias, b.dskip = dpar[0].data_ptr(), dpar[1].data_ptr(), dpar[2].data_ptr()
+        ws_bytes = lib.mlstm_b200_cellout_workspace_bytes(C.byref(a))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        b.workspace, b.workspace_bytes = ws.data_ptr(), ws_bytes
+        st = lib.mlstm_b200_cellout_bw(C.byref(b), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+        _cabi.check(st, "mlstm_b200_cellout_bw")
+    if hk is not h:
+        dh = torch.empty_strided(h.shape, h.stride(), dtype=h.dtype, device=dev).copy_(dh)
+    return dh, dpar, dx
 
 
 class _CellOut(torch.autograd.Function):
@@ -85,12 +138,7 @@ class _CellOut(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, h, weight, bias, skip, x, eps, out_dtype):
-        if not h.is_cuda:
-            raise RuntimeError("cell_out: h is on the CPU; this backend has no CPU path")
-        h = h if _vec_ok(h) else h.contiguous()
-        if x is not None:  # x, y, dy, dx all move as dense (B, S, H) rows
-            x = x if (x.dtype == out_dtype and x.is_contiguous() and x.data_ptr() % 16 == 0) else x.to(out_dtype).contiguous()
-        y = _cellout_fw_call(h, x, weight, bias, skip, eps, out_dtype)
+        y, h, x = _cellout_fw_call(h, x, weight, bias, skip, eps, out_dtype)
         ctx.save_for_backward(h, x, weight, bias, skip)
         ctx.eps, ctx.out_dtype = float(eps), out_dtype
         return y
@@ -99,19 +147,17 @@ class _CellOut(torch.autograd.Function):
     def backward(ctx, dy):
         h, x, weight, bias, skip = ctx.saved_tensors
         dh, dpar, dx = _cellout_bw_call(h, x, weight, skip, dy, ctx.eps, ctx.out_dtype, ctx.needs_input_grad[4])
-        return (dh,
-                None if weight is None else dpar[0].to(weight.dtype),
-                None if bias is None else dpar[1].to(bias.dtype),
-                None if skip is None else dpar[2].to(skip.dtype),
-                dx, None, None)
+        return (dh, *_param_grads(dpar, weight, bias, skip), dx, None, None)
 
 
 def cell_out(h, weight=None, bias=None, skip=None, x=None, eps=1e-6, out_dtype=None):
     """Fused MultiHeadLayerNorm (+ skip): see the module docstring.  ``weight`` is the effective scale
     (the reference's ``weight_proxy`` = 1 + weight, vision_lstm2.py:900-907)."""
     out_dtype = out_dtype or (x.dtype if x is not None else h.dtype)
+    if not h.is_cuda:
+        raise RuntimeError("cell_out: h is on the CPU; this backend has no CPU path")
     if torch.compiler.is_compiling():
-        return _ops.cell_out(h, weight, bias, skip, x, eps, out_dtype)
+        return _ops.cellout_fw(h, weight, bias, skip, x, float(eps), out_dtype)
     return _CellOut.apply(h, weight, bias, skip, x, eps, out_dtype)
 
 
@@ -135,10 +181,13 @@ def _rmsnorm_fw_call(x2, weight, eps, out_dtype):
     return y, rstd
 
 
-def _rmsnorm_bw_call(x2, weight, rstd, dy2, eps, out_dtype):
-    """mlstm_b200_rmsnorm_bw: dx (rows, C) in x2's dtype and dweight (C,) fp32; ``dy2`` contiguous in ``out_dtype``."""
+def _rmsnorm_bw_call(x2, weight, rstd, dy, eps, out_dtype):
+    """mlstm_b200_rmsnorm_bw: dx (rows, C) in x2's dtype and dweight (C,) fp32; ``dy`` has x2's number of elements and
+    is read as contiguous (rows, C) in ``out_dtype``."""
     lib = _cabi.load_library()
     rows, Cdim = x2.shape
+    dy2 = dy.reshape(rows, Cdim)
+    dy2 = dy2 if (dy2.dtype == out_dtype and dy2.is_contiguous()) else dy2.to(out_dtype).contiguous()
     w32 = _f32c(weight)
     dev = x2.device
     with _on_device(dev):
@@ -177,10 +226,7 @@ class _RmsNorm(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         x2, weight, rstd = ctx.saved_tensors
-        rows, Cdim = x2.shape
-        dy2 = dy.reshape(rows, Cdim)
-        dy2 = dy2 if (dy2.dtype == ctx.out_dtype and dy2.is_contiguous()) else dy2.to(ctx.out_dtype).contiguous()
-        dx, dw = _rmsnorm_bw_call(x2, weight, rstd, dy2, ctx.eps, ctx.out_dtype)
+        dx, dw = _rmsnorm_bw_call(x2, weight, rstd, dy, ctx.eps, ctx.out_dtype)
         return dx.view(ctx.shp), (None if weight is None else dw.to(weight.dtype)), None, None
 
 
@@ -205,21 +251,33 @@ def _head_dims(qk, v, NH):
     return qk.shape[-1] // (2 * NH), v.shape[-1] // NH
 
 
-def _grad_dtype(in_dtypes, qk_k, v_k, NH):
-    """dtype the backward kernel writes d_qk / d_v / d_gates in: the dtype the layer's tensors had before they were
-    re-rounded to the kernel dtype (fp16 under ultralytics' AMP with the bf16 kernels) when the tensor-core route runs
-    and the three agree -- ``shape.grad_dtype`` of the C-ABI -- else the kernel dtype (and a cast afterwards)."""
-    return _grad_dtype_of(in_dtypes, v_k.dtype, _head_dims(qk_k, v_k, NH), v_k.shape[1])
-
-
-def _grad_dtype_of(in_dtypes, kdt, head_dims, S):
-    """``_grad_dtype`` from the kernel dtype, (DHQK, DHHV) and S alone."""
+def _layer_grad_dtype(in_dtypes, kernel_dtype, head_dims, S):
+    """``backend._grad_dtype`` of a layer-layout call: the dtype the layer's tensors had before they were re-rounded to
+    the kernel dtype (fp16 under ultralytics' AMP with the bf16 kernels) when the three agree, on the tensor-core route
+    as the head dims, S and the implementation choice determine it (no query)."""
     dt = in_dtypes[0]
-    if (dt is not kdt and dt in (torch.float16, torch.bfloat16) and kdt in (torch.float16, torch.bfloat16)
-            and all(t is dt for t in in_dtypes) and head_dims in TENSOR_HEAD_DIMS and S % 4 == 0
-            and _backend._default_impl != _cabi.IMPL_EXACT):
-        return dt
-    return kdt
+    caller = dt if all(t is dt for t in in_dtypes) else None
+    tensor_route = head_dims in TENSOR_HEAD_DIMS and S % 4 == 0 and _backend._default_impl != _cabi.IMPL_EXACT
+    return _backend._grad_dtype(kernel_dtype, caller, tensor_route)
+
+
+@torch.compiler.assume_constant_result
+def _tensor_path_supported(NH: int, S: int, DK: int, DV: int, dtype: torch.dtype, chunk_size: int) -> bool:
+    """``backend.tensor_path_supported`` for B = 1 (the support matrix does not depend on B), a constant while
+    torch.compile traces."""
+    return tensor_path_supported(1, NH, S, DK, DV, dtype, chunk_size)
+
+
+def _layer_chunking(S, NH, head_dims, chunk_size, kernel_dtype):
+    """(chunk_size, pad) of a layer-layout call.  The tcgen05 kernels walk 128-token tiles whatever the chunk size is
+    and handle a ragged last tile themselves (the result does not depend on chunk_size: the stabiliser equals the
+    step-recurrent one), so on the tensor-core route S = 400 / 100 run as they are with a chunk size that divides them;
+    elsewhere the tensors are zero-padded to a multiple of ``chunk_size``."""
+    if S % chunk_size and kernel_dtype in (torch.float16, torch.bfloat16):
+        g = math.gcd(S, chunk_size)
+        if _tensor_path_supported(NH, S, *head_dims, kernel_dtype, g):
+            chunk_size = g
+    return chunk_size, (-S) % chunk_size
 
 
 def _heads(qk, v, gates, NH):
@@ -234,6 +292,29 @@ def _heads(qk, v, gates, NH):
     return q, k, vv, gates[..., :NH].transpose(1, 2), gates[..., NH:].transpose(1, 2)
 
 
+def _kernel_tensors(qk, v, gates, kernel_dtype):
+    return tuple(_backend.convert16(t, kernel_dtype) for t in (qk, v, gates))  # (fp32 inputs: torch's cast)
+
+
+def _layer_fw(qk, v, gates, NH, kernel_dtype, chunk_size, eps, impl, save_states, reverse, siging, soft_cap, epi=None):
+    """Forward of the chunkwise mLSTM on the layer's tensors (S a multiple of ``chunk_size``), rounded to
+    ``kernel_dtype`` here; ``epi``: the fused cell-output epilogue.  Returns the rounded (qk, v, gates), h, nm, c_states."""
+    ts = _kernel_tensors(qk, v, gates, kernel_dtype)
+    h, nm, _, c_states = _backend._fw_launch(*_heads(*ts, NH), None, None, None, None, False, chunk_size, eps, impl,
+                                             save_states, reverse, siging, soft_cap, epi)
+    return ts, h, nm, c_states
+
+
+def _layer_bw(qk, v, gates, nm, dh, c_states, NH, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype):
+    """Gradients of ``_layer_fw`` from its rounded tensors, written by the kernel in ``grad_dtype`` straight into
+    tensors of the layer's layouts: d_qk, d_v, d_gates."""
+    grads = tuple(torch.empty_like(t, dtype=grad_dtype) for t in (qk, v, gates))
+    n_ptr, m_ptr = _backend._nm_ptrs(nm)
+    _backend._bw_launch(*_heads(qk, v, gates, NH), n_ptr, m_ptr, dh, None, None, None, None, None, chunk_size, eps, impl,
+                        False, c_states, reverse, siging, _heads(*grads, NH), soft_cap)
+    return grads
+
+
 class _MlstmLayerLayout(torch.autograd.Function):
     """Chunkwise mLSTM on the tensors the layer already owns -- qk (B, S, 2H) = [q | k] from qk_proj, v (B, S, H),
     gates (B, S, 2NH) = [i | f] -- with the gradients written by the kernel straight into tensors of those
@@ -242,77 +323,58 @@ class _MlstmLayerLayout(torch.autograd.Function):
 
     @staticmethod
     @custom_fwd(device_type="cuda")
-    def forward(ctx, qk, v, gates, NH, reverse, siging, chunk_size, eps, kernel_dtype, soft_cap=0.0):
-        B, S, H = v.shape
+    def forward(ctx, qk, v, gates, NH, kernel_dtype, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype):
+        ts, h, nm, c_states = _layer_fw(qk, v, gates, NH, kernel_dtype, chunk_size, eps, impl,
+                                        any(ctx.needs_input_grad[:3]), reverse, siging, soft_cap)
+        ctx.save_for_backward(*ts, nm, c_states)
+        ctx.cfg = (NH, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype)
         ctx.in_dtypes = (qk.dtype, v.dtype, gates.dtype)
-        qk_k, v_k, g_k = (_backend.convert16(t, kernel_dtype) for t in (qk, v, gates))  # (fp32 inputs: torch's cast)
-        if S % chunk_size and kernel_dtype in (torch.float16, torch.bfloat16):
-            # The tcgen05 kernels walk 128-token tiles whatever the chunk size is and handle a ragged last tile
-            # themselves (the result does not depend on chunk_size: the stabiliser equals the step-recurrent one),
-            # so S = 400 / 100 run as they are with a chunk size that divides them -- no zero-padding copies.
-            g = math.gcd(S, chunk_size)
-            if tensor_path_supported(B, NH, S, *_head_dims(qk, v, NH), kernel_dtype, chunk_size=g):
-                chunk_size = g
-        pad = (-S) % chunk_size
-        if pad:  # zero padding as wrap_chunkwise__pad_zeros (kernel_wrappers.py:227-247); padded tokens come last
-            pp = (0, 0, pad, 0) if reverse else (0, 0, 0, pad)  # in scan order = first in memory when reversed
-            qk_k, v_k, g_k = (F.pad(t, pp) for t in (qk_k, v_k, g_k))
-        q, k, vv, i, f = _heads(qk_k, v_k, g_k, NH)
-        need_bw = any(ctx.needs_input_grad[:3])
-        h, n_out, m_out, _, c_states = mlstm_chunkwise_fw(q, k, vv, i, f, chunk_size=chunk_size, eps=eps,
-                                                          save_states=need_bw, reverse=reverse, siging=siging,
-                                                          gate_soft_cap=soft_cap)
-        ctx.save_for_backward(qk_k, v_k, g_k, n_out, m_out, c_states)
-        ctx.cfg = (NH, reverse, siging, chunk_size, eps, pad, S, soft_cap)
-        if pad:
-            h = h[:, :, pad:] if reverse else h[:, :, :S]
         return h
 
     @staticmethod
     @custom_bwd(device_type="cuda")
     def backward(ctx, dh):
-        qk_k, v_k, g_k, n_out, m_out, c_states = ctx.saved_tensors
-        NH, reverse, siging, chunk_size, eps, pad, S, soft_cap = ctx.cfg
-        if pad:
-            dh = F.pad(dh, (0, 0, pad, 0) if reverse else (0, 0, 0, pad))
-        gdt = _grad_dtype(ctx.in_dtypes, qk_k, v_k, NH)  # the caller's 16-bit dtype: no cast pass over the gradients
-        d_qk, d_v, d_g = (torch.empty_like(t, dtype=gdt) for t in (qk_k, v_k, g_k))
-        q, k, vv, i, f = _heads(qk_k, v_k, g_k, NH)
-        mlstm_chunkwise_bw(q, k, vv, i, f, n_out, m_out, dh, chunk_size=chunk_size, eps=eps, c_states=c_states,
-                           reverse=reverse, siging=siging, out=_heads(d_qk, d_v, d_g, NH), gate_soft_cap=soft_cap)
-        if pad:
-            d_qk, d_v, d_g = ((t[:, pad:] if reverse else t[:, :S]) for t in (d_qk, d_v, d_g))
-        d_qk, d_v, d_g = (t if t.dtype == dt else t.to(dt) for t, dt in zip((d_qk, d_v, d_g), ctx.in_dtypes))
-        return d_qk, d_v, d_g, None, None, None, None, None, None, None
+        qk_k, v_k, g_k, nm, c_states = ctx.saved_tensors
+        grads = _layer_bw(qk_k, v_k, g_k, nm, dh, c_states, *ctx.cfg)
+        return (*_to_dtypes(grads, ctx.in_dtypes), None, None, None, None, None, None, None, None, None)
 
 
-def _cellout_bw_call(h, x, weight, skip, dy, eps, out_dtype, want_dx):
-    """mlstm_b200_cellout_bw on saved tensors: returns dh (h's strides), dpar (3, H) fp32 = [dweight, dbias, dskip], dx."""
-    lib = _cabi.load_library()
-    B, NH, S, D = h.shape
-    dy = dy if (dy.dtype == out_dtype and dy.is_contiguous() and dy.data_ptr() % 16 == 0) else dy.to(out_dtype).contiguous()
-    w32, s32 = _f32c(weight), _f32c(skip)
-    dev = h.device
-    with _on_device(dev):
-        dh = torch.empty_strided(h.shape, h.stride(), dtype=h.dtype, device=dev)  # the kernel walks h and dh together
-        dx = torch.empty_like(dy) if (x is not None and want_dx) else None
-        dpar = torch.empty(3, NH * D, dtype=torch.float32, device=dev)
-        b = _cabi.CellOutBwArgs()
-        a = b.fw
-        a.B, a.NH, a.S, a.D = B, NH, S, D
-        a.h_dtype, a.x_dtype, a.y_dtype = _DTYPES[h.dtype], _DTYPES[out_dtype], _DTYPES[out_dtype]
-        a.eps = eps
-        a.h, a.x = _tensor(h), _tensor(x)
-        a.weight = None if w32 is None else w32.data_ptr()
-        a.skip = None if s32 is None else s32.data_ptr()
-        b.dy, b.dh, b.dx = _tensor(dy), _tensor(dh), _tensor(dx)
-        b.dweight, b.dbias, b.dskip = dpar[0].data_ptr(), dpar[1].data_ptr(), dpar[2].data_ptr()
-        ws_bytes = lib.mlstm_b200_cellout_workspace_bytes(C.byref(a))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        b.workspace, b.workspace_bytes = ws.data_ptr(), ws_bytes
-        st = lib.mlstm_b200_cellout_bw(C.byref(b), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
-        _cabi.check(st, "mlstm_b200_cellout_bw")
-    return dh, dpar, dx
+def _layer_layout(qk, v, gates, NH, reverse, siging, chunk_size, eps, kernel_dtype, soft_cap):
+    """h (B, NH, S, DHHV) of the chunkwise mLSTM on the layer's tensors: ``_MlstmLayerLayout``, or the ``layer_fw`` op
+    while torch.compile traces."""
+    S = v.shape[1]
+    head_dims = _head_dims(qk, v, NH)
+    chunk_size, pad = _layer_chunking(S, NH, head_dims, chunk_size, kernel_dtype)
+    gdt = _layer_grad_dtype((qk.dtype, v.dtype, gates.dtype), kernel_dtype, head_dims, S + pad)
+    if pad:  # zero padding as wrap_chunkwise__pad_zeros (kernel_wrappers.py:227-247); padded tokens come last
+        pp = (0, 0, pad, 0) if reverse else (0, 0, 0, pad)  # in scan order = first in memory when reversed
+        qk, v, gates = (F.pad(t, pp) for t in (qk, v, gates))
+    args = (qk, v, gates, NH, kernel_dtype, chunk_size, eps, _backend._default_impl)
+    if torch.compiler.is_compiling():
+        need_bw = torch.is_grad_enabled() and any(t.requires_grad for t in (qk, v, gates))
+        h = _ops.layer_fw(*args, need_bw, reverse, siging, soft_cap, gdt)[0]
+    else:
+        h = _MlstmLayerLayout.apply(*args, reverse, siging, soft_cap, gdt)
+    if pad:
+        h = h[:, :, pad:] if reverse else h[:, :, :S]
+    return h
+
+
+def _cell_fused_fw(qk, v, gates, x_skip, weight, bias, skip, NH, kernel_dtype, chunk_size, eps, impl, save_states, reverse,
+                   siging, soft_cap, ln_eps, out_dtype):
+    """``_layer_fw`` with MultiHeadLayerNorm, the relayout and the skip (``x_skip`` prepared as ``_rows``, or None) in
+    the kernel's epilogue.  Returns the rounded (qk, v, gates), the skip input read, y (B, S, NH DHHV), h (None unless
+    ``save_states``: the LayerNorm backward reads it), nm, c_states."""
+    B, S, H = v.shape
+    D = H // NH
+    xs = _rows(x_skip, out_dtype)
+    y = torch.empty(B, S, H, dtype=out_dtype, device=v.device)
+    as_heads = lambda t: t.view(B, S, NH, D).transpose(1, 2)  # noqa: E731  (B, NH, S, D) view of a (B, S, H) tensor
+    epi = _backend.FwEpilogue(as_heads(y), None if xs is None else as_heads(xs), _f32c(weight), _f32c(bias),
+                              None if xs is None else _f32c(skip), ln_eps, save_states)
+    ts, h, nm, c_states = _layer_fw(qk, v, gates, NH, kernel_dtype, chunk_size, eps, impl, save_states, reverse, siging,
+                                    soft_cap, epi)
+    return ts, xs, y, h, nm, c_states
 
 
 class _MlstmCellFused(torch.autograd.Function):
@@ -324,48 +386,45 @@ class _MlstmCellFused(torch.autograd.Function):
 
     @staticmethod
     @custom_fwd(device_type="cuda")
-    def forward(ctx, qk, v, gates, x_skip, weight, bias, skip, NH, reverse, siging, chunk_size, eps, kernel_dtype, soft_cap,
-                ln_eps, out_dtype):
-        B, S, H = v.shape
-        D = H // NH
+    def forward(ctx, qk, v, gates, x_skip, weight, bias, skip, NH, kernel_dtype, chunk_size, eps, impl, reverse, siging,
+                soft_cap, ln_eps, out_dtype, grad_dtype):
+        ts, xs, y, h, nm, c_states = _cell_fused_fw(qk, v, gates, x_skip, weight, bias, skip, NH, kernel_dtype, chunk_size,
+                                                    eps, impl, any(ctx.needs_input_grad[:7]), reverse, siging, soft_cap,
+                                                    ln_eps, out_dtype)
+        ctx.save_for_backward(*ts, nm, c_states, h, xs, weight, bias, skip)
+        ctx.cfg = (NH, chunk_size, eps, impl, reverse, siging, soft_cap, grad_dtype)
+        ctx.ln = (ln_eps, out_dtype)
         ctx.in_dtypes = (qk.dtype, v.dtype, gates.dtype)
-        qk_k, v_k, g_k = (_backend.convert16(t, kernel_dtype) for t in (qk, v, gates))  # (fp32 inputs: torch's cast)
-        if S % chunk_size:
-            chunk_size = math.gcd(S, chunk_size)  # any S % 4 == 0 runs unpadded (see _MlstmLayerLayout)
-        q, k, vv, i, f = _heads(qk_k, v_k, g_k, NH)
-        need_bw = any(ctx.needs_input_grad[:7])
-        y = torch.empty(B, S, H, dtype=out_dtype, device=v.device)
-        xs = None
-        if x_skip is not None and skip is not None:
-            xs = x_skip if (x_skip.dtype == out_dtype and x_skip.is_contiguous()) else x_skip.to(out_dtype).contiguous()
-        as_heads = lambda t: t.view(B, S, NH, D).transpose(1, 2)  # noqa: E731  (B, NH, S, D) view of a (B, S, H) tensor
-        epi = _backend.FwEpilogue(as_heads(y), None if xs is None else as_heads(xs), _f32c(weight), _f32c(bias),
-                                  None if xs is None else _f32c(skip), ln_eps, need_bw)
-        h, nm, _, c_states = _backend._fw_launch(q, k, vv, i, f, None, None, None, None, False, chunk_size, eps, None, need_bw,
-                                                 reverse, siging, soft_cap, epi)
-        ctx.save_for_backward(qk_k, v_k, g_k, nm, c_states, h, xs, weight, bias, skip)
-        ctx.cfg = (NH, reverse, siging, chunk_size, eps, soft_cap, ln_eps, out_dtype)
         return y
 
     @staticmethod
     @custom_bwd(device_type="cuda")
     def backward(ctx, dy):
         qk_k, v_k, g_k, nm, c_states, h, xs, weight, bias, skip = ctx.saved_tensors
-        NH, reverse, siging, chunk_size, eps, soft_cap, ln_eps, out_dtype = ctx.cfg
-        dh, dpar, dx = _cellout_bw_call(h, xs, weight, skip if xs is not None else None, dy, ln_eps, out_dtype,
-                                        ctx.needs_input_grad[3])
-        gdt = _grad_dtype(ctx.in_dtypes, qk_k, v_k, NH)  # the caller's 16-bit dtype: no cast pass over the gradients
-        d_qk, d_v, d_g = (torch.empty_like(t, dtype=gdt) for t in (qk_k, v_k, g_k))
-        q, k, vv, i, f = _heads(qk_k, v_k, g_k, NH)
-        nmp = nm.data_ptr()
-        _backend._bw_launch(q, k, vv, i, f, nmp, nmp + nm.stride(0) * 4, dh, None, None, None, None, None, chunk_size, eps, None,
-                            False, c_states, reverse, siging, _heads(d_qk, d_v, d_g, NH), soft_cap)
-        d_qk, d_v, d_g = (t if t.dtype == dt else t.to(dt) for t, dt in zip((d_qk, d_v, d_g), ctx.in_dtypes))
-        return (d_qk, d_v, d_g, dx,
-                None if weight is None else dpar[0].to(weight.dtype),
-                None if bias is None else dpar[1].to(bias.dtype),
-                None if (skip is None or xs is None) else dpar[2].to(skip.dtype),
-                None, None, None, None, None, None, None, None, None)
+        dh, dpar, dx = _cellout_bw_call(h, xs, weight, skip, dy, *ctx.ln, ctx.needs_input_grad[3])
+        grads = _layer_bw(qk_k, v_k, g_k, nm, dh, c_states, *ctx.cfg)
+        return (*_to_dtypes(grads, ctx.in_dtypes), dx, *_param_grads(dpar, weight, bias, skip),
+                None, None, None, None, None, None, None, None, None, None, None)
+
+
+def _cell_fused(qk, v, gates, x_skip, weight, bias, skip, NH, reverse, siging, chunk_size, eps, kernel_dtype, soft_cap,
+                ln_eps, out_dtype):
+    """y (B, S, NH DHHV) of the one-launch cell: ``_MlstmCellFused``, or the ``chunkwise_fw_epilogue`` op while
+    torch.compile traces.  The skip is added only with both ``skip`` and ``x_skip``."""
+    S = v.shape[1]
+    head_dims = _head_dims(qk, v, NH)
+    chunk_size, pad = _layer_chunking(S, NH, head_dims, chunk_size, kernel_dtype)
+    if pad:
+        raise RuntimeError("the fused cell-output epilogue exists on the tensor-core route only")
+    if x_skip is None or skip is None:
+        x_skip = skip = None
+    gdt = _layer_grad_dtype((qk.dtype, v.dtype, gates.dtype), kernel_dtype, head_dims, S)
+    args = (qk, v, gates, x_skip, weight, bias, skip, NH, kernel_dtype, chunk_size, eps, _backend._default_impl)
+    if torch.compiler.is_compiling():
+        need_bw = torch.is_grad_enabled() and any(
+            t is not None and t.requires_grad for t in (qk, v, gates, x_skip, weight, bias, skip))
+        return _ops.chunkwise_fw_epilogue(*args, need_bw, reverse, siging, soft_cap, ln_eps, out_dtype, gdt)[0]
+    return _MlstmCellFused.apply(*args, reverse, siging, soft_cap, ln_eps, out_dtype, gdt)
 
 
 def _is_reverse(layer) -> bool:
@@ -449,13 +508,10 @@ def mlstm_cell_b200(cell, q, k, v, reverse=False, skip=None, x_skip=None, siging
         fuse = one_launch == "always" or (one_launch == "auto" and auto_fuse)
         if (fuse and in_kernel_cap and S % 4 == 0 and out_dtype in (torch.float16, torch.bfloat16)
                 and cellout_supported(NH, D) and (x_skip is None or x_skip.shape == (B, S, H))):
-            fused = _ops.cell_fused if torch.compiler.is_compiling() else _MlstmCellFused.apply
-            return fused(qk_c, v_c, g_c, x_skip if skip is not None else None, norm.weight_proxy, norm.bias,
-                                         skip, NH, bool(reverse), bool(siging), int(chunk_size), float(eps), kdt,
-                                         float(cell.gate_soft_cap), float(norm.eps), out_dtype)
-        layer = _ops.layer_layout if torch.compiler.is_compiling() else _MlstmLayerLayout.apply
-        h = layer(qk_c, v_c, g_c, NH, bool(reverse), bool(siging), int(chunk_size), float(eps), kdt,
-                                    float(cell.gate_soft_cap) if in_kernel_cap else 0.0)
+            return _cell_fused(qk_c, v_c, g_c, x_skip, norm.weight_proxy, norm.bias, skip, NH, bool(reverse), bool(siging),
+                               int(chunk_size), float(eps), kdt, float(cell.gate_soft_cap), float(norm.eps), out_dtype)
+        h = _layer_layout(qk_c, v_c, g_c, NH, bool(reverse), bool(siging), int(chunk_size), float(eps), kdt,
+                          float(cell.gate_soft_cap) if in_kernel_cap else 0.0)
     else:
         capped = cell.gate_soft_cap * torch.tanh(if_preact / cell.gate_soft_cap)  # soft_cap, vision_lstm2.py:755-756
         i_pre, f_pre = torch.chunk(capped, 2, dim=-1)
