@@ -249,7 +249,8 @@ int mlstm_b200_recurrent_sequence(const mlstm_b200_recurrent_args* args, void* c
  *   x, y, dy, dx (B, S, NH*D)  element strides [b, s, 1];  x and y share one dtype (x_dtype == y_dtype)
  *   weight (= 1 + MultiHeadLayerNorm.weight, the reference's weight_proxy, vision_lstm2.py:900-907),
  *   bias, skip: contiguous fp32 (NH*D); weight / bias may be NULL (1 / 0); x.ptr == NULL drops the skip term.
- * Supported: D in {32, 64, 128}, NH*D a multiple of 128 and <= 2048; pointers 8-byte (16-bit types) or
+ * Supported: D in {32, 64, 128} and any NH >= 1 with NH*D <= 2048 (every YOLO-ViL width whose qkv_block_size is one of
+ * those head dims, up to dim 1024; NH*D need not be a multiple of 128); pointers 8-byte (16-bit types) or
  * 16-byte (fp32) aligned, strides multiples of 4 elements; x has y's strides; in the backward dh has h's strides
  * and x / dx have dy's (the kernels walk each family with one running offset).
  */
@@ -286,7 +287,8 @@ int mlstm_b200_cellout_bw(const mlstm_b200_cellout_bw_args* args, void* cuda_str
  * (vision_lstm2.py:277-278, applied at :318-327).  y = round_x(x * rsqrt(mean(x^2) + eps)) * weight over the last
  * dimension of a dense (rows, C) matrix -- the rounding of the normalised row to the input dtype is what torch's
  * composite rms_norm does when input and weight dtypes differ (fp16 autocast).  rstd (rows) fp32 is written by the
- * forward and read by the backward.  C in {192, 256, 384, 512}; x / dx of x_dtype, y / dy of y_dtype.
+ * forward and read by the backward.  C any multiple of 32 from 64 to 2048 (every ViL width dim in that range); x / dx of
+ * x_dtype, y / dy of y_dtype.
  */
 typedef struct mlstm_b200_rmsnorm_args {
   int64_t rows;

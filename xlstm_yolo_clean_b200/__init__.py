@@ -13,7 +13,8 @@ mlstm_kernels/torch/chunkwise/__init__.py:9-15 of the reference):
 """
 from ._cabi import LIB_PATH, LibraryMissing, load_library  # noqa: F401
 from .host_pipeline import HostFwBw  # noqa: F401
-from .vil import cell_out, cellout_supported, mlstm_branch_b200, mlstm_cell_b200, patch_layers, rms_norm_b200  # noqa: F401
+from .vil import (cell_out, cellout_supported, mlstm_branch_b200, mlstm_cell_b200, patch_layers, rms_norm_b200,  # noqa: F401
+                  rmsnorm_supported)
 from .backend import (  # noqa: F401
     KERNEL_NAME,
     last_launch_count,

@@ -12,7 +12,10 @@
 //
 // HBM-bound elementwise + small-group reduction work: no tensor cores.  One warp covers 128 consecutive
 // channels of one token row (4 channels per lane: 8-byte loads for 16-bit types), so x / y / dy / dx move
-// as fully coalesced 256-byte warp transactions and every h / dh access is one whole head row.  Group
+// as fully coalesced 256-byte warp transactions and every h / dh access is one whole head row.  A row whose
+// width H is not a multiple of 128 ends in a tail warp covering H mod 128 (= 32, 64 or 96) channels: its lanes
+// past the row's end load and store nothing (TAIL instantiations; D divides 128, so no head straddles two
+// warps and the idle lanes form whole head groups of their own).  Group
 // statistics are xor-shuffle reductions over the D/4 lanes of a head; the per-channel parameter gradients
 // stay in registers across a persistent row loop and are reduced deterministically in two stages
 // (CTA partials in the caller's workspace, then one small kernel) -- no atomics.
@@ -31,7 +34,7 @@ constexpr int kFwRows = MLSTM_CELL_FW_ROWS, kBwRows = MLSTM_CELL_BW_ROWS;  // (f
 constexpr int kMaxWarps = 16;
 
 struct CellP {
-  int B, NH, S, D, H, W, lpg;  // H = NH*D channels, W = H/128 warps per token row, lpg = D/4 lanes per head
+  int B, NH, S, D, H, W, lpg;  // H = NH*D channels, W = ceil(H/128) warps per token row, lpg = D/4 lanes per head
   float eps, inv_d;
   const void *h, *x, *dy;
   void *y, *dh, *dx;
@@ -130,17 +133,18 @@ template <typename TH, typename TX, int U> struct FwRegs {
 
 // Software-pipelined persistent loop: the loads of the next U rows are in flight while the current U rows are
 // normalised and stored (two register sets, ping-pong), so every warp keeps U*(h + x) loads outstanding.
-template <typename TH, typename TX, int U, int LPG>
+template <typename TH, typename TX, int U, int LPG, bool TAIL = false>
 __global__ void __launch_bounds__(kMaxWarps * 32, 1) k_cellout_fw(const CellP p) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int slot = warp % p.W, r = warp / p.W, R = (blockDim.x >> 5) / p.W;
   const int c0 = slot * 128 + lane * 4, head = c0 / p.D, d0 = c0 % p.D;
+  const bool act = !TAIL || c0 < p.H;  // lane inside the row (idle lanes still walk the rows: the shuffles need them)
   float w[4], b[4], sk[4];
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
-    w[e] = p.weight ? p.weight[c0 + e] : 1.f;
-    b[e] = p.bias ? p.bias[c0 + e] : 0.f;
-    sk[e] = p.skip ? p.skip[c0 + e] : 0.f;
+    w[e] = act && p.weight ? p.weight[c0 + e] : 1.f;
+    b[e] = act && p.bias ? p.bias[c0 + e] : 0.f;
+    sk[e] = act && p.skip ? p.skip[c0 + e] : 0.f;
   }
   const TH* hp = reinterpret_cast<const TH*>(p.h) + head * p.hs[1] + d0;
   const TX* xp = reinterpret_cast<const TX*>(p.x);
@@ -154,8 +158,10 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) k_cellout_fw(const CellP p)
       g.yoff[u] = -1;
       g.hv[u] = zraw<TH>(), g.xv[u] = zraw<TX>();
       if (it.valid()) {
-        g.hv[u] = ldraw<TH>(hp + it.off_a);
-        if (xp) g.xv[u] = ldraw<TX>(xp + it.off_c + c0);  // x shares y's strides (checked on the host)
+        if (act) {
+          g.hv[u] = ldraw<TH>(hp + it.off_a);
+          if (xp) g.xv[u] = ldraw<TX>(xp + it.off_c + c0);  // x shares y's strides (checked on the host)
+        }
         g.yoff[u] = it.off_c + c0;
       }
       it.next();
@@ -170,7 +176,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) k_cellout_fw(const CellP p)
       group_stats<LPG>(hv, p.inv_d, p.eps, mean, rstd);  // row validity is warp-uniform
 #pragma unroll
       for (int e = 0; e < 4; ++e) o[e] = (hv[e] - mean) * rstd * w[e] + b[e] + sk[e] * xv[e];
-      if (g.yoff[u] >= 0) store4<TX>(yp + g.yoff[u], o);
+      if (act && g.yoff[u] >= 0) store4<TX>(yp + g.yoff[u], o);
     }
   };
   Regs ga, gb;
@@ -190,17 +196,18 @@ template <typename TH, typename TX, int U> struct BwRegs {
   int64_t oa[U], oc[U];  // element offsets of the row in h / dh and in dy / x / dx; oa < 0: no row
 };
 
-template <typename TH, typename TX, int U, int LPG>
+template <typename TH, typename TX, int U, int LPG, bool TAIL = false>
 __global__ void __launch_bounds__(kMaxWarps * 32, 1) k_cellout_bw(const CellP p) {
   __shared__ float red[3][kMaxWarps][128];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int slot = warp % p.W, r = warp / p.W, R = (blockDim.x >> 5) / p.W;
   const int c0 = slot * 128 + lane * 4, head = c0 / p.D, d0 = c0 % p.D;
+  const bool act = !TAIL || c0 < p.H;  // as in the forward; idle lanes accumulate zeros
   float w[4], sk[4], aw[4] = {0.f, 0.f, 0.f, 0.f}, ab[4] = {0.f, 0.f, 0.f, 0.f}, as[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
   for (int e = 0; e < 4; ++e) {
-    w[e] = p.weight ? p.weight[c0 + e] : 1.f;
-    sk[e] = p.skip ? p.skip[c0 + e] : 0.f;
+    w[e] = act && p.weight ? p.weight[c0 + e] : 1.f;
+    sk[e] = act && p.skip ? p.skip[c0 + e] : 0.f;
   }
   const TH* hp = reinterpret_cast<const TH*>(p.h) + head * p.hs[1] + d0;
   TH* dhp = reinterpret_cast<TH*>(p.dh) + head * p.hs[1] + d0;
@@ -217,9 +224,11 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) k_cellout_bw(const CellP p)
       g.hv[u] = zraw<TH>(), g.xv[u] = zraw<TX>(), g.gv[u] = zraw<TX>();
       if (it.valid()) {
         g.oa[u] = it.off_a, g.oc[u] = it.off_c + c0;  // dh shares h's strides, x / dx share dy's (host-checked)
-        g.hv[u] = ldraw<TH>(hp + it.off_a);
-        g.gv[u] = ldraw<TX>(dyp + g.oc[u]);
-        if (xp) g.xv[u] = ldraw<TX>(xp + g.oc[u]);
+        if (act) {
+          g.hv[u] = ldraw<TH>(hp + it.off_a);
+          g.gv[u] = ldraw<TX>(dyp + g.oc[u]);
+          if (xp) g.xv[u] = ldraw<TX>(xp + g.oc[u]);
+        }
       }
       it.next();
     }
@@ -245,7 +254,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) k_cellout_bw(const CellP p)
       }
       s1 = group_sum<LPG>(s1) * p.inv_d;
       s2 = group_sum<LPG>(s2) * p.inv_d;
-      if (g.oa[u] >= 0) {
+      if (act && g.oa[u] >= 0) {
 #pragma unroll
         for (int e = 0; e < 4; ++e) o[e] = rstd * (gw[e] - s1 - xh[e] * s2);
         store4<TH>(dhp + g.oa[u], o);
@@ -276,7 +285,7 @@ __global__ void __launch_bounds__(kMaxWarps * 32, 1) k_cellout_bw(const CellP p)
     red[2][warp][lane * 4 + e] = as[e];
   }
   __syncthreads();
-  if (r == 0) {
+  if (r == 0 && act) {
 #pragma unroll
     for (int q = 0; q < 3; ++q) {
       float acc[4] = {0.f, 0.f, 0.f, 0.f};
@@ -425,6 +434,124 @@ __global__ void __launch_bounds__(512, 1) k_rmsnorm_bw(const RmsP p) {
   }
 }
 
+// Every other width (C a multiple of 32, 64 <= C <= 2048): the row as m = C/32 slots of 32 consecutive channels, one
+// element per lane and slot (64-byte warp accesses for 16-bit types, 128-byte for fp32).  A team of T warps shares a
+// row, warp t taking slots t, t + T, t + 2T, ... (at most K of them), so no lane holds more than K elements of a row
+// whatever C is: registers stay bounded at C = 2048 (K = 16, T = 4).  The team combines its warps' sums through
+// shared memory and one named barrier per row (double-buffered by row parity, so one barrier is enough: a warp
+// rewrites a buffer only after the whole team has passed the next barrier, i.e. has read it).  The arithmetic is
+// the pair kernels': fp32 statistics, one rounding at the store.  T = 1 needs no barrier at all.
+template <int T>
+__device__ __forceinline__ float team_sum(float v, float* tsum, int wib, int tib) {  // v: this warp's sum (warp-uniform)
+  if constexpr (T == 1) {
+    return v;
+  } else {
+    if ((threadIdx.x & 31) == 0) tsum[wib] = v;
+    asm volatile("bar.sync %0, %1;" ::"r"(1 + tib), "r"(T * 32) : "memory");
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < T; ++i) s += tsum[tib * T + i];  // same order in every warp of the team
+    return s;
+  }
+}
+
+template <typename TX, typename TY, int K, int T>
+__global__ void __launch_bounds__(512, 1) k_rmsnorm_fw_slots(const RmsP p) {
+  __shared__ float tsum[2][2][16];  // [row parity][row a / b][warp]
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, t = wib % T, tib = wib / T;
+  const int teams = (blockDim.x >> 5) / T, m = p.C >> 5;
+  const int64_t team = (int64_t)blockIdx.x * teams + tib, nteam = (int64_t)gridDim.x * teams;
+  float w[K];
+#pragma unroll
+  for (int k = 0; k < K; ++k) w[k] = (k * T + t < m && p.w) ? p.w[(k * T + t) * 32 + lane] : 1.f;
+  const float inv_c = 1.f / (float)p.C;
+  const int64_t c0 = t * 32 + lane;
+  int par = 0;
+  for (int64_t r0 = team; r0 < p.rows; r0 += 2 * nteam, par ^= 1) {  // two rows per iteration: their loads overlap
+    float xa[K], xb[K];
+    const int64_t r1 = r0 + nteam;
+    const bool has_b = r1 < p.rows;
+    const TX* pa = reinterpret_cast<const TX*>(p.x) + r0 * p.C + c0;
+    const TX* pb = reinterpret_cast<const TX*>(p.x) + (has_b ? r1 : r0) * p.C + c0;
+#pragma unroll
+    for (int k = 0; k < K; ++k) xa[k] = k * T + t < m ? to_f32<TX>(__ldg(pa + k * T * 32)) : 0.f;
+#pragma unroll
+    for (int k = 0; k < K; ++k) xb[k] = k * T + t < m ? to_f32<TX>(__ldg(pb + k * T * 32)) : 0.f;
+    float sa = 0.f, sb = 0.f;
+#pragma unroll
+    for (int k = 0; k < K; ++k) sa += xa[k] * xa[k], sb += xb[k] * xb[k];
+    sa = team_sum<T>(warp_all_sum(sa), tsum[par][0], wib, tib);
+    sb = team_sum<T>(warp_all_sum(sb), tsum[par][1], wib, tib);
+    const float ra = rsqrtf(sa * inv_c + p.eps), rb = rsqrtf(sb * inv_c + p.eps);
+    TY* ya = reinterpret_cast<TY*>(p.y) + r0 * p.C + c0;
+    TY* yb = reinterpret_cast<TY*>(p.y) + r1 * p.C + c0;
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+      if (k * T + t < m) ya[k * T * 32] = from_f32<TY>(xa[k] * ra * w[k]);
+    if (has_b) {
+#pragma unroll
+      for (int k = 0; k < K; ++k)
+        if (k * T + t < m) yb[k * T * 32] = from_f32<TY>(xb[k] * rb * w[k]);
+    }
+    if (t == 0 && lane == 0) {
+      p.rstd[r0] = ra;
+      if (has_b) p.rstd[r1] = rb;
+    }
+  }
+}
+
+// Dynamic shared memory: (16 / T) teams x C floats <= 32 KB for every C (T = ceil(C / 512) rounded up to 1, 2, 4).
+template <typename TX, typename TY, int K, int T>
+__global__ void __launch_bounds__(512, 1) k_rmsnorm_bw_slots(const RmsP p) {
+  extern __shared__ float red[];    // [teams][C]
+  __shared__ float tsum[2][16];     // [row parity][warp]
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, t = wib % T, tib = wib / T;
+  const int teams = (blockDim.x >> 5) / T, m = p.C >> 5;
+  const int64_t team = (int64_t)blockIdx.x * teams + tib, nteam = (int64_t)gridDim.x * teams;
+  float w[K], acc[K];
+#pragma unroll
+  for (int k = 0; k < K; ++k) {
+    w[k] = (k * T + t < m && p.w) ? p.w[(k * T + t) * 32 + lane] : 1.f;
+    acc[k] = 0.f;
+  }
+  const float inv_c = 1.f / (float)p.C;
+  const int64_t c0 = t * 32 + lane;
+  int par = 0;
+  for (int64_t r = team; r < p.rows; r += nteam, par ^= 1) {
+    const TX* px = reinterpret_cast<const TX*>(p.x) + r * p.C + c0;
+    const TY* pg = reinterpret_cast<const TY*>(p.dy) + r * p.C + c0;
+    float x[K], g[K];
+#pragma unroll
+    for (int k = 0; k < K; ++k) x[k] = k * T + t < m ? to_f32<TX>(__ldg(px + k * T * 32)) : 0.f;
+#pragma unroll
+    for (int k = 0; k < K; ++k) g[k] = k * T + t < m ? to_f32<TY>(__ldg(pg + k * T * 32)) : 0.f;
+    const float rs = p.rstd[r];
+    float dot = 0.f;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      const float hx = x[k] * rs;
+      acc[k] += g[k] * hx;  // d/dw of (x rstd) * w
+      g[k] *= w[k];         // gradient w.r.t. the normalised row
+      dot += g[k] * hx;
+      x[k] = hx;
+    }
+    dot = team_sum<T>(warp_all_sum(dot), tsum[par], wib, tib) * inv_c;
+    TX* pd = reinterpret_cast<TX*>(p.dx) + r * p.C + c0;
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+      if (k * T + t < m) pd[k * T * 32] = from_f32<TX>(rs * (g[k] - x[k] * dot));
+  }
+#pragma unroll
+  for (int k = 0; k < K; ++k)
+    if (k * T + t < m) red[tib * p.C + (k * T + t) * 32 + lane] = acc[k];
+  __syncthreads();
+  for (int c = threadIdx.x; c < p.C; c += blockDim.x) {
+    float a = 0.f;
+    for (int q = 0; q < teams; ++q) a += red[q * p.C + c];
+    p.partial[(int64_t)blockIdx.x * p.C + c] = a;
+  }
+}
+
 __global__ void k_rmsnorm_reduce(const float* __restrict__ partial, int n_cta, int C, float* dw) {
   const int idx = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (idx >= C) return;
@@ -449,8 +576,8 @@ int fill(const mlstm_b200_cellout_args& a, CellP& p) {
     return MLSTM_B200_EINVAL;
   }
   const int H = a.NH * a.D;
-  if ((a.D != 32 && a.D != 64 && a.D != 128) || H % 128 != 0 || H / 128 > kMaxWarps) {
-    set_error("cellout: needs D in {32,64,128} and NH*D a multiple of 128 (got D=%d NH=%d)", a.D, a.NH);
+  if ((a.D != 32 && a.D != 64 && a.D != 128) || H > kMaxWarps * 128) {
+    set_error("cellout: needs D in {32,64,128} and NH*D <= %d (got D=%d NH=%d)", kMaxWarps * 128, a.D, a.NH);
     return MLSTM_B200_EUNSUPPORTED;
   }
   if (!a.h.ptr || a.h.stride[3] != 1) {
@@ -461,7 +588,7 @@ int fill(const mlstm_b200_cellout_args& a, CellP& p) {
     set_error("cellout: x needs a skip vector and a unit innermost stride");
     return MLSTM_B200_EINVAL;
   }
-  p.B = a.B, p.NH = a.NH, p.S = a.S, p.D = a.D, p.H = H, p.W = H / 128, p.lpg = a.D / 4;
+  p.B = a.B, p.NH = a.NH, p.S = a.S, p.D = a.D, p.H = H, p.W = (H + 127) / 128, p.lpg = a.D / 4;
   p.eps = a.eps, p.inv_d = 1.f / (float)a.D;
   p.h = a.h.ptr, p.x = a.x.ptr;
   for (int i = 0; i < 3; ++i) p.hs[i] = a.h.stride[i];
@@ -528,10 +655,18 @@ int cellout_fw(const mlstm_b200_cellout_args& a, cudaStream_t st) {
   const int grid = grid_ctas(), block = block_threads(p);
   int rc = dispatch2(a.h_dtype, a.y_dtype, [&](auto th, auto tx) {
     constexpr int kRows = (sizeof(th) + sizeof(tx)) <= 4 ? kFwRows : kFwRows / 2;
-    switch (p.lpg) {
-      case 8: k_cellout_fw<decltype(th), decltype(tx), kRows, 8><<<grid, block, 0, st>>>(p); break;
-      case 16: k_cellout_fw<decltype(th), decltype(tx), kRows, 16><<<grid, block, 0, st>>>(p); break;
-      default: k_cellout_fw<decltype(th), decltype(tx), kRows, 32><<<grid, block, 0, st>>>(p); break;
+    using TH = decltype(th);
+    using TX = decltype(tx);
+    switch (p.lpg) {  // (D = 128 rows are always whole warps)
+      case 8:
+        if (p.H % 128) k_cellout_fw<TH, TX, kRows, 8, true><<<grid, block, 0, st>>>(p);
+        else k_cellout_fw<TH, TX, kRows, 8><<<grid, block, 0, st>>>(p);
+        break;
+      case 16:
+        if (p.H % 128) k_cellout_fw<TH, TX, kRows, 16, true><<<grid, block, 0, st>>>(p);
+        else k_cellout_fw<TH, TX, kRows, 16><<<grid, block, 0, st>>>(p);
+        break;
+      default: k_cellout_fw<TH, TX, kRows, 32><<<grid, block, 0, st>>>(p); break;
     }
     return 0;
   });
@@ -582,10 +717,18 @@ int cellout_bw(const mlstm_b200_cellout_bw_args& b, cudaStream_t st) {
   const int grid = grid_ctas(), block = block_threads(p);
   int rc = dispatch2(a.h_dtype, a.y_dtype, [&](auto th, auto tx) {
     constexpr int kRows = (sizeof(th) + 2 * sizeof(tx)) <= 6 ? kBwRows : 2;  // register budget per pipeline stage
+    using TH = decltype(th);
+    using TX = decltype(tx);
     switch (p.lpg) {
-      case 8: k_cellout_bw<decltype(th), decltype(tx), kRows, 8><<<grid, block, 0, st>>>(p); break;
-      case 16: k_cellout_bw<decltype(th), decltype(tx), kRows, 16><<<grid, block, 0, st>>>(p); break;
-      default: k_cellout_bw<decltype(th), decltype(tx), kRows, 32><<<grid, block, 0, st>>>(p); break;
+      case 8:
+        if (p.H % 128) k_cellout_bw<TH, TX, kRows, 8, true><<<grid, block, 0, st>>>(p);
+        else k_cellout_bw<TH, TX, kRows, 8><<<grid, block, 0, st>>>(p);
+        break;
+      case 16:
+        if (p.H % 128) k_cellout_bw<TH, TX, kRows, 16, true><<<grid, block, 0, st>>>(p);
+        else k_cellout_bw<TH, TX, kRows, 16><<<grid, block, 0, st>>>(p);
+        break;
+      default: k_cellout_bw<TH, TX, kRows, 32><<<grid, block, 0, st>>>(p); break;
     }
     return 0;
   });
@@ -605,8 +748,8 @@ int rms_check(const mlstm_b200_rmsnorm_args& a) {
     set_error("rmsnorm: bad arguments");
     return MLSTM_B200_EINVAL;
   }
-  if (a.C != 192 && a.C != 256 && a.C != 384 && a.C != 512) {
-    set_error("rmsnorm: dim %d not covered (192, 256, 384, 512)", a.C);
+  if (a.C % 32 != 0 || a.C < 64 || a.C > 2048) {
+    set_error("rmsnorm: dim %d not covered (a multiple of 32 from 64 to 2048)", a.C);
     return MLSTM_B200_EUNSUPPORTED;
   }
   return 0;
@@ -619,15 +762,31 @@ void rms_launch(const RmsP& p, bool backward, cudaStream_t st) {
   else
     k_rmsnorm_fw<TX, TY, J><<<grid, 512, 0, st>>>(p);
 }
+template <typename TX, typename TY, int K, int T>
+void rms_launch_slots(const RmsP& p, bool backward, cudaStream_t st) {
+  const int grid = grid_ctas();
+  if (backward)
+    k_rmsnorm_bw_slots<TX, TY, K, T><<<grid, 512, (16 / T) * p.C * sizeof(float), st>>>(p);
+  else
+    k_rmsnorm_fw_slots<TX, TY, K, T><<<grid, 512, 0, st>>>(p);
+}
 template <typename TX, typename TY>
 int rms_dispatch_j(const RmsP& p, bool backward, cudaStream_t st) {
-  switch (p.C / 64) {
-    case 3: rms_launch<TX, TY, 3>(p, backward, st); return 0;
-    case 4: rms_launch<TX, TY, 4>(p, backward, st); return 0;
-    case 6: rms_launch<TX, TY, 6>(p, backward, st); return 0;
-    case 8: rms_launch<TX, TY, 8>(p, backward, st); return 0;
+  if (p.C % 64 == 0) {
+    switch (p.C / 64) {  // the model widths 192 / 256 / 384 / 512: one element pair per lane and 64 channels
+      case 3: rms_launch<TX, TY, 3>(p, backward, st); return 0;
+      case 4: rms_launch<TX, TY, 4>(p, backward, st); return 0;
+      case 6: rms_launch<TX, TY, 6>(p, backward, st); return 0;
+      case 8: rms_launch<TX, TY, 8>(p, backward, st); return 0;
+    }
   }
-  return MLSTM_B200_EUNSUPPORTED;
+  const int m = p.C / 32;  // every other width (rms_check): 32-channel slots, K per warp, T warps per row
+  if (m <= 4) rms_launch_slots<TX, TY, 4, 1>(p, backward, st);
+  else if (m <= 8) rms_launch_slots<TX, TY, 8, 1>(p, backward, st);
+  else if (m <= 16) rms_launch_slots<TX, TY, 16, 1>(p, backward, st);
+  else if (m <= 32) rms_launch_slots<TX, TY, 16, 2>(p, backward, st);
+  else rms_launch_slots<TX, TY, 16, 4>(p, backward, st);
+  return 0;
 }
 int rms_dispatch(int tx, int ty, const RmsP& p, bool backward, cudaStream_t st) {
   return dispatch2(tx, ty, [&](auto a, auto b) { return rms_dispatch_j<decltype(a), decltype(b)>(p, backward, st); });

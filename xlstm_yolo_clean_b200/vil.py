@@ -37,7 +37,14 @@ from .backend import (_DTYPES, _cell_uses_siging, _on_device, _tensor, mlstm_chu
 
 
 def cellout_supported(NH: int, D: int) -> bool:
-    return D in (32, 64, 128) and (NH * D) % 128 == 0 and NH * D <= 2048
+    """The cell-output kernels (and so the fused layer path) cover head dim ``D`` in {32, 64, 128} and any ``NH >= 1``
+    with NH * D <= 2048: every YOLO-ViL width whose ``qkv_block_size`` is one of those head dims, up to dim 1024."""
+    return D in (32, 64, 128) and NH >= 1 and NH * D <= 2048
+
+
+def rmsnorm_supported(C: int) -> bool:
+    """The fused RMSNorm covers every width ``C`` that is a multiple of 32 from 64 to 2048."""
+    return C % 32 == 0 and 64 <= C <= 2048
 
 
 # one_launch="auto" for rectangular heads, by (DHQK, DHHV, gradients wanted): True = the cell as one forward launch (the
@@ -159,9 +166,6 @@ def cell_out(h, weight=None, bias=None, skip=None, x=None, eps=1e-6, out_dtype=N
     if torch.compiler.is_compiling():
         return _ops.cellout_fw(h, weight, bias, skip, x, float(eps), out_dtype)
     return _CellOut.apply(h, weight, bias, skip, x, eps, out_dtype)
-
-
-RMSNORM_DIMS = (192, 256, 384, 512)
 
 
 def _rmsnorm_fw_call(x2, weight, eps, out_dtype):
@@ -742,8 +746,10 @@ class _GraphedLayer(_Graphed):
 def patch_layers(model: torch.nn.Module, siging=None, kernel_dtype: str = "bfloat16", one_launch: str = "auto",
                  graphs: bool = False) -> int:
     """Rebind ``mlstm_branch`` of every ViLLayer-shaped module (``proj_up``, ``qk_proj``, ``v_proj``, ``mlstm_cell``,
-    ``learnable_skip``, ``proj_down``; vision_lstm2.py:218-290) whose head geometry the fused output kernel covers to
-    ``mlstm_branch_b200``.  Parameters and state-dict keys are untouched.  Returns the number of layers rebound.
+    ``learnable_skip``, ``proj_down``; vision_lstm2.py:218-290) whose head geometry the fused output kernel covers
+    (``cellout_supported``) to ``mlstm_branch_b200``, and its RMSNorms where ``rmsnorm_supported``.  Parameters and
+    state-dict keys are untouched.  Returns the number of layers rebound; a warning names the ViLLayer-shaped modules
+    left as they are.
     ``siging=None`` keeps the gate function of each layer's cell (sigmoid input gate iff the cell's CUDA backend is
     a ``*siging*`` kernel, as in the reference model); True / False force it.
 
@@ -754,13 +760,15 @@ def patch_layers(model: torch.nn.Module, siging=None, kernel_dtype: str = "bfloa
     training forward / backward of every such layer replay as CUDA graphs (``_GraphedLayer`` bound as ``layer.forward``
     for a full ViLLayer, ``_GraphedBranch`` as ``layer.mlstm_branch`` otherwise; see ``_Graphed``)."""
     import functools
+    import warnings
 
-    n = 0
-    for mod in model.modules():
+    n, skipped = 0, []
+    for name, mod in model.named_modules():
         cell = getattr(mod, "mlstm_cell", None)
         if cell is None or not all(hasattr(mod, a) for a in ("proj_up", "qk_proj", "v_proj", "learnable_skip", "proj_down")):
             continue
         if not cellout_supported(cell.num_heads, cell.dim // cell.num_heads):
+            skipped.append(f"{name or '<root>'} (NH={cell.num_heads}, D={cell.dim // cell.num_heads})")
             continue
         sig = _cell_uses_siging(cell) if siging is None else bool(siging)
         whole_layer = graphs and all(hasattr(mod, a) for a in ("norm", "ffn_norm", "ffn", "drop_path"))
@@ -772,7 +780,10 @@ def patch_layers(model: torch.nn.Module, siging=None, kernel_dtype: str = "bfloa
             mod.forward = _GraphedLayer(mod)
         for norm in (getattr(mod, "norm", None), getattr(mod, "ffn_norm", None)):  # the RMSNorms in front of the branches
             if (isinstance(norm, torch.nn.RMSNorm) and len(norm.normalized_shape) == 1
-                    and norm.normalized_shape[0] in RMSNORM_DIMS):
+                    and rmsnorm_supported(norm.normalized_shape[0])):
                 norm.forward = functools.partial(_norm_entry, norm)
         n += 1
+    if skipped:
+        warnings.warn(f"patch_layers: {len(skipped)} ViL layer(s) left unpatched (the fused kernels need head dim 32 / 64 / "
+                      f"128 and NH * D <= 2048): {', '.join(skipped)}", stacklevel=2)
     return n
