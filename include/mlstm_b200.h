@@ -173,10 +173,11 @@ size_t mlstm_b200_workspace_bytes(const mlstm_b200_shape* shape, int backward);
 size_t mlstm_b200_states_bytes(const mlstm_b200_shape* shape);
 
 /* 1 if the tensor-core (tcgen05) kernels cover this shape/dtype forward AND backward, else 0
- * (16-bit dtypes, S % 4 == 0, and DHQK == DHHV in {32, 64, 128} or (DHQK, DHHV) in {(32, 64), (64, 128)}; the
- * head-dim-128 backward runs as four head-dim-64 block problems inside the call, a rectangular (D, 2 D) call as two
- * square head-dim-D problems on the two column halves of v / h / dh / dv).  The forward's fused cell-output epilogue
- * (mlstm_b200_fw_epilogue) is available for every shape this returns 1 for. */
+ * (16-bit dtypes, S % 4 == 0, and DHQK == DHHV in {32, 64, 128} or (DHQK, DHHV) in {(32, 64), (64, 128), (256, 512)};
+ * the head-dim-128 backward runs as four head-dim-64 block problems inside the call, a rectangular (D, 2 D) call as two
+ * square head-dim-D problems on the two column halves of v / h / dh / dv, and (256, 512) -- xLSTM-Large's heads -- as
+ * 4 x 8 head-dim-64 block problems).  The forward's fused cell-output epilogue (mlstm_b200_fw_epilogue) is available
+ * for every shape this returns 1 for except (256, 512), where it is refused with MLSTM_B200_EUNSUPPORTED. */
 int mlstm_b200_tensor_path_supported(const mlstm_b200_shape* shape);
 
 /* Forward: h, n_out, m_out and optionally the last (C, n, m) states. */

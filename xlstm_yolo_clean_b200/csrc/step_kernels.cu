@@ -31,21 +31,26 @@ struct StepParams {
   float *c1, *n1, *m1;
 };
 
-template <typename T, int DK, int DV>
+// VB > 1: column-split form, DHHV = VB * DV.  CTA x holds the DV-wide column block x % VB of C of (batch, head) x / VB
+// (v, h and C are offset by the block); n and m do not depend on v, so every block computes them and block 0 writes them.
+// (DHQK, DHHV) = (256, 512), xLSTM-Large's heads, runs as <256, 64, 8>: the 256 x 512 fp32 state does not fit one CTA's
+// registers, so each of 8 CTAs per head holds a 64-column block (4 threads per column, 64 rows each).
+template <typename T, int DK, int DV, int VB = 1>
 __global__ void __launch_bounds__(kStepThreads) k_recurrent(StepParams p) {
   constexpr int TPC = kStepThreads / DV;  // threads per column of C
   constexpr int RPT = DK / TPC;           // rows of that column per thread
-  static_assert(TPC >= 2 && TPC <= 8 && RPT >= 1, "geometry");
+  constexpr int LDC = VB * DV;            // row stride of C
+  static_assert(TPC >= 2 && TPC <= 8 && RPT >= 1 && DK <= kStepThreads, "geometry");
   __shared__ float sq[DK], sk[DK], sv[DV], sn[DK], s_red[8], s_gate[2];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int bh = blockIdx.x, b = bh / p.NH, hd = bh % p.NH;
+  const int bh = blockIdx.x / VB, vb = blockIdx.x % VB, b = bh / p.NH, hd = bh % p.NH;
   const int j = tid / TPC, rg = tid % TPC;  // column of C, row group: rows rg, rg + TPC, ...
 
   float C[RPT];
   if (p.c0) {
-    const float* src = p.c0 + (int64_t)bh * DK * DV;
+    const float* src = p.c0 + (int64_t)bh * DK * LDC + vb * DV;
 #pragma unroll
-    for (int r = 0; r < RPT; ++r) C[r] = src[(int64_t)(rg + r * TPC) * DV + j];
+    for (int r = 0; r < RPT; ++r) C[r] = src[(int64_t)(rg + r * TPC) * LDC + j];
   } else {
 #pragma unroll
     for (int r = 0; r < RPT; ++r) C[r] = 0.f;
@@ -55,10 +60,10 @@ __global__ void __launch_bounds__(kStepThreads) k_recurrent(StepParams p) {
 
   const T* qp = (const T*)p.q + b * p.q_sb + hd * p.q_sh;
   const T* kp = (const T*)p.k + b * p.k_sb + hd * p.k_sh;
-  const T* vp = (const T*)p.v + b * p.v_sb + hd * p.v_sh;
+  const T* vp = (const T*)p.v + b * p.v_sb + hd * p.v_sh + vb * DV;
   const T* ip = (const T*)p.ig + b * p.i_sb + hd * p.i_sh;
   const T* fp = (const T*)p.fg + b * p.f_sb + hd * p.f_sh;
-  T* hp = (T*)p.h + b * p.h_sb + hd * p.h_sh;
+  T* hp = (T*)p.h + b * p.h_sb + hd * p.h_sh + vb * DV;
 
   for (int t = 0; t < p.S; ++t) {
     __syncthreads();  // the previous step's readers of sq / sk / sv / s_red are done
@@ -116,18 +121,21 @@ __global__ void __launch_bounds__(kStepThreads) k_recurrent(StepParams p) {
     m = m_new;
   }
   if (p.c1) {
-    float* dst = p.c1 + (int64_t)bh * DK * DV;
+    float* dst = p.c1 + (int64_t)bh * DK * LDC + vb * DV;
 #pragma unroll
-    for (int r = 0; r < RPT; ++r) dst[(int64_t)(rg + r * TPC) * DV + j] = C[r];
+    for (int r = 0; r < RPT; ++r) dst[(int64_t)(rg + r * TPC) * LDC + j] = C[r];
     __syncthreads();
-    if (tid < DK) p.n1[(int64_t)bh * DK + tid] = sn[tid];
-    if (tid == 0) p.m1[bh] = m;
+    if (vb == 0) {
+      if (tid < DK) p.n1[(int64_t)bh * DK + tid] = sn[tid];
+      if (tid == 0) p.m1[bh] = m;
+    }
   }
 }
 
 // (DHQK, DHHV) pairs with a k_recurrent instantiation
 bool recurrent_pair_ok(int DK, int DV) {
-  return (DK == DV && (DK == 32 || DK == 64 || DK == 128)) || (DK == 32 && DV == 64) || (DK == 64 && DV == 128);
+  return (DK == DV && (DK == 32 || DK == 64 || DK == 128)) || (DK == 32 && DV == 64) || (DK == 64 && DV == 128) ||
+         (DK == 256 && DV == 512);
 }
 
 template <typename T>
@@ -139,6 +147,8 @@ int launch(const StepParams& p, int DK, int DV, cudaStream_t st) {
       case 64: k_recurrent<T, 64, 64><<<grid, kStepThreads, 0, st>>>(p); break;
       case 128: k_recurrent<T, 128, 128><<<grid, kStepThreads, 0, st>>>(p); break;
     }
+  } else if (DK == 256) {
+    k_recurrent<T, 256, 64, 8><<<8 * grid, kStepThreads, 0, st>>>(p);
   } else if (DK == 32) {
     k_recurrent<T, 32, 64><<<grid, kStepThreads, 0, st>>>(p);
   } else {
@@ -153,7 +163,8 @@ int launch(const StepParams& p, int DK, int DV, cudaStream_t st) {
 
 int recurrent_sequence(const mlstm_b200_recurrent_args& a, cudaStream_t st) {
   if (!recurrent_pair_ok(a.DHQK, a.DHHV)) {
-    set_error("recurrent kernels cover (DHQK, DHHV) = (32, 32), (64, 64), (128, 128), (32, 64) and (64, 128) (got %d, %d)",
+    set_error("recurrent kernels cover (DHQK, DHHV) = (32, 32), (64, 64), (128, 128), (32, 64), (64, 128) and (256, 512) "
+              "(got %d, %d)",
               a.DHQK, a.DHHV);
     return MLSTM_B200_EUNSUPPORTED;
   }

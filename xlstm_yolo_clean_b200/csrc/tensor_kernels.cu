@@ -1358,6 +1358,408 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
 }
 
 // =============================================================================================
+// Forward, wide heads (DHQK, DHHV) = (256, 512): xLSTM-Large's mLSTM layer (qk_dim_factor 0.5, v_dim_factor 1.0) at
+// embedding 4096 with 8 heads.  CTA x runs column block vb = x % 8 of v / h / C of (batch, head) x / 8 (the 8 CTAs of a
+// head are adjacent, so their Q / K / gate reads meet in L2); n and m do not depend on v, so every block computes them
+// and block 0 writes them.  Same algorithm and warp roles as tc_fw_d128, with these differences:
+//   * Q and K are resident as four [128][64] swizzled K-blocks (S = Q K^T and Q C have K = 256); v is one 64-wide block.
+//   * dC = (abar.K)^T V is computed as K^T (abar.V) -- abar is a per-token factor -- so the scaled operand is the 16 KB
+//     V block instead of a 64 KB copy of K: two M128 N64 K128 MMAs (dqk rows 0-127 and 128-255).  dn = K^T abar (the
+//     ones-tile MMA of tc_fw with abar in row 0 of the B tile) gives n in fp32 (two M128 N16 MMAs).
+//   * P never goes through shared memory (packed into the S columns of TMEM, as tc_fw), and h is written straight from
+//     the registers (64 bytes per thread and row), so one Q / K / V stage fits (213 KB); the next tile is pulled into
+//     L2 two tiles ahead as in tc_fw_d128.
+//   * C: every worker thread owns dqk row 128 ch + row of the 256 x 64 block, 64 fp32 registers (M128 TMEM layout).
+// The saved states go out as the four 64 x 64 blocks (qa, vb) of this CTA's column block, in the layout of
+// make_states_map_blocks with bd = 64 (rows (8 qa + vb) 64 of a tile), which the 4 x 8 block problems of the backward
+// load.  TMEM: S 128 | Hintra 64 | Hinter 64 | dC 2 x 64 | dn 2 x 16 = 416 of 512 columns.
+// =============================================================================================
+struct FwSmemWide {
+  static constexpr int DK = 256, DV = 64, VB = 8;  // DV: the column block of one CTA
+  static constexpr int kTile = LT * 128;           // one [128][64] sub-tile
+  static constexpr int oQ = 0, oK = 4 * kTile, oV = 8 * kTile;
+  static constexpr int oVb = 9 * kTile;            // abar . V
+  static constexpr int oC = 10 * kTile;            // bf16 copy of the C block: [256 dqk rows][64 dv cols]
+  static constexpr int oA = 12 * kTile;            // abar as row 0 of a K-major [16][128 tokens] B tile (rows 1-15 zero)
+  static constexpr int oSmall = oA + 4096;
+  // floats: gates[2], srs[2][2][LT], sqn[2][2][LT], sN[2][DK]
+  static constexpr int fGates = 0, fRs = 2 * GateBuf::kFloats, fQn = fRs + 4 * LT, fN = fQn + 4 * LT,
+                       kSmallFloats = fN + 2 * DK;
+  static constexpr int kBytes = oSmall + kSmallFloats * 4 + 1024;
+  static constexpr uint32_t kLoadBytes = 9 * kTile;
+  static constexpr uint32_t cS = 0, cHi = 128, cHx = 192, cDC = 256, cDN = 384;
+  static_assert(kBytes + 1024 <= 228 * 1024, "shared memory");
+};
+
+template <typename T, bool REV>
+__global__ void __launch_bounds__(kTcThreads, 1)
+tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
+           const __grid_constant__ CUtensorMap mapV, const __grid_constant__ CUtensorMap mapCs, TcFwParams p) {
+  using SM = FwSmemWide;
+  constexpr int DK = SM::DK, DV = SM::DV, VB = SM::VB;
+  constexpr bool kBf16 = std::is_same<T, __nv_bfloat16>::value;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+  float* fsm = (float*)(smem + SM::oSmall);
+  uint8_t* sQ = smem + SM::oQ;
+  uint8_t* sK = smem + SM::oK;
+  uint8_t* sV = smem + SM::oV;
+  uint8_t* sVb = smem + SM::oVb;
+  uint8_t* sC = smem + SM::oC;
+  uint8_t* sA = smem + SM::oA;
+  __shared__ uint64_t bar_full, bar_s, bar_dc, bar_h, bar_g[2], bar_n;
+  __shared__ uint32_t tmem_base_s;
+
+  const int tid = threadIdx.x, lane = tid & 31;
+  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
+  const int bh = blockIdx.x / VB, vb = blockIdx.x % VB, b = bh / p.NH, hh = bh % p.NH;
+
+  if (tid == 0) {
+    mbar_init(&bar_full, 1);
+    mbar_init(&bar_s, 1);
+    mbar_init(&bar_dc, 1);
+    mbar_init(&bar_h, 1);
+    mbar_init(&bar_g[0], 1);
+    mbar_init(&bar_g[1], 1);
+    mbar_init(&bar_n, kWorkers);
+    fence_mbar_init();
+  }
+  if (warp == kCtlWarp) {
+    tmem_alloc<512>(&tmem_base_s);
+    if (lane == 0) {
+      prefetch_tmap(&mapQ); prefetch_tmap(&mapK); prefetch_tmap(&mapV); prefetch_tmap(&mapCs);
+    }
+  }
+  const int rb = warp & 3, ch = (warp >> 2) & 1;
+  const int row = rb * 32 + lane;  // tile row == TMEM lane
+  const int drow = ch * 128 + row;  // the dqk row of C (and entry of n) this thread owns
+  const uint32_t lane_base = (uint32_t)(rb * 32) << 16;
+  float Creg[DV];                  // C[drow][64 vb .. 64 vb + 63], fp32 master copy
+#pragma unroll
+  for (int j = 0; j < DV; ++j) Creg[j] = 0.f;
+  if (warp < kCtlWarp) {
+    if (p.c0) {
+      const float* src = p.c0 + ((int64_t)bh * DK + drow) * (VB * DV) + vb * DV;
+#pragma unroll
+      for (int j = 0; j < DV; ++j) Creg[j] = src[j];
+    }
+#pragma unroll
+    for (int hf = 0; hf < 2; ++hf) {
+      float t32[32];
+#pragma unroll
+      for (int j = 0; j < 32; ++j) t32[j] = Creg[hf * 32 + j];
+      store_row32<T>(sC, drow, hf * 32, t32);
+    }
+    fsm[SM::fN + tid] = p.n0 ? p.n0[(int64_t)bh * DK + tid] : 0.f;  // kWorkers == DK
+    for (int e = tid; e < 4096 / 16; e += kWorkers) reinterpret_cast<uint4*>(sA)[e] = make_uint4(0, 0, 0, 0);
+    fence_proxy_async_smem();
+  }
+  tc_fence_before_sync();
+  __syncthreads();
+  tc_fence_after_sync();
+  const uint32_t tmem = tmem_base_s;
+  const uint32_t tS = tmem + SM::cS, tHi = tmem + SM::cHi, tHx = tmem + SM::cHx, tDC = tmem + SM::cDC, tDN = tmem + SM::cDN;
+
+  const T* ip = (const T*)p.ig + b * p.ig_sb + hh * p.ig_sh;
+  const T* fp = (const T*)p.fg + b * p.fg_sb + hh * p.fg_sh;
+  auto mt = [&](int c) { return REV ? p.NT - 1 - c : c; };
+
+  if (warp == kCtlWarp) {
+    // =========================== control warp ===================================================
+    auto load_tile = [&](int c) {
+      mbar_expect_tx(&bar_full, SM::kLoadBytes);
+#pragma unroll
+      for (int kb = 0; kb < 4; ++kb) {
+        tma_load_4d(sQ + kb * SM::kTile, &mapQ, &bar_full, kb * 64, mt(c) * LT, hh, b);
+        tma_load_4d(sK + kb * SM::kTile, &mapK, &bar_full, kb * 64, mt(c) * LT, hh, b);
+      }
+      tma_load_4d(sV, &mapV, &bar_full, vb * DV, mt(c) * LT, hh, b);
+    };
+    auto prefetch_tile = [&](int c) {
+#pragma unroll
+      for (int kb = 0; kb < 4; ++kb) {
+        tma_prefetch_4d(&mapQ, kb * 64, mt(c) * LT, hh, b);
+        tma_prefetch_4d(&mapK, kb * 64, mt(c) * LT, hh, b);
+      }
+      tma_prefetch_4d(&mapV, vb * DV, mt(c) * LT, hh, b);
+    };
+    constexpr uint32_t id_s = umma_idesc(128, 128, false, false, kBf16);  // Q K^T: A, B K-major
+    constexpr uint32_t id_hx = umma_idesc(128, DV, false, true, kBf16);   // Q C: A K-major, B MN-major
+    constexpr uint32_t id_h = umma_idesc(128, DV, false, true, kBf16);    // P V: A from TMEM, B MN-major
+    constexpr uint32_t id_dc = umma_idesc(128, DV, true, true, kBf16);    // K^T Vbar: A, B MN-major
+    constexpr uint32_t id_dn = umma_idesc(128, 16, true, false, kBf16);   // K^T abar: A MN-major, B K-major
+    const uint64_t dQ = umma_smem_desc(smem_u32(sQ), 0, 1024), dK = umma_smem_desc(smem_u32(sK), 0, 1024);
+    const uint64_t dKm = umma_smem_desc(smem_u32(sK), SM::kTile, 1024);  // K as an MN-major A (dqk 0-127; +2 tiles: 128-255)
+    const uint64_t dV = umma_smem_desc(smem_u32(sV), 0, 1024), dVb = umma_smem_desc(smem_u32(sVb), 0, 1024);
+    const uint64_t dC = umma_smem_desc(smem_u32(sC), 0, 1024);
+    const uint64_t dA = umma_smem_desc(smem_u32(sA), 0, 1024);
+    // the four 64 x 64 blocks of the state entering tile c (64 consecutive dqk rows of sC each)
+    auto store_state = [&](int c) {
+#pragma unroll
+      for (int qa = 0; qa < 4; ++qa)
+        tma_store_4d(&mapCs, sC + qa * 8192, 0, mt(c) * (4 * VB * 64) + (qa * VB + vb) * 64, hh, b);
+    };
+    if (lane == 0) {
+      if (p.store_states) {
+        store_state(0);
+        tma_store_commit();
+      }
+      load_tile(0);
+      if (p.NT > 1) prefetch_tile(1);
+    }
+    __syncwarp();
+    for (int c = 0; c < p.NT; ++c) {
+      const uint32_t par = c & 1;
+      if (lane == 0 && c + 2 < p.NT) prefetch_tile(c + 2);
+      __syncwarp();
+      if (elect_one()) {
+        mbar_wait(&bar_full, par, 1);
+        tc_fence_after_sync();
+#pragma unroll
+        for (int kk = 0; kk < DK / 16; ++kk)  // S = Q K^T
+          umma_f16(tS, umma_desc_advance(dQ, (kk / 4) * SM::kTile + (kk % 4) * 32),
+                   umma_desc_advance(dK, (kk / 4) * SM::kTile + (kk % 4) * 32), id_s, kk > 0);
+        umma_commit(&bar_s);
+#pragma unroll
+        for (int kk = 0; kk < DK / 16; ++kk)  // Hinter = Q C_{k-1} (sC was written before the previous NB_C)
+          umma_f16(tHx, umma_desc_advance(dQ, (kk / 4) * SM::kTile + (kk % 4) * 32), umma_desc_advance(dC, kk * 2048), id_hx,
+                   kk > 0);
+      }
+      __syncwarp();
+      named_sync(NB_B, kNbAB);  // P(c) written
+      // the store of the state entering tile c has read sC before the workers rewrite it (after bar_dc below)
+      if (lane == 0) tma_store_wait_read<0>();
+      __syncwarp();
+      if (elect_one()) {
+        tc_fence_after_sync();
+#pragma unroll
+        for (int kk = 0; kk < LT / 16; ++kk)  // Hintra = P V, A = P from TMEM (packed inside the S columns)
+          umma_f16_ts(tHi, tS + 32 * (kk / 2) + 8 * (kk % 2), umma_desc_advance(dV, kk * 2048), id_h, kk > 0);
+        umma_commit(&bar_h);  // also covers Hinter
+      }
+      __syncwarp();
+      named_sync(NB_A, kNbAB);  // Vbar(c) and abar(c) written
+      if (elect_one()) {
+#pragma unroll
+        for (int hq = 0; hq < 2; ++hq) {
+#pragma unroll
+          for (int kk = 0; kk < LT / 16; ++kk)  // dC = K^T Vbar, dqk rows 128 hq ..
+            umma_f16(tDC + hq * DV, umma_desc_advance(dKm, 2 * hq * SM::kTile + kk * 2048), umma_desc_advance(dVb, kk * 2048),
+                     id_dc, kk > 0);
+#pragma unroll
+          for (int kk = 0; kk < LT / 16; ++kk)  // dn = K^T abar
+            umma_f16(tDN + hq * 16, umma_desc_advance(dKm, 2 * hq * SM::kTile + kk * 2048),
+                     umma_desc_advance(dA, (kk / 4) * 2048 + (kk % 4) * 32), id_dn, kk > 0);
+        }
+        umma_commit(&bar_dc);
+        mbar_wait(&bar_h, par, 8);  // every MMA of this tile has read Q / K / V: refill the single stage
+        mbar_wait(&bar_dc, par, 9);
+        if (c + 1 < p.NT) load_tile(c + 1);
+      }
+      __syncwarp();
+      named_sync(NB_C, kNbC);  // h written, C_k written
+      if (lane == 0 && p.store_states && c + 1 < p.NT) {
+        store_state(c + 1);  // C_k = state entering tile c+1
+        tma_store_commit();
+      }
+      __syncwarp();
+    }
+    if (lane == 0) tma_store_wait_all<0>();
+  } else if (warp == kScanWarp) {
+    // =========================== scan warp: gate vectors two tiles ahead ===========================
+    auto raw_of = [&](int c) {
+      const int t1 = mt(c) * LT;
+      return load_gate_raw<T>(ip + (int64_t)t1 * p.ig_ss, p.ig_ss, fp + (int64_t)t1 * p.fg_ss, p.fg_ss, min(LT, p.S - t1));
+    };
+    GateRaw<T> raw = raw_of(0);
+    for (int n = 0; n < p.NT; ++n) {
+      if (n >= 2) named_sync(NB_C, kNbC);
+      gate_scan_regs(fsm + SM::fGates + (n & 1) * GateBuf::kFloats, raw, REV, p.sig != 0, p.cap);
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bar_g[n & 1]);
+      if (n + 1 < p.NT) raw = raw_of(n + 1);
+    }
+    for (int n = max(p.NT - 2, 0); n < p.NT; ++n) named_sync(NB_C, kNbC);
+  } else {
+    // =========================== worker warps ===================================================
+    float m_run = p.m0 ? p.m0[bh] : 0.f;
+    int cur = 0;
+    T* hbase = (T*)p.h_plain + b * p.h_sb + hh * p.h_sh + vb * DV + ch * 32;
+    for (int c = 0; c < p.NT; ++c) {
+      const int pb = c & 1;
+      const uint32_t par = c & 1;
+      const float* gb = fsm + SM::fGates + pb * GateBuf::kFloats;
+      float* srs = fsm + SM::fRs + pb * 2 * LT;
+      float* sqn = fsm + SM::fQn + pb * 2 * LT;
+      const float* sNc = fsm + SM::fN + cur * DK;
+      float* sNn = fsm + SM::fN + (cur ^ 1) * DK;
+      const int t0 = mt(c) * LT;
+      const int n_valid = min(LT, p.S - t0);
+
+      mbar_wait(&bar_g[pb], (c >> 1) & 1, 2);
+      const float g = gb[GateBuf::oScal], amax = gb[GateBuf::oScal + 1];
+      const float m_next = p.sig ? 0.f : fmaxf(g + m_run, g + amax);    // fw.py:96-98
+      const float gbar = __expf(g + m_run - m_next);                    // fw.py:106
+      const float b_t = gb[GateBuf::oB + row], i_t = gb[GateBuf::oI + row];
+      const float m_t = p.sig ? 0.f : b_t + fmaxf(m_run, gb[GateBuf::oPm + row]);  // fw.py:178-184
+      mbar_wait(&bar_full, par, 3);
+      if (c > 0) mbar_wait(&bar_n, (c - 1) & 1, 4);
+      {  // partial q . n_{k-1} over this thread's 128 dqk columns (K-blocks 2 ch, 2 ch + 1)
+        float qn = 0.f;
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf) {
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            uint4 q = *reinterpret_cast<const uint4*>(sQ + (2 * ch + hf) * SM::kTile + swz128(row, 8 * j));
+            float2 q0 = unpack2<T>(q.x), q1 = unpack2<T>(q.y), q2 = unpack2<T>(q.z), q3 = unpack2<T>(q.w);
+            const float* nn = sNc + ch * 128 + hf * 64 + 8 * j;
+            const float4 n0 = *reinterpret_cast<const float4*>(nn);
+            const float4 n1 = *reinterpret_cast<const float4*>(nn + 4);
+            qn += q0.x * n0.x + q0.y * n0.y + q1.x * n0.z + q1.y * n0.w + q2.x * n1.x + q2.y * n1.y + q3.x * n1.z + q3.y * n1.w;
+          }
+        }
+        sqn[ch * LT + row] = qn;
+      }
+      // ---- P = S . D (causal), row sums, packed into the S columns (as tc_fw) ------------------------
+      mbar_wait(&bar_s, par, 5);
+      tc_fence_after_sync();
+      {
+        const float x_t = (b_t - m_t) * kLog2e + log2f(p.scale);
+        const float* sy = gb + GateBuf::oY;
+        const float* scf = gb + GateBuf::oCf;
+        float rs = 0.f;
+#pragma unroll 1
+        for (int u = ch; u < 4; u += 2) {
+          float v[32];
+          const bool off_diag = REV ? u > rb : u < rb;
+          if (off_diag) {
+            tmem_ld32(tS + lane_base + u * 32, v);
+            const float r_t = ex2_approx(x_t + gb[GateBuf::oScal + 4 + u]);
+#pragma unroll
+            for (int j4 = 0; j4 < 8; ++j4) {
+              const float4 cf = *reinterpret_cast<const float4*>(scf + u * 32 + 4 * j4);
+              v[4 * j4 + 0] *= cf.x * r_t;
+              v[4 * j4 + 1] *= cf.y * r_t;
+              v[4 * j4 + 2] *= cf.z * r_t;
+              v[4 * j4 + 3] *= cf.w * r_t;
+              rs += (v[4 * j4 + 0] + v[4 * j4 + 1]) + (v[4 * j4 + 2] + v[4 * j4 + 3]);
+            }
+          } else if (u == rb) {
+            tmem_ld32(tS + lane_base + u * 32, v);
+#pragma unroll
+            for (int j4 = 0; j4 < 8; ++j4) {
+              const float4 y = *reinterpret_cast<const float4*>(sy + u * 32 + 4 * j4);
+              const float yy[4] = {y.x, y.y, y.z, y.w};
+#pragma unroll
+              for (int e = 0; e < 4; ++e) {
+                const int j = 4 * j4 + e;
+                float pv = v[j] * ex2_approx(x_t + yy[e]);
+                pv = (REV ? j >= lane : j <= lane) ? pv : 0.f;
+                rs += pv;
+                v[j] = pv;
+              }
+            }
+          } else {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] = 0.f;
+          }
+          uint32_t pk[16];
+#pragma unroll
+          for (int j = 0; j < 16; ++j) pk[j] = pack2<T>(v[2 * j], v[2 * j + 1]);
+          tmem_st16(tS + lane_base + u * 32, pk);
+        }
+        srs[ch * LT + row] = rs;
+      }
+      tmem_st_wait();
+      tc_fence_before_sync();
+      named_arrive(NB_B, kNbAB);
+      {  // Vbar = abar . V (row, 32 columns); abar into row 0 of the dn operand
+        const float ab = __expf(g - b_t + i_t - m_next);  // fw.py:102 (exp(-inf) = 0 for tail tokens)
+        float vb32[32];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          uint4 u = *reinterpret_cast<const uint4*>(sV + swz128(row, ch * 32 + 8 * j));
+          float2 a0 = unpack2<T>(u.x), a1 = unpack2<T>(u.y), a2 = unpack2<T>(u.z), a3 = unpack2<T>(u.w);
+          vb32[8 * j + 0] = a0.x * ab; vb32[8 * j + 1] = a0.y * ab; vb32[8 * j + 2] = a1.x * ab; vb32[8 * j + 3] = a1.y * ab;
+          vb32[8 * j + 4] = a2.x * ab; vb32[8 * j + 5] = a2.y * ab; vb32[8 * j + 6] = a3.x * ab; vb32[8 * j + 7] = a3.y * ab;
+        }
+        store_cols<T, 64>(sVb, row, ch * 32, vb32);
+        if (ch == 0) *reinterpret_cast<T*>(sA + (row >> 6) * 2048 + swz128(0, row & 63)) = from_f32<T>(ab);
+        fence_proxy_async_smem();
+        named_arrive(NB_A, kNbAB);
+      }
+      // ---- epilogue: h (row, 32 columns) straight to global memory -------------------------------------
+      mbar_wait(&bar_h, par, 7);
+      tc_fence_after_sync();
+      {
+        uint32_t hi[32], hx[32];
+        tmem_ld32_nowait(tHi + lane_base + ch * 32, hi);
+        tmem_ld32_nowait(tHx + lane_base + ch * 32, hx);
+        const float bq = __expf(b_t + m_run - m_t) * p.scale;                          // fw.py:197-198
+        const float den = bq * (sqn[row] + sqn[LT + row]) + srs[row] + srs[LT + row];  // fw.py:204-206
+        const float nmax = fmaxf(fabsf(den), __expf(-m_t));                            // fw.py:208-210
+        const float inv = p.sig == 2 ? 1.f : 1.f / (nmax + p.eps);  // siging = 2: no normaliser
+        tmem_ld_wait();
+        if (row < n_valid) {
+          uint4* dst = reinterpret_cast<uint4*>(hbase + (int64_t)(t0 + row) * p.h_ss);
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            float o[8];
+#pragma unroll
+            for (int e = 0; e < 8; ++e) o[e] = (__uint_as_float(hi[8 * j + e]) + bq * __uint_as_float(hx[8 * j + e])) * inv;
+            uint4 u;
+            u.x = pack2<T>(o[0], o[1]);
+            u.y = pack2<T>(o[2], o[3]);
+            u.z = pack2<T>(o[4], o[5]);
+            u.w = pack2<T>(o[6], o[7]);
+            dst[j] = u;
+          }
+          if (ch == 0 && vb == 0) {
+            p.n_out[(int64_t)bh * p.S + t0 + row] = nmax;
+            p.m_out[(int64_t)bh * p.S + t0 + row] = m_t;
+          }
+        }
+      }
+      // ---- state update C_k = gbar C_{k-1} + dC (M128 layout: lane == dqk row within the half); n_k -------
+      mbar_wait(&bar_dc, par, 6);
+      tc_fence_after_sync();
+      {
+        uint32_t dn_u;
+        tmem_ld1_nowait(tDN + ch * 16 + lane_base, dn_u);
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf) {
+          float v[32], t32[32];
+          tmem_ld32(tDC + ch * DV + lane_base + hf * 32, v);  // (waits for dn_u too)
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            Creg[hf * 32 + j] = gbar * Creg[hf * 32 + j] + v[j];
+            t32[j] = Creg[hf * 32 + j];
+          }
+          store_row32<T>(sC, drow, hf * 32, t32);  // Q C_{k-1} (bar_h) has finished reading the old copy
+        }
+        sNn[drow] = gbar * sNc[drow] + __uint_as_float(dn_u);  // n_k = gbar n_{k-1} + K^T abar (fw.py:116)
+        mbar_arrive(&bar_n);
+      }
+      fence_proxy_async_smem();
+      tc_fence_before_sync();
+      named_arrive(NB_C, kNbC);
+      m_run = m_next;
+      cur ^= 1;
+    }
+    if (p.c_last) {  // final states (fw.py:302-309)
+      float* dst = p.c_last + ((int64_t)bh * DK + drow) * (VB * DV) + vb * DV;
+#pragma unroll
+      for (int j = 0; j < DV; ++j) dst[j] = Creg[j];
+      if (vb == 0) p.n_last[(int64_t)bh * DK + drow] = fsm[SM::fN + cur * DK + drow];  // this thread's own entry
+      if (tid == 0 && vb == 0) p.m_last[bh] = m_run;
+    }
+  }
+  tc_fence_before_sync();
+  __syncthreads();
+  if (warp == kCtlWarp) tmem_dealloc<512>(tmem);
+}
+
+// =============================================================================================
 // Backward: one reverse sweep per (batch, head) over 128-token tiles (reference native/bw.py).
 // dC lives on chip (fp32 registers + bf16 operand copy); C_{k-1} comes from the forward's
 // c_states.  n_out and every max state are constants (bw.py:44-47).  Per tile:
@@ -2120,6 +2522,17 @@ int launch_fw_d128(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap
   return 0;
 }
 
+template <typename T>
+int launch_fw_wide(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
+                   const CUtensorMap& mcs, cudaStream_t st) {
+  auto kern = p.rev ? tc_fw_wide<T, true> : tc_fw_wide<T, false>;
+  MLSTM_CUDA_CHECK(ensure_smem(kern, FwSmemWide::kBytes));
+  kern<<<FwSmemWide::VB * p.B * p.NH, kTcThreads, FwSmemWide::kBytes, st>>>(mq, mk, mv, mcs, p);
+  count_launch();
+  MLSTM_CUDA_CHECK(cudaGetLastError());
+  return 0;
+}
+
 template <typename T, int D, typename TO = T>
 int launch_bw(const TcBwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
               const CUtensorMap& mdh, const CUtensorMap& mcs, const CUtensorMap& mdq, const CUtensorMap& mdk,
@@ -2159,9 +2572,49 @@ int make_states_map_blocks(CUtensorMap* m, const void* ptr, const mlstm_b200_sha
                                    (int64_t)NT * rows * bd, bd, bd, bd);
 }
 bool rect_heads(const mlstm_b200_shape& s) { return s.DHQK != s.DHHV; }
+bool wide_heads(const mlstm_b200_shape& s) { return s.DHQK == 256 && s.DHHV == 512; }
+
+// (256, 512): tc_fw_wide, eight 64-wide column blocks of v / h / C per head; h is written from the registers
+int run_fw_wide(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
+  const mlstm_b200_shape& s = a.shape;
+  if (a.epilogue) {
+    set_error("the fused cell-output epilogue does not cover (DHQK, DHHV) = (256, 512)");
+    return MLSTM_B200_EUNSUPPORTED;
+  }
+  if (!tma_ok(a.q) || !tma_ok(a.k) || !tma_ok(a.v) || !tma_ok(a.h)) {
+    set_error("tensor path needs 16-byte aligned q/k/v/h with strides that are multiples of 8 elements");
+    return MLSTM_B200_EUNSUPPORTED;
+  }
+  CUtensorMap mq, mk, mv, mcs;
+  int r = make_map(&mq, a.q, s, s.DHQK) | make_map(&mk, a.k, s, s.DHQK) | make_map(&mv, a.v, s, s.DHHV, 64);
+  // without a c_states buffer the map is never used by the kernel; point it at v to keep it valid
+  r |= c_states ? make_states_map_blocks(&mcs, c_states, s, (s.DHQK / 64) * s.DHHV, 64) : make_map(&mcs, a.v, s, s.DHHV, 64);
+  if (r) {
+    set_error("cuTensorMapEncodeTiled failed (%d)", r);
+    return MLSTM_B200_ENODEVICE;
+  }
+  TcFwParams p{};
+  p.B = s.B; p.NH = s.NH; p.S = s.S; p.NT = (s.S + LT - 1) / LT;
+  p.eps = s.eps;
+  p.scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf((float)s.DHQK);
+  p.ig = a.i.ptr; p.ig_sb = a.i.stride[0]; p.ig_sh = a.i.stride[1]; p.ig_ss = a.i.stride[2];
+  p.fg = a.f.ptr; p.fg_sb = a.f.stride[0]; p.fg_sh = a.f.stride[1]; p.fg_ss = a.f.stride[2];
+  p.c0 = a.c_initial; p.n0 = a.n_initial; p.m0 = a.m_initial;
+  p.n_out = a.n_out; p.m_out = a.m_out;
+  p.c_last = a.c_last; p.n_last = a.n_last; p.m_last = a.m_last;
+  p.rev = s.reverse ? 1 : 0;
+  p.sig = s.siging;
+  p.store_states = c_states != nullptr;
+  p.cap = s.gate_soft_cap;
+  p.h_plain = a.h.ptr; p.h_sb = a.h.stride[0]; p.h_sh = a.h.stride[1]; p.h_ss = a.h.stride[2];  // h, stored by the workers
+  TC_SET_PROF(p, 0);
+  return s.dtype == MLSTM_B200_BF16 ? launch_fw_wide<__nv_bfloat16>(p, mq, mk, mv, mcs, st)
+                                    : launch_fw_wide<__half>(p, mq, mk, mv, mcs, st);
+}
 
 int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   const mlstm_b200_shape& s = a.shape;
+  if (wide_heads(s)) return run_fw_wide(a, c_states, st);
   const mlstm_b200_fw_epilogue* ep = a.epilogue;
   // with the fused epilogue the tensor map describes y (the un-normalised h, if wanted, is stored from registers)
   const mlstm_b200_tensor& out = ep ? ep->y : a.h;
@@ -2261,7 +2714,8 @@ BwWs bw_ws(const mlstm_b200_shape& s) {
 // (DHQK / bd) x (DHHV / bd) tc_bw<bd> problems on strided views of the same tensors (no copies of q/k/v/dh;
 // qk_scale = DHQK^-1/2 of the whole problem; each loads its block of the forward's saved states or recomputes it,
 // bw.py:251-266).  Head dim 128: bd = 64, a 2 x 2 grid (a 128-wide tile set does not fit the backward's shared memory
-// with 128-token tiles).  Rectangular heads (D, 2 D): bd = D, a 1 x 2 grid.  The first partial of every output block
+// with 128-token tiles).  Rectangular heads (D, 2 D): bd = D, a 1 x 2 grid.  Wide heads (256, 512): bd = 64, a 4 x 8
+// grid (dq / dk then take 8 partials, dv 4, di / df 32).  The first partial of every output block
 // is written in place, the second is added by the kernel that produces it (TMA reduce-add stores).
 // bd x bd block (a, b) of a (BH, DK, DV) fp32 state <-> contiguous (BH, bd, bd); vec: (BH, DK) <-> (BH, bd)
 __global__ void k_state_block(float* __restrict__ blk, float* __restrict__ full, int a, int b, int bd, int DK, int DV,
@@ -2278,6 +2732,20 @@ __global__ void k_state_vec_block(float* __restrict__ blk, const float* __restri
   if (idx >= n) return;
   blk[idx] = full[(idx / bd) * DK + a * bd + idx % bd];
 }
+// Wide heads: di / df as the fp32 sum of the block problems' partials (part: [2][nparts][B NH S], di then df), rounded once
+template <typename TO>
+__global__ void k_sum_gate_partials(const TO* __restrict__ part, int nparts, int64_t n, int NH, int S, TO* di, int64_t di_sb,
+                                    int64_t di_sh, int64_t di_ss, TO* df, int64_t df_sb, int64_t df_sh, int64_t df_ss) {
+  const int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (idx >= 2 * n) return;
+  const int which = (int)(idx / n);
+  const int64_t e = idx % n, bh = e / S, t = e % S, b = bh / NH, h = bh % NH;
+  const TO* src = part + (int64_t)which * nparts * n + e;
+  float acc = 0.f;
+  for (int j = 0; j < nparts; ++j) acc += to_f32<TO>(src[(int64_t)j * n]);
+  if (which == 0) di[b * di_sb + h * di_sh + t * di_ss] = from_f32<TO>(acc);
+  else df[b * df_sb + h * df_sh + t * df_ss] = from_f32<TO>(acc);
+}
 
 }  // namespace
 int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, int nblocks, cudaStream_t st, int acc_qk = 0,
@@ -2286,7 +2754,7 @@ int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int b
                      int acc_v, int acc_g);
 namespace {
 
-int block_dim(const mlstm_b200_shape& s) { return s.DHQK == 128 ? 64 : s.DHQK; }
+int block_dim(const mlstm_b200_shape& s) { return s.DHQK >= 128 ? 64 : s.DHQK; }
 mlstm_b200_shape block_shape(const mlstm_b200_shape& s) {
   mlstm_b200_shape b = s;
   b.DHQK = b.DHHV = block_dim(s);
@@ -2294,7 +2762,7 @@ mlstm_b200_shape block_shape(const mlstm_b200_shape& s) {
   return b;
 }
 struct BlocksWs {
-  size_t off_sub, sub_bytes, off_c0, off_n0, off_dcl, off_dc0, total;
+  size_t off_sub, sub_bytes, off_c0, off_n0, off_dcl, off_dc0, off_g, total;
 };
 BlocksWs blocks_ws(const mlstm_b200_shape& s) {
   BlocksWs w{};
@@ -2306,6 +2774,10 @@ BlocksWs blocks_ws(const mlstm_b200_shape& s) {
   w.off_n0 = o; o += align_up(bh * bd * 4, 256);
   w.off_dcl = o; o += align_up(bh * bd * bd * 4, 256);
   w.off_dc0 = o; o += align_up(bh * bd * bd * 4, 256);
+  // wide heads: the 16-bit di / df partial of every block problem, summed in fp32 by k_sum_gate_partials (the in-kernel
+  // accumulation would round the running sum to 16 bits 31 times)
+  w.off_g = o;
+  if (wide_heads(s)) o += align_up(2 * (size_t)(s.DHQK / bd) * (s.DHHV / bd) * bh * s.S * 2, 256);
   w.total = o;
   return w;
 }
@@ -2332,12 +2804,20 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
   };
   int launches = 0;
   bool first = true;
+  const bool gate_parts = wide_heads(s);
+  const int64_t ntok = bh * s.S;
+  auto gate_part = [&](int which, int j) {  // (B, NH, S) view of partial j of di (which = 0) or df (1)
+    mlstm_b200_tensor t{};
+    t.ptr = ws + w.off_g + ((size_t)which * nq * nv + j) * ntok * 2;
+    t.stride[0] = (int64_t)s.NH * s.S; t.stride[1] = s.S; t.stride[2] = 1; t.stride[3] = 1;
+    return t;
+  };
   for (int qa = 0; qa < nq; ++qa) {
     for (int vb = 0; vb < nv; ++vb) {
       mlstm_b200_bw_args sub = a;
       sub.shape = block_shape(s);
       sub.q = cols(a.q, qa); sub.k = cols(a.k, qa); sub.v = cols(a.v, vb); sub.dh = cols(a.dh, vb);
-      // With the forward's saved states (tc_fw_d128 / tc_fw_rect store them block-wise) every problem loads its
+      // With the forward's saved states (tc_fw_d128 / tc_fw_rect / tc_fw_wide store them block-wise) every problem loads its
       // block; without them it recomputes its slice.
       const bool saved = a.c_states != nullptr;
       sub.c_states = nullptr;
@@ -2363,10 +2843,10 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
       sub.dq = cols(a.dq, qa);
       sub.dk = cols(a.dk, qa);
       sub.dv = cols(a.dv, vb);
-      sub.di = a.di;
-      sub.df = a.df;
+      sub.di = gate_parts ? gate_part(0, qa * nv + vb) : a.di;
+      sub.df = gate_parts ? gate_part(1, qa * nv + vb) : a.df;
       if (int e = tensor_bw_blocks(sub, saved ? a.c_states : nullptr, saved ? qa * nv + vb : -1, nq * nv, st, vb > 0, qa > 0,
-                                   !first))
+                                   !first && !gate_parts))
         return e;
       if (a.dc_initial) {
         state_block(w.off_dc0, a.dc_initial, qa, vb, 1);
@@ -2374,6 +2854,19 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
       }
       first = false;
     }
+  }
+  if (gate_parts) {
+    const int gdt = s.grad_dtype ? s.grad_dtype : s.dtype;
+    const unsigned grid = (unsigned)((2 * ntok + 255) / 256);
+    if (gdt == MLSTM_B200_BF16)
+      k_sum_gate_partials<__nv_bfloat16><<<grid, 256, 0, st>>>(
+          (const __nv_bfloat16*)(ws + w.off_g), nq * nv, ntok, s.NH, s.S, (__nv_bfloat16*)a.di.ptr, a.di.stride[0],
+          a.di.stride[1], a.di.stride[2], (__nv_bfloat16*)a.df.ptr, a.df.stride[0], a.df.stride[1], a.df.stride[2]);
+    else
+      k_sum_gate_partials<__half><<<grid, 256, 0, st>>>((const __half*)(ws + w.off_g), nq * nv, ntok, s.NH, s.S,
+                                                        (__half*)a.di.ptr, a.di.stride[0], a.di.stride[1], a.di.stride[2],
+                                                        (__half*)a.df.ptr, a.df.stride[0], a.df.stride[1], a.df.stride[2]);
+    ++launches;
   }
   MLSTM_CUDA_CHECK(cudaGetLastError());
   count_launch(launches);  // the block problems counted their own launches
@@ -2401,9 +2894,11 @@ bool tensor_context_is_current() { return sm100_host::context_is_current(); }
 
 // forward: d = 32, 64 and 128; backward: d = 32 and 64 natively, d = 128 as four d = 64 block problems (bw_by_blocks).
 // Rectangular heads (DHQK, DHHV) = (32, 64) and (64, 128): the forward as two square column-block problems in one launch
-// (tc_fw_rect), the backward as two tc_bw<DHQK> block problems.
+// (tc_fw_rect), the backward as two tc_bw<DHQK> block problems.  Wide heads (256, 512) (xLSTM-Large): the forward as eight
+// 64-wide column blocks in one launch (tc_fw_wide), the backward as 4 x 8 tc_bw<64> block problems.
 bool tensor_supported(const mlstm_b200_shape& s, int backward) {
   if (s.dtype != MLSTM_B200_BF16 && s.dtype != MLSTM_B200_F16) return false;
+  if (wide_heads(s)) return s.S % 4 == 0;
   if (s.DHQK != s.DHHV && !((s.DHQK == 32 || s.DHQK == 64) && s.DHHV == 2 * s.DHQK)) return false;
   if (s.DHQK != 64 && s.DHQK != 32 && s.DHQK != 128) return false;  // d = 128 backward: four d = 64 block problems
   // Tiles are 128 tokens whatever chunk_size is (h and the states do not depend on it: the stabiliser equals the
@@ -2431,7 +2926,7 @@ int tensor_fw(const mlstm_b200_fw_args& a, cudaStream_t st) { return run_fw(a, a
 // cudaOccupancyMaxActiveClusters of the rectangular forward with the fused epilogue ({2, 1, 1} clusters) on the current
 // device; 0 for a shape that does not launch it, -1 on a CUDA error
 int tensor_fw_epilogue_clusters(const mlstm_b200_shape& s) {
-  if (!tensor_supported(s, 0) || !rect_heads(s)) return 0;
+  if (!tensor_supported(s, 0) || !rect_heads(s) || wide_heads(s)) return 0;
   auto query = [&](auto kern, int smem) {
     if (ensure_smem(kern, smem) != cudaSuccess) return -1;
     cudaLaunchConfig_t cfg = {};

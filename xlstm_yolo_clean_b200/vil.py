@@ -247,7 +247,8 @@ def rms_norm_b200(x, weight=None, eps=1e-6, out_dtype=None):
     return _RmsNorm.apply(x, weight, eps, out_dtype)
 
 
-TENSOR_HEAD_DIMS = ((32, 32), (64, 64), (128, 128), (32, 64), (64, 128))  # (DHQK, DHHV) of the tensor-core kernels
+TENSOR_HEAD_DIMS = ((32, 32), (64, 64), (128, 128), (32, 64), (64, 128), (256, 512))  # (DHQK, DHHV) of the tensor-core kernels
+NO_EPILOGUE_HEAD_DIMS = ((256, 512),)  # tensor-core head dims whose forward has no fused cell-output epilogue
 
 
 def _head_dims(qk, v, NH):
@@ -511,6 +512,7 @@ def mlstm_cell_b200(cell, q, k, v, reverse=False, skip=None, x_skip=None, siging
             auto_fuse = RECT_ONE_LAUNCH.get((DK, D, needs_grad), False)
         fuse = one_launch == "always" or (one_launch == "auto" and auto_fuse)
         if (fuse and in_kernel_cap and S % 4 == 0 and out_dtype in (torch.float16, torch.bfloat16)
+                and (DK, D) not in NO_EPILOGUE_HEAD_DIMS
                 and cellout_supported(NH, D) and (x_skip is None or x_skip.shape == (B, S, H))):
             return _cell_fused(qk_c, v_c, g_c, x_skip, norm.weight_proxy, norm.bias, skip, NH, bool(reverse), bool(siging),
                                int(chunk_size), float(eps), kdt, float(cell.gate_soft_cap), float(norm.eps), out_dtype)
