@@ -478,6 +478,135 @@ struct FwSmem {
   static_assert(cDN + 8 <= kTmemCols, "TMEM budget");
 };
 
+// ---------------------------------------------------------------------------------------------
+// Stages shared by the three forward kernels (tc_fw_body, tc_fw_d128, tc_fw_wide)
+// ---------------------------------------------------------------------------------------------
+
+// Scan warp: the gate vectors of tile n go into buffer n & 1 of `gates` two tiles ahead of the workers, announced on
+// bar_g[n & 1]; tiles 0 and 1 need no buffer hand-back, tile n >= 2 waits until every worker is done with tile n - 2.
+// X_ROW_BYTES > 0 (fused epilogue): the skip-input rows of tile n (xbase, p.x_ss elements apart) are pulled into L2
+// two tiles before the workers read them.
+template <bool REV, int X_ROW_BYTES, typename T, typename MT>
+__device__ __forceinline__ void fw_scan_warp(const TcFwParams& p, const T* ip, const T* fp, MT mt, float* gates,
+                                             uint64_t* bar_g, const uint16_t* xbase) {
+  const int lane = threadIdx.x & 31;
+  auto raw_of = [&](int c) {
+    const int t1 = mt(c) * LT;
+    return load_gate_raw<T>(ip + (int64_t)t1 * p.ig_ss, p.ig_ss, fp + (int64_t)t1 * p.fg_ss, p.fg_ss, min(LT, p.S - t1));
+  };
+  GateRaw<T> raw = raw_of(0);
+  for (int n = 0; n < p.NT; ++n) {
+    if constexpr (X_ROW_BYTES > 0) {
+      if (p.x) prefetch_rows_l2<X_ROW_BYTES>(xbase, p.x_ss, mt(n) * LT, min(LT, p.S - mt(n) * LT), lane);
+    }
+    if (n >= 2) named_sync(NB_C, kNbC);  // every worker is done with tile n-2: its gate buffer can be reused
+    gate_scan_regs(gates + (n & 1) * GateBuf::kFloats, raw, REV, p.sig != 0, p.cap);
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&bar_g[n & 1]);
+    if (n + 1 < p.NT) raw = raw_of(n + 1);  // stays in flight until the next hand-back
+  }
+  for (int n = max(p.NT - 2, 0); n < p.NT; ++n) named_sync(NB_C, kNbC);  // match the workers' remaining arrivals
+}
+
+// Gate scalars of one tile for tile row `row`: g = b_L, the stabilisers m_next (end of the tile) and m_t (this row), the
+// state decay gbar, and the row's b_t and i_t.  sig != 0: every max state is 0.
+struct TileGates {
+  float g, m_next, gbar, b_t, i_t, m_t;
+};
+__device__ __forceinline__ TileGates tile_gates(const float* gb, int row, float m_run, int sig) {
+  const float g = gb[GateBuf::oScal], amax = gb[GateBuf::oScal + 1];
+  const float m_next = sig ? 0.f : fmaxf(g + m_run, g + amax);    // fw.py:96-98
+  const float gbar = __expf(g + m_run - m_next);                    // fw.py:106
+  const float b_t = gb[GateBuf::oB + row], i_t = gb[GateBuf::oI + row];
+  const float m_t = sig ? 0.f : b_t + fmaxf(m_run, gb[GateBuf::oPm + row]);  // fw.py:178-184
+  return {g, m_next, gbar, b_t, i_t, m_t};
+}
+
+// P = S . D (causal) of tile row rb * 32 + lane over this thread's two 32-column units u = ch, ch + 2 (warp-uniform
+// branches).  S is read from TMEM at tS_row (this row's lane, column 0).  sink(u, v) stores each finished unit; returns
+// the row sum of P over both units.  Called by tc_fw_d128 and tc_fw_wide; tc_fw_body writes the same loop out (see there).
+template <bool REV, typename Sink>
+__device__ __forceinline__ float causal_p(uint32_t tS_row, const float* gb, float b_t, float m_t, float scale, int rb, int ch,
+                                          int lane, Sink sink) {
+  const float x_t = (b_t - m_t) * kLog2e + log2f(scale);
+  const float* sy = gb + GateBuf::oY;
+  const float* scf = gb + GateBuf::oCf;
+  float rs = 0.f;
+#pragma unroll 1
+  for (int u = ch; u < 4; u += 2) {
+    float v[32];
+    const bool off_diag = REV ? u > rb : u < rb;  // fully unmasked 32x32 block
+    if (off_diag) {  // rank-1 decay, one exp per row
+      tmem_ld32(tS_row + u * 32, v);
+      const float r_t = ex2_approx(x_t + gb[GateBuf::oScal + 4 + u]);
+#pragma unroll
+      for (int j4 = 0; j4 < 8; ++j4) {
+        const float4 cf = *reinterpret_cast<const float4*>(scf + u * 32 + 4 * j4);
+        v[4 * j4 + 0] *= cf.x * r_t;
+        v[4 * j4 + 1] *= cf.y * r_t;
+        v[4 * j4 + 2] *= cf.z * r_t;
+        v[4 * j4 + 3] *= cf.w * r_t;
+        rs += (v[4 * j4 + 0] + v[4 * j4 + 1]) + (v[4 * j4 + 2] + v[4 * j4 + 3]);
+      }
+    } else if (u == rb) {  // diagonal block: causal mask, one exp per entry
+      tmem_ld32(tS_row + u * 32, v);
+#pragma unroll
+      for (int j4 = 0; j4 < 8; ++j4) {
+        const float4 y = *reinterpret_cast<const float4*>(sy + u * 32 + 4 * j4);
+        const float yy[4] = {y.x, y.y, y.z, y.w};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const int j = 4 * j4 + e;
+          float pv = v[j] * ex2_approx(x_t + yy[e]);
+          pv = (REV ? j >= lane : j <= lane) ? pv : 0.f;
+          rs += pv;
+          v[j] = pv;
+        }
+      }
+    } else {  // above the diagonal: zeros (the S MMA of every tile overwrites these columns)
+#pragma unroll
+      for (int j = 0; j < 32; ++j) v[j] = 0.f;
+    }
+    sink(u, v);
+  }
+  return rs;
+}
+
+// One 32-column unit of P packed to 16 bits into the TMEM columns of its S unit (see FwSmem: P stays in TMEM)
+template <typename T>
+__device__ __forceinline__ void tmem_st_p(uint32_t taddr, const float (&v)[32]) {
+  uint32_t pk[16];
+#pragma unroll
+  for (int j = 0; j < 16; ++j) pk[j] = pack2<T>(v[2 * j], v[2 * j + 1]);
+  tmem_st16(taddr, pk);
+}
+
+// Normaliser of row t (fw.py:197-212): bq = exp(b_t + m_{k-1} - m_t) scale scales Hinter, nmax = max(|den|, exp(-m_t)) is
+// n_out, and h = (Hintra + bq Hinter) inv.  den_of(bq) returns bq (q . n_{k-1}) + the row sum of P; it runs after bq,
+// so a body may wait for the TMEM loads of q . n there.
+struct Normaliser {
+  float bq, nmax, inv;
+};
+template <typename DenOf>
+__device__ __forceinline__ Normaliser normaliser(const TcFwParams& p, float b_t, float m_run, float m_t, DenOf den_of) {
+  const float bq = __expf(b_t + m_run - m_t) * p.scale;       // fw.py:197-198
+  const float den = den_of(bq);                                // fw.py:204-206
+  const float nmax = fmaxf(fabsf(den), __expf(-m_t));          // fw.py:208-210
+  const float inv = p.sig == 2 ? 1.f : 1.f / (nmax + p.eps);  // siging = 2: no normaliser
+  return {bq, nmax, inv};
+}
+
+// Per-channel parameters of the fused cell-output epilogue, channels col0 .. col0 + D - 1 of the layer row (spar: [3][D]
+// = weight, bias, skip; a missing tensor reads as 1, 0, 0)
+template <int D>
+__device__ __forceinline__ void load_ln_params(const TcFwParams& p, float* spar, int col0, int tid) {
+  for (int e = tid; e < D; e += kWorkers) {
+    spar[e] = p.ln_w ? p.ln_w[col0 + e] : 1.f;
+    spar[D + e] = p.ln_b ? p.ln_b[col0 + e] : 0.f;
+    spar[2 * D + e] = p.ln_skip ? p.ln_skip[col0 + e] : 0.f;
+  }
+}
+
 // VB > 1: rectangular heads, DHQK = D and DHHV = VB * D.  CTA x runs the square problem of (batch, head) x / VB on
 // the D-wide column block vb = x % VB of v / h / C (see tc_fw_rect); n and m do not depend on v, so every block
 // computes them and block 0 writes them.  With the fused epilogue the two blocks of a head are one {2, 1, 1} cluster
@@ -574,14 +703,7 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
       const uint32_t one2 = pack2<T>(1.f, 1.f);
       for (int e = tid; e < 2048 / 16; e += kWorkers) reinterpret_cast<uint4*>(sOnes)[e] = make_uint4(one2, one2, one2, one2);
     }
-    if (EPI) {  // per-channel parameters of the fused cell-output epilogue for this head's column block
-      float* spar = fsm + SM::fPar;
-      for (int e = tid; e < D; e += kWorkers) {
-        spar[e] = p.ln_w ? p.ln_w[hh * (VB * D) + vb * D + e] : 1.f;
-        spar[D + e] = p.ln_b ? p.ln_b[hh * (VB * D) + vb * D + e] : 0.f;
-        spar[2 * D + e] = p.ln_skip ? p.ln_skip[hh * (VB * D) + vb * D + e] : 0.f;
-      }
-    }
+    if (EPI) load_ln_params<D>(p, fsm + SM::fPar, hh * (VB * D) + vb * D, tid);  // this head's column block
     named_sync(NB_PAIR0, kWorkers);  // sNt zeroed before the owners write column 0
     if (owns_c && ch == 0) {
       n_reg = p.n0 ? p.n0[(int64_t)bh * D + drow] : 0.f;
@@ -707,23 +829,8 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
     }
     if (lane == 0) tma_store_wait_all<0>();
   } else if (warp == kScanWarp) {
-    // =========================== scan warp: gate vectors two tiles ahead ===========================
-    auto raw_of = [&](int c) {
-      const int t1 = mt(c) * LT;
-      return load_gate_raw<T>(ip + (int64_t)t1 * p.ig_ss, p.ig_ss, fp + (int64_t)t1 * p.fg_ss, p.fg_ss, min(LT, p.S - t1));
-    };
-    // skip-input rows of this head (fused epilogue): pulled into L2 two tiles before the workers read them
-    const uint16_t* xbase = p.x ? (const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh + vb * D : nullptr;
-    GateRaw<T> raw = raw_of(0);
-    for (int n = 0; n < p.NT; ++n) {  // vectors of tile n; tiles 0 and 1 need no buffer hand-back
-      if (EPI && p.x) prefetch_rows_l2<D * 2>(xbase, p.x_ss, mt(n) * LT, min(LT, p.S - mt(n) * LT), lane);
-      if (n >= 2) named_sync(NB_C, kNbC);  // every worker is done with tile n-2: its gate buffer can be reused
-      gate_scan_regs(fsm + SM::fGates + (n & 1) * GateBuf::kFloats, raw, REV, p.sig != 0, p.cap);
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bar_g[n & 1]);
-      if (n + 1 < p.NT) raw = raw_of(n + 1);  // stays in flight until the next hand-back
-    }
-    for (int n = max(p.NT - 2, 0); n < p.NT; ++n) named_sync(NB_C, kNbC);  // match the workers' remaining arrivals
+    fw_scan_warp<REV, EPI ? D * 2 : 0>(p, ip, fp, mt, fsm + SM::fGates, bar_g,
+                                       p.x ? (const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh + vb * D : nullptr);
   } else {
     // =========================== worker warps ===================================================
     float m_run = p.m0 ? p.m0[bh] : 0.f;
@@ -740,13 +847,9 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
 
       TC_PROF(c, 0);
       mbar_wait(&bar_g[pb], (c >> 1) & 1, 2);
-      const float g = gb[GateBuf::oScal], amax = gb[GateBuf::oScal + 1];
-      const float m_next = p.sig ? 0.f : fmaxf(g + m_run, g + amax);    // fw.py:96-98
-      const float gbar = __expf(g + m_run - m_next);                    // fw.py:106
-      const float b_t = gb[GateBuf::oB + row], i_t = gb[GateBuf::oI + row];
-      const float m_t = p.sig ? 0.f : b_t + fmaxf(m_run, gb[GateBuf::oPm + row]);  // fw.py:178-184
+      const auto [g, m_next, gbar, b_t, i_t, m_t] = tile_gates(gb, row, m_run, p.sig);
       TC_PROF(c, 1);
-      // ---- P = S . D (causal), row sums ----------------------------------------------------------
+      // ---- P = S . D (causal), row sums; P packed into the S columns ----------------------------
       mbar_wait(&bar_s, par, 5);
       tc_fence_after_sync();
       TC_PROF(c, 2);
@@ -756,6 +859,8 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
         const float* scf = gb + GateBuf::oCf;
         float rs = 0.f;
 #pragma unroll 1
+        // causal_p's loop, written out here: called, it changes this kernel's register allocation and costs the (64, 128)
+        // forward 0.4 % at S = 6400 (B200); keep the two copies in step
         for (int u = ch; u < 4; u += 2) {  // this thread's two 32-column units (warp-uniform branches)
           float v[32];
           const bool off_diag = REV ? u > rb : u < rb;  // fully unmasked 32x32 block
@@ -831,12 +936,11 @@ __device__ __forceinline__ void tc_fw_body(const CUtensorMap& mapQ, const CUtens
         tmem_ld_nowait(tHi + lane_base + ch * CW, hi);
         tmem_ld_nowait(tHx + lane_base + ch * CW, hx);
         tmem_ld1_nowait(tHx + lane_base + D, qn_u);  // q . n_{k-1}
-        const float bq = __expf(b_t + m_run - m_t) * p.scale;  // fw.py:197-198
-        const float rs = srs[row] + srs[LT + row];
-        tmem_ld_wait();
-        const float den = bq * __uint_as_float(qn_u) + rs;       // fw.py:204-206
-        const float nmax = fmaxf(fabsf(den), __expf(-m_t));    // fw.py:208-210
-        const float inv = p.sig == 2 ? 1.f : 1.f / (nmax + p.eps);  // siging = 2: no normaliser
+        const auto [bq, nmax, inv] = normaliser(p, b_t, m_run, m_t, [&](float bq_t) {
+          const float rs = srs[row] + srs[LT + row];
+          tmem_ld_wait();
+          return bq_t * __uint_as_float(qn_u) + rs;
+        });
         float o[CW];
 #pragma unroll
         for (int j = 0; j < CW; ++j) o[j] = (__uint_as_float(hi[j]) + bq * __uint_as_float(hx[j])) * inv;  // fw.py:200-212
@@ -946,7 +1050,7 @@ tc_fw(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensor
 // (grid 2 B NH, the two blocks of a head on adjacent CTAs so that their Q / K reads meet in L2).  Shared memory, TMEM
 // columns and CTAs per SM are those of tc_fw<T, D>; mapV / mapH are DHHV wide with D-wide boxes, and mapCs is the
 // block layout of make_states_map_blocks (the state entering tile c, column block vb, at rows (2 c + vb) D).
-// EPI: fused cell-output epilogue, launched as {2, 1, 1} clusters (launch_fw_rect) with FwSmem<D>::kBytesPair.
+// EPI: fused cell-output epilogue, launched as {2, 1, 1} clusters (run_fw) with FwSmem<D>::kBytesPair.
 template <typename T, int D, bool REV, bool EPI>
 __global__ void __launch_bounds__(kTcThreads, D == 32 ? 2 : 1)
 tc_fw_rect(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapK,
@@ -957,7 +1061,8 @@ tc_fw_rect(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
 
 // =============================================================================================
 // Forward, head dim 128 (640-base384.yaml: NH=6, DH=128; the inference config of BASELINE.json).
-// Same algorithm and warp roles as tc_fw_d64; differences: every Q/K/V/H/C tile is two [128][64]
+// Same algorithm, warp roles and shared stages (fw_scan_warp, tile_gates, normaliser) as tc_fw_body;
+// differences: every Q/K/V/H/C tile is two [128][64]
 // swizzled sub-tiles (column halves), dC = Kbar^T V is M128 N128 so C lives in the plain TMEM
 // lane == row layout (every worker thread owns C[row][64 columns] in 64 registers), shared memory
 // (192 KB of tiles) leaves room for ONE Q/K/V stage and S is single-buffered in TMEM (4 x 128 columns).
@@ -976,6 +1081,68 @@ struct FwSmem128 {
   static constexpr int kBytes = oSmall + kSmallFloats * 4 + 1024;
   static constexpr uint32_t kLoadBytes = 6 * kTile;
 };
+
+// ---- pieces of the M128-layout forwards (tc_fw_d128, tc_fw_wide): C in the plain TMEM lane == row layout, every worker
+// thread keeps 64 fp32 columns of one C row in registers (Creg) ---------------------------------------------------------
+
+// Set-up: thread 0 initialises the mbarriers (bar_n takes n_arrivals per phase, the others one), the control warp
+// allocates the 512 TMEM columns and prefetches the four tensor maps.
+__device__ __forceinline__ void fw128_prologue(int warp, uint64_t& bar_full, uint64_t& bar_s, uint64_t& bar_dc, uint64_t& bar_h,
+                                               uint64_t (&bar_g)[2], uint64_t& bar_n, uint32_t n_arrivals, uint32_t& tmem_base_s,
+                                               const CUtensorMap& m0, const CUtensorMap& m1, const CUtensorMap& m2,
+                                               const CUtensorMap& m3) {
+  if (threadIdx.x == 0) {
+    mbar_init(&bar_full, 1);
+    mbar_init(&bar_s, 1);
+    mbar_init(&bar_dc, 1);
+    mbar_init(&bar_h, 1);
+    mbar_init(&bar_g[0], 1);
+    mbar_init(&bar_g[1], 1);
+    mbar_init(&bar_n, n_arrivals);
+    fence_mbar_init();
+  }
+  if (warp == kCtlWarp) {
+    tmem_alloc<512>(&tmem_base_s);
+    if ((threadIdx.x & 31) == 0) {
+      prefetch_tmap(&m0); prefetch_tmap(&m1); prefetch_tmap(&m2); prefetch_tmap(&m3);
+    }
+  }
+}
+
+// C_0: Creg = the row at c0 + off (c0 NULL: Creg keeps its zeros), and its 16-bit operand copy into row srow, columns
+// col0 .. col0 + 63 of sC
+template <typename T>
+__device__ __forceinline__ void fw128_load_c0(float (&Creg)[64], const float* c0, int64_t off, uint8_t* sC, int srow, int col0) {
+  if (c0) {
+    const float* src = c0 + off;
+#pragma unroll
+    for (int j = 0; j < 64; ++j) Creg[j] = src[j];
+  }
+#pragma unroll
+  for (int hf = 0; hf < 2; ++hf) {
+    float t32[32];
+#pragma unroll
+    for (int j = 0; j < 32; ++j) t32[j] = Creg[hf * 32 + j];
+    store_row32<T>(sC, srow, col0 + hf * 32, t32);
+  }
+}
+
+// C_k = gbar C_{k-1} + dC (dC: this thread's 64 columns in TMEM from tDC_row) and its 16-bit operand copy, placed as in
+// fw128_load_c0
+template <typename T>
+__device__ __forceinline__ void fw128_update_c(float (&Creg)[64], float gbar, uint32_t tDC_row, uint8_t* sC, int srow, int col0) {
+#pragma unroll
+  for (int hf = 0; hf < 2; ++hf) {
+    float v[32], t32[32];
+    tmem_ld32(tDC_row + hf * 32, v);
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      Creg[hf * 32 + j] = gbar * Creg[hf * 32 + j] + v[j];
+      t32[j] = Creg[hf * 32 + j];
+    }
+    store_row32<T>(sC, srow, col0 + hf * 32, t32);  // Q C_{k-1} (bar_h) has finished reading the old copy
+  }
+}
 
 template <typename T, bool REV, bool EPI>
 __global__ void __launch_bounds__(kTcThreads, 1)
@@ -1002,22 +1169,7 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int bh = blockIdx.x, b = bh / p.NH, hh = bh % p.NH;
 
-  if (tid == 0) {
-    mbar_init(&bar_full, 1);
-    mbar_init(&bar_s, 1);
-    mbar_init(&bar_dc, 1);
-    mbar_init(&bar_h, 1);
-    mbar_init(&bar_g[0], 1);
-    mbar_init(&bar_g[1], 1);
-    mbar_init(&bar_n, D);
-    fence_mbar_init();
-  }
-  if (warp == kCtlWarp) {
-    tmem_alloc<512>(&tmem_base_s);
-    if (lane == 0) {
-      prefetch_tmap(&mapQ); prefetch_tmap(&mapK); prefetch_tmap(&mapV); prefetch_tmap(&mapH);
-    }
-  }
+  fw128_prologue(warp, bar_full, bar_s, bar_dc, bar_h, bar_g, bar_n, D, tmem_base_s, mapQ, mapK, mapV, mapH);
   const int rb = warp & 3, ch = (warp >> 2) & 1;
   const int row = rb * 32 + lane;  // tile row == TMEM lane; also the dqk row of C this thread owns
   const uint32_t lane_base = (uint32_t)(rb * 32) << 16;
@@ -1025,25 +1177,9 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
 #pragma unroll
   for (int j = 0; j < 64; ++j) Creg[j] = 0.f;
   if (warp < kCtlWarp) {
-    if (p.c0) {
-      const float* src = p.c0 + ((int64_t)bh * D + row) * D + ch * 64;
-#pragma unroll
-      for (int j = 0; j < 64; ++j) Creg[j] = src[j];
-    }
-#pragma unroll
-    for (int hf = 0; hf < 2; ++hf) {
-      float t32[32];
-#pragma unroll
-      for (int j = 0; j < 32; ++j) t32[j] = Creg[hf * 32 + j];
-      store_row32<T>(sC, row, ch * 64 + hf * 32, t32);
-    }
+    fw128_load_c0<T>(Creg, p.c0, ((int64_t)bh * D + row) * D + ch * 64, sC, row, ch * 64);
     if (tid < D) fsm[SM::fN + tid] = p.n0 ? p.n0[(int64_t)bh * D + tid] : 0.f;
-    if (EPI && tid < D) {  // per-channel parameters of the fused cell-output epilogue for this head
-      float* spar = fsm + SM::fPar;
-      spar[tid] = p.ln_w ? p.ln_w[hh * D + tid] : 1.f;
-      spar[D + tid] = p.ln_b ? p.ln_b[hh * D + tid] : 0.f;
-      spar[2 * D + tid] = p.ln_skip ? p.ln_skip[hh * D + tid] : 0.f;
-    }
+    if (EPI) load_ln_params<D>(p, fsm + SM::fPar, hh * D, tid);  // this head
     fence_proxy_async_smem();
   }
   tc_fence_before_sync();
@@ -1159,23 +1295,8 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
     }
     if (lane == 0) tma_store_wait_all<0>();
   } else if (warp == kScanWarp) {
-    // =========================== scan warp: gate vectors two tiles ahead ===========================
-    auto raw_of = [&](int c) {
-      const int t1 = mt(c) * LT;
-      return load_gate_raw<T>(ip + (int64_t)t1 * p.ig_ss, p.ig_ss, fp + (int64_t)t1 * p.fg_ss, p.fg_ss, min(LT, p.S - t1));
-    };
-    // skip-input rows of this head (fused epilogue): pulled into L2 two tiles before the workers read them
-    const uint16_t* xbase = p.x ? (const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh : nullptr;
-    GateRaw<T> raw = raw_of(0);
-    for (int n = 0; n < p.NT; ++n) {
-      if (EPI && p.x) prefetch_rows_l2<D * 2>(xbase, p.x_ss, mt(n) * LT, min(LT, p.S - mt(n) * LT), lane);
-      if (n >= 2) named_sync(NB_C, kNbC);
-      gate_scan_regs(fsm + SM::fGates + (n & 1) * GateBuf::kFloats, raw, REV, p.sig != 0, p.cap);
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bar_g[n & 1]);
-      if (n + 1 < p.NT) raw = raw_of(n + 1);
-    }
-    for (int n = max(p.NT - 2, 0); n < p.NT; ++n) named_sync(NB_C, kNbC);
+    fw_scan_warp<REV, EPI ? D * 2 : 0>(p, ip, fp, mt, fsm + SM::fGates, bar_g,
+                                       p.x ? (const uint16_t*)p.x + b * p.x_sb + hh * p.x_sh : nullptr);
   } else {
     // =========================== worker warps ===================================================
     float m_run = p.m0 ? p.m0[bh] : 0.f;
@@ -1193,11 +1314,7 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
       const int n_valid = min(LT, p.S - t0);
 
       mbar_wait(&bar_g[pb], (c >> 1) & 1, 2);
-      const float g = gb[GateBuf::oScal], amax = gb[GateBuf::oScal + 1];
-      const float m_next = p.sig ? 0.f : fmaxf(g + m_run, g + amax);    // fw.py:96-98
-      const float gbar = __expf(g + m_run - m_next);                    // fw.py:106
-      const float b_t = gb[GateBuf::oB + row], i_t = gb[GateBuf::oI + row];
-      const float m_t = p.sig ? 0.f : b_t + fmaxf(m_run, gb[GateBuf::oPm + row]);  // fw.py:178-184
+      const auto [g, m_next, gbar, b_t, i_t, m_t] = tile_gates(gb, row, m_run, p.sig);
       mbar_wait(&bar_full, par, 3);
       if (c > 0) mbar_wait(&bar_n, (c - 1) & 1, 4);
       {  // partial q . n_{k-1} over this thread's 64 columns
@@ -1212,53 +1329,11 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
         }
         sqn[ch * LT + row] = qn;
       }
-      // ---- P = S . D (causal), row sums -- identical to the d=64 kernel (S is 128 x 128 either way) ----
+      // ---- P = S . D (causal), row sums; P written swizzled to sP -----------------------------------
       mbar_wait(&bar_s, par, 5);
       tc_fence_after_sync();
-      {
-        const float x_t = (b_t - m_t) * kLog2e + log2f(p.scale);
-        const float* sy = gb + GateBuf::oY;
-        const float* scf = gb + GateBuf::oCf;
-        float rs = 0.f;
-#pragma unroll 1
-        for (int u = ch; u < 4; u += 2) {
-          float v[32];
-          const bool off_diag = REV ? u > rb : u < rb;
-          if (off_diag) {
-            tmem_ld32(tS + lane_base + u * 32, v);
-            const float r_t = ex2_approx(x_t + gb[GateBuf::oScal + 4 + u]);
-#pragma unroll
-            for (int j4 = 0; j4 < 8; ++j4) {
-              const float4 cf = *reinterpret_cast<const float4*>(scf + u * 32 + 4 * j4);
-              v[4 * j4 + 0] *= cf.x * r_t;
-              v[4 * j4 + 1] *= cf.y * r_t;
-              v[4 * j4 + 2] *= cf.z * r_t;
-              v[4 * j4 + 3] *= cf.w * r_t;
-              rs += (v[4 * j4 + 0] + v[4 * j4 + 1]) + (v[4 * j4 + 2] + v[4 * j4 + 3]);
-            }
-          } else if (u == rb) {
-            tmem_ld32(tS + lane_base + u * 32, v);
-#pragma unroll
-            for (int j4 = 0; j4 < 8; ++j4) {
-              const float4 y = *reinterpret_cast<const float4*>(sy + u * 32 + 4 * j4);
-              const float yy[4] = {y.x, y.y, y.z, y.w};
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                const int j = 4 * j4 + e;
-                float pv = v[j] * ex2_approx(x_t + yy[e]);
-                pv = (REV ? j >= lane : j <= lane) ? pv : 0.f;
-                rs += pv;
-                v[j] = pv;
-              }
-            }
-          } else {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] = 0.f;
-          }
-          store_row32<T>(sP, row, u * 32, v);
-        }
-        srs[ch * LT + row] = rs;
-      }
+      srs[ch * LT + row] = causal_p<REV>(tS + lane_base, gb, b_t, m_t, p.scale, rb, ch, lane,
+                                         [&](int u, const float(&v)[32]) { store_row32<T>(sP, row, u * 32, v); });
       fence_proxy_async_smem();
       tc_fence_before_sync();
       named_arrive(NB_B, kNbAB);
@@ -1285,10 +1360,8 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
       mbar_wait(&bar_h, par, 7);
       tc_fence_after_sync();
       {
-        const float bq = __expf(b_t + m_run - m_t) * p.scale;                          // fw.py:197-198
-        const float den = bq * (sqn[row] + sqn[LT + row]) + srs[row] + srs[LT + row];  // fw.py:204-206
-        const float nmax = fmaxf(fabsf(den), __expf(-m_t));                            // fw.py:208-210
-        const float inv = p.sig == 2 ? 1.f : 1.f / (nmax + p.eps);  // siging = 2: no normaliser
+        const auto [bq, nmax, inv] = normaliser(
+            p, b_t, m_run, m_t, [&](float bq_t) { return bq_t * (sqn[row] + sqn[LT + row]) + srs[row] + srs[LT + row]; });
 #pragma unroll 1
         for (int hf = 0; hf < 2; ++hf) {
           uint32_t hi[32], hx[32];
@@ -1322,17 +1395,7 @@ tc_fw_d128(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
       mbar_wait(&bar_dc, par, 6);
       tc_fence_after_sync();
       {
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-          float v[32], t32[32];
-          tmem_ld32(tDC + lane_base + ch * 64 + hf * 32, v);
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            Creg[hf * 32 + j] = gbar * Creg[hf * 32 + j] + v[j];
-            t32[j] = Creg[hf * 32 + j];
-          }
-          store_row32<T>(sC, row, ch * 64 + hf * 32, t32);  // Q C_{k-1} (bar_h) has finished reading the old copy
-        }
+        fw128_update_c<T>(Creg, gbar, tDC + lane_base + ch * 64, sC, row, ch * 64);
         if (tid < D) {  // n_k = gbar n_{k-1} + column sums of Kbar (fw.py:116)
           sNn[tid] = gbar * sNc[tid] + ((snp[tid] + snp[D + tid]) + (snp[2 * D + tid] + snp[3 * D + tid]));
           mbar_arrive(&bar_n);
@@ -1414,22 +1477,7 @@ tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int bh = blockIdx.x / VB, vb = blockIdx.x % VB, b = bh / p.NH, hh = bh % p.NH;
 
-  if (tid == 0) {
-    mbar_init(&bar_full, 1);
-    mbar_init(&bar_s, 1);
-    mbar_init(&bar_dc, 1);
-    mbar_init(&bar_h, 1);
-    mbar_init(&bar_g[0], 1);
-    mbar_init(&bar_g[1], 1);
-    mbar_init(&bar_n, kWorkers);
-    fence_mbar_init();
-  }
-  if (warp == kCtlWarp) {
-    tmem_alloc<512>(&tmem_base_s);
-    if (lane == 0) {
-      prefetch_tmap(&mapQ); prefetch_tmap(&mapK); prefetch_tmap(&mapV); prefetch_tmap(&mapCs);
-    }
-  }
+  fw128_prologue(warp, bar_full, bar_s, bar_dc, bar_h, bar_g, bar_n, kWorkers, tmem_base_s, mapQ, mapK, mapV, mapCs);
   const int rb = warp & 3, ch = (warp >> 2) & 1;
   const int row = rb * 32 + lane;  // tile row == TMEM lane
   const int drow = ch * 128 + row;  // the dqk row of C (and entry of n) this thread owns
@@ -1438,18 +1486,7 @@ tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
 #pragma unroll
   for (int j = 0; j < DV; ++j) Creg[j] = 0.f;
   if (warp < kCtlWarp) {
-    if (p.c0) {
-      const float* src = p.c0 + ((int64_t)bh * DK + drow) * (VB * DV) + vb * DV;
-#pragma unroll
-      for (int j = 0; j < DV; ++j) Creg[j] = src[j];
-    }
-#pragma unroll
-    for (int hf = 0; hf < 2; ++hf) {
-      float t32[32];
-#pragma unroll
-      for (int j = 0; j < 32; ++j) t32[j] = Creg[hf * 32 + j];
-      store_row32<T>(sC, drow, hf * 32, t32);
-    }
+    fw128_load_c0<T>(Creg, p.c0, ((int64_t)bh * DK + drow) * (VB * DV) + vb * DV, sC, drow, 0);
     fsm[SM::fN + tid] = p.n0 ? p.n0[(int64_t)bh * DK + tid] : 0.f;  // kWorkers == DK
     for (int e = tid; e < 4096 / 16; e += kWorkers) reinterpret_cast<uint4*>(sA)[e] = make_uint4(0, 0, 0, 0);
     fence_proxy_async_smem();
@@ -1566,20 +1603,7 @@ tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
     }
     if (lane == 0) tma_store_wait_all<0>();
   } else if (warp == kScanWarp) {
-    // =========================== scan warp: gate vectors two tiles ahead ===========================
-    auto raw_of = [&](int c) {
-      const int t1 = mt(c) * LT;
-      return load_gate_raw<T>(ip + (int64_t)t1 * p.ig_ss, p.ig_ss, fp + (int64_t)t1 * p.fg_ss, p.fg_ss, min(LT, p.S - t1));
-    };
-    GateRaw<T> raw = raw_of(0);
-    for (int n = 0; n < p.NT; ++n) {
-      if (n >= 2) named_sync(NB_C, kNbC);
-      gate_scan_regs(fsm + SM::fGates + (n & 1) * GateBuf::kFloats, raw, REV, p.sig != 0, p.cap);
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bar_g[n & 1]);
-      if (n + 1 < p.NT) raw = raw_of(n + 1);
-    }
-    for (int n = max(p.NT - 2, 0); n < p.NT; ++n) named_sync(NB_C, kNbC);
+    fw_scan_warp<REV, 0>(p, ip, fp, mt, fsm + SM::fGates, bar_g, nullptr);
   } else {
     // =========================== worker warps ===================================================
     float m_run = p.m0 ? p.m0[bh] : 0.f;
@@ -1597,11 +1621,7 @@ tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
       const int n_valid = min(LT, p.S - t0);
 
       mbar_wait(&bar_g[pb], (c >> 1) & 1, 2);
-      const float g = gb[GateBuf::oScal], amax = gb[GateBuf::oScal + 1];
-      const float m_next = p.sig ? 0.f : fmaxf(g + m_run, g + amax);    // fw.py:96-98
-      const float gbar = __expf(g + m_run - m_next);                    // fw.py:106
-      const float b_t = gb[GateBuf::oB + row], i_t = gb[GateBuf::oI + row];
-      const float m_t = p.sig ? 0.f : b_t + fmaxf(m_run, gb[GateBuf::oPm + row]);  // fw.py:178-184
+      const auto [g, m_next, gbar, b_t, i_t, m_t] = tile_gates(gb, row, m_run, p.sig);
       mbar_wait(&bar_full, par, 3);
       if (c > 0) mbar_wait(&bar_n, (c - 1) & 1, 4);
       {  // partial q . n_{k-1} over this thread's 128 dqk columns (K-blocks 2 ch, 2 ch + 1)
@@ -1623,53 +1643,8 @@ tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
       // ---- P = S . D (causal), row sums, packed into the S columns (as tc_fw) ------------------------
       mbar_wait(&bar_s, par, 5);
       tc_fence_after_sync();
-      {
-        const float x_t = (b_t - m_t) * kLog2e + log2f(p.scale);
-        const float* sy = gb + GateBuf::oY;
-        const float* scf = gb + GateBuf::oCf;
-        float rs = 0.f;
-#pragma unroll 1
-        for (int u = ch; u < 4; u += 2) {
-          float v[32];
-          const bool off_diag = REV ? u > rb : u < rb;
-          if (off_diag) {
-            tmem_ld32(tS + lane_base + u * 32, v);
-            const float r_t = ex2_approx(x_t + gb[GateBuf::oScal + 4 + u]);
-#pragma unroll
-            for (int j4 = 0; j4 < 8; ++j4) {
-              const float4 cf = *reinterpret_cast<const float4*>(scf + u * 32 + 4 * j4);
-              v[4 * j4 + 0] *= cf.x * r_t;
-              v[4 * j4 + 1] *= cf.y * r_t;
-              v[4 * j4 + 2] *= cf.z * r_t;
-              v[4 * j4 + 3] *= cf.w * r_t;
-              rs += (v[4 * j4 + 0] + v[4 * j4 + 1]) + (v[4 * j4 + 2] + v[4 * j4 + 3]);
-            }
-          } else if (u == rb) {
-            tmem_ld32(tS + lane_base + u * 32, v);
-#pragma unroll
-            for (int j4 = 0; j4 < 8; ++j4) {
-              const float4 y = *reinterpret_cast<const float4*>(sy + u * 32 + 4 * j4);
-              const float yy[4] = {y.x, y.y, y.z, y.w};
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                const int j = 4 * j4 + e;
-                float pv = v[j] * ex2_approx(x_t + yy[e]);
-                pv = (REV ? j >= lane : j <= lane) ? pv : 0.f;
-                rs += pv;
-                v[j] = pv;
-              }
-            }
-          } else {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] = 0.f;
-          }
-          uint32_t pk[16];
-#pragma unroll
-          for (int j = 0; j < 16; ++j) pk[j] = pack2<T>(v[2 * j], v[2 * j + 1]);
-          tmem_st16(tS + lane_base + u * 32, pk);
-        }
-        srs[ch * LT + row] = rs;
-      }
+      srs[ch * LT + row] = causal_p<REV>(tS + lane_base, gb, b_t, m_t, p.scale, rb, ch, lane,
+                                         [&](int u, const float(&v)[32]) { tmem_st_p<T>(tS + lane_base + u * 32, v); });
       tmem_st_wait();
       tc_fence_before_sync();
       named_arrive(NB_B, kNbAB);
@@ -1695,10 +1670,8 @@ tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
         uint32_t hi[32], hx[32];
         tmem_ld32_nowait(tHi + lane_base + ch * 32, hi);
         tmem_ld32_nowait(tHx + lane_base + ch * 32, hx);
-        const float bq = __expf(b_t + m_run - m_t) * p.scale;                          // fw.py:197-198
-        const float den = bq * (sqn[row] + sqn[LT + row]) + srs[row] + srs[LT + row];  // fw.py:204-206
-        const float nmax = fmaxf(fabsf(den), __expf(-m_t));                            // fw.py:208-210
-        const float inv = p.sig == 2 ? 1.f : 1.f / (nmax + p.eps);  // siging = 2: no normaliser
+        const auto [bq, nmax, inv] = normaliser(
+            p, b_t, m_run, m_t, [&](float bq_t) { return bq_t * (sqn[row] + sqn[LT + row]) + srs[row] + srs[LT + row]; });
         tmem_ld_wait();
         if (row < n_valid) {
           uint4* dst = reinterpret_cast<uint4*>(hbase + (int64_t)(t0 + row) * p.h_ss);
@@ -1726,17 +1699,7 @@ tc_fw_wide(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUt
       {
         uint32_t dn_u;
         tmem_ld1_nowait(tDN + ch * 16 + lane_base, dn_u);
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf) {
-          float v[32], t32[32];
-          tmem_ld32(tDC + ch * DV + lane_base + hf * 32, v);  // (waits for dn_u too)
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            Creg[hf * 32 + j] = gbar * Creg[hf * 32 + j] + v[j];
-            t32[j] = Creg[hf * 32 + j];
-          }
-          store_row32<T>(sC, drow, hf * 32, t32);  // Q C_{k-1} (bar_h) has finished reading the old copy
-        }
+        fw128_update_c<T>(Creg, gbar, tDC + ch * DV + lane_base, sC, drow, 0);  // (its first TMEM load waits for dn_u too)
         sNn[drow] = gbar * sNc[drow] + __uint_as_float(dn_u);  // n_k = gbar n_{k-1} + K^T abar (fw.py:116)
         mbar_arrive(&bar_n);
       }
@@ -2403,16 +2366,6 @@ std::atomic<long long*> g_prof{nullptr};
 #define TC_SET_PROF(p, off)
 #endif
 
-int num_sms() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-  }
-  return n;
-}
-
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) once per (kernel, device) instead of on every launch
 // (a runtime call of a few microseconds on the host path of a launch-bound training step)
 template <typename K>
@@ -2445,89 +2398,53 @@ int pdl_mode() {  // 0 off, 1 forward and backward, 2 forward only
   }
   return v;
 }
+// cudaLaunchKernelEx with programmatic stream serialisation (use_pdl) and, with pair, the two column blocks of a head
+// (adjacent CTAs) as one {2, 1, 1} cluster: co-scheduled, and each can reach the other's shared memory.
 template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(bool use_pdl, void (*kern)(KArgs...), int grid, int block, size_t smem, cudaStream_t st, Args&&... args) {
+cudaError_t launch_ex(bool use_pdl, bool pair, void (*kern)(KArgs...), int grid, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid), cfg.blockDim = dim3(block), cfg.dynamicSmemBytes = smem, cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr, cfg.numAttrs = use_pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
-}
-
-template <typename T, int D>
-int launch_fw(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
-              const CUtensorMap& mh, const CUtensorMap& mcs, cudaStream_t st) {
-  using SM = FwSmem<D>;
-  // the fused cell-output epilogue is a template parameter: the plain kernel carries none of its code (the worker loop is
-  // several instruction-cache lines shorter: 33.7 vs 34.3 us at config 2)
-  auto kern = p.epi ? (p.rev ? tc_fw<T, D, true, true> : tc_fw<T, D, false, true>)
-                    : (p.rev ? tc_fw<T, D, true, false> : tc_fw<T, D, false, false>);
-  MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytes));
-  MLSTM_CUDA_CHECK(launch_pdl(pdl_mode() != 0, kern, p.B * p.NH, kTcThreads, SM::kBytes, st, mq, mk, mv, mh, mcs, p));
-  count_launch();
-  MLSTM_CUDA_CHECK(cudaGetLastError());
-  return 0;
-}
-
-// The two column blocks of a head (adjacent CTAs) as one {2, 1, 1} cluster: co-scheduled, and each can reach the other's
-// shared memory.  Programmatic stream serialisation as launch_pdl.
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pair_pdl(bool use_pdl, void (*kern)(KArgs...), int grid, int block, size_t smem, cudaStream_t st,
-                            Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid), cfg.blockDim = dim3(block), cfg.dynamicSmemBytes = smem, cfg.stream = st;
+  cfg.gridDim = dim3(grid), cfg.blockDim = dim3(kTcThreads), cfg.dynamicSmemBytes = smem, cfg.stream = st;
   cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr, cfg.numAttrs = use_pdl ? 2 : 1;
+  unsigned n = 0;
+  if (pair) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = 2, attr[n].val.clusterDim.y = 1, attr[n].val.clusterDim.z = 1;
+    ++n;
+  }
+  if (use_pdl) {
+    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
+  }
+  cfg.attrs = attr, cfg.numAttrs = n;
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 
-template <typename T, int D>
-auto fw_rect_kernel(bool epi, bool rev) {
-  return epi ? (rev ? tc_fw_rect<T, D, true, true> : tc_fw_rect<T, D, false, true>)
-             : (rev ? tc_fw_rect<T, D, true, false> : tc_fw_rect<T, D, false, false>);
+// The call's 16-bit element type and square head dim 32 / 64 as types: f(T{}), g(std::integral_constant<int, D>{})
+template <typename F>
+int with_dtype(int dtype, F f) {
+  return dtype == MLSTM_B200_BF16 ? f(__nv_bfloat16{}) : f(__half{});
+}
+template <typename F>
+int with_d32_64(int D, F f) {
+  return D == 32 ? f(std::integral_constant<int, 32>{}) : f(std::integral_constant<int, 64>{});
+}
+// The instantiation of a forward kernel template for the call's (epi, rev): pick(std::bool_constant<EPI>,
+// std::bool_constant<REV>) returns it.  The fused cell-output epilogue is a template parameter: the plain kernel carries
+// none of its code (the worker loop is several instruction-cache lines shorter: 33.7 vs 34.3 us at config 2).
+template <typename Pick>
+auto fw_kernel(bool epi, bool rev, Pick pick) {
+  using F = std::false_type;
+  using TT = std::true_type;
+  return epi ? (rev ? pick(TT{}, TT{}) : pick(TT{}, F{})) : (rev ? pick(F{}, TT{}) : pick(F{}, F{}));
 }
 
-template <typename T, int D>
-int launch_fw_rect(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
-                   const CUtensorMap& mh, const CUtensorMap& mcs, cudaStream_t st) {
-  using SM = FwSmem<D>;
-  auto kern = fw_rect_kernel<T, D>(p.epi != 0, p.rev != 0);
-  if (p.epi) {  // fused epilogue: LayerNorm statistics exchanged between the two blocks of a head
-    MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytesPair));
-    MLSTM_CUDA_CHECK(launch_pair_pdl(pdl_mode() != 0, kern, 2 * p.B * p.NH, kTcThreads, SM::kBytesPair, st, mq, mk, mv, mh, mcs, p));
-  } else {
-    MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytes));
-    MLSTM_CUDA_CHECK(launch_pdl(pdl_mode() != 0, kern, 2 * p.B * p.NH, kTcThreads, SM::kBytes, st, mq, mk, mv, mh, mcs, p));
-  }
-  count_launch();
-  MLSTM_CUDA_CHECK(cudaGetLastError());
-  return 0;
-}
-
-template <typename T>
-int launch_fw_d128(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
-                   const CUtensorMap& mh, const CUtensorMap& mcs, cudaStream_t st) {
-  auto kern = p.epi ? (p.rev ? tc_fw_d128<T, true, true> : tc_fw_d128<T, false, true>)
-                    : (p.rev ? tc_fw_d128<T, true, false> : tc_fw_d128<T, false, false>);
-  MLSTM_CUDA_CHECK(ensure_smem(kern, FwSmem128::kBytes));
-  kern<<<p.B * p.NH, kTcThreads, FwSmem128::kBytes, st>>>(mq, mk, mv, mh, mcs, p);
-  count_launch();
-  MLSTM_CUDA_CHECK(cudaGetLastError());
-  return 0;
-}
-
-template <typename T>
-int launch_fw_wide(const TcFwParams& p, const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mv,
-                   const CUtensorMap& mcs, cudaStream_t st) {
-  auto kern = p.rev ? tc_fw_wide<T, true> : tc_fw_wide<T, false>;
-  MLSTM_CUDA_CHECK(ensure_smem(kern, FwSmemWide::kBytes));
-  kern<<<FwSmemWide::VB * p.B * p.NH, kTcThreads, FwSmemWide::kBytes, st>>>(mq, mk, mv, mcs, p);
+// One forward launch of ctas_per_head CTAs per (batch, head); maps: the kernel's tensor maps, in its parameter order.
+template <typename K, typename... Maps>
+int launch_fw(K kern, const TcFwParams& p, int ctas_per_head, int smem, bool pair, bool use_pdl, cudaStream_t st,
+              const Maps&... maps) {
+  MLSTM_CUDA_CHECK(ensure_smem(kern, smem));
+  MLSTM_CUDA_CHECK(launch_ex(use_pdl, pair, kern, ctas_per_head * p.B * p.NH, smem, st, maps..., p));
   count_launch();
   MLSTM_CUDA_CHECK(cudaGetLastError());
   return 0;
@@ -2540,7 +2457,7 @@ int launch_bw(const TcBwParams& p, const CUtensorMap& mq, const CUtensorMap& mk,
   using SM = BwSmem<D>;
   auto kern = p.rev ? tc_bw<T, D, true, TO> : tc_bw<T, D, false, TO>;
   MLSTM_CUDA_CHECK(ensure_smem(kern, SM::kBytes));
-  MLSTM_CUDA_CHECK(launch_pdl(pdl_mode() == 1, kern, p.B * p.NH, kTcThreads, SM::kBytes, st, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, p));
+  MLSTM_CUDA_CHECK(launch_ex(pdl_mode() == 1, false, kern, p.B * p.NH, SM::kBytes, st, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, p));
   MLSTM_CUDA_CHECK(cudaGetLastError());
   return 0;
 }
@@ -2574,6 +2491,45 @@ int make_states_map_blocks(CUtensorMap* m, const void* ptr, const mlstm_b200_sha
 bool rect_heads(const mlstm_b200_shape& s) { return s.DHQK != s.DHHV; }
 bool wide_heads(const mlstm_b200_shape& s) { return s.DHQK == 256 && s.DHHV == 512; }
 
+// Gate, scale and direction fields that TcFwParams and TcBwParams share
+template <typename P>
+void set_gate_params(P& p, const mlstm_b200_shape& s, const mlstm_b200_tensor& i, const mlstm_b200_tensor& f) {
+  p.B = s.B; p.NH = s.NH; p.S = s.S; p.NT = (s.S + LT - 1) / LT;
+  p.eps = s.eps;
+  p.scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf((float)s.DHQK);
+  p.ig = i.ptr; p.ig_sb = i.stride[0]; p.ig_sh = i.stride[1]; p.ig_ss = i.stride[2];
+  p.fg = f.ptr; p.fg_sb = f.stride[0]; p.fg_sh = f.stride[1]; p.fg_ss = f.stride[2];
+  p.rev = s.reverse ? 1 : 0;
+  p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
+  p.cap = s.gate_soft_cap;
+}
+
+// Forward parameters of a call that stores the state entering every tile into c_states (NULL: no states)
+TcFwParams fw_params(const mlstm_b200_fw_args& a, const void* c_states) {
+  TcFwParams p{};
+  set_gate_params(p, a.shape, a.i, a.f);
+  p.c0 = a.c_initial; p.n0 = a.n_initial; p.m0 = a.m_initial;
+  p.n_out = a.n_out; p.m_out = a.m_out;
+  p.c_last = a.c_last; p.n_last = a.n_last; p.m_last = a.m_last;
+  p.store_states = c_states != nullptr;
+  // h stored from the registers: always by tc_fw_wide, by the other kernels only with the fused epilogue
+  p.h_plain = a.h.ptr; p.h_sb = a.h.stride[0]; p.h_sh = a.h.stride[1]; p.h_ss = a.h.stride[2];
+  if (const mlstm_b200_fw_epilogue* ep = a.epilogue) {
+    p.epi = 1;
+    p.xy_f16 = ep->xy_dtype == MLSTM_B200_F16;
+    p.ln_eps = ep->eps;
+    p.ln_w = ep->weight; p.ln_b = ep->bias; p.ln_skip = ep->skip;
+    p.x = ep->x.ptr; p.x_sb = ep->x.stride[0]; p.x_sh = ep->x.stride[1]; p.x_ss = ep->x.stride[2];
+  }
+  TC_SET_PROF(p, 0);
+  return p;
+}
+
+template <typename T, int D>
+auto fw_rect_kernel(bool epi, bool rev) {
+  return fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw_rect<T, D, decltype(r)::value, decltype(e)::value>; });
+}
+
 // (256, 512): tc_fw_wide, eight 64-wide column blocks of v / h / C per head; h is written from the registers
 int run_fw_wide(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   const mlstm_b200_shape& s = a.shape;
@@ -2593,23 +2549,12 @@ int run_fw_wide(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
     set_error("cuTensorMapEncodeTiled failed (%d)", r);
     return MLSTM_B200_ENODEVICE;
   }
-  TcFwParams p{};
-  p.B = s.B; p.NH = s.NH; p.S = s.S; p.NT = (s.S + LT - 1) / LT;
-  p.eps = s.eps;
-  p.scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf((float)s.DHQK);
-  p.ig = a.i.ptr; p.ig_sb = a.i.stride[0]; p.ig_sh = a.i.stride[1]; p.ig_ss = a.i.stride[2];
-  p.fg = a.f.ptr; p.fg_sb = a.f.stride[0]; p.fg_sh = a.f.stride[1]; p.fg_ss = a.f.stride[2];
-  p.c0 = a.c_initial; p.n0 = a.n_initial; p.m0 = a.m_initial;
-  p.n_out = a.n_out; p.m_out = a.m_out;
-  p.c_last = a.c_last; p.n_last = a.n_last; p.m_last = a.m_last;
-  p.rev = s.reverse ? 1 : 0;
-  p.sig = s.siging;
-  p.store_states = c_states != nullptr;
-  p.cap = s.gate_soft_cap;
-  p.h_plain = a.h.ptr; p.h_sb = a.h.stride[0]; p.h_sh = a.h.stride[1]; p.h_ss = a.h.stride[2];  // h, stored by the workers
-  TC_SET_PROF(p, 0);
-  return s.dtype == MLSTM_B200_BF16 ? launch_fw_wide<__nv_bfloat16>(p, mq, mk, mv, mcs, st)
-                                    : launch_fw_wide<__half>(p, mq, mk, mv, mcs, st);
+  const TcFwParams p = fw_params(a, c_states);
+  return with_dtype(s.dtype, [&](auto t) {
+    using T = decltype(t);
+    auto kern = fw_kernel(false, p.rev, [](auto, auto r) { return tc_fw_wide<T, decltype(r)::value>; });
+    return launch_fw(kern, p, FwSmemWide::VB, FwSmemWide::kBytes, false, false, st, mq, mk, mv, mcs);
+  });
 }
 
 int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
@@ -2648,45 +2593,23 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
     set_error("cuTensorMapEncodeTiled failed (%d)", r);
     return MLSTM_B200_ENODEVICE;
   }
-  TcFwParams p{};
-  p.B = s.B; p.NH = s.NH; p.S = s.S; p.NT = (s.S + LT - 1) / LT;
-  p.eps = s.eps;
-  p.scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf((float)s.DHQK);
-  p.ig = a.i.ptr; p.ig_sb = a.i.stride[0]; p.ig_sh = a.i.stride[1]; p.ig_ss = a.i.stride[2];
-  p.fg = a.f.ptr; p.fg_sb = a.f.stride[0]; p.fg_sh = a.f.stride[1]; p.fg_ss = a.f.stride[2];
-  p.c0 = a.c_initial; p.n0 = a.n_initial; p.m0 = a.m_initial;
-  p.n_out = a.n_out; p.m_out = a.m_out;
-  p.c_last = a.c_last; p.n_last = a.n_last; p.m_last = a.m_last;
-  p.rev = s.reverse ? 1 : 0;
-  p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
-  p.store_states = c_states != nullptr;
-  p.cap = s.gate_soft_cap;
-  if (ep) {
-    p.epi = 1;
-    p.xy_f16 = ep->xy_dtype == MLSTM_B200_F16;
-    p.ln_eps = ep->eps;
-    p.ln_w = ep->weight; p.ln_b = ep->bias; p.ln_skip = ep->skip;
-    p.x = ep->x.ptr; p.x_sb = ep->x.stride[0]; p.x_sh = ep->x.stride[1]; p.x_ss = ep->x.stride[2];
-    p.h_plain = a.h.ptr; p.h_sb = a.h.stride[0]; p.h_sh = a.h.stride[1]; p.h_ss = a.h.stride[2];
-  }
-  TC_SET_PROF(p, 0);
-  if (rect) {
-    if (s.DHQK == 32)
-      return s.dtype == MLSTM_B200_BF16 ? launch_fw_rect<__nv_bfloat16, 32>(p, mq, mk, mv, mh, mcs, st)
-                                        : launch_fw_rect<__half, 32>(p, mq, mk, mv, mh, mcs, st);
-    return s.dtype == MLSTM_B200_BF16 ? launch_fw_rect<__nv_bfloat16, 64>(p, mq, mk, mv, mh, mcs, st)
-                                      : launch_fw_rect<__half, 64>(p, mq, mk, mv, mh, mcs, st);
-  }
-  if (s.DHQK == 128) {
-    if (s.dtype == MLSTM_B200_BF16) return launch_fw_d128<__nv_bfloat16>(p, mq, mk, mv, mh, mcs, st);
-    return launch_fw_d128<__half>(p, mq, mk, mv, mh, mcs, st);
-  }
-  if (s.DHQK == 32) {
-    if (s.dtype == MLSTM_B200_BF16) return launch_fw<__nv_bfloat16, 32>(p, mq, mk, mv, mh, mcs, st);
-    return launch_fw<__half, 32>(p, mq, mk, mv, mh, mcs, st);
-  }
-  if (s.dtype == MLSTM_B200_BF16) return launch_fw<__nv_bfloat16, 64>(p, mq, mk, mv, mh, mcs, st);
-  return launch_fw<__half, 64>(p, mq, mk, mv, mh, mcs, st);
+  const TcFwParams p = fw_params(a, c_states);
+  const bool epi = p.epi != 0, rev = p.rev != 0, pdl = pdl_mode() != 0;
+  return with_dtype(s.dtype, [&](auto t) {
+    using T = decltype(t);
+    if (s.DHQK == 128) {
+      auto kern = fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw_d128<T, decltype(r)::value, decltype(e)::value>; });
+      return launch_fw(kern, p, 1, FwSmem128::kBytes, false, false, st, mq, mk, mv, mh, mcs);
+    }
+    return with_d32_64(s.DHQK, [&](auto d) {
+      constexpr int D = decltype(d)::value;
+      using SM = FwSmem<D>;
+      if (rect)  // with the fused epilogue the two blocks of a head exchange their LayerNorm statistics: a cluster
+        return launch_fw(fw_rect_kernel<T, D>(epi, rev), p, 2, epi ? SM::kBytesPair : SM::kBytes, epi, pdl, st, mq, mk, mv, mh, mcs);
+      auto kern = fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw<T, D, decltype(r)::value, decltype(e)::value>; });
+      return launch_fw(kern, p, 1, SM::kBytes, false, pdl, st, mq, mk, mv, mh, mcs);
+    });
+  });
 }
 
 struct BwWs {
@@ -2938,12 +2861,12 @@ int tensor_fw_epilogue_clusters(const mlstm_b200_shape& s) {
     int n = 0;
     return cudaOccupancyMaxActiveClusters(&n, kern, &cfg) == cudaSuccess ? n : -1;
   };
-  const bool bf = s.dtype == MLSTM_B200_BF16, rev = s.reverse != 0;
-  if (s.DHQK == 32)
-    return bf ? query(fw_rect_kernel<__nv_bfloat16, 32>(true, rev), FwSmem<32>::kBytesPair)
-              : query(fw_rect_kernel<__half, 32>(true, rev), FwSmem<32>::kBytesPair);
-  return bf ? query(fw_rect_kernel<__nv_bfloat16, 64>(true, rev), FwSmem<64>::kBytesPair)
-            : query(fw_rect_kernel<__half, 64>(true, rev), FwSmem<64>::kBytesPair);
+  return with_dtype(s.dtype, [&](auto t) {
+    return with_d32_64(s.DHQK, [&](auto d) {
+      constexpr int D = decltype(d)::value;
+      return query(fw_rect_kernel<decltype(t), D>(true, s.reverse != 0), FwSmem<D>::kBytesPair);
+    });
+  });
 }
 
 int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st) { return tensor_bw_blocks(a, a.c_states, -1, 1, st, 0, 0, 0); }
@@ -3002,37 +2925,26 @@ int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, int nbl
     return MLSTM_B200_ENODEVICE;
   }
   TcBwParams p{};
-  p.B = s.B; p.NH = s.NH; p.S = s.S; p.NT = (s.S + LT - 1) / LT;
-  p.eps = s.eps;
-  p.scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf((float)s.DHQK);
-  p.ig = a.i.ptr; p.ig_sb = a.i.stride[0]; p.ig_sh = a.i.stride[1]; p.ig_ss = a.i.stride[2];
-  p.fg = a.f.ptr; p.fg_sb = a.f.stride[0]; p.fg_sh = a.f.stride[1]; p.fg_ss = a.f.stride[2];
+  set_gate_params(p, s, a.i, a.f);
   p.m0 = a.m_initial;
   p.n_out = a.n_out; p.m_out = a.m_out; p.dc_last = a.dc_last;
   p.di = a.di.ptr; p.di_sb = a.di.stride[0]; p.di_sh = a.di.stride[1]; p.di_ss = a.di.stride[2];
   p.df = a.df.ptr; p.df_sb = a.df.stride[0]; p.df_sh = a.df.stride[1]; p.df_ss = a.df.stride[2];
   p.dc0 = a.dc_initial;
-  p.rev = s.reverse ? 1 : 0;
-  p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
-  p.cap = s.gate_soft_cap;
   p.acc_qk = acc_qk; p.acc_v = acc_v; p.acc_g = acc_g;
   p.cs_rows = block < 0 ? D : nblocks * D;
   p.cs_off = block < 0 ? 0 : D * block;
   TC_SET_PROF(p, 4096);
-  int e;
-  if (mixed) {  // kernel operands in one 16-bit dtype, gradients rounded once from fp32 to the other
-    if (s.DHQK == 32)
-      e = s.dtype == MLSTM_B200_BF16 ? launch_bw<__nv_bfloat16, 32, __half>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st)
-                                     : launch_bw<__half, 32, __nv_bfloat16>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st);
-    else
-      e = s.dtype == MLSTM_B200_BF16 ? launch_bw<__nv_bfloat16, 64, __half>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st)
-                                     : launch_bw<__half, 64, __nv_bfloat16>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st);
-  } else if (s.DHQK == 32)
-    e = s.dtype == MLSTM_B200_BF16 ? launch_bw<__nv_bfloat16, 32>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st)
-                                   : launch_bw<__half, 32>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st);
-  else
-    e = s.dtype == MLSTM_B200_BF16 ? launch_bw<__nv_bfloat16, 64>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st)
-                                   : launch_bw<__half, 64>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st);
+  const int e = with_dtype(s.dtype, [&](auto t) {
+    using T = decltype(t);
+    using TX = std::conditional_t<std::is_same<T, __half>::value, __nv_bfloat16, __half>;  // the other 16-bit type
+    return with_d32_64(D, [&](auto d) {
+      constexpr int DD = decltype(d)::value;
+      // mixed: kernel operands in one 16-bit dtype, gradients rounded once from fp32 to the other
+      return mixed ? launch_bw<T, DD, TX>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st)
+                   : launch_bw<T, DD>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st);
+    });
+  });
   if (e) return e;
   count_launch();
   MLSTM_CUDA_CHECK(cudaGetLastError());
