@@ -57,7 +57,9 @@ enum {
 
 /* kernel families; AUTO picks tensor-core (tcgen05) kernels for 16-bit inputs with
  * supported head dims and the exact fp32 FFMA kernels otherwise.  This selects between
- * precision modes of the SAME sm_100a path, not between backends. */
+ * precision modes of the SAME sm_100a path, not between backends.  The exact kernels take
+ * every dtype and any head dims that are multiples of 4 with DHQK <= 256 and DHHV <= 512
+ * (outside that: MLSTM_B200_EUNSUPPORTED). */
 enum { MLSTM_B200_IMPL_AUTO = 0, MLSTM_B200_IMPL_EXACT = 1, MLSTM_B200_IMPL_TENSOR = 2 };
 
 typedef struct mlstm_b200_tensor {
@@ -177,7 +179,9 @@ size_t mlstm_b200_states_bytes(const mlstm_b200_shape* shape);
  * the head-dim-128 backward runs as four head-dim-64 block problems inside the call, a rectangular (D, 2 D) call as two
  * square head-dim-D problems on the two column halves of v / h / dh / dv, and (256, 512) -- xLSTM-Large's heads -- as
  * 4 x 8 head-dim-64 block problems).  The forward's fused cell-output epilogue (mlstm_b200_fw_epilogue) is available
- * for every shape this returns 1 for except (256, 512), where it is refused with MLSTM_B200_EUNSUPPORTED. */
+ * for every shape this returns 1 for except (256, 512), where it is refused with MLSTM_B200_EUNSUPPORTED.  A shape this
+ * returns 0 for runs on the exact kernels (fp32 FFMA) when its head dims are multiples of 4 with DHQK <= 256 and
+ * DHHV <= 512 -- fp32 at (256, 512), square 256 and (128, 256) included -- and is refused otherwise. */
 int mlstm_b200_tensor_path_supported(const mlstm_b200_shape* shape);
 
 /* Forward: h, n_out, m_out and optionally the last (C, n, m) states. */

@@ -48,7 +48,8 @@ struct ExactParams {
   int64_t dq_s[3], dk_s[3], dv_s[3], di_s[3], df_s[3];
   float* dc0;
   int DVT;  // dv slice width of the recurrent kernels
-  int rev;  // 1: anti-causal scan -- processing index t lives at memory token S-1-t (no data is moved)
+  int DVB;  // v column block of k_fw_h / k_bw_dqkv (= DV when the whole of v fits in shared memory)
+  int rev; // 1: anti-causal scan -- processing index t lives at memory token S-1-t (no data is moved)
   int sig;  // mlstm_b200_shape::siging: 1 sigmoid input gate, every max state 0; 2 the same without the normaliser
 };
 // memory token of processing index t, and the signed token step
@@ -191,18 +192,19 @@ __global__ void __launch_bounds__(kThreads) k_states(ExactParams p) {
 }
 
 // -------------------------------------------------------------------------------------------
-// k_fw_h: one CTA per (chunk, b*h)
+// k_fw_h: one CTA per (chunk, b*h).  P and the denominators are computed once; h is then written in column blocks
+// of width DVB, the V and C_{k-1} blocks taking turns in shared memory (one block when the whole of v fits).
 // -------------------------------------------------------------------------------------------
 template <typename T>
 __global__ void __launch_bounds__(kThreads) k_fw_h(ExactParams p) {
   extern __shared__ float smem[];
   const int c = blockIdx.x, bh = blockIdx.y, b = bh / p.NH, hh = bh % p.NH;
-  const int L = p.L, DK = p.DK, DV = p.DV;
-  const int ldk = DK + 1, ldv = DV + 1, ldp = L + 1;
+  const int L = p.L, DK = p.DK, DV = p.DV, DVB = p.DVB;
+  const int ldk = DK + 1, ldv = DVB + 1, ldp = L + 1;
   float* sQ = smem;
   float* sK = sQ + L * ldk;
-  float* sV = sK + L * ldk;
-  float* sC = sV + L * ldv;   // DK x ldv
+  float* sV = sK + L * ldk;   // L x ldv: one column block of V
+  float* sC = sV + L * ldv;   // DK x ldv: the same block of C_{k-1}
   float* sP = sC + DK * ldv;  // L x ldp
   float* sN = sP + L * ldp;   // DK
   float* sb = sN + DK;
@@ -215,12 +217,10 @@ __global__ void __launch_bounds__(kThreads) k_fw_h(ExactParams p) {
   const int64_t t0 = tok(p, (int64_t)c * L), sg = sgn(p);  // memory token of the chunk's first processed row
   load_tile<T>(sQ, ldk, (const T*)p.q.ptr + b * p.q.sb + hh * p.q.sh + t0 * p.q.ss, sg * p.q.ss, L, DK);
   load_tile<T>(sK, ldk, (const T*)p.k.ptr + b * p.k.sb + hh * p.k.sh + t0 * p.k.ss, sg * p.k.ss, L, DK);
-  load_tile<T>(sV, ldv, (const T*)p.v.ptr + b * p.v.sb + hh * p.v.sh + t0 * p.v.ss, sg * p.v.ss, L, DV);
+  const T* vp = (const T*)p.v.ptr + b * p.v.sb + hh * p.v.sh + t0 * p.v.ss;
   const float* Cs = p.Cst + ((int64_t)bh * (p.NC + 1) + c) * DK * DV;
-  for (int e = threadIdx.x; e < DK * DV; e += blockDim.x) {
-    int d = e / DV, x = e - d * DV;
-    sC[d * ldv + x] = Cs[e];
-  }
+  load_tile<T>(sV, ldv, vp, sg * p.v.ss, L, DVB);  // column block 0
+  load_tile<float>(sC, ldv, Cs, DV, DK, DVB);
   for (int d = threadIdx.x; d < DK; d += blockDim.x) sN[d] = p.Nst[((int64_t)bh * (p.NC + 1) + c) * DK + d];
   const float m_prev = p.Mst[(int64_t)bh * (p.NC + 1) + c];
   if (threadIdx.x < 32) {
@@ -264,9 +264,16 @@ __global__ void __launch_bounds__(kThreads) k_fw_h(ExactParams p) {
     p.m_out[(int64_t)bh * p.S + t0 + sg * t] = smt[t];
   }
   __syncthreads();
-  {  // h = (qbar C + P V) / (n + eps), fw.py:200-212
-    const int MS = L / 4, NS = DV / 4;
-    T* hp = (T*)p.h + b * p.h_sb + hh * p.h_sh + t0 * p.h_ss;
+  T* hp = (T*)p.h + b * p.h_sb + hh * p.h_sh + t0 * p.h_ss;
+  for (int e0 = 0; e0 < DV; e0 += DVB) {  // h = (qbar C + P V) / (n + eps), fw.py:200-212
+    const int W = min(DVB, DV - e0);
+    if (e0) {
+      __syncthreads();
+      load_tile<T>(sV, ldv, vp + e0, sg * p.v.ss, L, W);
+      load_tile<float>(sC, ldv, Cs + e0, DV, DK, W);
+      __syncthreads();
+    }
+    const int MS = L / 4, NS = W / 4;
     for (int idx = threadIdx.x; idx < MS * NS; idx += blockDim.x) {
       int tm = idx / NS, tn = idx - tm * NS;
       float a1[4][4], a2[4][4];
@@ -279,7 +286,7 @@ __global__ void __launch_bounds__(kThreads) k_fw_h(ExactParams p) {
 #pragma unroll
         for (int y = 0; y < 4; ++y) {
           int t = tm + x * MS, e = tn + y * NS;
-          hp[(int64_t)t * sg * p.h_ss + e] = from_f32<T>((sbq[t] * a1[x][y] + a2[x][y]) / sden[t]);
+          hp[(int64_t)t * sg * p.h_ss + e0 + e] = from_f32<T>((sbq[t] * a1[x][y] + a2[x][y]) / sden[t]);
         }
     }
   }
@@ -370,44 +377,77 @@ __global__ void __launch_bounds__(kThreads) k_bw_dc(ExactParams p) {
 }
 
 // -------------------------------------------------------------------------------------------
-// k_bw_dqkv: one CTA per (chunk, b*h)
+// k_bw_dqkv: one CTA per (chunk, b*h).  v is taken in column blocks of width DVB (one block when the whole of v
+// fits in shared memory).  Each block writes its columns of dV and adds its part to dS and dI; every block but the
+// last also adds its part of the inter-chunk terms of dK and dQ, which sum over v, to the accumulators sWk / sWq.
+// The final dK / dQ passes add the last block's part, so one block needs neither the accumulators nor extra passes.
 // -------------------------------------------------------------------------------------------
-template <typename T>
+__host__ __device__ __forceinline__ int spart_width(int DK, int DVB) { return max(32, max(DK, DVB) / 4); }
+
+__device__ __forceinline__ void load_acc(float (&acc)[4][4], const float* src, int ld, int tm, int MS, int tn, int NS) {
+#pragma unroll
+  for (int x = 0; x < 4; ++x)
+#pragma unroll
+    for (int y = 0; y < 4; ++y) acc[x][y] = src[(tm + x * MS) * ld + tn + y * NS];
+}
+__device__ __forceinline__ void store_acc(const float (&acc)[4][4], float* dst, int ld, int tm, int MS, int tn, int NS) {
+#pragma unroll
+  for (int x = 0; x < 4; ++x)
+#pragma unroll
+    for (int y = 0; y < 4; ++y) dst[(tm + x * MS) * ld + tn + y * NS] = acc[x][y];
+}
+
+template <typename T, bool kBlocked>  // kBlocked = false: DVB == DV, the loop below runs once
 __global__ void __launch_bounds__(kThreads) k_bw_dqkv(ExactParams p) {
   extern __shared__ float smem[];
   const int c = blockIdx.x, bh = blockIdx.y, b = bh / p.NH, hh = bh % p.NH;
-  const int L = p.L, DK = p.DK, DV = p.DV;
-  const int ldk = DK + 1, ldv = DV + 1, ldp = L + 1;
+  const int L = p.L, DK = p.DK, DV = p.DV, DVB = p.DVB, nblk = kBlocked ? (DV + DVB - 1) / DVB : 1;
+  const int ldk = DK + 1, ldv = DVB + 1, ldp = L + 1, spw = spart_width(DK, DVB);
   float* sQ = smem;
   float* sK = sQ + L * ldk;
-  float* sV = sK + L * ldk;
-  float* sH = sV + L * ldv;    // dH / (n + eps)
-  float* sC = sH + L * ldv;    // C_{k-1}   DK x ldv
-  float* sdC = sC + DK * ldv;  // dC_k      DK x ldv
+  float* sV = sK + L * ldk;    // V block               L x ldv
+  float* sH = sV + L * ldv;    // dH / (n + eps) block  L x ldv
+  float* sC = sH + L * ldv;    // C_{k-1} block         DK x ldv
+  float* sdC = sC + DK * ldv;  // dC_k block            DK x ldv
   float* sS = sdC + DK * ldv;  // Sbar      L x ldp
   float* sdS = sS + L * ldp;   // dS        L x ldp
-  float* spart = sdS + L * ldp;  // L x 32 row-dot partials
-  float* sb = spart + L * 32;
+  float* spart = sdS + L * ldp;  // L x spw row-dot partials
+  float* sb = spart + L * spw;
   float* si = sb + L;
   float* spm = si + L;
   float* sab = spm + L;   // abar
   float* sbb = sab + L;   // bbar
   float* smt = sbb + L;   // m_out
   float* sacc = smt + L;  // q.dq - k.dk
+  float* sWk = sacc + L;       // nblk > 1: V dC_k^T over the blocks before the last        L x ldk
+  float* sWq = sWk + L * ldk;  // nblk > 1: dHt C_{k-1}^T over the blocks before the last  L x ldk
+  float* sdi = sWq + L * ldk;  // nblk > 1: v . dv over the blocks before the last
   __shared__ float s_g;
 
   const int64_t t0 = tok(p, (int64_t)c * L), sg = sgn(p);
-  load_tile<T>(sQ, ldk, (const T*)p.q.ptr + b * p.q.sb + hh * p.q.sh + t0 * p.q.ss, sg * p.q.ss, L, DK);
-  load_tile<T>(sK, ldk, (const T*)p.k.ptr + b * p.k.sb + hh * p.k.sh + t0 * p.k.ss, sg * p.k.ss, L, DK);
-  load_tile<T>(sV, ldv, (const T*)p.v.ptr + b * p.v.sb + hh * p.v.sh + t0 * p.v.ss, sg * p.v.ss, L, DV);
-  load_tile<T>(sH, ldv, (const T*)p.dh.ptr + b * p.dh.sb + hh * p.dh.sh + t0 * p.dh.ss, sg * p.dh.ss, L, DV);
+  const T* vp = (const T*)p.v.ptr + b * p.v.sb + hh * p.v.sh + t0 * p.v.ss;
+  const T* dhp = (const T*)p.dh.ptr + b * p.dh.sb + hh * p.dh.sh + t0 * p.dh.ss;
   const float* Cs = p.Cst + ((int64_t)bh * (p.NC + 1) + c) * DK * DV;
   const float* dCs = p.dCst + ((int64_t)bh * (p.NC + 1) + c + 1) * DK * DV;
-  for (int e = threadIdx.x; e < DK * DV; e += blockDim.x) {
-    int d = e / DV, x = e - d * DV;
-    sC[d * ldv + x] = Cs[e];
-    sdC[d * ldv + x] = dCs[e];
-  }
+  auto load_block = [&](int e0, int W) {
+    load_tile<T>(sV, ldv, vp + e0, sg * p.v.ss, L, W);
+    load_tile<T>(sH, ldv, dhp + e0, sg * p.dh.ss, L, W);
+    for (int e = threadIdx.x; e < DK * W; e += blockDim.x) {
+      int d = e / W, x = e - d * W;
+      sC[d * ldv + x] = Cs[(int64_t)d * DV + e0 + x];
+      sdC[d * ldv + x] = dCs[(int64_t)d * DV + e0 + x];
+    }
+  };
+  auto normalise_dh = [&](int W) {  // bw.py:135; siging = 2: no normaliser, dh is used as it is
+    if (p.sig == 2) return;
+    for (int e = threadIdx.x; e < L * W; e += blockDim.x) {
+      int t = e / W, x = e - t * W;
+      sH[t * ldv + x] /= (p.n_out_in[(int64_t)bh * p.S + t0 + sg * t] + p.eps);
+    }
+  };
+  load_tile<T>(sQ, ldk, (const T*)p.q.ptr + b * p.q.sb + hh * p.q.sh + t0 * p.q.ss, sg * p.q.ss, L, DK);
+  load_tile<T>(sK, ldk, (const T*)p.k.ptr + b * p.k.sb + hh * p.k.sh + t0 * p.k.ss, sg * p.k.ss, L, DK);
+  load_block(0, DVB);
   if (threadIdx.x < 32) {
     float amax;
     float g = chunk_gate_scan<T>((const T*)p.ig.ptr + b * p.ig.sb + hh * p.ig.sh + t0 * p.ig.ss, sg * p.ig.ss,
@@ -423,74 +463,104 @@ __global__ void __launch_bounds__(kThreads) k_bw_dqkv(ExactParams p) {
     sab[t] = expf(s_g - sb[t] + si[t] - m_next);  // bw.py:181,187
     sbb[t] = expf(sb[t] + m_prev - mt);           // bw.py:186
   }
-  if (p.sig != 2) {  // siging = 2: no normaliser, dh is used as it is
-    for (int e = threadIdx.x; e < L * DV; e += blockDim.x) {
-      int t = e / DV, x = e - t * DV;
-      sH[t * ldv + x] /= (p.n_out_in[(int64_t)bh * p.S + t0 + sg * t] + p.eps);  // bw.py:135
-    }
-  }
-  __syncthreads();
-
-  {  // Sbar and dS, bw.py:153-167
-    const int MS = L / 4, NS = L / 4;
-    for (int idx = threadIdx.x; idx < MS * NS; idx += blockDim.x) {
-      int tm = idx / NS, tn = idx - tm * NS;
-      float a1[4][4], a2[4][4];
-      zero_tile(a1);
-      zero_tile(a2);
-      mm_tile<false, true>(sQ, ldk, sK, ldk, DK, tm, MS, tn, NS, a1);
-      mm_tile<false, true>(sH, ldv, sV, ldv, DV, tm, MS, tn, NS, a2);
-#pragma unroll
-      for (int x = 0; x < 4; ++x)
-#pragma unroll
-        for (int y = 0; y < 4; ++y) {
-          int t = tm + x * MS, s = tn + y * NS;
-          float d = (s <= t) ? expf(sb[t] - sb[s] + si[s] - smt[t]) : 0.f;
-          sS[t * ldp + s] = a1[x][y] * p.scale * d;
-          sdS[t * ldp + s] = a2[x][y] * d;
-        }
-    }
-  }
+  normalise_dh(DVB);
   __syncthreads();
 
   const int64_t tok0 = (int64_t)bh * p.S + (int64_t)c * L;  // the q.dq - k.dk workspace is in processing order
-  {  // dV = Sbar^T dHt + abar (K dC_k); dI = v . dv   (bw.py:164,190,326)
-    const int MS = L / 4, NS = DV / 4;
-    T* op = (T*)p.dv + b * p.dv_s[0] + hh * p.dv_s[1] + t0 * p.dv_s[2];
-    for (int idx0 = 0; idx0 < MS * NS; idx0 += blockDim.x) {
-      int idx = idx0 + threadIdx.x;
-      if (idx < MS * NS) {
+  T* dvp = (T*)p.dv + b * p.dv_s[0] + hh * p.dv_s[1] + t0 * p.dv_s[2];
+  T* dip = (T*)p.di + b * p.di_s[0] + hh * p.di_s[1] + t0 * p.di_s[2];
+  int e0 = 0, W = DVB;  // the block in shared memory: columns [e0, e0 + W)
+  for (int blk = 0; blk < nblk; ++blk) {
+    const bool last = blk == nblk - 1;
+    if (blk) {
+      e0 += DVB;
+      W = min(DVB, DV - e0);
+      __syncthreads();
+      load_block(e0, W);
+      __syncthreads();
+      normalise_dh(W);
+      __syncthreads();
+    }
+    {  // Sbar (first block) and dS (summed over the blocks, times D after the last), bw.py:153-167
+      const int MS = L / 4, NS = L / 4;
+      for (int idx = threadIdx.x; idx < MS * NS; idx += blockDim.x) {
         int tm = idx / NS, tn = idx - tm * NS;
         float a1[4][4], a2[4][4];
         zero_tile(a1);
-        zero_tile(a2);
-        mm_tile<true, false>(sS, ldp, sH, ldv, L, tm, MS, tn, NS, a1);
-        mm_tile<false, false>(sK, ldk, sdC, ldv, DK, tm, MS, tn, NS, a2);
+        if (blk) load_acc(a2, sdS, ldp, tm, MS, tn, NS);
+        else zero_tile(a2);
+        if (!blk) mm_tile<false, true>(sQ, ldk, sK, ldk, DK, tm, MS, tn, NS, a1);
+        mm_tile<false, true>(sH, ldv, sV, ldv, W, tm, MS, tn, NS, a2);
 #pragma unroll
-        for (int x = 0; x < 4; ++x) {
-          int s = tm + x * MS;
-          float part = 0.f;
+        for (int x = 0; x < 4; ++x)
 #pragma unroll
           for (int y = 0; y < 4; ++y) {
-            int e = tn + y * NS;
-            float val = a1[x][y] + sab[s] * a2[x][y];
-            op[(int64_t)s * sg * p.dv_s[2] + e] = from_f32<T>(val);
-            part = fmaf(sV[s * ldv + e], val, part);
+            int t = tm + x * MS, s = tn + y * NS;
+            float d = (s <= t && (!blk || last)) ? expf(sb[t] - sb[s] + si[s] - smt[t]) : 0.f;
+            if (!blk) sS[t * ldp + s] = a1[x][y] * p.scale * d;
+            sdS[t * ldp + s] = last ? a2[x][y] * d : a2[x][y];
           }
-          spart[s * 32 + tn] = part;
-        }
       }
     }
     __syncthreads();
-    T* dip = (T*)p.di + b * p.di_s[0] + hh * p.di_s[1] + t0 * p.di_s[2];
-    for (int s = threadIdx.x; s < L; s += blockDim.x) {
-      float r = 0.f;
-      for (int x = 0; x < NS; ++x) r += spart[s * 32 + x];
-      if (p.sig) r *= 1.f - expf(si[s]);  // d logsigmoid(i)/di = sigmoid(-i) = 1 - exp(logsigmoid(i))
-      dip[(int64_t)s * sg * p.di_s[2]] = from_f32<T>(r);
+    {  // dV = Sbar^T dHt + abar (K dC_k); dI = v . dv   (bw.py:164,190,326)
+      const int MS = L / 4, NS = W / 4;
+      for (int idx0 = 0; idx0 < MS * NS; idx0 += blockDim.x) {
+        int idx = idx0 + threadIdx.x;
+        if (idx < MS * NS) {
+          int tm = idx / NS, tn = idx - tm * NS;
+          float a1[4][4], a2[4][4];
+          zero_tile(a1);
+          zero_tile(a2);
+          mm_tile<true, false>(sS, ldp, sH, ldv, L, tm, MS, tn, NS, a1);
+          mm_tile<false, false>(sK, ldk, sdC, ldv, DK, tm, MS, tn, NS, a2);
+#pragma unroll
+          for (int x = 0; x < 4; ++x) {
+            int s = tm + x * MS;
+            float part = 0.f;
+#pragma unroll
+            for (int y = 0; y < 4; ++y) {
+              int e = tn + y * NS;
+              float val = a1[x][y] + sab[s] * a2[x][y];
+              dvp[(int64_t)s * sg * p.dv_s[2] + e0 + e] = from_f32<T>(val);
+              part = fmaf(sV[s * ldv + e], val, part);
+            }
+            spart[s * spw + tn] = part;
+          }
+        }
+      }
+      __syncthreads();
+      for (int s = threadIdx.x; s < L; s += blockDim.x) {
+        float r = blk ? sdi[s] : 0.f;
+        for (int x = 0; x < NS; ++x) r += spart[s * spw + x];
+        if (!last) {
+          sdi[s] = r;
+          continue;
+        }
+        if (p.sig) r *= 1.f - expf(si[s]);  // d logsigmoid(i)/di = sigmoid(-i) = 1 - exp(logsigmoid(i))
+        dip[(int64_t)s * sg * p.di_s[2]] = from_f32<T>(r);
+      }
     }
-    __syncthreads();
+    if (!last) {  // this block's part of V dC_k^T and dHt C_{k-1}^T
+      const int MS = L / 4, NS = DK / 4;
+      for (int idx = threadIdx.x; idx < MS * NS; idx += blockDim.x) {
+        int tm = idx / NS, tn = idx - tm * NS;
+        float a1[4][4], a2[4][4];
+        if (blk) {
+          load_acc(a1, sWk, ldk, tm, MS, tn, NS);
+          load_acc(a2, sWq, ldk, tm, MS, tn, NS);
+        } else {
+          zero_tile(a1);
+          zero_tile(a2);
+        }
+        mm_tile<false, true>(sV, ldv, sdC, ldv, W, tm, MS, tn, NS, a1);
+        mm_tile<false, true>(sH, ldv, sC, ldv, W, tm, MS, tn, NS, a2);
+        store_acc(a1, sWk, ldk, tm, MS, tn, NS);
+        store_acc(a2, sWq, ldk, tm, MS, tn, NS);
+      }
+    }
   }
+  __syncthreads();
   {  // dK = scale dS^T Q + abar (V dC_k^T)   (bw.py:170,192)
     const int MS = L / 4, NS = DK / 4;
     T* op = (T*)p.dk + b * p.dk_s[0] + hh * p.dk_s[1] + t0 * p.dk_s[2];
@@ -500,9 +570,10 @@ __global__ void __launch_bounds__(kThreads) k_bw_dqkv(ExactParams p) {
         int tm = idx / NS, tn = idx - tm * NS;
         float a1[4][4], a2[4][4];
         zero_tile(a1);
-        zero_tile(a2);
+        if (nblk > 1) load_acc(a2, sWk, ldk, tm, MS, tn, NS);
+        else zero_tile(a2);
         mm_tile<true, false>(sdS, ldp, sQ, ldk, L, tm, MS, tn, NS, a1);
-        mm_tile<false, true>(sV, ldv, sdC, ldv, DV, tm, MS, tn, NS, a2);
+        mm_tile<false, true>(sV, ldv, sdC, ldv, W, tm, MS, tn, NS, a2);
 #pragma unroll
         for (int x = 0; x < 4; ++x) {
           int s = tm + x * MS;
@@ -514,14 +585,14 @@ __global__ void __launch_bounds__(kThreads) k_bw_dqkv(ExactParams p) {
             op[(int64_t)s * sg * p.dk_s[2] + d] = from_f32<T>(val);
             part = fmaf(sK[s * ldk + d], val, part);
           }
-          spart[s * 32 + tn] = part;
+          spart[s * spw + tn] = part;
         }
       }
     }
     __syncthreads();
     for (int s = threadIdx.x; s < L; s += blockDim.x) {
       float r = 0.f;
-      for (int x = 0; x < NS; ++x) r += spart[s * 32 + x];
+      for (int x = 0; x < NS; ++x) r += spart[s * spw + x];
       sacc[s] = -r;
     }
     __syncthreads();
@@ -535,9 +606,10 @@ __global__ void __launch_bounds__(kThreads) k_bw_dqkv(ExactParams p) {
         int tm = idx / NS, tn = idx - tm * NS;
         float a1[4][4], a2[4][4];
         zero_tile(a1);
-        zero_tile(a2);
+        if (nblk > 1) load_acc(a2, sWq, ldk, tm, MS, tn, NS);
+        else zero_tile(a2);
         mm_tile<false, false>(sdS, ldp, sK, ldk, L, tm, MS, tn, NS, a1);
-        mm_tile<false, true>(sH, ldv, sC, ldv, DV, tm, MS, tn, NS, a2);
+        mm_tile<false, true>(sH, ldv, sC, ldv, W, tm, MS, tn, NS, a2);
 #pragma unroll
         for (int x = 0; x < 4; ++x) {
           int t = tm + x * MS;
@@ -549,14 +621,14 @@ __global__ void __launch_bounds__(kThreads) k_bw_dqkv(ExactParams p) {
             op[(int64_t)t * sg * p.dq_s[2] + d] = from_f32<T>(val);
             part = fmaf(sQ[t * ldk + d], val, part);
           }
-          spart[t * 32 + tn] = part;
+          spart[t * spw + tn] = part;
         }
       }
     }
     __syncthreads();
     for (int t = threadIdx.x; t < L; t += blockDim.x) {
       float r = 0.f;
-      for (int x = 0; x < NS; ++x) r += spart[t * 32 + x];
+      for (int x = 0; x < NS; ++x) r += spart[t * spw + x];
       p.acc[tok0 + t] = r + sacc[t];  // q.dq - k.dk, bw.py:321
     }
   }
@@ -593,28 +665,48 @@ __global__ void k_bw_df(ExactParams p) {
 // -------------------------------------------------------------------------------------------
 // host side
 // -------------------------------------------------------------------------------------------
-constexpr size_t kMaxSmem = 227 * 1024;
+// Dynamic shared memory a CTA may use: the 227 KB per-block limit less the kernels' static __shared__ scalars.
+constexpr size_t kMaxSmem = 227 * 1024 - 128;
 
 size_t smem_states(int L, int DK, int DVT) {
   return sizeof(float) * ((size_t)L * (DK + 1) + (size_t)L * (DVT | 1) + (size_t)DK * (DVT | 1) + DK + 4 * L);
 }
-size_t smem_fw_h(int L, int DK, int DV) {
-  return sizeof(float) * ((size_t)2 * L * (DK + 1) + (size_t)L * (DV + 1) + (size_t)DK * (DV + 1) + (size_t)L * (L + 1) +
-                          DK + 6 * L);
+size_t smem_fw_h(int L, int DK, int DVB) {
+  return sizeof(float) * ((size_t)2 * L * (DK + 1) + (size_t)L * (DVB + 1) + (size_t)DK * (DVB + 1) +
+                          (size_t)L * (L + 1) + DK + 6 * L);
 }
 size_t smem_bw_dc(int L, int DK, int DVT) {
   return sizeof(float) * ((size_t)L * (DK + 1) + (size_t)L * (DVT | 1) + (size_t)DK * (DVT | 1) + 3 * L);
 }
-size_t smem_bw_dqkv(int L, int DK, int DV) {
-  return sizeof(float) * ((size_t)2 * L * (DK + 1) + (size_t)2 * L * (DV + 1) + (size_t)2 * DK * (DV + 1) +
-                          (size_t)2 * L * (L + 1) + (size_t)L * 32 + 7 * L);
+size_t smem_bw_dqkv(int L, int DK, int DV, int DVB) {
+  size_t n = (size_t)2 * L * (DK + 1) + (size_t)2 * L * (DVB + 1) + (size_t)2 * DK * (DVB + 1) + (size_t)2 * L * (L + 1) +
+             (size_t)L * spart_width(DK, DVB) + 7 * L;
+  if (DVB < DV) n += (size_t)2 * L * (DK + 1) + L;  // the accumulators over the v blocks
+  return sizeof(float) * n;
 }
 
-// Largest internal chunk (dividing the requested one) whose tiles fit in shared memory.
+constexpr int kMaxDK = 256, kMaxDV = 512;
+
+// v column block of k_fw_h (backward = 0) or k_bw_dqkv (1) at internal chunk L: the widest that fits in shared
+// memory, from splitting v into as few near-equal blocks of a multiple of 4 columns as possible; 0 if none fits.
+int pick_dvb(int L, int DK, int DV, int backward) {
+  for (int n = 1; n <= DV / 4; ++n) {
+    const int dvb = ((DV + n - 1) / n + 3) & ~3;
+    if ((backward ? smem_bw_dqkv(L, DK, DV, dvb) : smem_fw_h(L, DK, dvb)) <= kMaxSmem) return dvb;
+  }
+  return 0;
+}
+
+// Largest internal chunk (dividing the requested one) whose tiles fit in shared memory.  A chunk that keeps the
+// whole of v resident in both kernels is preferred over a larger one that needs v blocks.
 int pick_chunk(const mlstm_b200_shape& s) {
-  for (int L = s.chunk_size < 64 ? s.chunk_size : 64; L >= 4; --L) {
-    if ((s.chunk_size % L) || (L & 3)) continue;
-    if (smem_bw_dqkv(L, s.DHQK, s.DHHV) <= kMaxSmem && smem_fw_h(L, s.DHQK, s.DHHV) <= kMaxSmem) return L;
+  if ((s.DHQK & 3) || (s.DHHV & 3) || s.DHQK > kMaxDK || s.DHHV > kMaxDV) return 0;
+  for (int blocked = 0; blocked < 2; ++blocked) {
+    for (int L = s.chunk_size < 64 ? s.chunk_size : 64; L >= 4; --L) {
+      if ((s.chunk_size % L) || (L & 3)) continue;
+      const int fw = pick_dvb(L, s.DHQK, s.DHHV, 0), bw = pick_dvb(L, s.DHQK, s.DHHV, 1);
+      if (fw && bw && (blocked || (fw == s.DHHV && bw == s.DHHV))) return L;
+    }
   }
   return 0;
 }
@@ -628,8 +720,9 @@ int check_shape(const mlstm_b200_shape& s) {
     set_error("Sequence length %d is not divisible by chunk size %d.", s.S, s.chunk_size);
     return MLSTM_B200_EINVAL;
   }
-  if ((s.DHQK & 3) || (s.DHHV & 3) || s.DHQK > 128 || s.DHHV > 128) {
-    set_error("exact path needs head dims that are multiples of 4 and <= 128 (got %d, %d)", s.DHQK, s.DHHV);
+  if ((s.DHQK & 3) || (s.DHHV & 3) || s.DHQK > kMaxDK || s.DHHV > kMaxDV) {
+    set_error("exact path needs head dims that are multiples of 4 with DHQK <= %d and DHHV <= %d (got %d, %d)", kMaxDK,
+              kMaxDV, s.DHQK, s.DHHV);
     return MLSTM_B200_EUNSUPPORTED;
   }
   if (pick_chunk(s) == 0) {
@@ -672,10 +765,13 @@ int set_smem(K kernel, size_t bytes) {
   return 0;
 }
 
-int pick_dvt(const mlstm_b200_shape& s) {
-  // slice dv so that the sequential kernels expose more CTAs; keep slices multiples of 4
+int pick_dvt(const mlstm_b200_shape& s, int L) {
+  // slice dv so that the sequential kernels expose more CTAs and their tiles fit in shared memory; keep slices
+  // multiples of 4 (the last one may be narrower)
+  auto fits = [&](int d) { return smem_states(L, s.DHQK, d) <= kMaxSmem && smem_bw_dc(L, s.DHQK, d) <= kMaxSmem; };
   int dvt = s.DHHV;
-  while (dvt > 16 && (dvt % 8) == 0 && (long)s.B * s.NH * (s.DHHV / dvt) < 592) dvt /= 2;
+  while (dvt > 16 && (dvt % 8) == 0 && ((long)s.B * s.NH * (s.DHHV / dvt) < 592 || !fits(dvt))) dvt /= 2;
+  while (!fits(dvt)) dvt = (dvt / 2 + 3) & ~3;
   return dvt;
 }
 
@@ -719,12 +815,13 @@ int exact_fw(const mlstm_b200_fw_args& a, cudaStream_t st) {
   p.h = a.h.ptr; p.h_sb = a.h.stride[0]; p.h_sh = a.h.stride[1]; p.h_ss = a.h.stride[2];
   p.n_out = a.n_out; p.m_out = a.m_out;
   p.c_last = a.c_last; p.n_last = a.n_last; p.m_last = a.m_last;
-  p.DVT = pick_dvt(s);
+  p.DVT = pick_dvt(s, L);
+  p.DVB = pick_dvb(L, p.DK, p.DV, 0);
   p.rev = s.reverse ? 1 : 0;
   p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
   MLSTM_DISPATCH_DTYPE(s.dtype, T, {
     if (int e = launch_states<T>(p, st)) return e;
-    size_t sm = smem_fw_h(L, p.DK, p.DV);
+    size_t sm = smem_fw_h(L, p.DK, p.DVB);
     if (int e = set_smem(k_fw_h<T>, sm)) return e;
     k_fw_h<T><<<dim3(p.NC, p.B * p.NH), kThreads, sm, st>>>(p);
     count_launch();
@@ -759,7 +856,8 @@ int exact_bw(const mlstm_b200_bw_args& a, cudaStream_t st) {
     p.di_s[x] = a.di.stride[x]; p.df_s[x] = a.df.stride[x];
   }
   p.dc0 = a.dc_initial;
-  p.DVT = pick_dvt(s);
+  p.DVT = pick_dvt(s, L);
+  p.DVB = pick_dvb(L, p.DK, p.DV, 1);
   p.rev = s.reverse ? 1 : 0;
   p.sig = s.siging;  // 0, 1 or 2 (checked at the C-ABI)
   MLSTM_DISPATCH_DTYPE(s.dtype, T, {
@@ -769,9 +867,10 @@ int exact_bw(const mlstm_b200_bw_args& a, cudaStream_t st) {
     k_bw_dc<T><<<dim3(p.B * p.NH, (p.DV + p.DVT - 1) / p.DVT), kThreads, sm, st>>>(p);
     count_launch();
     MLSTM_CUDA_CHECK(cudaGetLastError());
-    sm = smem_bw_dqkv(L, p.DK, p.DV);
-    if (int e = set_smem(k_bw_dqkv<T>, sm)) return e;
-    k_bw_dqkv<T><<<dim3(p.NC, p.B * p.NH), kThreads, sm, st>>>(p);
+    sm = smem_bw_dqkv(L, p.DK, p.DV, p.DVB);
+    auto dqkv = p.DVB < p.DV ? k_bw_dqkv<T, true> : k_bw_dqkv<T, false>;
+    if (int e = set_smem(dqkv, sm)) return e;
+    dqkv<<<dim3(p.NC, p.B * p.NH), kThreads, sm, st>>>(p);
     count_launch();
     MLSTM_CUDA_CHECK(cudaGetLastError());
     k_bw_df<T><<<p.B * p.NH, 32, 0, st>>>(p);
