@@ -4,6 +4,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace mlstm {
@@ -79,16 +81,102 @@ int require_device() {
   return 0;
 }
 
-bool use_tensor(const mlstm_b200_shape& s, int backward, int* err) {
+bool use_tensor(const mlstm_b200_shape& s, int* err) {
   *err = 0;
   if (s.impl == MLSTM_B200_IMPL_EXACT) return false;
-  bool ok = tensor_supported(s, backward);
+  bool ok = tensor_supported(s);
   if (s.impl == MLSTM_B200_IMPL_TENSOR && !ok) {
     set_error("tensor-core path does not cover dtype=%d DHQK=%d DHHV=%d chunk=%d", s.dtype, s.DHQK, s.DHHV,
               s.chunk_size);
     *err = MLSTM_B200_EUNSUPPORTED;
   }
   return ok;
+}
+
+// Validation and route choice of mlstm_b200_chunkwise_fw (Args = mlstm_b200_fw_args) and _bw (mlstm_b200_bw_args), in
+// the order the checks run; *tc: the call goes to the tensor-core kernels, otherwise to the exact ones.
+template <typename Args>
+int chunkwise_route(const Args& a, bool* tc) {
+  constexpr bool bw = std::is_same<Args, mlstm_b200_bw_args>::value;
+  const mlstm_b200_shape& s = a.shape;
+  if (int e = check_qkv(a.q, "q")) return e;
+  if (int e = check_qkv(a.k, "k")) return e;
+  if (int e = check_qkv(a.v, "v")) return e;
+  if constexpr (bw) {
+    if (int e = check_qkv(a.dh, "dh")) return e;
+    if (int e = check_qkv(a.dq, "dq")) return e;
+    if (int e = check_qkv(a.dk, "dk")) return e;
+    if (int e = check_qkv(a.dv, "dv")) return e;
+  } else if (a.epilogue) {  // fused cell-output epilogue: y is mandatory, the un-normalised h optional
+    if (int e = check_qkv(a.epilogue->y, "epilogue.y")) return e;
+    if (a.h.ptr)
+      if (int e = check_qkv(a.h, "h")) return e;
+  } else if (int e = check_qkv(a.h, "h")) {
+    return e;
+  }
+  if (int e = check_vec(a.i, "i")) return e;
+  if (int e = check_vec(a.f, "f")) return e;
+  if constexpr (bw) {
+    if (int e = check_vec(a.di, "di")) return e;
+    if (int e = check_vec(a.df, "df")) return e;
+  }
+  if (!a.n_out || !a.m_out) {
+    set_error("n_out / m_out are NULL");
+    return MLSTM_B200_EINVAL;
+  }
+  int ninit = (a.c_initial != 0) + (a.n_initial != 0) + (a.m_initial != 0);
+  if constexpr (bw) {
+    if (ninit != 0 && ninit != 3) {
+      set_error("initial states must be given all three or none");
+      return MLSTM_B200_EINVAL;
+    }
+  } else {
+    int nlast = (a.c_last != 0) + (a.n_last != 0) + (a.m_last != 0);
+    if ((ninit != 0 && ninit != 3) || (nlast != 0 && nlast != 3)) {
+      set_error("initial / last states must be given all three or none");
+      return MLSTM_B200_EINVAL;
+    }
+  }
+  if (s.S % (s.chunk_size > 0 ? s.chunk_size : 1)) {
+    set_error("Sequence length %d is not divisible by chunk size %d.", s.S, s.chunk_size);
+    return MLSTM_B200_EINVAL;
+  }
+  if (int e = check_siging(s.siging)) return e;
+  if constexpr (!bw) {
+    if (a.epilogue && s.siging == 2) {  // the cell it fuses (MatrixLSTMCell) always normalises
+      set_error("the fused cell-output epilogue does not cover siging = 2 (no normaliser)");
+      return MLSTM_B200_EUNSUPPORTED;
+    }
+  }
+  if (int e = require_device()) return e;
+  int err = 0;
+  *tc = use_tensor(s, &err);
+  if (err) return err;
+  // AUTO accepts any strides like the reference does (torch/utils.py:30-42): views a TMA tensor map cannot describe
+  // (odd offsets, strides that are not multiples of 16 bytes) go to the exact kernels, which take any stride.  The
+  // exact family needs its own (larger) workspace: mlstm_b200_workspace_bytes with impl = EXACT.
+  if (*tc && s.impl == MLSTM_B200_IMPL_AUTO && !tensor_views_ok(a)) *tc = false;
+  if (!*tc && s.gate_soft_cap > 0.f) {
+    set_error("gate_soft_cap is applied by the tensor-core kernels only; cap the gates before an exact-route call");
+    return MLSTM_B200_EUNSUPPORTED;
+  }
+  if constexpr (bw) {
+    const int gd = s.grad_dtype;
+    if (gd != 0 && gd != s.dtype) {
+      if (gd != MLSTM_B200_BF16 && gd != MLSTM_B200_F16) {
+        set_error("grad_dtype must be 0, MLSTM_B200_BF16 or MLSTM_B200_F16 (got %d)", gd);
+        return MLSTM_B200_EINVAL;
+      }
+      if (!*tc) {
+        set_error("gradients in a dtype other than shape.dtype are written by the tensor-core kernels only");
+        return MLSTM_B200_EUNSUPPORTED;
+      }
+    }
+  } else if (!*tc && a.epilogue) {
+    set_error("the fused cell-output epilogue exists on the tensor-core route only (use mlstm_b200_cellout_fw)");
+    return MLSTM_B200_EUNSUPPORTED;
+  }
+  return 0;
 }
 
 }  // namespace
@@ -118,19 +206,19 @@ int mlstm_b200_debug_fw_epilogue_clusters(const mlstm_b200_shape* shape) {
 
 int mlstm_b200_tensor_path_supported(const mlstm_b200_shape* shape) {
   if (!shape) return 0;
-  return (tensor_supported(*shape, 0) && tensor_supported(*shape, 1)) ? 1 : 0;
+  return tensor_supported(*shape) ? 1 : 0;
 }
 
 size_t mlstm_b200_states_bytes(const mlstm_b200_shape* shape) {
   if (!shape) return 0;
   int err = 0;
-  return use_tensor(*shape, 1, &err) ? tensor_states_bytes(*shape) : 0;
+  return use_tensor(*shape, &err) ? tensor_states_bytes(*shape) : 0;
 }
 
 size_t mlstm_b200_workspace_bytes(const mlstm_b200_shape* shape, int backward) {
   if (!shape) return 0;
   int err = 0;
-  size_t n = use_tensor(*shape, backward, &err) ? tensor_workspace_bytes(*shape, backward)
+  size_t n = use_tensor(*shape, &err) ? tensor_workspace_bytes(*shape, backward)
                                       : exact_workspace_bytes(*shape, backward);
   return n < 256 ? 256 : n;
 }
@@ -142,53 +230,8 @@ int mlstm_b200_chunkwise_fw(const mlstm_b200_fw_args* a, void* stream) {
     set_error("args is NULL");
     return MLSTM_B200_EINVAL;
   }
-  if (int e = check_qkv(a->q, "q")) return e;
-  if (int e = check_qkv(a->k, "k")) return e;
-  if (int e = check_qkv(a->v, "v")) return e;
-  if (a->epilogue) {  // fused cell-output epilogue: y is mandatory, the un-normalised h optional
-    if (int e = check_qkv(a->epilogue->y, "epilogue.y")) return e;
-    if (a->h.ptr)
-      if (int e = check_qkv(a->h, "h")) return e;
-  } else if (int e = check_qkv(a->h, "h")) {
-    return e;
-  }
-  if (int e = check_vec(a->i, "i")) return e;
-  if (int e = check_vec(a->f, "f")) return e;
-  if (!a->n_out || !a->m_out) {
-    set_error("n_out / m_out are NULL");
-    return MLSTM_B200_EINVAL;
-  }
-  int ninit = (a->c_initial != 0) + (a->n_initial != 0) + (a->m_initial != 0);
-  int nlast = (a->c_last != 0) + (a->n_last != 0) + (a->m_last != 0);
-  if ((ninit != 0 && ninit != 3) || (nlast != 0 && nlast != 3)) {
-    set_error("initial / last states must be given all three or none");
-    return MLSTM_B200_EINVAL;
-  }
-  if (a->shape.S % (a->shape.chunk_size > 0 ? a->shape.chunk_size : 1)) {
-    set_error("Sequence length %d is not divisible by chunk size %d.", a->shape.S, a->shape.chunk_size);
-    return MLSTM_B200_EINVAL;
-  }
-  if (int e = check_siging(a->shape.siging)) return e;
-  if (a->epilogue && a->shape.siging == 2) {  // the cell it fuses (MatrixLSTMCell) always normalises
-    set_error("the fused cell-output epilogue does not cover siging = 2 (no normaliser)");
-    return MLSTM_B200_EUNSUPPORTED;
-  }
-  if (int e = require_device()) return e;
-  int err = 0;
-  bool tc = use_tensor(a->shape, 0, &err);
-  if (err) return err;
-  // AUTO accepts any strides like the reference does (torch/utils.py:30-42): views a TMA tensor map cannot describe
-  // (odd offsets, strides that are not multiples of 16 bytes) go to the exact kernels, which take any stride.  The
-  // exact family needs its own (larger) workspace: mlstm_b200_workspace_bytes with impl = EXACT.
-  if (tc && a->shape.impl == MLSTM_B200_IMPL_AUTO && !tensor_fw_views_ok(*a)) tc = false;
-  if (!tc && a->shape.gate_soft_cap > 0.f) {
-    set_error("gate_soft_cap is applied by the tensor-core kernels only; cap the gates before an exact-route call");
-    return MLSTM_B200_EUNSUPPORTED;
-  }
-  if (!tc && a->epilogue) {
-    set_error("the fused cell-output epilogue exists on the tensor-core route only (use mlstm_b200_cellout_fw)");
-    return MLSTM_B200_EUNSUPPORTED;
-  }
+  bool tc = false;
+  if (int e = chunkwise_route(*a, &tc)) return e;
   return tc ? tensor_fw(*a, (cudaStream_t)stream) : exact_fw(*a, (cudaStream_t)stream);
 }
 
@@ -199,51 +242,8 @@ int mlstm_b200_chunkwise_bw(const mlstm_b200_bw_args* a, void* stream) {
     set_error("args is NULL");
     return MLSTM_B200_EINVAL;
   }
-  if (int e = check_qkv(a->q, "q")) return e;
-  if (int e = check_qkv(a->k, "k")) return e;
-  if (int e = check_qkv(a->v, "v")) return e;
-  if (int e = check_qkv(a->dh, "dh")) return e;
-  if (int e = check_qkv(a->dq, "dq")) return e;
-  if (int e = check_qkv(a->dk, "dk")) return e;
-  if (int e = check_qkv(a->dv, "dv")) return e;
-  if (int e = check_vec(a->i, "i")) return e;
-  if (int e = check_vec(a->f, "f")) return e;
-  if (int e = check_vec(a->di, "di")) return e;
-  if (int e = check_vec(a->df, "df")) return e;
-  if (!a->n_out || !a->m_out) {
-    set_error("n_out / m_out are NULL");
-    return MLSTM_B200_EINVAL;
-  }
-  int ninit = (a->c_initial != 0) + (a->n_initial != 0) + (a->m_initial != 0);
-  if (ninit != 0 && ninit != 3) {
-    set_error("initial states must be given all three or none");
-    return MLSTM_B200_EINVAL;
-  }
-  if (a->shape.S % (a->shape.chunk_size > 0 ? a->shape.chunk_size : 1)) {
-    set_error("Sequence length %d is not divisible by chunk size %d.", a->shape.S, a->shape.chunk_size);
-    return MLSTM_B200_EINVAL;
-  }
-  if (int e = check_siging(a->shape.siging)) return e;
-  if (int e = require_device()) return e;
-  int err = 0;
-  bool tc = use_tensor(a->shape, 1, &err);
-  if (err) return err;
-  if (tc && a->shape.impl == MLSTM_B200_IMPL_AUTO && !tensor_bw_views_ok(*a)) tc = false;  // see the forward
-  if (!tc && a->shape.gate_soft_cap > 0.f) {
-    set_error("gate_soft_cap is applied by the tensor-core kernels only; cap the gates before an exact-route call");
-    return MLSTM_B200_EUNSUPPORTED;
-  }
-  const int gd = a->shape.grad_dtype;
-  if (gd != 0 && gd != a->shape.dtype) {
-    if (gd != MLSTM_B200_BF16 && gd != MLSTM_B200_F16) {
-      set_error("grad_dtype must be 0, MLSTM_B200_BF16 or MLSTM_B200_F16 (got %d)", gd);
-      return MLSTM_B200_EINVAL;
-    }
-    if (!tc) {
-      set_error("gradients in a dtype other than shape.dtype are written by the tensor-core kernels only");
-      return MLSTM_B200_EUNSUPPORTED;
-    }
-  }
+  bool tc = false;
+  if (int e = chunkwise_route(*a, &tc)) return e;
   return tc ? tensor_bw(*a, (cudaStream_t)stream) : exact_bw(*a, (cudaStream_t)stream);
 }
 

@@ -178,13 +178,13 @@ size_t exact_workspace_bytes(const mlstm_b200_shape& s, int backward);
 int exact_fw(const mlstm_b200_fw_args& a, cudaStream_t st);
 int exact_bw(const mlstm_b200_bw_args& a, cudaStream_t st);
 
-bool tensor_supported(const mlstm_b200_shape& s, int backward);
+bool tensor_supported(const mlstm_b200_shape& s);
 size_t tensor_workspace_bytes(const mlstm_b200_shape& s, int backward);
 size_t tensor_states_bytes(const mlstm_b200_shape& s);
 void tensor_set_clock_buffer(void* dev_ptr);
 bool tensor_context_is_current();  // a CUDA context is current on the calling thread (driver-level query)
-bool tensor_fw_views_ok(const mlstm_b200_fw_args& a);
-bool tensor_bw_views_ok(const mlstm_b200_bw_args& a);
+bool tensor_views_ok(const mlstm_b200_fw_args& a);
+bool tensor_views_ok(const mlstm_b200_bw_args& a);
 int tensor_fw(const mlstm_b200_fw_args& a, cudaStream_t st);
 int tensor_fw_epilogue_clusters(const mlstm_b200_shape& s);
 int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st);

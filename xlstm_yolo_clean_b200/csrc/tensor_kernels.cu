@@ -2468,28 +2468,53 @@ bool tma_ok(const mlstm_b200_tensor& t) {
 }
 
 // [128 tokens][min(D, 64)] boxes: D = 32 -> 64-byte rows / SWIZZLE_64B, otherwise 128-byte rows / SWIZZLE_128B.
-// `box` < D: D-wide rows read or written in box-wide column blocks (v / h of the rectangular forward).
+// `box` < D: D-wide rows read or written in box-wide column blocks (v / h of the rectangular and wide forwards).
 int make_map(CUtensorMap* m, const mlstm_b200_tensor& t, const mlstm_b200_shape& s, int D, int box = 0) {
   return sm100_host::make_map_bhsd(m, t.ptr, s.dtype == MLSTM_B200_BF16, s.B, s.NH, s.S, D, t.stride[0], t.stride[1],
                                    t.stride[2], LT, box ? box : D == 32 ? 32 : 64);
 }
-// c_states: (B, NH, NT, D, D) 16-bit, one [D][D] box per tile
-int make_states_map(CUtensorMap* m, const void* ptr, const mlstm_b200_shape& s) {
-  const int NT = (s.S + LT - 1) / LT, D = s.DHQK;
-  return sm100_host::make_map_bhsd(m, ptr, s.dtype == MLSTM_B200_BF16, s.B, s.NH, NT * D, D, (int64_t)s.NH * NT * D * D,
-                                   (int64_t)NT * D * D, D, D, D);
-}
 
-// states stored as bd x bd blocks: (B, NH, NT * rows, bd), `rows` = (DHQK / bd) (DHHV / bd) bd rows per tile, block
-// (a, b) of a tile at rows (a DHHV / bd + b) bd.  Head dim 128: bd = 64, four blocks (see tc_fw_d128::store_state);
-// rectangular heads (D, 2 D): bd = D, two blocks (tc_fw_rect).
+// c_states: the state entering every tile stored as bd x bd blocks, (B, NH, NT * rows, bd) 16-bit with `rows` = nq nv bd
+// rows per tile and block (a, b) of a tile at rows (a nv + b) bd (tc_fw_d128::store_state, tc_fw_rect, tc_fw_wide).  A
+// square head is block 0 of 1: one [D][D] box per tile.
 int make_states_map_blocks(CUtensorMap* m, const void* ptr, const mlstm_b200_shape& s, int rows, int bd) {
   const int NT = (s.S + LT - 1) / LT;
   return sm100_host::make_map_bhsd(m, ptr, s.dtype == MLSTM_B200_BF16, s.B, s.NH, NT * rows, bd, (int64_t)s.NH * NT * rows * bd,
                                    (int64_t)NT * rows * bd, bd, bd, bd);
 }
-bool rect_heads(const mlstm_b200_shape& s) { return s.DHQK != s.DHHV; }
-bool wide_heads(const mlstm_b200_shape& s) { return s.DHQK == 256 && s.DHHV == 512; }
+
+enum class TcFw { none, square, d128, rect, wide };  // the forward kernel families (none: not on the tensor-core route)
+
+// How the tensor-core route cuts a head geometry: a (DHQK, DHHV) head is an nq x nv grid of bd x bd blocks.  The forward
+// reads and writes v / h in bd-wide column boxes and stores each tile's state as those blocks (make_states_map_blocks);
+// the backward runs one tc_bw<bd> problem per block (bw_by_blocks), or one native problem when the grid is 1 x 1.
+struct TcGeometry {
+  TcFw fw;
+  int bd, nq, nv;
+  int ctas;         // forward CTAs per (batch, head)
+  bool epilogue;    // the fused cell-output epilogue exists ...
+  bool cluster;     // ... and exchanges LayerNorm statistics between the two CTAs of a head: a {2, 1, 1} cluster
+  bool gate_parts;  // the backward sums the block problems' dI / dF in fp32 (k_sum_gate_partials)
+};
+
+// The one place that knows which (DHQK, DHHV) the tensor-core kernels cover and how each is cut.
+TcGeometry tc_geometry(const mlstm_b200_shape& s) {
+  // Tiles are 128 tokens whatever chunk_size is (h and the states do not depend on it: the stabiliser equals the
+  // step-recurrent one), and ragged last tiles are handled in-kernel (TMA zero-fill, gates masked at scan time),
+  // so any S that keeps the fp32 n_out / m_out rows 16-byte aligned is covered; S % chunk_size == 0 is enforced
+  // at the C-ABI like the reference does (native/fw.py:252-254).
+  if ((s.dtype != MLSTM_B200_BF16 && s.dtype != MLSTM_B200_F16) || s.S % 4 != 0) return {TcFw::none};
+  const int dk = s.DHQK, dv = s.DHHV;
+  const bool d32_64 = dk == 32 || dk == 64;
+  //                                       fw          bd  nq nv  ctas            epilogue cluster gate_parts
+  if (d32_64 && dv == dk)       return {TcFw::square, dk, 1, 1, 1,              true,    false,  false};
+  // a 128-wide tile set does not fit the backward's shared memory with 128-token tiles: 2 x 2 blocks of 64
+  if (dk == 128 && dv == 128)   return {TcFw::d128,   64, 2, 2, 1,              true,    false,  false};
+  if (d32_64 && dv == 2 * dk)   return {TcFw::rect,   dk, 1, 2, 2,              true,    true,   false};
+  // xLSTM-Large; the in-kernel accumulation of dI / dF would round their running sum to 16 bits 31 times
+  if (dk == 256 && dv == 512)   return {TcFw::wide,   64, 4, 8, FwSmemWide::VB, false,   false,  true};
+  return {TcFw::none};
+}
 
 // Gate, scale and direction fields that TcFwParams and TcBwParams share
 template <typename P>
@@ -2530,40 +2555,15 @@ auto fw_rect_kernel(bool epi, bool rev) {
   return fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw_rect<T, D, decltype(r)::value, decltype(e)::value>; });
 }
 
-// (256, 512): tc_fw_wide, eight 64-wide column blocks of v / h / C per head; h is written from the registers
-int run_fw_wide(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
-  const mlstm_b200_shape& s = a.shape;
-  if (a.epilogue) {
-    set_error("the fused cell-output epilogue does not cover (DHQK, DHHV) = (256, 512)");
-    return MLSTM_B200_EUNSUPPORTED;
-  }
-  if (!tma_ok(a.q) || !tma_ok(a.k) || !tma_ok(a.v) || !tma_ok(a.h)) {
-    set_error("tensor path needs 16-byte aligned q/k/v/h with strides that are multiples of 8 elements");
-    return MLSTM_B200_EUNSUPPORTED;
-  }
-  CUtensorMap mq, mk, mv, mcs;
-  int r = make_map(&mq, a.q, s, s.DHQK) | make_map(&mk, a.k, s, s.DHQK) | make_map(&mv, a.v, s, s.DHHV, 64);
-  // without a c_states buffer the map is never used by the kernel; point it at v to keep it valid
-  r |= c_states ? make_states_map_blocks(&mcs, c_states, s, (s.DHQK / 64) * s.DHHV, 64) : make_map(&mcs, a.v, s, s.DHHV, 64);
-  if (r) {
-    set_error("cuTensorMapEncodeTiled failed (%d)", r);
-    return MLSTM_B200_ENODEVICE;
-  }
-  const TcFwParams p = fw_params(a, c_states);
-  return with_dtype(s.dtype, [&](auto t) {
-    using T = decltype(t);
-    auto kern = fw_kernel(false, p.rev, [](auto, auto r) { return tc_fw_wide<T, decltype(r)::value>; });
-    return launch_fw(kern, p, FwSmemWide::VB, FwSmemWide::kBytes, false, false, st, mq, mk, mv, mcs);
-  });
-}
-
 int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   const mlstm_b200_shape& s = a.shape;
-  if (wide_heads(s)) return run_fw_wide(a, c_states, st);
+  const TcGeometry g = tc_geometry(s);
   const mlstm_b200_fw_epilogue* ep = a.epilogue;
-  // with the fused epilogue the tensor map describes y (the un-normalised h, if wanted, is stored from registers)
-  const mlstm_b200_tensor& out = ep ? ep->y : a.h;
-  if (!tma_ok(a.q) || !tma_ok(a.k) || !tma_ok(a.v) || !tma_ok(out)) {
+  if (ep && !g.epilogue) {
+    set_error("the fused cell-output epilogue does not cover (DHQK, DHHV) = (%d, %d)", s.DHQK, s.DHHV);
+    return MLSTM_B200_EUNSUPPORTED;
+  }
+  if (!tensor_views_ok(a)) {
     set_error("tensor path needs 16-byte aligned q/k/v/h with strides that are multiples of 8 elements");
     return MLSTM_B200_EUNSUPPORTED;
   }
@@ -2577,18 +2577,19 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
       return MLSTM_B200_EUNSUPPORTED;
     }
   }
-  CUtensorMap mq, mk, mv, mh, mcs;
+  // with the fused epilogue the h map describes y (the un-normalised h, if wanted, is stored from registers); tc_fw_wide
+  // stores h from the registers and takes no h map
+  const mlstm_b200_tensor& out = ep ? ep->y : a.h;
   mlstm_b200_shape so = s;  // the y map carries y's element type
   if (ep) so.dtype = ep->xy_dtype;
-  const bool rect = rect_heads(s);
-  const int vbox = rect ? s.DHQK : 0;  // rectangular heads: v / h in DHQK-wide column blocks
-  int r = make_map(&mq, a.q, s, s.DHQK) | make_map(&mk, a.k, s, s.DHQK) | make_map(&mv, a.v, s, s.DHHV, vbox) |
-          make_map(&mh, out, so, s.DHHV, vbox);
-  // without a c_states buffer the map is never used by the kernel; point it at the output to keep it valid
-  r |= !c_states ? make_map(&mcs, out, so, s.DHHV, vbox)
-       : s.DHQK == 128 ? make_states_map_blocks(&mcs, c_states, s, 256, 64)
-       : rect          ? make_states_map_blocks(&mcs, c_states, s, s.DHHV, s.DHQK)
-                       : make_states_map(&mcs, c_states, s);
+  CUtensorMap mq, mk, mv, mh, mcs;
+  int r = make_map(&mq, a.q, s, s.DHQK) | make_map(&mk, a.k, s, s.DHQK) | make_map(&mv, a.v, s, s.DHHV, g.bd) |
+          make_map(&mh, out, so, s.DHHV, g.bd);
+  // without a c_states buffer the map is never used by the kernel; a copy of the h map keeps it valid
+  if (c_states)
+    r |= make_states_map_blocks(&mcs, c_states, s, g.nq * g.nv * g.bd, g.bd);
+  else
+    mcs = mh;
   if (r) {
     set_error("cuTensorMapEncodeTiled failed (%d)", r);
     return MLSTM_B200_ENODEVICE;
@@ -2597,18 +2598,29 @@ int run_fw(const mlstm_b200_fw_args& a, void* c_states, cudaStream_t st) {
   const bool epi = p.epi != 0, rev = p.rev != 0, pdl = pdl_mode() != 0;
   return with_dtype(s.dtype, [&](auto t) {
     using T = decltype(t);
-    if (s.DHQK == 128) {
-      auto kern = fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw_d128<T, decltype(r)::value, decltype(e)::value>; });
-      return launch_fw(kern, p, 1, FwSmem128::kBytes, false, false, st, mq, mk, mv, mh, mcs);
+    switch (g.fw) {
+      case TcFw::wide: {
+        auto kern = fw_kernel(false, rev, [](auto, auto r) { return tc_fw_wide<T, decltype(r)::value>; });
+        return launch_fw(kern, p, g.ctas, FwSmemWide::kBytes, false, false, st, mq, mk, mv, mcs);
+      }
+      case TcFw::d128: {
+        auto kern = fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw_d128<T, decltype(r)::value, decltype(e)::value>; });
+        return launch_fw(kern, p, g.ctas, FwSmem128::kBytes, false, false, st, mq, mk, mv, mh, mcs);
+      }
+      case TcFw::rect:
+        return with_d32_64(g.bd, [&](auto d) {
+          constexpr int D = decltype(d)::value;
+          const bool pair = epi && g.cluster;
+          return launch_fw(fw_rect_kernel<T, D>(epi, rev), p, g.ctas, pair ? FwSmem<D>::kBytesPair : FwSmem<D>::kBytes, pair,
+                           pdl, st, mq, mk, mv, mh, mcs);
+        });
+      default:  // TcFw::square
+        return with_d32_64(g.bd, [&](auto d) {
+          constexpr int D = decltype(d)::value;
+          auto kern = fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw<T, D, decltype(r)::value, decltype(e)::value>; });
+          return launch_fw(kern, p, g.ctas, FwSmem<D>::kBytes, false, pdl, st, mq, mk, mv, mh, mcs);
+        });
     }
-    return with_d32_64(s.DHQK, [&](auto d) {
-      constexpr int D = decltype(d)::value;
-      using SM = FwSmem<D>;
-      if (rect)  // with the fused epilogue the two blocks of a head exchange their LayerNorm statistics: a cluster
-        return launch_fw(fw_rect_kernel<T, D>(epi, rev), p, 2, epi ? SM::kBytesPair : SM::kBytes, epi, pdl, st, mq, mk, mv, mh, mcs);
-      auto kern = fw_kernel(epi, rev, [](auto e, auto r) { return tc_fw<T, D, decltype(r)::value, decltype(e)::value>; });
-      return launch_fw(kern, p, 1, SM::kBytes, false, pdl, st, mq, mk, mv, mh, mcs);
-    });
   });
 }
 
@@ -2626,9 +2638,8 @@ BwWs bw_ws(const mlstm_b200_shape& s) {
   return w;
 }
 
-
 // ---------------------------------------------------------------------------------------------
-// Head dim 128 and rectangular-head backward as square block problems.
+// The backward of a head geometry with more than one block (tc_geometry) as square block problems.
 //
 // With n_out and every max state held constant (the definition of this backward, native/bw.py:44-47) every term
 // of bw.py:106-203 is bilinear in (a bd-wide block of q / k, a bd-wide block of v / dh): dS = (dH V^T) . D and
@@ -2636,10 +2647,8 @@ BwWs bw_ws(const mlstm_b200_shape& s) {
 // blocks with the same decay, and the stabilisers depend on the gates only.  So a (DHQK, DHHV) problem is the sum of
 // (DHQK / bd) x (DHHV / bd) tc_bw<bd> problems on strided views of the same tensors (no copies of q/k/v/dh;
 // qk_scale = DHQK^-1/2 of the whole problem; each loads its block of the forward's saved states or recomputes it,
-// bw.py:251-266).  Head dim 128: bd = 64, a 2 x 2 grid (a 128-wide tile set does not fit the backward's shared memory
-// with 128-token tiles).  Rectangular heads (D, 2 D): bd = D, a 1 x 2 grid.  Wide heads (256, 512): bd = 64, a 4 x 8
-// grid (dq / dk then take 8 partials, dv 4, di / df 32).  The first partial of every output block
-// is written in place, the second is added by the kernel that produces it (TMA reduce-add stores).
+// bw.py:251-266).  dq / dk then take nv partials, dv nq and di / df nq nv.  The first partial of every output block
+// is written in place, the others are added by the kernel that produces them (TMA reduce-add stores).
 // bd x bd block (a, b) of a (BH, DK, DV) fp32 state <-> contiguous (BH, bd, bd); vec: (BH, DK) <-> (BH, bd)
 __global__ void k_state_block(float* __restrict__ blk, float* __restrict__ full, int a, int b, int bd, int DK, int DV,
                               int64_t n, int scatter) {
@@ -2670,51 +2679,107 @@ __global__ void k_sum_gate_partials(const TO* __restrict__ part, int nparts, int
   else df[b * df_sb + h * df_sh + t * df_ss] = from_f32<TO>(acc);
 }
 
-}  // namespace
-int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, int nblocks, cudaStream_t st, int acc_qk = 0,
-           int acc_v = 0, int acc_g = 0);
-int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int block, int nblocks, cudaStream_t st, int acc_qk,
-                     int acc_v, int acc_g);
-namespace {
-
-int block_dim(const mlstm_b200_shape& s) { return s.DHQK >= 128 ? 64 : s.DHQK; }
-mlstm_b200_shape block_shape(const mlstm_b200_shape& s) {
+// One bd x bd block problem of s; qk_scale stays that of the whole problem
+mlstm_b200_shape block_shape(const mlstm_b200_shape& s, int bd) {
   mlstm_b200_shape b = s;
-  b.DHQK = b.DHHV = block_dim(s);
+  b.DHQK = b.DHHV = bd;
   b.qk_scale = s.qk_scale > 0.f ? s.qk_scale : 1.f / sqrtf((float)s.DHQK);
   return b;
 }
 struct BlocksWs {
   size_t off_sub, sub_bytes, off_c0, off_n0, off_dcl, off_dc0, off_g, total;
 };
-BlocksWs blocks_ws(const mlstm_b200_shape& s) {
+BlocksWs blocks_ws(const mlstm_b200_shape& s, const TcGeometry& g) {
   BlocksWs w{};
-  const size_t bh = (size_t)s.B * s.NH, bd = block_dim(s);
+  const size_t bh = (size_t)s.B * s.NH, bd = g.bd;
   size_t o = 0;
-  w.sub_bytes = bw_ws(block_shape(s)).total;
+  w.sub_bytes = bw_ws(block_shape(s, g.bd)).total;
   w.off_sub = o; o += align_up(w.sub_bytes, 256);
   w.off_c0 = o; o += align_up(bh * bd * bd * 4, 256);
   w.off_n0 = o; o += align_up(bh * bd * 4, 256);
   w.off_dcl = o; o += align_up(bh * bd * bd * 4, 256);
   w.off_dc0 = o; o += align_up(bh * bd * bd * 4, 256);
-  // wide heads: the 16-bit di / df partial of every block problem, summed in fp32 by k_sum_gate_partials (the in-kernel
-  // accumulation would round the running sum to 16 bits 31 times)
+  // gate_parts: the 16-bit di / df partial of every block problem, summed in fp32 by k_sum_gate_partials
   w.off_g = o;
-  if (wide_heads(s)) o += align_up(2 * (size_t)(s.DHQK / bd) * (s.DHHV / bd) * bh * s.S * 2, 256);
+  if (g.gate_parts) o += align_up(2 * (size_t)g.nq * g.nv * bh * s.S * 2, 256);
   w.total = o;
   return w;
 }
 
-template <typename T>
-int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
+// One tc_bw launch of a square problem (DHQK = DHHV = D).  c_states: the forward's saved states as nblocks D x D blocks per
+// tile, of which this problem reads block `block`; NULL: recompute them into the workspace first (bw.py:251-266), as
+// block 0 of 1.  acc_*: add into dq / dk, dv, di / df instead of overwriting them.
+int bw_square(const mlstm_b200_bw_args& a, const void* c_states, int block, int nblocks, cudaStream_t st, int acc_qk,
+              int acc_v, int acc_g) {
   const mlstm_b200_shape& s = a.shape;
-  const BlocksWs w = blocks_ws(s);
+  if (!c_states) {
+    BwWs w = bw_ws(s);
+    if (!a.workspace || a.workspace_bytes < w.total) {
+      set_error("workspace too small: need %zu bytes, got %zu", w.total, a.workspace_bytes);
+      return MLSTM_B200_EWORKSPACE;
+    }
+    char* ws = (char*)a.workspace;
+    mlstm_b200_fw_args f{};
+    f.shape = s;
+    f.q = a.q; f.k = a.k; f.v = a.v; f.i = a.i; f.f = a.f;
+    f.c_initial = a.c_initial; f.n_initial = a.n_initial; f.m_initial = a.m_initial;
+    f.h.ptr = ws + w.off_h;
+    f.h.stride[0] = (int64_t)s.NH * s.S * s.DHHV; f.h.stride[1] = (int64_t)s.S * s.DHHV; f.h.stride[2] = s.DHHV;
+    f.h.stride[3] = 1;
+    f.n_out = (float*)(ws + w.off_n); f.m_out = (float*)(ws + w.off_m);
+    if (int e = run_fw(f, ws + w.off_states, st)) return e;
+    c_states = ws + w.off_states;
+    block = 0, nblocks = 1;
+  }
+  CUtensorMap mq, mk, mv, mdh, mcs, mdq, mdk, mdv;
+  const int D = s.DHQK;
+  mlstm_b200_shape sg = s;  // the gradients' tensor maps carry THEIR dtype (it matters for the reduce-add stores)
+  if (s.grad_dtype) sg.dtype = s.grad_dtype;
+  const bool mixed = sg.dtype != s.dtype;
+  int r = make_map(&mq, a.q, s, D) | make_map(&mk, a.k, s, D) | make_map(&mv, a.v, s, D) | make_map(&mdh, a.dh, s, D) |
+          make_states_map_blocks(&mcs, c_states, s, nblocks * D, D) | make_map(&mdq, a.dq, sg, D) |
+          make_map(&mdk, a.dk, sg, D) | make_map(&mdv, a.dv, sg, D);
+  if (r) {
+    set_error("cuTensorMapEncodeTiled failed (%d)", r);
+    return MLSTM_B200_ENODEVICE;
+  }
+  TcBwParams p{};
+  set_gate_params(p, s, a.i, a.f);
+  p.m0 = a.m_initial;
+  p.n_out = a.n_out; p.m_out = a.m_out; p.dc_last = a.dc_last;
+  p.di = a.di.ptr; p.di_sb = a.di.stride[0]; p.di_sh = a.di.stride[1]; p.di_ss = a.di.stride[2];
+  p.df = a.df.ptr; p.df_sb = a.df.stride[0]; p.df_sh = a.df.stride[1]; p.df_ss = a.df.stride[2];
+  p.dc0 = a.dc_initial;
+  p.acc_qk = acc_qk; p.acc_v = acc_v; p.acc_g = acc_g;
+  p.cs_rows = nblocks * D;
+  p.cs_off = block * D;
+  TC_SET_PROF(p, 4096);
+  const int e = with_dtype(s.dtype, [&](auto t) {
+    using T = decltype(t);
+    using TX = std::conditional_t<std::is_same<T, __half>::value, __nv_bfloat16, __half>;  // the other 16-bit type
+    return with_d32_64(D, [&](auto d) {
+      constexpr int DD = decltype(d)::value;
+      // mixed: kernel operands in one 16-bit dtype, gradients rounded once from fp32 to the other
+      return mixed ? launch_bw<T, DD, TX>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st)
+                   : launch_bw<T, DD>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st);
+    });
+  });
+  if (e) return e;
+  count_launch();
+  MLSTM_CUDA_CHECK(cudaGetLastError());
+  return 0;
+}
+
+template <typename T>
+int bw_by_blocks(const mlstm_b200_bw_args& a, const TcGeometry& g, cudaStream_t st) {
+  const mlstm_b200_shape& s = a.shape;
+  const BlocksWs w = blocks_ws(s, g);
   if (!a.workspace || a.workspace_bytes < w.total) {
     set_error("workspace too small: need %zu bytes, got %zu", w.total, a.workspace_bytes);
     return MLSTM_B200_EWORKSPACE;
   }
   char* ws = (char*)a.workspace;
-  const int bd = block_dim(s), nq = s.DHQK / bd, nv = s.DHHV / bd;
+  const int bd = g.bd, nq = g.nq, nv = g.nv;
   const int64_t bh = (int64_t)s.B * s.NH, nst = bh * bd * bd, nvec = bh * bd;
   auto cols = [&](const mlstm_b200_tensor& t, int j) {  // columns bd j .. bd j + bd - 1 of a wider tensor: a view
     mlstm_b200_tensor v = t;
@@ -2727,7 +2792,6 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
   };
   int launches = 0;
   bool first = true;
-  const bool gate_parts = wide_heads(s);
   const int64_t ntok = bh * s.S;
   auto gate_part = [&](int which, int j) {  // (B, NH, S) view of partial j of di (which = 0) or df (1)
     mlstm_b200_tensor t{};
@@ -2735,15 +2799,14 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
     t.stride[0] = (int64_t)s.NH * s.S; t.stride[1] = s.S; t.stride[2] = 1; t.stride[3] = 1;
     return t;
   };
+  // With the forward's saved states (stored block-wise, make_states_map_blocks) every problem loads its block; without
+  // them it recomputes its slice.
+  const bool saved = a.c_states != nullptr;
   for (int qa = 0; qa < nq; ++qa) {
     for (int vb = 0; vb < nv; ++vb) {
       mlstm_b200_bw_args sub = a;
-      sub.shape = block_shape(s);
+      sub.shape = block_shape(s, bd);
       sub.q = cols(a.q, qa); sub.k = cols(a.k, qa); sub.v = cols(a.v, vb); sub.dh = cols(a.dh, vb);
-      // With the forward's saved states (tc_fw_d128 / tc_fw_rect / tc_fw_wide store them block-wise) every problem loads its
-      // block; without them it recomputes its slice.
-      const bool saved = a.c_states != nullptr;
-      sub.c_states = nullptr;
       sub.workspace = ws + w.off_sub; sub.workspace_bytes = w.sub_bytes;
       if (a.c_initial && !saved) {
         state_block(w.off_c0, a.c_initial, qa, vb, 0);
@@ -2766,11 +2829,9 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
       sub.dq = cols(a.dq, qa);
       sub.dk = cols(a.dk, qa);
       sub.dv = cols(a.dv, vb);
-      sub.di = gate_parts ? gate_part(0, qa * nv + vb) : a.di;
-      sub.df = gate_parts ? gate_part(1, qa * nv + vb) : a.df;
-      if (int e = tensor_bw_blocks(sub, saved ? a.c_states : nullptr, saved ? qa * nv + vb : -1, nq * nv, st, vb > 0, qa > 0,
-                                   !first && !gate_parts))
-        return e;
+      sub.di = g.gate_parts ? gate_part(0, qa * nv + vb) : a.di;
+      sub.df = g.gate_parts ? gate_part(1, qa * nv + vb) : a.df;
+      if (int e = bw_square(sub, a.c_states, qa * nv + vb, nq * nv, st, vb > 0, qa > 0, !first && !g.gate_parts)) return e;
       if (a.dc_initial) {
         state_block(w.off_dc0, a.dc_initial, qa, vb, 1);
         ++launches;
@@ -2778,17 +2839,15 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
       first = false;
     }
   }
-  if (gate_parts) {
-    const int gdt = s.grad_dtype ? s.grad_dtype : s.dtype;
+  if (g.gate_parts) {
     const unsigned grid = (unsigned)((2 * ntok + 255) / 256);
-    if (gdt == MLSTM_B200_BF16)
-      k_sum_gate_partials<__nv_bfloat16><<<grid, 256, 0, st>>>(
-          (const __nv_bfloat16*)(ws + w.off_g), nq * nv, ntok, s.NH, s.S, (__nv_bfloat16*)a.di.ptr, a.di.stride[0],
-          a.di.stride[1], a.di.stride[2], (__nv_bfloat16*)a.df.ptr, a.df.stride[0], a.df.stride[1], a.df.stride[2]);
-    else
-      k_sum_gate_partials<__half><<<grid, 256, 0, st>>>((const __half*)(ws + w.off_g), nq * nv, ntok, s.NH, s.S,
-                                                        (__half*)a.di.ptr, a.di.stride[0], a.di.stride[1], a.di.stride[2],
-                                                        (__half*)a.df.ptr, a.df.stride[0], a.df.stride[1], a.df.stride[2]);
+    with_dtype(s.grad_dtype ? s.grad_dtype : s.dtype, [&](auto t) {
+      using TO = decltype(t);
+      k_sum_gate_partials<TO><<<grid, 256, 0, st>>>((const TO*)(ws + w.off_g), nq * nv, ntok, s.NH, s.S, (TO*)a.di.ptr,
+                                                    a.di.stride[0], a.di.stride[1], a.di.stride[2], (TO*)a.df.ptr,
+                                                    a.df.stride[0], a.df.stride[1], a.df.stride[2]);
+      return 0;
+    });
     ++launches;
   }
   MLSTM_CUDA_CHECK(cudaGetLastError());
@@ -2799,10 +2858,10 @@ int bw_by_blocks(const mlstm_b200_bw_args& a, cudaStream_t st) {
 }  // namespace
 
 // the views a call hands in can be described by TMA tensor maps (16-byte aligned base, 16-byte-multiple strides)
-bool tensor_fw_views_ok(const mlstm_b200_fw_args& a) {
+bool tensor_views_ok(const mlstm_b200_fw_args& a) {
   return tma_ok(a.q) && tma_ok(a.k) && tma_ok(a.v) && tma_ok(a.epilogue ? a.epilogue->y : a.h);
 }
-bool tensor_bw_views_ok(const mlstm_b200_bw_args& a) {
+bool tensor_views_ok(const mlstm_b200_bw_args& a) {
   return tma_ok(a.q) && tma_ok(a.k) && tma_ok(a.v) && tma_ok(a.dh) && tma_ok(a.dq) && tma_ok(a.dk) && tma_ok(a.dv);
 }
 
@@ -2815,25 +2874,10 @@ void tensor_set_clock_buffer(void* dev_ptr) {
 }
 bool tensor_context_is_current() { return sm100_host::context_is_current(); }
 
-// forward: d = 32, 64 and 128; backward: d = 32 and 64 natively, d = 128 as four d = 64 block problems (bw_by_blocks).
-// Rectangular heads (DHQK, DHHV) = (32, 64) and (64, 128): the forward as two square column-block problems in one launch
-// (tc_fw_rect), the backward as two tc_bw<DHQK> block problems.  Wide heads (256, 512) (xLSTM-Large): the forward as eight
-// 64-wide column blocks in one launch (tc_fw_wide), the backward as 4 x 8 tc_bw<64> block problems.
-bool tensor_supported(const mlstm_b200_shape& s, int backward) {
-  if (s.dtype != MLSTM_B200_BF16 && s.dtype != MLSTM_B200_F16) return false;
-  if (wide_heads(s)) return s.S % 4 == 0;
-  if (s.DHQK != s.DHHV && !((s.DHQK == 32 || s.DHQK == 64) && s.DHHV == 2 * s.DHQK)) return false;
-  if (s.DHQK != 64 && s.DHQK != 32 && s.DHQK != 128) return false;  // d = 128 backward: four d = 64 block problems
-  // Tiles are 128 tokens whatever chunk_size is (h and the states do not depend on it: the stabiliser equals the
-  // step-recurrent one), and ragged last tiles are handled in-kernel (TMA zero-fill, gates masked at scan time),
-  // so any S that keeps the fp32 n_out / m_out rows 16-byte aligned is covered; S % chunk_size == 0 is enforced
-  // at the C-ABI like the reference does (native/fw.py:252-254).
-  if (s.S % 4 != 0) return false;
-  return true;
-}
+bool tensor_supported(const mlstm_b200_shape& s) { return tc_geometry(s).fw != TcFw::none; }
 
 size_t tensor_states_bytes(const mlstm_b200_shape& s) {
-  if (!tensor_supported(s, 1)) return 0;
+  if (!tensor_supported(s)) return 0;
   const size_t NT = (s.S + LT - 1) / LT;
   return (size_t)s.B * s.NH * NT * s.DHQK * s.DHHV * 2;
 }
@@ -2841,19 +2885,21 @@ size_t tensor_states_bytes(const mlstm_b200_shape& s) {
 // forward needs no scratch; backward needs room to recompute the states when c_states is absent
 size_t tensor_workspace_bytes(const mlstm_b200_shape& s, int backward) {
   if (!backward) return 256;
-  return s.DHQK == 128 || rect_heads(s) ? blocks_ws(s).total : bw_ws(s).total;
+  const TcGeometry g = tc_geometry(s);
+  return g.nq * g.nv > 1 ? blocks_ws(s, g).total : bw_ws(s).total;
 }
 
 int tensor_fw(const mlstm_b200_fw_args& a, cudaStream_t st) { return run_fw(a, a.c_states, st); }
 
-// cudaOccupancyMaxActiveClusters of the rectangular forward with the fused epilogue ({2, 1, 1} clusters) on the current
-// device; 0 for a shape that does not launch it, -1 on a CUDA error
+// cudaOccupancyMaxActiveClusters of the forward with the fused epilogue in {2, 1, 1} clusters on the current device; 0 for
+// a shape that does not launch it, -1 on a CUDA error
 int tensor_fw_epilogue_clusters(const mlstm_b200_shape& s) {
-  if (!tensor_supported(s, 0) || !rect_heads(s) || wide_heads(s)) return 0;
+  const TcGeometry g = tc_geometry(s);
+  if (!g.cluster) return 0;
   auto query = [&](auto kern, int smem) {
     if (ensure_smem(kern, smem) != cudaSuccess) return -1;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * s.B * s.NH), cfg.blockDim = dim3(kTcThreads), cfg.dynamicSmemBytes = smem;
+    cfg.gridDim = dim3(g.ctas * s.B * s.NH), cfg.blockDim = dim3(kTcThreads), cfg.dynamicSmemBytes = smem;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = 2, attr[0].val.clusterDim.y = 1, attr[0].val.clusterDim.z = 1;
@@ -2862,93 +2908,21 @@ int tensor_fw_epilogue_clusters(const mlstm_b200_shape& s) {
     return cudaOccupancyMaxActiveClusters(&n, kern, &cfg) == cudaSuccess ? n : -1;
   };
   return with_dtype(s.dtype, [&](auto t) {
-    return with_d32_64(s.DHQK, [&](auto d) {
+    return with_d32_64(g.bd, [&](auto d) {
       constexpr int D = decltype(d)::value;
       return query(fw_rect_kernel<decltype(t), D>(true, s.reverse != 0), FwSmem<D>::kBytesPair);
     });
   });
 }
 
-int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st) { return tensor_bw_blocks(a, a.c_states, -1, 1, st, 0, 0, 0); }
-
-// c_states: the forward's saved states (block < 0: this problem's own; block = 0 .. nblocks - 1: block `block` of the
-// block-wise buffer of a head-dim-128 or rectangular forward) or NULL = recompute; acc_*: add into dq / dk, dv, di / df
-// instead of overwriting them
-int tensor_bw_blocks(const mlstm_b200_bw_args& a, const void* c_states_in, int block, int nblocks, cudaStream_t st, int acc_qk,
-                     int acc_v, int acc_g) {
-  const mlstm_b200_shape& s = a.shape;
-  if (!tma_ok(a.q) || !tma_ok(a.k) || !tma_ok(a.v) || !tma_ok(a.dh) || !tma_ok(a.dq) || !tma_ok(a.dk) || !tma_ok(a.dv)) {
+int tensor_bw(const mlstm_b200_bw_args& a, cudaStream_t st) {
+  if (!tensor_views_ok(a)) {
     set_error("tensor path needs 16-byte aligned q/k/v/dh/dq/dk/dv with strides that are multiples of 8 elements");
     return MLSTM_B200_EUNSUPPORTED;
   }
-  if (s.DHQK == 128 || rect_heads(s))
-    return s.dtype == MLSTM_B200_BF16 ? bw_by_blocks<__nv_bfloat16>(a, st) : bw_by_blocks<__half>(a, st);
-  const void* c_states = c_states_in;
-  if (!c_states) {  // recompute the states with a forward pass into the workspace (bw.py:251-266)
-    block = -1;
-    BwWs w = bw_ws(s);
-    if (!a.workspace || a.workspace_bytes < w.total) {
-      set_error("workspace too small: need %zu bytes, got %zu", w.total, a.workspace_bytes);
-      return MLSTM_B200_EWORKSPACE;
-    }
-    char* ws = (char*)a.workspace;
-    mlstm_b200_fw_args f{};
-    f.shape = s;
-    f.q = a.q; f.k = a.k; f.v = a.v; f.i = a.i; f.f = a.f;
-    f.c_initial = a.c_initial; f.n_initial = a.n_initial; f.m_initial = a.m_initial;
-    f.h.ptr = ws + w.off_h;
-    f.h.stride[0] = (int64_t)s.NH * s.S * s.DHHV; f.h.stride[1] = (int64_t)s.S * s.DHHV; f.h.stride[2] = s.DHHV;
-    f.h.stride[3] = 1;
-    f.n_out = (float*)(ws + w.off_n); f.m_out = (float*)(ws + w.off_m);
-    if (int e = run_fw(f, ws + w.off_states, st)) return e;
-    c_states = ws + w.off_states;
-  }
-  return run_bw(a, c_states, block, nblocks, st, acc_qk, acc_v, acc_g);
-}
-
-// block < 0: c_states holds this problem's own (B, NH, NT, D, D) states.  block = 0 .. nblocks - 1: c_states is a
-// block-wise buffer (nblocks D x D blocks per tile, make_states_map_blocks) and this problem reads block `block` of
-// every tile.
-int run_bw(const mlstm_b200_bw_args& a, const void* c_states, int block, int nblocks, cudaStream_t st, int acc_qk, int acc_v,
-           int acc_g) {
-  const mlstm_b200_shape& s = a.shape;
-  CUtensorMap mq, mk, mv, mdh, mcs, mdq, mdk, mdv;
-  const int D = s.DHQK;
-  mlstm_b200_shape sg = s;  // the gradients' tensor maps carry THEIR dtype (it matters for the reduce-add stores)
-  if (s.grad_dtype) sg.dtype = s.grad_dtype;
-  const bool mixed = sg.dtype != s.dtype;
-  int r = make_map(&mq, a.q, s, D) | make_map(&mk, a.k, s, D) | make_map(&mv, a.v, s, D) | make_map(&mdh, a.dh, s, D) |
-          (block < 0 ? make_states_map(&mcs, c_states, s) : make_states_map_blocks(&mcs, c_states, s, nblocks * D, D)) |
-          make_map(&mdq, a.dq, sg, D) | make_map(&mdk, a.dk, sg, D) | make_map(&mdv, a.dv, sg, D);
-  if (r) {
-    set_error("cuTensorMapEncodeTiled failed (%d)", r);
-    return MLSTM_B200_ENODEVICE;
-  }
-  TcBwParams p{};
-  set_gate_params(p, s, a.i, a.f);
-  p.m0 = a.m_initial;
-  p.n_out = a.n_out; p.m_out = a.m_out; p.dc_last = a.dc_last;
-  p.di = a.di.ptr; p.di_sb = a.di.stride[0]; p.di_sh = a.di.stride[1]; p.di_ss = a.di.stride[2];
-  p.df = a.df.ptr; p.df_sb = a.df.stride[0]; p.df_sh = a.df.stride[1]; p.df_ss = a.df.stride[2];
-  p.dc0 = a.dc_initial;
-  p.acc_qk = acc_qk; p.acc_v = acc_v; p.acc_g = acc_g;
-  p.cs_rows = block < 0 ? D : nblocks * D;
-  p.cs_off = block < 0 ? 0 : D * block;
-  TC_SET_PROF(p, 4096);
-  const int e = with_dtype(s.dtype, [&](auto t) {
-    using T = decltype(t);
-    using TX = std::conditional_t<std::is_same<T, __half>::value, __nv_bfloat16, __half>;  // the other 16-bit type
-    return with_d32_64(D, [&](auto d) {
-      constexpr int DD = decltype(d)::value;
-      // mixed: kernel operands in one 16-bit dtype, gradients rounded once from fp32 to the other
-      return mixed ? launch_bw<T, DD, TX>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st)
-                   : launch_bw<T, DD>(p, mq, mk, mv, mdh, mcs, mdq, mdk, mdv, st);
-    });
-  });
-  if (e) return e;
-  count_launch();
-  MLSTM_CUDA_CHECK(cudaGetLastError());
-  return 0;
+  const TcGeometry g = tc_geometry(a.shape);
+  if (g.nq * g.nv == 1) return bw_square(a, a.c_states, 0, 1, st, 0, 0, 0);
+  return with_dtype(a.shape.dtype, [&](auto t) { return bw_by_blocks<decltype(t)>(a, g, st); });
 }
 
 }  // namespace mlstm
